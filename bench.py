@@ -2,7 +2,7 @@
 """bench.py — headline benchmark of the hot path (BASELINE.json: "YOLOv2-416 pruned-fwd images/sec ...; prune-mask ms vs
 HBM roofline").
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1]): YOLOv2-VOC, seed-0 default init, 40 % global filter pruning
 (quick_filter_prune) with the pruned filters PHYSICALLY removed, bf16 forward, batch 64 per GPU, 416x416 synthetic
@@ -13,6 +13,9 @@ events on the launching stream, and the elapsed time is the max over ranks.
 
 `--impl reference` times the CPU path (oracle port of the reference's PyTorch forward: same F.conv2d / batch_norm /
 leaky_relu / max_pool2d calls, same masked weights) on the host cores, on a bounded sample per step.
+
+`--dump-outputs DIR` writes the head the last timed step returned (rank 0's) as DIR/head.npy, float32 [B, 125, 13, 13].
+Weights and inputs are seeded, so two builds run with the same arguments can be compared output for output.
 
 Extras in the same JSON line (rank 0): roofline against the BURST bf16 peak (the timed region is milliseconds long) with
 the sustained fraction beside it, whole-net fractions, per-op times, decode / NMS microseconds per image, the mask
@@ -39,6 +42,7 @@ CPU_SAMPLE_BATCH = 4
 PER_OP_REPS = 6  # launches per event pair in the per-kernel timing (amortises the events' own cost)
 N_INPUT_BUFFERS = 6  # 6 x 33 MB uint8 batches = 199 MB > 126 MB L2
 DENSE_GFLOP_PER_IMAGE = 29.360
+DUMP_MAX_BYTES = 64 * 1000 * 1000
 
 
 def profiled_traffic():
@@ -153,9 +157,25 @@ def build_pruned_model(device):
     return model, masks, keep
 
 
+def dump_head(out_dir, head):
+    """Write one step's head as out_dir/head.npy (float32).  A head larger than DUMP_MAX_BYTES keeps a seeded sample of
+    whole images in batch order (the same images for the same --batch), so that the file stays comparable across runs."""
+    import numpy as np
+    import torch
+    head = head.detach().float().cpu()
+    per_image = head[0].numel() * 4
+    n = max(1, (DUMP_MAX_BYTES - 128) // per_image)  # 128: the .npy header
+    if n < head.shape[0]:
+        idx = torch.randperm(head.shape[0], generator=torch.Generator().manual_seed(0))[:n].sort().values
+        head = head[idx]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, 'head.npy'), head.numpy())
+
+
 # ----------------------------------------------------------------------------------------------------- CPU legs
 def cpu_forward_sample(state, blocks, batch, steps, warmup=1):
-    """Oracle port of the reference forward on the host cores.  Returns (images/s, seconds per step)."""
+    """Oracle port of the reference forward on the host cores.  Returns (images/s, seconds per step, head of the last
+    step)."""
     import torch
     from oracle import forward_oracle
     torch.manual_seed(1)
@@ -165,9 +185,9 @@ def cpu_forward_sample(state, blocks, batch, steps, warmup=1):
             forward_oracle.darknet_forward_fp32(blocks, state, x)
         t0 = time.perf_counter()
         for _ in range(steps):
-            forward_oracle.darknet_forward_fp32(blocks, state, x)
+            y, _ = forward_oracle.darknet_forward_fp32(blocks, state, x)
         dt = time.perf_counter() - t0
-    return batch * steps / dt, dt / steps
+    return batch * steps / dt, dt / steps, y
 
 
 def cpu_stage_legs(dense_state, blocks, anchors):
@@ -235,7 +255,9 @@ def run_reference_arm(args, rank):
     for (name, p), m in zip([(n, p) for n, p in model.named_parameters() if p.dim() == 4], masks):
         state[name] = p.data * torch.from_numpy(m)  # set_mask: weight.data *= mask (layers.py:46)
     cores = torch.get_num_threads()
-    ips, sps = cpu_forward_sample(state, model.blocks, CPU_SAMPLE_BATCH, args.steps, args.warmup)
+    ips, sps, head = cpu_forward_sample(state, model.blocks, CPU_SAMPLE_BATCH, args.steps, args.warmup)
+    if args.dump_outputs:
+        dump_head(args.dump_outputs, head)
     line = {
         "impl": "reference", "metric": METRIC, "value": ips, "unit": "images/s", "n_gpus": args.gpus,
         "steps": args.steps, "warmup": args.warmup, "ms_per_step": sps * 1e3, "higher_is_better": True,
@@ -674,7 +696,10 @@ def main():
     ap.add_argument('--no-retrain', action='store_true', help='skip the extra retrain-step timings (configs[2], N4)')
     ap.add_argument('--no-eval', action='store_true', help='skip the extra evaluation-pipeline timing (configs[4])')
     ap.add_argument('--no-library', action='store_true', help='skip the ATen/cuDNN library baseline')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='write the head of the last timed step as DIR/head.npy')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     args.warmup = max(args.warmup, 3) if args.impl == 'b200' else max(args.warmup, 1)
 
     rank = int(os.environ.get('RANK', '0'))
@@ -742,7 +767,7 @@ def main():
             torch.cuda._sleep(max(3000000, 130000 * K))
             ev[0].record()
             for i in range(K):
-                step(i)
+                out = step(i)
                 ev[i + 1].record()
             gc.enable()
             # NVML queries perturb the GPU: polling every 0.5 ms cost 1.2 % of the step (79.9 k vs 80.95 k img/s, same
@@ -753,7 +778,7 @@ def main():
                 time.sleep(poll_s)
             probe.sample()
             barrier()
-            return [ev[i].elapsed_time(ev[i + 1]) for i in range(K)]
+            return [ev[i].elapsed_time(ev[i + 1]) for i in range(K)], out
 
         # A timed region in which ONE step is many times the median (seen once: a 70 ms step among 99 of 0.79 ms, i.e. the
         # host stalled longer than the spin kernel covers and the GPU sat idle waiting for launches) is not a measurement
@@ -761,7 +786,7 @@ def main():
         # stay in the JSON line ("rejected_attempts").  All ranks decide together.
         rejected_attempts = []
         for attempt in range(3):
-            step_ms = timed_region()
+            step_ms, last_head = timed_region()
             med = statistics.median(step_ms)
             stalled = 1.0 if (K >= 4 and max(step_ms) > 5.0 * med) else 0.0
             if world > 1:
@@ -772,6 +797,8 @@ def main():
                 break
             rejected_attempts.append({"rank": rank, "total_ms": ev[0].elapsed_time(ev[K]), "median_step_ms": med,
                                       "max_step_ms": max(step_ms), "why": "a step > 5x the median: host stall"})
+        if args.dump_outputs and rank == 0:
+            dump_head(args.dump_outputs, last_head)
         y = step(0)
         clocks = probe.result()
         elapsed_ms = ev[0].elapsed_time(ev[K])
@@ -1007,7 +1034,7 @@ def main():
                 line["retrain"] = time_retrain(device, peaks, B)
             if not args.no_cpu_baseline:
                 state = {k: v.detach().cpu() for k, v in model.state_dict().items()}
-                ips, sps = cpu_forward_sample(state, model.blocks, CPU_SAMPLE_BATCH, 6, 1)
+                ips, sps, _ = cpu_forward_sample(state, model.blocks, CPU_SAMPLE_BATCH, 6, 1)
                 line["cpu_baseline"] = {"value": ips, "unit": "images/s", "cores": torch.get_num_threads(),
                                         "kind": "port", "sample": "6 forwards of batch %d of the same pruned network "
                                         "(oracle port of the reference PyTorch CPU path)" % CPU_SAMPLE_BATCH,

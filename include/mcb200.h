@@ -240,7 +240,7 @@ size_t mc_workspace_bytes_conv_fwd(const mc_conv_desc* desc);
 /* Which launch configuration the LAST mc_conv_fwd call of this host thread chose (tests / bench reporting):
  * info[0] = 1 CTA-pair kernel (tcgen05 cta_group::2, 256-row tiles, half of each weight tile per CTA), 0 single CTA
  * info[1] = tile width block_n      info[2] = resident CTAs per SM requested (1..3)
- * info[3] = single CTA: 1 weights resident in shared memory; CTA pair: units in the stream-K tail
+ * info[3] = CTA pair: units in the stream-K tail; 0 otherwise
  * info[4] = 1 shared activation box (3x3)
  * info[5] = smem ring stages         info[6] = grid size                   info[7] = k-block (32 or 64)           */
 int mc_conv_last_plan(int info[8]);
@@ -296,10 +296,6 @@ int mc_conv_window_supported(int Cin, int in_kind, int N, int pool);
 int mc_conv_window_geometry(int Cin, int in_kind, int N, int pool, int* npos, int* nb, int* kcols);
 int mc_conv_window_fwd(const void* d_in, int in_kind, const void* d_w, const float* d_scale, const float* d_shift,
                        void* d_out, int B, int H, int W, int Cin, int N, int ldc, int leaky, int pool, void* stream);
-
-/* Debug aid (tuning builds, make TUNING=1): later mc_conv_window_fwd launches record clock64 stamps of CTA 0 into
- * d_buf (128 x uint64); NULL switches it off.  A product build ignores the buffer.                              */
-int mc_debug_window_trace(void* d_buf);
 
 /* Debug aid: later single-CTA mc_conv_fwd launches record globaltimer stamps (32 x uint64 per CTA: entry, set-up done,
  * first operands landed, per-tile MMA issue / accumulator ready / epilogue done, exit) into d_buf (32*8*grid bytes);

@@ -93,7 +93,6 @@ _SIGNATURES = {
     "mc_conv_im2col_fwd": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int,
                                    c_int, c_int, c_int, c_int, c_int, c_void_p]),
     "mc_debug_im2col_timeout": (c_int, []),
-    "mc_debug_window_trace": (c_int, [c_void_p]),
     "mc_debug_conv_trace": (c_int, [c_void_p]),
     "mc_conv_window_supported": (c_int, [c_int, c_int, c_int, c_int]),
     "mc_conv_window_geometry": (c_int, [c_int, c_int, c_int, c_int, POINTER(c_int), POINTER(c_int), POINTER(c_int)]),

@@ -35,18 +35,6 @@ int mc_set_error(int code, const char* fmt, ...);
                           cudaGetErrorString(e_));                                          \
   } while (0)
 
-// A/B switches of the launch planners (MCB200_* environment variables, listed in tools/ab.sh) exist only in a tuning
-// build (make TUNING=1 -> -DMCB200_TUNING).  The product build never reads the environment: every decision is the
-// measured default.
-static inline const char* mc_tune_env(const char* name) {
-#ifdef MCB200_TUNING
-  return getenv(name);
-#else
-  (void)name;
-  return nullptr;
-#endif
-}
-
 static inline int mc_num_sms() {
   static int n = 0;
   if (n == 0) {

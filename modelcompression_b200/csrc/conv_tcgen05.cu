@@ -17,8 +17,7 @@
 //   conv_gemm_tcgen05_kernel<MINB>   persistent, 1..3 CTAs per SM (MINB = register budget), every layer shape;
 //   conv_gemm_tcgen05_pair_kernel    cluster of 2 CTAs, tcgen05 cta_group::2: 256-row tiles, each CTA loads half of every
 //                                    weight tile — the wide 3x3 layers (block_n >= 192, >= 36 k-blocks).
-// mc_conv_fwd picks kernel, tile width, ring depth and CTAs per SM (mc_conv_last_plan reports the choice;
-// MCB200_CONV_TRACE=1 prints it; the MCB200_* switches listed in tools/ab.sh override single decisions for A/B runs).
+// mc_conv_fwd picks kernel, tile width, ring depth and CTAs per SM (mc_conv_last_plan reports the choice).
 #include <cuda.h>
 #include <stdio.h>
 #include <stdlib.h>
@@ -31,12 +30,11 @@ namespace {
 
 constexpr int BLOCK_M = 128;  // k-block: 64 bf16 (128-byte swizzle rows) or 32 bf16 (64-byte swizzle rows), per launch
 constexpr int MAX_STAGES = 8;
-constexpr int MAX_A_STAGES = 8;   // activation-box ring: 3 beside a weight ring, up to 8 when the weights are resident
-constexpr int DEF_A_STAGES = 3;
+constexpr int MAX_A_STAGES = 3;  // activation-box ring: 3 boxes with one CTA per SM, 2 with several
 constexpr int A_BOX_ROWS = BLOCK_M + 8;          // rows m0-1 .. m0+134: the dx = -1, 0, +1 windows of a 128-row tile
 constexpr int A_BOX_BYTES = A_BOX_ROWS * 128;   // 17,408 B landed by TMA
 constexpr int A_BOX_STRIDE = 18 * 1024;         // ring pitch (1024-byte aligned for the 128-byte swizzle)
-constexpr int MAX_ACC = 8;  // accumulator stages in TMEM (2 for wide tiles; up to 8 for narrow one-N-tile layers)
+constexpr int ACC_STAGES = 2;  // accumulator stages in TMEM: the MMA issuer runs this many tiles ahead of the epilogue
 constexpr int NUM_THREADS = 192;
 
 struct ConvKParams {
@@ -49,7 +47,6 @@ struct ConvKParams {
   int ksize;       // 1 or 3
   int Wp, Hp, W, H;  // Wp = W+1, Hp = H+1
   int block_n, stages, tmem_cols, acc_stride;  // acc_stride: TMEM columns between accumulator stages
-  int acc_stages;  // accumulator stages: the MMA issuer runs this many tiles ahead of the epilogue
   int out_pitch;   // > 0: PNHWC epilogue stages each warp's 32 rows in shared memory (row pitch in bytes) and writes them out coalesced
   int out_chunk;   // columns staged at a time (<= 64)
   int tma_bufs;    // > 0: PNHWC epilogue writes whole 64-column chunks with TMA stores from this many 4 KB slabs per warp
@@ -57,7 +54,6 @@ struct ConvKParams {
   float* stat_sumsq;  // accumulated from the TMA-store slabs (the batch statistics of BatchNorm); nullptr: off
   unsigned int wp_mul, wp_shr, hp_mul, hp_shr;  // magic-number division by Wp and Hp (row -> x, y, b)
   int last_ksteps;  // UMMA K steps (16 channels) that hold real channels in the LAST channel block of a tap
-  int b_resident;   // share_dx only: all weight tiles stay in shared memory for the whole launch (one N tile, small K)
   int share_dx, a_stages;  // 3x3 only: one A box (136 rows) serves the three dx taps of a filter row; separate A / B rings
   int m_tiles, n_tiles;
   uint32_t idesc;
@@ -394,7 +390,7 @@ __device__ __forceinline__ void epilogue_loop(const ConvKParams& p, uint32_t tme
                                      vec_ok, s_out + (size_t)quarter * p.tma_bufs * 4096, slab_buf, &tmem_empty_bar[as],
                                      [](uint32_t (&)[16], int) {}, stat_acc);
       if (!PAIR && et == 0 && ti < 8) conv_stamp(p, 13 + 2 * ti);
-      if (++as == p.acc_stages) { as = 0; aphase ^= 1u; }
+      if (++as == ACC_STAGES) { as = 0; aphase ^= 1u; }
       continue;
     }
 
@@ -455,7 +451,7 @@ __device__ __forceinline__ void epilogue_loop(const ConvKParams& p, uint32_t tme
         __syncwarp();  // wbuf is rewritten by the next chunk / tile
       }
       if (!PAIR && et == 0 && ti < 8) conv_stamp(p, 13 + 2 * ti);
-      if (++as == p.acc_stages) { as = 0; aphase ^= 1u; }
+      if (++as == ACC_STAGES) { as = 0; aphase ^= 1u; }
       continue;
     }
 
@@ -502,7 +498,7 @@ __device__ __forceinline__ void epilogue_loop(const ConvKParams& p, uint32_t tme
         }
       }
       __syncwarp();  // the rows are rewritten by the next tile
-      if (++as == p.acc_stages) { as = 0; aphase ^= 1u; }
+      if (++as == ACC_STAGES) { as = 0; aphase ^= 1u; }
       continue;
     }
 
@@ -529,7 +525,7 @@ __device__ __forceinline__ void epilogue_loop(const ConvKParams& p, uint32_t tme
       else ptx::mbar_arrive(&tmem_empty_bar[as]);
     }
     if (!PAIR && et == 0 && ti < 8) conv_stamp(p, 13 + 2 * ti);
-    if (++as == p.acc_stages) { as = 0; aphase ^= 1u; }
+    if (++as == ACC_STAGES) { as = 0; aphase ^= 1u; }
   }
   if (stat_acc != nullptr && stat_n0 >= 0) flush_stats(p, stat_acc, stat_n0, lane);
   if (MODE == MC_EPI_PNHWC && p.tma_bufs > 0 && lane == 0) ptx::bulk_wait_group_read<0>();  // slabs read before the CTA exits
@@ -564,13 +560,12 @@ conv_gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __gri
   const uint32_t a_box_bytes = (uint32_t)A_BOX_ROWS * a_row_bytes;
   const uint32_t a_box_stride = p.block_k == 64 ? (uint32_t)A_BOX_STRIDE : (uint32_t)A_BOX_STRIDE / 2u;
   uint8_t* b_ring = tiles + (size_t)p.a_stages * a_box_stride;
-  uint8_t* aux = p.share_dx ? b_ring + (size_t)(p.b_resident ? p.num_kb : p.stages) * b_tile_bytes
-                            : tiles + (size_t)p.stages * stage_bytes;
+  uint8_t* aux = p.share_dx ? b_ring + (size_t)p.stages * b_tile_bytes : tiles + (size_t)p.stages * stage_bytes;
   uint64_t* full_bar = reinterpret_cast<uint64_t*>(aux);
   uint64_t* empty_bar = full_bar + MAX_STAGES;
-  uint64_t* tmem_full_bar = empty_bar + MAX_STAGES;   // [MAX_ACC]
-  uint64_t* tmem_empty_bar = tmem_full_bar + MAX_ACC; // [MAX_ACC]
-  uint64_t* afull_bar = tmem_empty_bar + MAX_ACC;     // [MAX_A_STAGES]
+  uint64_t* tmem_full_bar = empty_bar + MAX_STAGES;      // [ACC_STAGES]
+  uint64_t* tmem_empty_bar = tmem_full_bar + ACC_STAGES; // [ACC_STAGES]
+  uint64_t* afull_bar = tmem_empty_bar + ACC_STAGES;     // [MAX_A_STAGES]
   uint64_t* aempty_bar = afull_bar + MAX_A_STAGES;    // [MAX_A_STAGES]
   uint32_t* tmem_ptr_smem = reinterpret_cast<uint32_t*>(aempty_bar + MAX_A_STAGES);
   float* s_ss = reinterpret_cast<float*>(aux + 512);  // [2 acc stages][scale|shift][256]
@@ -589,7 +584,7 @@ conv_gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __gri
       ptx::mbar_init(&full_bar[s], 1);
       ptx::mbar_init(&empty_bar[s], 1);
     }
-    for (int a = 0; a < p.acc_stages; ++a) {
+    for (int a = 0; a < ACC_STAGES; ++a) {
       ptx::mbar_init(&tmem_full_bar[a], 1);
       ptx::mbar_init(&tmem_empty_bar[a], 4);  // one arrive per epilogue warp
     }
@@ -618,11 +613,6 @@ conv_gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __gri
       // the activations cross L2 -> smem 3 times per tile instead of 9.  B: one tile per tap, its own ring.
       int s = 0, sa = 0;
       uint32_t phase = 0, pha = 0;
-      if (p.b_resident) {  // every weight tile of the layer, once: [num_kb][block_n rows x 128 B]
-        ptx::mbar_arrive_expect_tx(&full_bar[0], (uint32_t)p.num_kb * b_tile_bytes);
-        for (int kb = 0; kb < p.num_kb; ++kb)
-          ptx::tma_load_2d(b_ring + (size_t)kb * b_tile_bytes, &tmap_b, &full_bar[0], kb * p.block_k, 0);
-      }
       for (int tile = blockIdx.x; tile < total_tiles; tile += gridDim.x) {
         const int n0 = (tile % p.n_tiles) * p.block_n;
         const int m0 = (tile / p.n_tiles) * BLOCK_M;
@@ -633,7 +623,6 @@ conv_gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __gri
           ptx::tma_load_2d(tiles + (size_t)sa * a_box_stride, &tmap_abox, &afull_bar[sa], cb * p.block_k,
                            m0 + (dy - 1) * p.Wp - 1);
           if (++sa == p.a_stages) { sa = 0; pha ^= 1u; }
-          if (p.b_resident) continue;
           for (int dx = 0; dx < 3; ++dx) {
             const int kb = (dy * 3 + dx) * p.kb_per_tap + cb;
             ptx::mbar_wait(&empty_bar[s], phase ^ 1u);
@@ -675,7 +664,6 @@ conv_gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __gri
     if (p.share_dx) {
       int s = 0, sa = 0, as = 0;
       uint32_t phase = 0, pha = 0, aphase = 0;
-      bool b_loaded = false;
       int ti = 0;
       for (int tile = blockIdx.x; tile < total_tiles; tile += gridDim.x, ++ti) {
         ptx::mbar_wait(&tmem_empty_bar[as], aphase ^ 1u);
@@ -689,15 +677,9 @@ conv_gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __gri
           if (ti == 0 && g == 0 && lane == 0) conv_stamp(p, 4);
           const uint32_t a_addr = ptx::smem_u32(tiles + (size_t)sa * a_box_stride);
           for (int dx = 0; dx < 3; ++dx) {
-            uint32_t b_addr;
-            if (p.b_resident) {
-              if (!b_loaded) { ptx::mbar_wait(&full_bar[0], 0); b_loaded = true; }
-              b_addr = ptx::smem_u32(b_ring + (size_t)((dy * 3 + dx) * p.kb_per_tap + cb) * b_tile_bytes);
-            } else {
-              ptx::mbar_wait(&full_bar[s], phase);
-              b_addr = ptx::smem_u32(b_ring + (size_t)s * b_tile_bytes);
-            }
+            ptx::mbar_wait(&full_bar[s], phase);
             ptx::tc_fence_after();
+            const uint32_t b_addr = ptx::smem_u32(b_ring + (size_t)s * b_tile_bytes);
             // the window of tap dx starts dx rows (dx * 128 B) into the box.  The start is then not aligned to the
             // 1024-byte swizzle pattern; measured on B200: the tensor core applies the 128-byte swizzle to the absolute
             // shared-memory address (as TMA did when it wrote the box), so the descriptor's base-offset field must stay
@@ -715,19 +697,17 @@ conv_gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __gri
                 if (k < nk)
                   ptx::umma_bf16_ss(tmem_acc, adesc + (uint64_t)(2 * k), bdesc + (uint64_t)(2 * k), p.idesc,
                                     (g > 0 || dx > 0 || k > 0) ? 1u : 0u);
-              if (!p.b_resident) ptx::umma_commit(&empty_bar[s]);
+              ptx::umma_commit(&empty_bar[s]);
               if (dx == 2) ptx::umma_commit(&aempty_bar[sa]);  // the box may be refilled once its three taps retire
               if (dx == 2 && g == 3 * p.kb_per_tap - 1) ptx::umma_commit(&tmem_full_bar[as]);
             }
             __syncwarp();
-            if (!p.b_resident) {
-              if (++s == p.stages) { s = 0; phase ^= 1u; }
-            }
+            if (++s == p.stages) { s = 0; phase ^= 1u; }
           }
           if (++sa == p.a_stages) { sa = 0; pha ^= 1u; }
         }
         if (lane == 0 && ti < 6) conv_stamp(p, 5 + ti);
-        if (++as == p.acc_stages) { as = 0; aphase ^= 1u; }
+        if (++as == ACC_STAGES) { as = 0; aphase ^= 1u; }
       }
     } else {
       int s = 0;
@@ -766,7 +746,7 @@ conv_gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __gri
           if (++s == p.stages) { s = 0; phase ^= 1u; }
         }
         if (lane == 0 && ti < 6) conv_stamp(p, 5 + ti);
-        if (++as == p.acc_stages) { as = 0; aphase ^= 1u; }
+        if (++as == ACC_STAGES) { as = 0; aphase ^= 1u; }
       }
     }
   } else {
@@ -1008,7 +988,7 @@ __device__ __forceinline__ void epilogue_loop_pair(const ConvKParams& p, uint32_
                                          }
                                        }, stat_acc);
         if (et == 0 && ti < 8) conv_stamp(p, 13 + 2 * ti);
-        if (++as == p.acc_stages) { as = 0; aphase ^= 1u; }
+        if (++as == ACC_STAGES) { as = 0; aphase ^= 1u; }
         continue;
       }
       for (int c0 = 0; c0 < p.block_n; c0 += 32) {
@@ -1051,7 +1031,7 @@ __device__ __forceinline__ void epilogue_loop_pair(const ConvKParams& p, uint32_
       if (lane == 0) ptx::mbar_arrive_leader(&tmem_empty_bar[as]);
     }
     if (et == 0 && ti < 8) conv_stamp(p, 13 + 2 * ti);
-    if (++as == p.acc_stages) { as = 0; aphase ^= 1u; }
+    if (++as == ACC_STAGES) { as = 0; aphase ^= 1u; }
   }
   if (stat_acc != nullptr && stat_n0 >= 0) flush_stats(p, stat_acc, stat_n0, lane);
   if (MODE == MC_EPI_PNHWC && p.tma_bufs > 0 && lane == 0) ptx::bulk_wait_group_read<0>();  // slabs read before the CTA exits
@@ -1081,9 +1061,9 @@ conv_gemm_tcgen05_pair_kernel(const __grid_constant__ CUtensorMap tmap_b, const 
   uint8_t* aux = b_ring + (size_t)p.stages * b_half_bytes;
   uint64_t* full_bar = reinterpret_cast<uint64_t*>(aux);
   uint64_t* empty_bar = full_bar + MAX_STAGES;
-  uint64_t* tmem_full_bar = empty_bar + MAX_STAGES;   // [MAX_ACC]
-  uint64_t* tmem_empty_bar = tmem_full_bar + MAX_ACC; // [MAX_ACC]
-  uint64_t* afull_bar = tmem_empty_bar + MAX_ACC;     // [MAX_A_STAGES]
+  uint64_t* tmem_full_bar = empty_bar + MAX_STAGES;      // [ACC_STAGES]
+  uint64_t* tmem_empty_bar = tmem_full_bar + ACC_STAGES; // [ACC_STAGES]
+  uint64_t* afull_bar = tmem_empty_bar + ACC_STAGES;     // [MAX_A_STAGES]
   uint64_t* aempty_bar = afull_bar + MAX_A_STAGES;    // [MAX_A_STAGES]
   uint32_t* tmem_ptr_smem = reinterpret_cast<uint32_t*>(aempty_bar + MAX_A_STAGES);
   float* s_ss = reinterpret_cast<float*>(aux + 512);
@@ -1103,7 +1083,7 @@ conv_gemm_tcgen05_pair_kernel(const __grid_constant__ CUtensorMap tmap_b, const 
       ptx::mbar_init(&full_bar[s], 1);
       ptx::mbar_init(&empty_bar[s], 1);
     }
-    for (int a = 0; a < p.acc_stages; ++a) {
+    for (int a = 0; a < ACC_STAGES; ++a) {
       ptx::mbar_init(&tmem_full_bar[a], 1);
       ptx::mbar_init(&tmem_empty_bar[a], 8);  // 4 epilogue warps of each CTA
     }
@@ -1195,7 +1175,7 @@ conv_gemm_tcgen05_pair_kernel(const __grid_constant__ CUtensorMap tmap_b, const 
           if (++sa == p.a_stages) { sa = 0; pha ^= 1u; }
         }
         if (lane == 0 && ti < 6) conv_stamp(p, 5 + ti);
-        if (++as == p.acc_stages) { as = 0; aphase ^= 1u; }
+        if (++as == ACC_STAGES) { as = 0; aphase ^= 1u; }
       }
     }
   } else {
@@ -1308,36 +1288,14 @@ extern "C" int mc_conv_fwd(const mc_conv_desc* d, void* stream_) {
   MC_CHECK_ARG(M_rows < (1ll << 31), "mc_conv_fwd: too many rows");
   const int m_tiles = (int)((M_rows + BLOCK_M - 1) / BLOCK_M);
 
-  // 3x3 with 64-wide k-blocks: share one activation box among the three dx taps (MCB200_SHARE_DX=0 disables)
-  static int share_env = -1, share_env32 = 1;
-  if (share_env < 0) {
-    const char* e = mc_tune_env("MCB200_SHARE_DX");
-    share_env = (e && e[0] == '0') ? 0 : 1;
-    share_env32 = (e && e[0] == '2') ? 0 : 1;
-  }
-  // (MCB200_SHARE_DX=2 restricts the shared box to 64-wide k-blocks, the state before the 64-byte-swizzle variant)
+  // 3x3 with 64-wide k-blocks: share one activation box among the three dx taps.
   // 32-wide k-blocks share the box only on long, feed-bound launches (dense conv2: 21,841 tiles, 306 -> 262 us); short
   // ones lose a little to the two-ring pipeline (shrunk conv13, 365 tiles: 18 -> 21 us)
-  const int share_dx = (d->ksize == 3 && share_env && (BLOCK_K == 64 || (share_env32 && m_tiles >= 2048))) ? 1 : 0;
+  const int share_dx = (d->ksize == 3 && (BLOCK_K == 64 || m_tiles >= 2048)) ? 1 : 0;
   const int a_box_stride = BLOCK_K == 64 ? A_BOX_STRIDE : A_BOX_STRIDE / 2;
   int block_n = d->block_n;
   // (the operand-feed term keeps the un-shared 16 KB A tile: with the shared-box figure the model picks narrower tiles
   //  that measured 4 % slower end to end on B200)
-  {  // experiment switch: MCB200_CONV_BN_BIG=<bn> forces the tile width of the wide 3x3 layers (Npad >= 960)
-    static int bn_big = -1;
-    if (bn_big < 0) {
-      const char* e = mc_tune_env("MCB200_CONV_BN_BIG");
-      bn_big = e ? atoi(e) : 0;
-    }
-    if (block_n <= 0 && bn_big >= 16 && bn_big <= 256 && (bn_big % 16) == 0 && d->Npad >= 960 && d->ksize == 3) block_n = bn_big;
-    static int bn_mid = -1;  // MCB200_CONV_BN_MID=<bn>: same for 3x3 layers with 512 <= Npad < 960
-    if (bn_mid < 0) {
-      const char* e = mc_tune_env("MCB200_CONV_BN_MID");
-      bn_mid = e ? atoi(e) : 0;
-    }
-    if (block_n <= 0 && bn_mid >= 16 && bn_mid <= 256 && (bn_mid % 16) == 0 && d->Npad >= 512 && d->Npad < 960 && d->ksize == 3)
-      block_n = bn_mid;
-  }
   if (decode) block_n = d->Npad;  // every logit of a cell in ONE accumulator row
   if (block_n <= 0) block_n = pick_block_n(d->Npad, m_tiles, (ntaps * Kc + 63) / 64, mc_num_sms(), false);  // 64-wide k-block units
   const bool want_stats = d->d_stat_sum != nullptr || d->d_stat_sumsq != nullptr;
@@ -1356,49 +1314,24 @@ extern "C" int mc_conv_fwd(const mc_conv_desc* d, void* stream_) {
   const long long total_tiles = (long long)n_tiles * m_tiles;
   const int acc_stride = block_n == 16 ? 16 : ((block_n + 31) / 32) * 32;
   int tmem_cols = 32;
-  while (tmem_cols < 2 * acc_stride) tmem_cols <<= 1;  // at least two accumulator stages (more below for narrow layers)
+  while (tmem_cols < ACC_STAGES * acc_stride) tmem_cols <<= 1;
   const int num_kb = ntaps * (Kc / BLOCK_K);
   constexpr size_t AUX_BYTES = 5120 + 1024;  // barriers (512), scale/shift staging (4096), pad to 1 KB; 1024-byte alignment slack
 
-  // smem ring of one CTA when `ctas` CTAs share an SM (each CTA also costs 1 KB of reserved shared memory)
-  // resident weights: one N tile and all taps' weight tiles fit beside the activation ring -> loaded once per CTA
-  // (narrow 3x3 layers: the per-tile weight re-load is otherwise as much TMA traffic as the activations)
-  const size_t b_res_bytes = (size_t)num_kb * block_n * BLOCK_K * 2;
-  // OFF by default (MCB200_CONV_RESIDENT=1 enables): measured on B200 it loses to the weight ring on every narrow
-  // 3x3 shape tried (64->64 @52x52: 37 us vs 25 us; 48->32 @104x104: 71 vs 58; 40->80 @52x52: 41 vs 33) because the
-  // resident tiles leave room for ONE CTA per SM, and three small CTAs per SM hide the per-tile latency chain better
-  // than the saved weight traffic.
-  static int res_env = -1;
-  if (res_env < 0) {
-    const char* e = mc_tune_env("MCB200_CONV_RESIDENT");
-    res_env = (e && e[0] == '1') ? 1 : 0;
-  }
-  const int b_resident = (res_env && share_dx && n_tiles == 1 && d->stages <= 0 && b_res_bytes <= 112 * 1024) ? 1 : 0;
   // staged epilogue (PNHWC, tiles up to 128 wide): 128 rows x (block_n bf16 + 16 B) of shared memory
-  static int stage_env = -1;  // MCB200_CONV_STAGE_OUT=0 disables (A/B switch)
-  if (stage_env < 0) {
-    const char* e = mc_tune_env("MCB200_CONV_STAGE_OUT");
-    stage_env = (e && e[0] == '0') ? 0 : ((e && e[0] == '2') ? 2 : 1);
-  }
   // (measured: tiles 32..96 wide gain — dense conv2 396 -> 300 us, conv4' 60 -> 54, shrunk conv8 33 -> 29; 128-wide tiles
   //  lose smem ring depth to the 34 KB staging buffer (133 -> 154 us) and 16-wide rows are two stores either way)
   // Wider tiles go through the buffer in 64-column chunks where it was measured to pay: 3x3 layers at high resolution
   // (dense conv3/conv5, 128 wide, 5513 tiles: 137 -> 123 us); wide 1x1 layers (conv7: 39 -> 47 us) and the short
-  // launches of the 26x26 / 13x13 stages do not.  MCB200_CONV_STAGE_OUT=2 stages every wide tile (A/B switch).
-  const bool wide_ok = stage_env == 2 || (d->ksize == 3 && m_tiles >= 1024);
+  // launches of the 26x26 / 13x13 stages do not.
+  const bool wide_ok = d->ksize == 3 && m_tiles >= 1024;
   // TMA-store epilogue (tiles >= 64 wide): whole 64-column chunks leave as bulk tensor stores from 4 KB slabs per
   // epilogue warp — two slabs per warp when the CTA has the SM to itself, one (16 KB per CTA) when several CTAs share
   // it (measured: dense conv4/conv6 at 104x104 run 113 us with 2 CTAs per SM + one slab, 158 us with one CTA + two
-  // slabs, 125 us with the staged epilogue).  MCB200_CONV_TMA_OUT=0 disables, =1 / =2 force the slab count.
-  static int tma_env = -1;
-  if (tma_env < 0) {
-    const char* e = mc_tune_env("MCB200_CONV_TMA_OUT");
-    tma_env = e ? atoi(e) : 3;
-    if (tma_env < 0 || tma_env > 3) tma_env = 3;
-  }
-  const bool tma_out = tma_env && d->epi_mode == MC_EPI_PNHWC && block_n >= 64 && ((d->ldc | d->ch_off) & 7) == 0;
-  auto tma_bufs_for = [&](int ctas_) -> int { return !tma_out ? 0 : (tma_env == 3 ? (ctas_ == 1 ? 2 : 1) : tma_env); };
-  const bool stage_out = !tma_out && stage_env && d->epi_mode == MC_EPI_PNHWC && block_n >= 32 && (block_n <= 96 || wide_ok) &&
+  // slabs, 125 us with the staged epilogue).
+  const bool tma_out = d->epi_mode == MC_EPI_PNHWC && block_n >= 64 && ((d->ldc | d->ch_off) & 7) == 0;
+  auto tma_bufs_for = [&](int ctas_) -> int { return tma_out ? (ctas_ == 1 ? 2 : 1) : 0; };
+  const bool stage_out = !tma_out && d->epi_mode == MC_EPI_PNHWC && block_n >= 32 && (block_n <= 96 || wide_ok) &&
                          ((d->ldc | d->ch_off) & 7) == 0;
   const int out_chunk = block_n <= 96 ? block_n : 64;
   const int out_pitch = stage_out ? out_chunk * 2 + 16 : 0;
@@ -1408,21 +1341,13 @@ extern "C" int mc_conv_fwd(const mc_conv_desc* d, void* stream_) {
                   : (tma_out ? (size_t)tma_bufs_for(ctas_) * 4 * 4096 + (want_stats ? 4 * 512 * sizeof(float) : 0)
                              : (size_t)128 * out_pitch);
   };
+  // smem ring of one CTA when `ctas` CTAs share an SM (each CTA also costs 1 KB of reserved shared memory)
   auto plan_ring = [&](int ctas, int* st, int* ast, size_t* bytes) -> bool {
     const size_t out_stage_bytes = out_stage_for(ctas);
     const long long cap = (ctas == 1 ? 220 * 1024 - (long long)AUX_BYTES : (227 * 1024) / ctas - 1024 - (long long)AUX_BYTES) - (long long)out_stage_bytes;
-    if (b_resident) {
-      // the activation ring is the only pipeline left: as deep as the smem beside the weights allows (a tile is 3 boxes)
-      long long a = (cap - (long long)b_res_bytes) / a_box_stride;
-      if (a > MAX_A_STAGES) a = MAX_A_STAGES;
-      if (a < (ctas == 1 ? 3 : 2)) return false;
-      *st = 1; *ast = (int)a;
-      *bytes = (size_t)a * a_box_stride + b_res_bytes + AUX_BYTES + out_stage_bytes;
-      return true;
-    }
     if (share_dx) {
       const int b_bytes = block_n * BLOCK_K * 2;
-      int a = ctas == 1 ? DEF_A_STAGES : 2;
+      int a = ctas == 1 ? MAX_A_STAGES : 2;
       long long stg = (cap - (long long)a * a_box_stride) / b_bytes;
       if (stg > MAX_STAGES) stg = MAX_STAGES;
       if (stg < 3) return false;
@@ -1440,28 +1365,16 @@ extern "C" int mc_conv_fwd(const mc_conv_desc* d, void* stream_) {
   };
   // CTAs per SM.  Wide, long-K tiles are tensor-bound: one CTA with the deepest ring.  Narrow layers are bound by the
   // per-tile latency chain, which only more CTAs (or tiles) in flight hide: up to 3 when the rings and the TMEM
-  // slices fit and every CTA still gets >= 2 tiles.  MCB200_CONV_CTAS=1|2|3 forces the upper limit.
-  static int ctas_env = -1;
-  if (ctas_env < 0) {
-    const char* e = mc_tune_env("MCB200_CONV_CTAS");
-    ctas_env = e ? atoi(e) : 0;
-    if (ctas_env < 0 || ctas_env > 3) ctas_env = 0;
-  }
-  static int min_tiles = -1;  // tiles every CTA must get before another CTA per SM is added (MCB200_CONV_MINTILES, A/B)
-  if (min_tiles < 0) {
-    const char* e = mc_tune_env("MCB200_CONV_MINTILES");
-    min_tiles = e ? atoi(e) : 1;  // measured: 1 beats 2 by 0.5 % on the shrunk step (the 365-tile 26x26 layers get 2 CTAs per SM)
-    if (min_tiles < 1) min_tiles = 1;
-  }
+  // slices fit and every CTA still gets at least one tile (measured: one beats two by 0.5 % on the shrunk step, the
+  // 365-tile 26x26 layers get 2 CTAs per SM).
   int ctas = 1;
   {
-    const int limit = ctas_env ? ctas_env : 3;
     const double main_cycles = (double)num_kb * (BLOCK_K / 64.0) * (2.0 * block_n > 128.0 + block_n ? 2.0 * block_n : 128.0 + block_n);
-    const bool narrow = ctas_env ? true : main_cycles < 6000.0;
-    for (int c = limit; c >= 2 && narrow; --c) {
+    const bool narrow = main_cycles < 6000.0;
+    for (int c = 3; c >= 2 && narrow; --c) {
       int st, ast;
       size_t bytes;
-      if (c * tmem_cols > 512 || total_tiles < (long long)min_tiles * c * mc_num_sms() || !plan_ring(c, &st, &ast, &bytes)) continue;
+      if (c * tmem_cols > 512 || total_tiles < (long long)c * mc_num_sms() || !plan_ring(c, &st, &ast, &bytes)) continue;
       ctas = c;
       break;
     }
@@ -1474,7 +1387,7 @@ extern "C" int mc_conv_fwd(const mc_conv_desc* d, void* stream_) {
   } else {
     ctas = 1;
     if (share_dx) {
-      a_stages = DEF_A_STAGES;
+      a_stages = MAX_A_STAGES;
       MC_CHECK_ARG(stages >= 2 && stages <= MAX_STAGES, "mc_conv_fwd: stages %d invalid", stages);
       smem_bytes = (size_t)a_stages * a_box_stride + (size_t)stages * block_n * BLOCK_K * 2 + AUX_BYTES + out_stage_for(1);
     } else {
@@ -1484,18 +1397,12 @@ extern "C" int mc_conv_fwd(const mc_conv_desc* d, void* stream_) {
   }
   MC_CHECK_ARG(smem_bytes <= 227 * 1024, "mc_conv_fwd: smem %zu too large", smem_bytes);
 
-  // CTA pair (cta_group::2) for the wide 3x3 layers: MCB200_CONV_2CTA=0 off, 1 auto (default), 2 wherever legal
-  static int pair_env = -1;
-  if (pair_env < 0) {
-    const char* e = mc_tune_env("MCB200_CONV_2CTA");
-    pair_env = e ? atoi(e) : 1;
-    if (pair_env < 0 || pair_env > 2) pair_env = 1;
-  }
+  // CTA pair (cta_group::2) for the wide 3x3 layers
   const bool pair_legal = share_dx && BLOCK_K == 64 && d->stages <= 0 && (block_n % 16) == 0 && block_n >= 64 && m_tiles >= 2;
-  const bool use_pair = !decode && pair_legal && (pair_env == 2 || (pair_env == 1 && block_n >= 192 && num_kb >= 36));
+  const bool use_pair = !decode && pair_legal && block_n >= 192 && num_kb >= 36;
   if (use_pair) {
     ctas = 1;
-    a_stages = DEF_A_STAGES;
+    a_stages = MAX_A_STAGES;
     const int b_half = block_n / 2 * 128;
     const int slab_bytes = tma_bufs_for(1) * 4 * 4096 + (want_stats ? 4 * 512 * (int)sizeof(float) : 0);
     stages = (220 * 1024 - a_stages * A_BOX_STRIDE - slab_bytes) / b_half;
@@ -1545,38 +1452,16 @@ extern "C" int mc_conv_fwd(const mc_conv_desc* d, void* stream_) {
   p.block_n = block_n;
   p.stages = stages;
   p.share_dx = share_dx;
-  p.b_resident = (b_resident && !use_pair) ? 1 : 0;
   {
     const int rem = d->Cin - (Kc / BLOCK_K - 1) * BLOCK_K;  // channels in the last channel block of a tap
     p.last_ksteps = (rem + 15) / 16;
   }
   p.a_stages = a_stages;
-  // Accumulator stages: two.  More (a narrow one-N-tile layer's tiles are small, the CTA's TMEM share holds up to 8) was
-  // measured on B200 and rejected: no gain on the narrow layers themselves (their epilogue warps, not the hand-back
-  // round trip, set the ~1 us per tile and CTA), and the larger TMEM allocations keep the next kernel's CTAs from
-  // co-residing with this kernel's tail (dense step 2.25 -> 2.35 ms).  MCB200_CONV_ACC=<n> (3..8) enables it for A/B.
-  static int acc_env = -1;
-  if (acc_env < 0) {
-    const char* e = mc_tune_env("MCB200_CONV_ACC");
-    acc_env = e ? atoi(e) : 0;
-  }
-  int acc_stages = 2;
-  if (n_tiles == 1 && !use_pair && acc_env > 2) {
-    int budget = ctas == 1 ? 512 : (ctas == 2 ? 256 : 128);
-    acc_stages = budget / acc_stride;
-    if (acc_stages > MAX_ACC) acc_stages = MAX_ACC;
-    if (acc_stages > acc_env) acc_stages = acc_env;
-    if (acc_stages < 2) acc_stages = 2;
-    tmem_cols = 32;
-    while (tmem_cols < acc_stages * acc_stride) tmem_cols <<= 1;
-  }
-  p.acc_stages = acc_stages;
   p.out_pitch = use_pair ? 0 : out_pitch;
   p.out_chunk = out_chunk;
   p.tma_bufs = tma_bufs;
   p.stat_sum = d->d_stat_sum;
   p.stat_sumsq = d->d_stat_sumsq;
-  MC_CHECK_ARG(!want_stats || tma_bufs > 0, "mc_conv_fwd: statistics need the TMA-store epilogue (tuning switch disabled it)");
   {
     auto magic = [](unsigned int dv, unsigned int* mul, unsigned int* shr) {
       unsigned int l = 0;
@@ -1622,10 +1507,9 @@ extern "C" int mc_conv_fwd(const mc_conv_desc* d, void* stream_) {
 
   if (use_pair) {
     p.idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(block_n >> 3) << 17) | ((uint32_t)(256 >> 4) << 24);
-    p.acc_stages = 2;
     p.acc_stride = ((block_n + 31) / 32) * 32;
     p.tmem_cols = 32;
-    while (p.tmem_cols < 2 * p.acc_stride) p.tmem_cols <<= 1;
+    while (p.tmem_cols < ACC_STAGES * p.acc_stride) p.tmem_cols <<= 1;
     static int max_clusters = -1;
     if (max_clusters < 0) {
       MC_CUDA(cudaFuncSetAttribute(conv_gemm_tcgen05_pair_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
@@ -1652,7 +1536,7 @@ extern "C" int mc_conv_fwd(const mc_conv_desc* d, void* stream_) {
     // clusters — without it the 26 left-over units cost a whole second round).  Measured on B200 for the bench shapes
     // (196 units = 2.65 waves): no gain, 0.8556 vs 0.8584 ms per step — the 48 clusters of a two-thirds-full last wave
     // run their units faster because the operand feed from L2 is shared by fewer SMs, so whole tiles are kept there.
-    // Needs the caller's workspace; MCB200_CONV_STREAMK=0 disables, =2 forces it for any remainder (tuning builds).
+    // Needs the caller's workspace.
     p.sk_first = (int)units;
     p.sk_units = 0;
     p.sk_gper = 3 * p.kb_per_tap;
@@ -1662,11 +1546,8 @@ extern "C" int mc_conv_fwd(const mc_conv_desc* d, void* stream_) {
     p.sk_part = nullptr;
     {
       const long long full = units / clusters, rem = units % clusters;
-      const char* e = mc_tune_env("MCB200_CONV_STREAMK");
-      const bool on = !(e && e[0] == '0');
-      const bool any_rem = e && e[0] == '2';
       const size_t need = mc_workspace_bytes_conv_fwd(d);
-      if (on && full >= 1 && rem > 0 && (rem * 2 <= (long long)clusters || any_rem) && d->d_ws != nullptr && need > 0 &&
+      if (full >= 1 && rem > 0 && rem * 2 <= (long long)clusters && d->d_ws != nullptr && need > 0 &&
           d->ws_bytes >= need && ((uintptr_t)d->d_ws & 255) == 0) {
         p.sk_first = (int)(full * clusters);
         p.sk_units = (int)rem;
@@ -1691,17 +1572,8 @@ extern "C" int mc_conv_fwd(const mc_conv_desc* d, void* stream_) {
     attr_set = true;
   }
   const long long max_ctas = (long long)mc_num_sms() * ctas;
-  int grid = (int)(total_tiles < max_ctas ? total_tiles : max_ctas);
-  static int trace_env = -1;  // MCB200_CONV_TRACE=1: one line per launch on stderr (tools/bench_layers.py)
-  if (trace_env < 0) {
-    const char* e = mc_tune_env("MCB200_CONV_TRACE");
-    trace_env = (e && e[0] == '1') ? 1 : 0;
-  }
-  if (trace_env)
-    fprintf(stderr, "[mc_conv_fwd] %dx%d k%d Cin %d N %d: m_tiles %d block_n %d n_tiles %d kb %d(x%d) ctas %d stages %d/%d share %d stage_out %d grid %d smem %zu\n",
-            d->H, d->W, d->ksize, d->Cin, d->N, m_tiles, block_n, n_tiles, num_kb, BLOCK_K, ctas, stages, a_stages, share_dx,
-            p.out_pitch, grid, smem_bytes);
-  g_last_plan[0] = 0; g_last_plan[1] = block_n; g_last_plan[2] = ctas; g_last_plan[3] = p.b_resident;
+  const int grid = (int)(total_tiles < max_ctas ? total_tiles : max_ctas);
+  g_last_plan[0] = 0; g_last_plan[1] = block_n; g_last_plan[2] = ctas; g_last_plan[3] = 0;
   g_last_plan[4] = share_dx; g_last_plan[5] = stages; g_last_plan[6] = grid; g_last_plan[7] = BLOCK_K;
   if (ctas >= 3)
     conv_gemm_tcgen05_kernel<3><<<grid, NUM_THREADS, smem_bytes, stream>>>(tm_a, tm_b, tm_abox, tm_out, p);

@@ -39,7 +39,7 @@ struct WgradParams {
   int m_tiles, n_tiles, ntaps;
   int block_n, nb64;  // N tile (multiple of 16, <= 256) and its number of 64-column boxes
   int stages, tmem_cols;
-  int Wp, ksize;
+  int Wp;
   int share3;       // 3x3: one CTA = one filter row (dy), three accumulators, the activation box shared by its 3 taps
   int merge3;       // share3 with <= 64 input channels: the three dx taps are ONE instruction of N = 192 (see the issuer)
   uint32_t idesc3;  // instruction descriptor of that N = 192 instruction
@@ -102,9 +102,8 @@ conv_wgrad_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_dz, const __g
   const int kb0 = (int)(((long long)p.num_kb * split) / p.nsplit);
   const int kb1 = (int)(((long long)p.num_kb * (split + 1)) / p.nsplit);
   const int m0 = m_tile * BLOCK_M, n0 = n_tile * p.block_n;
-  int row_off = 0;
-  if (p.share3) row_off = (tap - 1) * p.Wp - 1;  // first row of the box: tap dx reads it dx rows further down
-  else if (p.ksize == 3) row_off = (tap / 3 - 1) * p.Wp + (tap % 3 - 1);
+  // 3x3: first row of the box, tap dx reads it dx rows further down; 1x1: no offset
+  const int row_off = p.share3 ? (tap - 1) * p.Wp - 1 : 0;
 
   if (warp_idx == 0 && lane == 0) {
     ptx::prefetch_tensormap(&tmap_dz);
@@ -346,12 +345,7 @@ int plan_wgrad(WgradPlan* pl, int B, int H, int W, int C, int O, int ksize) {
   pl->num_kb = (int)((rows + BLOCK_K - 1) / BLOCK_K);
   pl->m_tiles = (O + BLOCK_M - 1) / BLOCK_M;
   const int c16 = (C + 15) / 16 * 16;
-  static int share_env = -1;
-  if (share_env < 0) {
-    const char* e = mc_tune_env("MCB200_WGRAD_SHARE");
-    share_env = (e && e[0] == '0') ? 0 : 1;
-  }
-  pl->share3 = (ksize == 3 && share_env) ? 1 : 0;
+  pl->share3 = ksize == 3 ? 1 : 0;
   const int max_n = pl->share3 ? 128 : 256;  // share3: three accumulators must fit the 512 TMEM columns
   pl->n_tiles = (c16 + max_n - 1) / max_n;
   pl->block_n = ((c16 + pl->n_tiles - 1) / pl->n_tiles + 15) / 16 * 16;
@@ -384,12 +378,7 @@ int plan_wgrad(WgradPlan* pl, int B, int H, int W, int C, int O, int ksize) {
   if (stages > MAX_STAGES) stages = MAX_STAGES;
   pl->stages = stages;
   pl->smem_bytes = (size_t)stages * stage_bytes + 256 + 1024;
-  static int merge_env = -1;
-  if (merge_env < 0) {
-    const char* e = mc_tune_env("MCB200_WGRAD_MERGE");
-    merge_env = (e && e[0] == '0') ? 0 : 1;
-  }
-  pl->merge3 = (pl->share3 && pl->nb64 == 1 && pl->n_tiles == 1 && merge_env) ? 1 : 0;
+  pl->merge3 = (pl->share3 && pl->nb64 == 1 && pl->n_tiles == 1) ? 1 : 0;
   int tc = 32;
   while (tc < (pl->merge3 ? 192 : (pl->share3 ? 3 : 1) * pl->block_n)) tc <<= 1;
   pl->tmem_cols = tc;
@@ -441,7 +430,6 @@ extern "C" int mc_conv_wgrad(const void* d_a, int lda, int C, const void* d_dz, 
   p.stages = pl.stages;
   p.tmem_cols = pl.tmem_cols;
   p.Wp = W + 1;
-  p.ksize = ksize;
   p.share3 = pl.share3;
   p.merge3 = pl.merge3;
   p.Opad = pl.Opad;

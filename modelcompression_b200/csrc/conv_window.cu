@@ -37,15 +37,6 @@
 
 namespace {
 
-// Attribution switches (tuning builds only, MCB200_WIN_X bit mask: 1 no MMA, 2 MMAs twice, 4 no epilogue math/stores,
-// 8 no image loads, 16 polling waits, 32/64 plain arrives instead of tcgen05.commit); a product build compiles them out.
-#ifdef MCB200_TUNING
-#define WIN_X(bit) ((p.xflags & (bit)) != 0)
-#else
-#define WIN_X(bit) false
-#endif
-#define WIN_WAIT(bar, parity) do { if (WIN_X(16)) ptx::mbar_wait_poll(bar, parity); else ptx::mbar_wait(bar, parity); } while (0)
-
 constexpr int WTY = 16, WTX = 8;  // GEMM rows of a tile: (ty, tx), row = ty*8 + tx = TMEM lane
 // CTA = FRONT warps (P8: TMA producer + MMA issuer; IMG: 4 warps that load + convert the image, warp 0 also issues the MMAs)
 // + 4 epilogue warps (one per TMEM lane quarter)
@@ -65,15 +56,7 @@ struct WinParams {
   int tiles_x, tiles_y, total_tiles;
   int tmem_cols, acc_stages, acc_shift;  // accumulator stages in TMEM (power of two, 1..8) and log2 of it
   uint32_t idesc;
-  unsigned long long* dbg;  // tuning builds: clock64 stamps of CTA 0 (mc_debug_window_trace), else nullptr
-  int xflags;               // tuning builds (MCB200_WIN_X): 1 no MMA, 2 MMAs issued twice, 4 no epilogue math/stores, 8 no conversion
 };
-
-#ifdef MCB200_TUNING
-#define WIN_STAMP(slot) do { if (p.dbg != nullptr && blockIdx.x == 0 && it >= 8 && it < 16) p.dbg[(it - 8) * 16 + (slot)] = clock64(); } while (0)
-#else
-#define WIN_STAMP(slot) do { } while (0)
-#endif
 
 // K-major operand without swizzle: 8-row core matrices, rows 16 B apart, groups `sbo` bytes apart, the instruction's
 // second K chunk `lbo` bytes after the first.
@@ -138,9 +121,11 @@ struct WinGeom {
 // These layers are LATENCY bound (clock64 traces: per tile and CTA the epilogue chain accumulator-ready -> tcgen05.ld ->
 // math -> stores -> hand-back takes ~1,900 cycles whatever the channel count), so the kernel is built for occupancy:
 // 6 warps per CTA, <= 42 registers (8 CTAs = 32 epilogue warps per SM) unless the tile is WIDE (> 16 output columns).
+// p is __grid_constant__ so that its fields are read from parameter space where they are used: passed by value, the
+// compiler loads the whole struct into registers at entry, and the image kernels then spill under their 64-register cap.
 template <int KIND, bool WIDE>
 __global__ void __launch_bounds__(WinGeom<KIND>::THREADS, WIDE ? 4 : (KIND == 0 ? 6 : 4))
-conv_window_kernel(const __grid_constant__ CUtensorMap tmap_in, const WinParams p) {
+conv_window_kernel(const __grid_constant__ CUtensorMap tmap_in, const __grid_constant__ WinParams p) {
   using G = WinGeom<KIND>;
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   uint8_t* smem = smem_raw;
@@ -235,13 +220,8 @@ conv_window_kernel(const __grid_constant__ CUtensorMap tmap_in, const WinParams 
   }
   auto issue_mma = [&](int ps, uint32_t tacc) {  // called by ONE elected lane
     const uint64_t soff = (uint64_t)((uint32_t)ps * (uint32_t)(G::PSTRIDE >> 4));
-    if (WIN_X(1)) return;
 #pragma unroll
     for (int i = 0; i < G::NMMA; ++i) ptx::umma_bf16_ss(tacc, adesc0[i] + soff, bdesc[i], p.idesc, i > 0 ? 1u : 0u);
-    if (WIN_X(2)) {
-#pragma unroll
-      for (int i = 0; i < G::NMMA; ++i) ptx::umma_bf16_ss(tacc, adesc0[i] + soff, bdesc[i], p.idesc, 1u);
-    }
   };
 
   if (warp_idx < G::FRONT_WARPS) {
@@ -272,7 +252,7 @@ conv_window_kernel(const __grid_constant__ CUtensorMap tmap_in, const WinParams 
 #pragma unroll
         for (int j = 0; j < 2; ++j) {
           const int y = 2 * ti.ty * WTY - 1 + qr[j], x = 2 * ti.tx * WTX - 4 + 4 * qk[j];
-          const bool ok = qok[j] && y >= 0 && y < p.H && x >= 0 && x + 4 <= p.W && !WIN_X(8);
+          const bool ok = qok[j] && y >= 0 && y < p.H && x >= 0 && x + 4 <= p.W;
           const uint8_t* src = img + (long long)ti.b * 3 * plane + ((long long)y * p.W + x) * EL;
 #pragma unroll
           for (int c = 0; c < 3; ++c) {
@@ -288,9 +268,7 @@ conv_window_kernel(const __grid_constant__ CUtensorMap tmap_in, const WinParams 
       for (unsigned int tile = tile_lo; tile < tile_hi; ++tile, ++it) {
         const int s = it & (G::NPATCH - 1);
         const uint32_t ph = (uint32_t)((it / G::NPATCH) & 1);
-        if (t == 0) WIN_STAMP(8);
-        WIN_WAIT(&patch_free[s], ph ^ 1u);  // MMAs of tile it-2 have read patch[s]
-        if (t == 0) WIN_STAMP(9);
+        ptx::mbar_wait(&patch_free[s], ph ^ 1u);  // MMAs of tile it-2 have read patch[s]
         uint8_t* patch = patch0 + (size_t)s * G::PSTRIDE;
         // quad k of row r -> patch pixels 4k+1 .. 4k+4 of patch row r, each pixel = (c0 c1 | c2 0) in bf16
 #pragma unroll
@@ -323,23 +301,18 @@ conv_window_kernel(const __grid_constant__ CUtensorMap tmap_in, const WinParams 
           tin.next(p.tiles_x, p.tiles_y);
           load_tile(tin);
         }
-        if (t == 0) WIN_STAMP(11);
         ptx::fence_proxy_async_smem();  // generic-proxy smem writes -> visible to the tensor core (async proxy)
         asm volatile("bar.sync 1, 128;" ::: "memory");  // patch[s] complete
-        if (t == 0) WIN_STAMP(12);
         if (warp_idx == 0) {
           const int a = it & (p.acc_stages - 1);
-          WIN_WAIT(&tmem_free[a], (uint32_t)(((it >> p.acc_shift) & 1) ^ 1));  // epilogue drained TMEM[a]
-          if (t == 0) WIN_STAMP(13);
+          ptx::mbar_wait(&tmem_free[a], (uint32_t)(((it >> p.acc_shift) & 1) ^ 1));  // epilogue drained TMEM[a]
           ptx::tc_fence_after();
           if (ptx::elect_one()) {
             issue_mma(s, tmem_base + (uint32_t)a * acc_stride);
-            if (WIN_X(32)) { ptx::mbar_arrive(&patch_free[s]); ptx::mbar_arrive(&tmem_full[a]); }
-            else if (WIN_X(64)) { ptx::mbar_arrive(&patch_free[s]); ptx::umma_commit(&tmem_full[a]); }
-            else { ptx::umma_commit(&patch_free[s]); ptx::umma_commit(&tmem_full[a]); }
+            ptx::umma_commit(&patch_free[s]);
+            ptx::umma_commit(&tmem_full[a]);
           }
           __syncwarp();
-          if (t == 0) WIN_STAMP(14);
         }
       }
     } else {
@@ -351,8 +324,7 @@ conv_window_kernel(const __grid_constant__ CUtensorMap tmap_in, const WinParams 
         for (unsigned int tile = tile_lo; tile < tile_hi; ++tile, ++it) {
           const int s = it & (G::NPATCH - 1);
           const uint32_t ph = (uint32_t)((it / G::NPATCH) & 1);
-          WIN_WAIT(&patch_free[s], ph ^ 1u);
-          if (lane == 0) WIN_STAMP(0);
+          ptx::mbar_wait(&patch_free[s], ph ^ 1u);
           if (ptx::elect_one()) issue_in(tin, s);
           __syncwarp();
           tin.next(p.tiles_x, p.tiles_y);
@@ -361,19 +333,15 @@ conv_window_kernel(const __grid_constant__ CUtensorMap tmap_in, const WinParams 
         int it = 0;
         for (unsigned int tile = tile_lo; tile < tile_hi; ++tile, ++it) {
           const int s = it & (G::NPATCH - 1), a = it & (p.acc_stages - 1);
-          WIN_WAIT(&in_full[s], (uint32_t)((it / G::NPATCH) & 1));
-          if (lane == 0) WIN_STAMP(1);
-          WIN_WAIT(&tmem_free[a], (uint32_t)(((it >> p.acc_shift) & 1) ^ 1));
-          if (lane == 0) WIN_STAMP(2);
+          ptx::mbar_wait(&in_full[s], (uint32_t)((it / G::NPATCH) & 1));
+          ptx::mbar_wait(&tmem_free[a], (uint32_t)(((it >> p.acc_shift) & 1) ^ 1));
           ptx::tc_fence_after();
           if (ptx::elect_one()) {
             issue_mma(s, tmem_base + (uint32_t)a * acc_stride);
-            if (WIN_X(32)) { ptx::mbar_arrive(&patch_free[s]); ptx::mbar_arrive(&tmem_full[a]); }
-            else if (WIN_X(64)) { ptx::mbar_arrive(&patch_free[s]); ptx::umma_commit(&tmem_full[a]); }
-            else { ptx::umma_commit(&patch_free[s]); ptx::umma_commit(&tmem_full[a]); }
+            ptx::umma_commit(&patch_free[s]);
+            ptx::umma_commit(&tmem_full[a]);
           }
           __syncwarp();
-          if (lane == 0) WIN_STAMP(3);
         }
       }
     }
@@ -410,9 +378,7 @@ conv_window_kernel(const __grid_constant__ CUtensorMap tmap_in, const WinParams 
       const bool valid = oy < Hout && ox < Wout && my_store;
       __nv_bfloat16* dst =
           reinterpret_cast<__nv_bfloat16*>(p.out) + (((long long)ti.b * (Hout + 1) + oy) * (Wout + 1) + ox) * ldc;
-      if (et == 0) WIN_STAMP(4);
-      WIN_WAIT(&tmem_full[a], aph);
-      if (et == 0) WIN_STAMP(5);
+      ptx::mbar_wait(&tmem_full[a], aph);
       ptx::tc_fence_after();
       const uint32_t trow = tmem_base + ((uint32_t)(quarter * 32) << 16) + (uint32_t)a * acc_stride;
 
@@ -444,8 +410,7 @@ conv_window_kernel(const __grid_constant__ CUtensorMap tmap_in, const WinParams 
         }
       };
 
-      if (WIN_X(4)) {
-      } else if constexpr (G::IMG) {
+      if constexpr (G::IMG) {
         const int np = p.npos;
         if (!WIDE && np == 4) {
           // all four window positions of the 4 filters in ONE 16-column load
@@ -531,13 +496,11 @@ conv_window_kernel(const __grid_constant__ CUtensorMap tmap_in, const WinParams 
         }
       }
       // the accumulator stage is drained: hand it back before the (possibly staged) copy-out
-      if (et == 0) WIN_STAMP(6);
       ptx::tc_fence_before();
       __syncwarp();
       if (lane == 0) ptx::mbar_arrive(&tmem_free[a]);
-      if (et == 0) WIN_STAMP(7);
 
-      if (staged && !WIN_X(4)) {
+      if (staged) {
         // the warp's pixels sit in shared memory [pixel][stage_pitch]; consecutive lanes write consecutive 16-byte
         // chunks of consecutive pixels: whole coalesced segments instead of 16-byte pieces one pixel pitch apart
         const int cpr = (n4 + 7) >> 3;  // 16-byte chunks per pixel that hold real channels
@@ -611,13 +574,6 @@ int launch_window(const WinParams& p, cudaStream_t stream) {
 
 }  // namespace
 
-static unsigned long long* g_window_dbg = nullptr;
-// Tuning builds: the next launches record clock64 stamps of CTA 0, tiles 8..15, 16 slots per tile, into d_buf (128 x u64).
-extern "C" int mc_debug_window_trace(void* d_buf) {
-  g_window_dbg = reinterpret_cast<unsigned long long*>(d_buf);
-  return 0;
-}
-
 // in_kind: 0 = bf16 PNHWC with pitch 8 (Cin <= 8), 1 = fp32 NCHW image, 2 = uint8 NCHW image (Cin <= 3, pool required)
 extern "C" int mc_conv_window_supported(int Cin, int in_kind, int N, int pool) {
   if (Cin < 1 || N < 1) return 0;
@@ -658,11 +614,6 @@ extern "C" int mc_conv_window_fwd(const void* d_in, int in_kind, const void* d_w
   MC_CHECK_ARG(((uintptr_t)d_w & 15) == 0 && ((uintptr_t)d_in & 15) == 0 && ((uintptr_t)d_out & 15) == 0,
                "mc_conv_window_fwd: pointers must be 16-byte aligned");
   WinParams p;
-  p.dbg = g_window_dbg;
-  {
-    const char* e = mc_tune_env("MCB200_WIN_X");
-    p.xflags = e ? atoi(e) : 0;
-  }
   p.in = d_in;
   p.w = reinterpret_cast<const __nv_bfloat16*>(d_w);
   p.out = d_out;

@@ -456,6 +456,10 @@ __global__ void __launch_bounds__(1024) filter_threshold_kernel(const float* __r
 // 31 rounds of "count keys below prefix|bit", both ranks at once, keys in shared memory — ~4 us for 10,461 values,
 // where a shared-memory radix histogram serialises on the few distinct high digits of values that all lie in (0,1].
 constexpr int FIN_THREADS = 1024;
+// Leaves of NumPy's pairwise recursion over one layer's values: at most 512 for the <= 51,200 values the kernel takes
+// (mc_filter_prune rejects more).  Every layer goes through the lane-parallel sum: thread 0 running the recursion itself
+// overflowed the 1 KB device stack on a layer of 27,000 filters.
+constexpr int FIN_MAX_LEAVES = 512;
 
 __device__ void block_count2(unsigned int c0, unsigned int c1, unsigned int* s_red /*[64]*/, unsigned int* out0,
                              unsigned int* out1) {
@@ -487,7 +491,7 @@ __global__ void __launch_bounds__(FIN_THREADS) filter_finish_kernel(const LayerT
   extern __shared__ __align__(16) unsigned char dsm[];
   float* s_v = reinterpret_cast<float*>(dsm);  // max(O_l, n) floats
   __shared__ float s_norm;
-  __shared__ float s_leaf[MAX_LEAVES];
+  __shared__ float s_leaf[FIN_MAX_LEAVES];
   __shared__ unsigned int s_red[64];
   __shared__ unsigned int s_last;
   const int l = blockIdx.x;
@@ -502,20 +506,16 @@ __global__ void __launch_bounds__(FIN_THREADS) filter_finish_kernel(const LayerT
   // ---- v /= sqrt(pairwise(v^2)); v /= max(v)   (methods.py:46-51)
   for (int o = threadIdx.x; o < O; o += FIN_THREADS) s_v[o] = v[o];
   __syncthreads();
-  if (O <= 128 * MAX_LEAVES) {
-    if (threadIdx.x < 32) {  // lane-parallel replay of NumPy's pairwise recursion (leaves are independent)
-      const int lane = threadIdx.x;
-      np_for_each_leaf(O, [&](int leaf, int st, int ln) {
-        if ((leaf & 31) == lane && leaf < MAX_LEAVES) s_leaf[leaf] = np_leaf_sum<true>(s_v + st, ln);
-      });
-      __syncwarp();
-      if (lane == 0) {
-        int next = 0;
-        s_norm = __fsqrt_rn(np_combine_leaves(s_leaf, O, &next));
-      }
+  if (threadIdx.x < 32) {  // lane-parallel replay of NumPy's pairwise recursion (leaves are independent)
+    const int lane = threadIdx.x;
+    np_for_each_leaf(O, [&](int leaf, int st, int ln) {
+      if ((leaf & 31) == lane) s_leaf[leaf] = np_leaf_sum<true>(s_v + st, ln);
+    });
+    __syncwarp();
+    if (lane == 0) {
+      int next = 0;
+      s_norm = __fsqrt_rn(np_combine_leaves(s_leaf, O, &next));
     }
-  } else if (threadIdx.x == 0) {
-    s_norm = __fsqrt_rn(np_pairwise<true>(s_v, O));
   }
   __syncthreads();
   const float nrm = s_norm;
@@ -1061,15 +1061,6 @@ int launch_sumsq(const LayerTable& lt, float* d_values, cudaStream_t stream) {
   const int n_generic = lt.toff[lt.nlayers] / SS_THREADS;
   const int first_wave = n_tiled < mc_num_sms() ? n_tiled : mc_num_sms();
   if (n_tiled + n_generic == 0) return 0;
-  const char* dbg = mc_tune_env("MCB200_SUMSQ_ONLY");  // timing experiments only (results are incomplete)
-  if (dbg && dbg[0] == 't') {
-    filter_sumsq_kernel<<<n_tiled, SS_THREADS, SUMSQ_SMEM, stream>>>(lt, d_values, n_tiled, first_wave);
-    return 0;
-  }
-  if (dbg && dbg[0] == 'g') {
-    filter_sumsq_kernel<<<n_generic, SS_THREADS, SUMSQ_SMEM, stream>>>(lt, d_values, 0, 0);
-    return 0;
-  }
   filter_sumsq_kernel<<<n_tiled + n_generic, SS_THREADS, SUMSQ_SMEM, stream>>>(lt, d_values, n_tiled, first_wave);
   MC_LAUNCH_CHECK("filter_sumsq_kernel");
   return 0;
@@ -1171,37 +1162,33 @@ extern "C" int mc_filter_prune(const float* const* h_w_ptrs, const int* h_O, con
   const int n = lt.voff[nlayers];
   MC_CHECK_ARG(k >= 0 && k < n, "mc_filter_prune: rank out of range");
   MC_CHECK_ARG(gamma >= 0.0 && gamma < 1.0, "mc_filter_prune: gamma must be in [0,1)");
-  {
-    const char* e = mc_tune_env("MCB200_FILTER_FUSED");  // =0: the three-launch path (A/B)
-    const bool fused_on = !(e && e[0] == '0');
-    if (fused_on && n <= FU_MAX_N) {
-      LayerTable lf;
-      rc = build_layers(&lf, h_w_ptrs, h_mask_ptrs, h_O, h_C, taps, nlayers, "mc_filter_prune", FU_THREADS, FU_F);
-      if (rc) return rc;
-      static int max_blocks = -1;
-      if (max_blocks < 0) {
-        MC_CUDA(cudaFuncSetAttribute(filter_prune_fused_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)FU_SMEM));
-        int per_sm = 0;
-        MC_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, filter_prune_fused_kernel, FU_THREADS, FU_SMEM));
-        if (per_sm < 1) return mc_set_error(MC_ERR_SHAPE, "mc_filter_prune: fused kernel does not fit an SM");
-        max_blocks = per_sm * mc_num_sms();
-      }
-      int n_tiled = lf.tblk[lf.ntiled];
-      int n_items = n_tiled + lf.toff[lf.nlayers] / FU_THREADS;
-      int n_big = 0;  // tiled items of the layers with >= 1024 input channels (torder is sorted by descending C)
-      for (int i2 = 0; i2 < lf.ntiled && h_C[lf.torder[i2]] >= 1024; ++i2) n_big = lf.tblk[i2 + 1];
-      int grid = n_items < max_blocks ? n_items : max_blocks;
-      if (grid < 1) grid = 1;
-      MC_CUDA(cudaMemsetAsync(d_ws, 0, sizeof(FusedState), stream));
-      long long kk = (long long)k;
-      FusedState* stp = reinterpret_cast<FusedState*>(d_ws);
-      float* d_raw = reinterpret_cast<float*>(reinterpret_cast<unsigned char*>(d_ws) + 2048);  // raw sums [n]
-      int fill = h_mask_ptrs ? 1 : 0;
-      void* args[] = {&lf, &d_raw, &d_values, &n_tiled, &n_big, &n_items, &kk, &gamma, &d_thr, &d_keep, &stp, &fill};
-      MC_CUDA(cudaLaunchCooperativeKernel(reinterpret_cast<void*>(filter_prune_fused_kernel), dim3((unsigned)grid),
-                                          dim3(FU_THREADS), args, FU_SMEM, stream));
-      return 0;
+  if (n <= FU_MAX_N) {
+    LayerTable lf;
+    rc = build_layers(&lf, h_w_ptrs, h_mask_ptrs, h_O, h_C, taps, nlayers, "mc_filter_prune", FU_THREADS, FU_F);
+    if (rc) return rc;
+    static int max_blocks = -1;
+    if (max_blocks < 0) {
+      MC_CUDA(cudaFuncSetAttribute(filter_prune_fused_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)FU_SMEM));
+      int per_sm = 0;
+      MC_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, filter_prune_fused_kernel, FU_THREADS, FU_SMEM));
+      if (per_sm < 1) return mc_set_error(MC_ERR_SHAPE, "mc_filter_prune: fused kernel does not fit an SM");
+      max_blocks = per_sm * mc_num_sms();
     }
+    int n_tiled = lf.tblk[lf.ntiled];
+    int n_items = n_tiled + lf.toff[lf.nlayers] / FU_THREADS;
+    int n_big = 0;  // tiled items of the layers with >= 1024 input channels (torder is sorted by descending C)
+    for (int i2 = 0; i2 < lf.ntiled && h_C[lf.torder[i2]] >= 1024; ++i2) n_big = lf.tblk[i2 + 1];
+    int grid = n_items < max_blocks ? n_items : max_blocks;
+    if (grid < 1) grid = 1;
+    MC_CUDA(cudaMemsetAsync(d_ws, 0, sizeof(FusedState), stream));
+    long long kk = (long long)k;
+    FusedState* stp = reinterpret_cast<FusedState*>(d_ws);
+    float* d_raw = reinterpret_cast<float*>(reinterpret_cast<unsigned char*>(d_ws) + 2048);  // raw sums [n]
+    int fill = h_mask_ptrs ? 1 : 0;
+    void* args[] = {&lf, &d_raw, &d_values, &n_tiled, &n_big, &n_items, &kk, &gamma, &d_thr, &d_keep, &stp, &fill};
+    MC_CUDA(cudaLaunchCooperativeKernel(reinterpret_cast<void*>(filter_prune_fused_kernel), dim3((unsigned)grid),
+                                        dim3(FU_THREADS), args, FU_SMEM, stream));
+    return 0;
   }
   const size_t fin_smem = (size_t)(n > max_o ? n : max_o) * sizeof(float);
   if (fin_smem > 200 * 1024) return mc_set_error(MC_ERR_SHAPE, "mc_filter_prune: %d filters exceed the single-block select", n);

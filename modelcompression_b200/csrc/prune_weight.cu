@@ -959,10 +959,8 @@ int launch_weight_prune(const float* const* h_w_ptrs, float* const* h_mask_ptrs,
   SelState* state = reinterpret_cast<SelState*>(d_ws);
   unsigned int* cand = reinterpret_cast<unsigned int*>(reinterpret_cast<char*>(d_ws) + state_bytes);
 
-  // MCB200_SELECT_EXACT=1 forces the exact radix path (used by the tests to cover the fallback on large inputs)
-  const char* force_exact = mc_tune_env("MCB200_SELECT_EXACT");
   // the fast path indexes elements with 32 bits and needs a sample much smaller than the data
-  int use_fast = (n >= 8 * SAMPLE && n < (1ll << 32) && !(force_exact && force_exact[0] == '1')) ? 1 : 0;
+  int use_fast = (n >= 8 * SAMPLE && n < (1ll << 32)) ? 1 : 0;
 
   static int blocks_per_sm[2] = {0, 0};
   const int which = h_mask_ptrs ? 1 : 0;

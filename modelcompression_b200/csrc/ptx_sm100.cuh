@@ -81,28 +81,6 @@ __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity, unsign
   }
 }
 
-// Polling wait (mbarrier.test_wait, never suspends): for pipelines whose stages are only a few hundred cycles long, where
-// the wake-up latency of a suspended try_wait would dominate.  Bounded like mbar_wait.
-__device__ __forceinline__ bool mbar_test_wait(uint64_t* bar, uint32_t parity) {
-  uint32_t ok;
-  asm volatile(
-      "{\n\t"
-      ".reg .pred P;\n\t"
-      "mbarrier.test_wait.parity.shared::cta.b64 P, [%1], %2;\n\t"
-      "selp.b32 %0, 1, 0, P;\n\t"
-      "}\n"
-      : "=r"(ok)
-      : "r"(smem_u32(bar)), "r"(parity)
-      : "memory");
-  return ok != 0;
-}
-__device__ __forceinline__ void mbar_wait_poll(uint64_t* bar, uint32_t parity) {
-  uint32_t spins = 0;
-  while (!mbar_test_wait(bar, parity)) {
-    if (++spins > (1u << 26)) __trap();
-  }
-}
-
 // ---------------- TMA ----------------
 __device__ __forceinline__ void prefetch_tensormap(const void* tmap) {
   asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(tmap)) : "memory");

@@ -99,7 +99,6 @@ class CompiledDarknet(object):
             if self.lib.mc_device_ok() != 1:
                 raise RuntimeError("Darknet.forward: " + self.lib.mc_last_error_string().decode())
         self.shrink = bool(shrink)
-        self.use_window = bool(getattr(model, 'b200_window', True))  # (False: the im2col-build kernels, for A/B runs)
         # CUDA-core kernel for the degenerate layers of a shrunk net (csrc/conv_thin.cu): 0 off, 1 on, 2 on + the 1x1 layer
         # behind a thin 3x3 layer applied in the same kernel
         self.use_thin = int(getattr(model, 'b200_thin', 2))
@@ -399,8 +398,8 @@ class CompiledDarknet(object):
 
         # ---- no-build window kernel (csrc/conv_window.cu): the image layer with its pool, and <= 8-channel PNHWC inputs
         win_kind = None
-        if self.use_window and plain_dst and k == 3 and (not pool or (H % 2 == 0 and W % 2 == 0)):
-            # Measured on B200 (tools/bench_window.py, batch 64): the window kernel wins for the narrow image layer
+        if plain_dst and k == 3 and (not pool or (H % 2 == 0 and W % 2 == 0)):
+            # Measured on B200 (batch 64): the window kernel wins for the narrow image layer
             # (3 -> <= 8 filters: 92 -> 68 us) and for un-pooled <= 8-channel layers (37 -> 31 us); with 32 filters its
             # epilogue (128 accumulator columns per pool window) costs what the im2col build saved (194 vs 192 us), and
             # pooled pitch-8 layers lose to the pool-window GEMM of conv_im2col_tc.cu (49 vs 39 us).
@@ -488,7 +487,7 @@ class CompiledDarknet(object):
             src = _TensorRef(bid_in, H, W, in_ch, list(range(in_ch)), torch.zeros(in_ch))
 
         # k-block of 32 (64-byte swizzle) where it halves K (<= 32 input channels).  Measured on B200: TMA cost follows the
-        # box AREA, not the valid channels, so a 64-wide box (shared activation box, resident weights) is slower than
+        # box AREA, not the valid channels, so a 64-wide box (shared activation box) is slower than
         # 32-wide boxes for <= 32 channels (dense conv2: 402 us vs 524 us; shrunk conv8: 33 us vs 39 us); and for
         # 69 -> 96 instead of 128 columns the extra pipeline steps cost more than the zero padding they remove.
         kblk = 32 if c_phys_in <= 32 else 64

@@ -202,11 +202,9 @@ class TrainPlan(object):
                 raise NotImplementedError("unresolved concat producer at block %d" % L.ind)
         # Pooled layers whose full-resolution activation feeds nothing but the pool: BatchNorm + leaky + pool run as one
         # pass each way (mc_bn_apply_pool / mc_bn_pool_backward) and the activation / its gradient are never stored
-        # (model.b200_fuse_pool = False keeps the separate passes: A/B runs, tests)
-        fuse = bool(getattr(model, 'b200_fuse_pool', True))
         for L in self.layers:
             L.fused_pool = False
-            if not (fuse and L.pool and not L.is_head and L.act is not None and L.act.name == 'a%d' % L.ind):
+            if not (L.pool and not L.is_head and L.act is not None and L.act.name == 'a%d' % L.ind):
                 continue
             if self.lib.mc_bn_pool_supported(L.O) != 1 or any(o.src is L.act for o in self.layers):
                 continue

@@ -73,7 +73,7 @@ def _last_plan():
     from modelcompression_b200 import _lib
     info = (ctypes.c_int * 8)()
     _lib.check(_lib.load().mc_conv_last_plan(info), "mc_conv_last_plan")
-    return dict(pair=info[0], block_n=info[1], ctas=info[2], resident=info[3], share=info[4], stages=info[5],
+    return dict(pair=info[0], block_n=info[1], ctas=info[2], sk_units=info[3], share=info[4], stages=info[5],
                 grid=info[6], block_k=info[7])
 
 
@@ -85,7 +85,7 @@ def _last_plan():
     (8, 32, 104, 104, 64, 3, dict(share=0, block_k=32)),  # same layer, short launch: one box per tap
     (8, 40, 52, 52, 72, 3, dict(share=1, block_k=64)),    # Cin 40 in a 64-wide k-block: 3 of 4 K steps issued
     (8, 16, 52, 52, 72, 3, dict(block_k=32)),
-    (16, 24, 104, 104, 8, 1, dict(pair=0, resident=0)),  # narrow 1x1: several CTAs per SM
+    (16, 24, 104, 104, 8, 1, dict(pair=0, sk_units=0)),  # narrow 1x1: several CTAs per SM
     (32, 80, 52, 52, 16, 1, dict(pair=0)),
 ])
 def test_conv_launch_paths(B, C, H, W, O, k, want):
@@ -307,8 +307,8 @@ def test_conv_stream_k_tail(B, C, H, W, O, sk):
     plan = _last_plan()
     conv.b200_no_workspace = True
     y_dp = conv(x)
-    assert plan['pair'] == 1 and (plan['resident'] > 0) == sk  # ('resident' slot = stream-K units of the pair kernel)
-    assert _last_plan()['pair'] == 1 and _last_plan()['resident'] == 0
+    assert plan['pair'] == 1 and (plan['sk_units'] > 0) == sk
+    assert _last_plan()['pair'] == 1 and _last_plan()['sk_units'] == 0
     ref = F.conv2d(_bf16(x), _bf16(conv.weight.data), conv.bias.data, 1, 1)
     for y in (y_sk, y_dp):
         err = (y - ref).abs()

@@ -63,14 +63,20 @@ def test_weight_prune_darknet_bit_exact(darknet, idx):
         assert m.shape == p.shape and m.device == p.device
 
 
-def test_weight_prune_uses_fast_path(darknet):
-    # on the 50.6 M-weight model the sample-pivot bracket holds: one pass over W (the exact path is the fallback)
+def _used_fast():
+    """1 when the last weight_prune on cuda:0 took the sample-pivot fast path, 0 when it fell back to the exact radix
+    select."""
     from modelcompression_b200 import _lib
     from modelcompression_b200.pruning.weightPruning import methods
-    mc.weight_prune(darknet, 70.)
     ws = methods._WS[('cuda', 0)]
     with torch.cuda.device(0):
-        assert _lib.load().mc_debug_select_used_fast(ws.data_ptr(), _lib.stream_ptr()) == 1
+        return _lib.load().mc_debug_select_used_fast(ws.data_ptr(), _lib.stream_ptr())
+
+
+def test_weight_prune_uses_fast_path(darknet):
+    # on the 50.6 M-weight model the sample-pivot bracket holds: one pass over W (the exact path is the fallback)
+    mc.weight_prune(darknet, 70.)
+    assert _used_fast() == 1
 
 
 class _ParamBag(torch.nn.Module):
@@ -134,6 +140,7 @@ def test_weight_prune_unaligned_and_degenerate_inputs():
     bagi = _ParamBag([bad.clone()]).to(DEV)
     _, masks_o = prune_oracle.weight_prune_np([bad.numpy()], 60.0)
     assert np.array_equal(mc.weight_prune(bagi, 60.0)[0].cpu().numpy(), masks_o[0])
+    assert _used_fast() == 0  # 400,000 elements would take the fast path; a non-finite value forces the exact one
     bad[5, 0] = float('nan')
     bagn = _ParamBag([bad.clone()]).to(DEV)
     import warnings
@@ -141,20 +148,12 @@ def test_weight_prune_unaligned_and_degenerate_inputs():
         warnings.simplefilter("ignore")
         _, masks_o = prune_oracle.weight_prune_np([bad.numpy()], 60.0)
     assert np.array_equal(mc.weight_prune(bagn, 60.0)[0].cpu().numpy(), masks_o[0])  # threshold NaN: nothing survives
+    assert _used_fast() == 0
     tiny = _ParamBag([torch.tensor([[3.0]]), torch.tensor([[1.0, -2.0]])]).to(DEV)
     for perc in (0.0, 50.0, 100.0):
         _, masks_o = prune_oracle.weight_prune_np([p.detach().cpu().numpy() for p in tiny.parameters()], perc)
         for a, b in zip(mc.weight_prune(tiny, perc), masks_o):
             assert np.array_equal(a.cpu().numpy(), b)
-
-
-def test_weight_prune_exact_radix_fallback(darknet, monkeypatch):
-    # the sample-pivot fast path falls back to the full radix select on the device when its bracket misses; force
-    # that path on the full model and check it gives the same (bit-exact) masks
-    g = load_golden('weight_prune_darknet.npz')
-    monkeypatch.setenv('MCB200_SELECT_EXACT', '1')
-    masks = mc.weight_prune(darknet, 80.)
-    assert [_sha(_bits(m.cpu().numpy())) for m in masks] == g['sha_2'].tolist()
 
 
 def test_weight_prune_vs_oracle_other_percentiles(darknet):
@@ -187,6 +186,7 @@ def test_set_masks_prune_rate_consistency(cfg_path):
     assert mc.are_masks_consistent(model, masks) is False
     # pruning an already-pruned model: >= 90 % of |w| are exactly 0 -> threshold 0, the zero bin holds the rank
     masks2 = mc.weight_prune(model, 50.)
+    assert _used_fast() == 0  # the zero keys overflow the fast path's candidate slices: the exact radix select runs
     ws = [p.detach().cpu().numpy() for p in model.parameters() if p.dim() != 1]
     _, masks_o = prune_oracle.weight_prune_np(ws, 50.)
     for a, b in zip(masks2, masks_o):
@@ -279,6 +279,27 @@ def test_filter_prune_tiled_and_generic_mix():
     _, keep = mc.quick_filter_prune(net, 50., return_keep=True)
     for a, b in zip(keep, keep_o):
         assert a.cpu().tolist() == np.nonzero(b)[0].tolist()
+
+
+def test_filter_prune_more_filters_than_the_fused_kernel_holds():
+    # 27,064 filters > 26,368 (the single cooperative launch's limit): the three-launch path (sums, select, mask fill)
+    torch.manual_seed(11)
+
+    class Net(torch.nn.Module):
+        def __init__(self):
+            super().__init__()
+            self.a = torch.nn.Conv2d(32, 64, 3)
+            self.b = torch.nn.Conv2d(4, 27000, 1)
+
+    net = Net().to(DEV)
+    cw = [p.detach().cpu().numpy() for p in net.parameters() if p.dim() == 4]
+    for perc in (10., 47.3, 90.):
+        masks, keep = mc.quick_filter_prune(net, perc, return_keep=True)
+        _, _, keep_o, masks_o = prune_oracle.quick_filter_prune_np(cw, perc)
+        for a, b in zip(masks, masks_o):
+            assert np.array_equal(a.cpu().numpy(), b), "perc %s" % perc
+        for a, b in zip(keep, keep_o):
+            assert a.cpu().tolist() == np.nonzero(b)[0].tolist(), "perc %s" % perc
 
 
 def test_count_zeros_and_unaligned_segments():

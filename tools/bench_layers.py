@@ -1,5 +1,5 @@
-"""Per-launch timing of the bench workload's forward (shrunk by default, `dense` for the un-pruned net) under the current
-environment (MCB200_* switches), for A/B runs inside one GPU lease.  Usage: bench_layers.py [dense] [tag]
+"""Per-launch timing of the bench workload's forward (shrunk by default, `dense` for the un-pruned net), for comparing
+builds inside one GPU lease.  Usage: bench_layers.py [dense] [tag]
 Prints one JSON line: {"tag":…, "ms_per_step": graph-replayed step, "per_op_us": {...}}"""
 import json
 import os

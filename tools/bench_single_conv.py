@@ -1,4 +1,4 @@
-"""Time mc_conv_fwd alone on given shapes (B C H W O k ...) under the current MCB200_* environment."""
+"""Time mc_conv_fwd alone on given shapes (B C H W O k ...) and report the launch plan it chose."""
 import ctypes, json, os, sys, statistics
 import torch
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))

@@ -119,6 +119,25 @@ int mc_filter_prune(const float* const* h_w_ptrs, const int* h_O, const int* h_C
                     float* const* h_mask_ptrs, uint8_t* d_keep, void* d_ws, size_t ws_bytes, void* stream);
 size_t mc_workspace_bytes_filter_prune(void);
 
+/* Greedy filter pruning — replaces methods.py:81-126 (prune_one_filter) and :129-142 (filter_prune), arXiv:1611.06440.
+ * Per layer v = raw / sqrt(pairwise_sum(raw^2)) (raw as in step 1 above, float32, NumPy's order); each layer offers
+ * arg_nonzero_min(v) (utils.py:96-120, with its tie rules; (inf, inf) when nothing or only index 0 is nonzero); the
+ * pick is np.argmin over those float64 values (the first NaN, else the first minimum); the picked filter's raw value
+ * becomes 0 and its nonzero weights are added to the zero count.  After each pick the walk stops when
+ * !(100. * zeros / total_params < perc) (float64; zeros starts at zeros0, so at least one filter is picked), or
+ * after max_picks picks (1 <= max_picks <= sum O).  sum O <= 20,480.
+ *   d_picks  [max_picks][2] int32, 8-byte aligned: (filter index over all layers, its count of nonzero weights)
+ *   d_result [3] int64: picks made, final zero count, status: 0 target reached, 1 max_picks made first, 2 a NaN pick
+ *            (it changes no value: the reference repeats it forever), 3 every layer reports (inf, inf) (no pick is
+ *            made), 4 a raw value is not finite (no pick is made)
+ * Full-shape masks (1 = kept, 0 = picked) are written when h_mask_ptrs != NULL.
+ * d_ws: mc_workspace_bytes_filter_prune_greedy(sum O) bytes, any content.                                         */
+int mc_filter_prune_greedy(const float* const* h_w_ptrs, const int* h_O, const int* h_C, const int* h_kh,
+                           const int* h_kw, int nlayers, int64_t zeros0, int64_t total_params, double perc,
+                           int max_picks, int32_t* d_picks, int64_t* d_result, float* const* h_mask_ptrs,
+                           void* d_ws, size_t ws_bytes, void* stream);
+size_t mc_workspace_bytes_filter_prune_greedy(int n_filters);
+
 /* ------------------------------------------------------------------------------------------
  * Region decode + NMS — replaces src/nets2_utils.py:141-234 (get_region_boxes) and :236-259 (nms),
  * :63-98 (bbox_iou, centre format).

@@ -15,7 +15,7 @@ from .nets import Darknet, EmptyModule, Reorg, RegionLoss, getYOLOv2, parse_cfg 
 from .nets2_utils import bbox_iou, bbox_ious, detect_batch, do_detect, get_region_boxes, nms  # noqa: F401
 from .optim import MaskedSGD  # noqa: F401
 from .pruning.weightPruning.layers import MaskedConv2d, MaskedLinear  # noqa: F401
-from .pruning.weightPruning.methods import quick_filter_prune, weight_prune  # noqa: F401
+from .pruning.weightPruning.methods import filter_prune, prune_one_filter, quick_filter_prune, weight_prune  # noqa: F401
 from .pruning.weightPruning.utils import are_masks_consistent, prune_rate, to_var  # noqa: F401
 
 __version__ = "0.1.0"

@@ -69,6 +69,10 @@ _SIGNATURES = {
                                 c_int64, c_double, c_void_p, c_void_p, POINTER(c_void_p), c_void_p, c_void_p, c_size_t,
                                 c_void_p]),
     "mc_workspace_bytes_filter_prune": (c_size_t, []),
+    "mc_filter_prune_greedy": (c_int, [POINTER(c_void_p), POINTER(c_int), POINTER(c_int), POINTER(c_int),
+                                       POINTER(c_int), c_int, c_int64, c_int64, c_double, c_int, c_void_p, c_void_p,
+                                       POINTER(c_void_p), c_void_p, c_size_t, c_void_p]),
+    "mc_workspace_bytes_filter_prune_greedy": (c_size_t, [c_int]),
     "mc_decode_region": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_int, POINTER(c_float), c_float, c_int,
                                  c_void_p, c_void_p, c_void_p, c_void_p]),
     "mc_nms_batched": (c_int, [c_void_p, c_void_p, c_int, c_int, c_float, c_void_p, c_void_p, c_void_p]),

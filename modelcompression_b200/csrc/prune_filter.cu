@@ -12,6 +12,7 @@
 //               n<8 sequential; n<=128: 8 strided accumulators, ((r0+r1)+(r2+r3))+((r4+r5)+(r6+r7)), tail;
 //               else split at n/2 rounded down to a multiple of 8).  sum(v^2) over O uses the same rule.
 // All products/sums use *_rn intrinsics so nvcc cannot contract them into FMAs.
+#include <limits.h>
 #include <stdlib.h>
 #include "common.cuh"
 
@@ -1209,6 +1210,311 @@ extern "C" int mc_filter_prune(const float* const* h_w_ptrs, const int* h_O, con
     const int cap = mc_num_sms() * 16;
     if (blocks > cap) blocks = cap;
     filter_mask_fill_kernel<<<blocks, 256, 0, stream>>>(lt, d_values, d_thr);
+    MC_LAUNCH_CHECK("filter_mask_fill_kernel");
+  }
+  return 0;
+}
+
+// ---- greedy filter pruning: prune_one_filter / filter_prune (methods.py:81-142, arXiv:1611.06440) ----------------------
+// The reference re-reads every weight for every filter it removes.  Surviving filters are only ever multiplied by 1.0,
+// so a filter's raw value (mean of squares, step 1 of quick_filter_prune) and its count of nonzero weights are computed
+// once (pass 1).  A pick sets one raw value to 0, which changes one leaf of its layer's pairwise sum of squares and
+// therefore only that layer's norm and candidate: the greedy walk (pass 2) re-sums that leaf, replays the combine and
+// rescans the one layer, in one warp with everything in shared memory.  Pass 3 fills the masks from the keep flags.
+namespace {
+
+
+// Nonzero weights per filter (-0.0 counts as zero, as `== 0` does in NumPy): one warp per filter.
+__global__ void __launch_bounds__(256) filter_nonzero_kernel(const LayerTable lt, int* __restrict__ nz) {
+  const int n = lt.voff[lt.nlayers];
+  const int lane = threadIdx.x & 31;
+  const int f = blockIdx.x * 8 + (threadIdx.x >> 5);
+  if (f >= n) return;
+  int l = 0;
+  while (l + 1 < lt.nlayers && f >= lt.voff[l + 1]) ++l;
+  const int per = lt.C[l] * lt.taps[l];
+  const float* w = lt.w[l] + (long long)(f - lt.voff[l]) * per;
+  int head = (int)(((16 - (reinterpret_cast<uintptr_t>(w) & 15)) & 15) >> 2);  // scalar head up to 16-byte alignment
+  if (head > per) head = per;
+  int c = (lane < head && w[lane] != 0.f) ? 1 : 0;
+  const int body4 = (per - head) >> 2;
+  const float4* w4 = reinterpret_cast<const float4*>(w + head);
+#pragma unroll 4
+  for (int i = lane; i < body4; i += 32) {
+    const float4 v = ld_stream_f4(w4 + i);
+    c += (v.x != 0.f) + (v.y != 0.f) + (v.z != 0.f) + (v.w != 0.f);
+  }
+  for (int i = head + body4 * 4 + lane; i < per; i += 32) c += (w[i] != 0.f) ? 1 : 0;
+  c = __reduce_add_sync(0xffffffffu, c);
+  if (lane == 0) nz[f] = c;
+}
+
+constexpr int GR_THREADS = 256;
+constexpr int GR_MAX_N = 20480;  // filters staged in shared memory: raw value, nonzero count, keep flag (9 bytes each)
+// Leaves of the pairwise recursion: one per layer of <= 128 filters, otherwise every leaf is at least 57 long.
+constexpr int GR_MAX_LEAVES = GR_MAX_N / 56 + 2 * MAX_LAYERS;
+constexpr size_t GR_SMEM = (size_t)GR_MAX_N * 9;
+
+// NumPy's pairwise sum of a[i]^2 over one leaf (n <= 128) by a warp: lane j & 7 runs accumulator j, the xor butterfly
+// performs ((r0+r1)+(r2+r3))+((r4+r5)+(r6+r7)), then the sequential tail.  The result is valid in every lane.
+__device__ __forceinline__ float warp_leaf_sumsq(const float* a, int n) {
+  const int j = threadIdx.x & 7;
+  const int body = n - (n % 8);
+  float r = 0.f;
+  if (n >= 8) {
+    float x = a[j];
+    r = __fmul_rn(x, x);
+    for (int i = 8; i < body; i += 8) {
+      x = a[i + j];
+      r = __fadd_rn(r, __fmul_rn(x, x));
+    }
+  }
+  float t = __fadd_rn(r, __shfl_xor_sync(0xffffffffu, r, 1));
+  t = __fadd_rn(t, __shfl_xor_sync(0xffffffffu, t, 2));
+  t = __fadd_rn(t, __shfl_xor_sync(0xffffffffu, t, 4));
+  float sum = n >= 8 ? t : 0.f;
+  for (int i = n >= 8 ? body : 0; i < n; ++i) sum = __fadd_rn(sum, __fmul_rn(a[i], a[i]));
+  return sum;
+}
+
+enum { GR_DONE = 0, GR_BUDGET = 1, GR_NAN_PICK = 2, GR_NO_CANDIDATE = 3, GR_NONFINITE = 4 };
+
+struct GreedyShared {
+  int lst[GR_MAX_LEAVES], lln[GR_MAX_LEAVES];  // leaf (start, length) inside its layer
+  float lsum[GR_MAX_LEAVES];                   // leaf sums of raw^2
+  int loff[MAX_LAYERS + 1];                    // first leaf of each layer
+  float cval[MAX_LAYERS];                      // per-layer arg_nonzero_min: value (inf when it reports (inf, inf))
+  int cidx[MAX_LAYERS];                        // ... and index (-1 for (inf, inf))
+};
+
+// Layer l's norm from its leaf sums, v = raw / norm, and arg_nonzero_min(list(v)) (utils.py:96-120) by one warp:
+// the start is the LAST entry with v != 0 (NaN != 0 too) and only a strict `<` replaces it, so that entry wins a tie
+// for the minimum and otherwise the first index of the minimum wins; a NaN start is never replaced; no nonzero entry,
+// or index 0 as the last one, reports (inf, inf).
+__device__ void greedy_refresh_layer(const LayerTable& lt, int l, const float* s_raw, GreedyShared& g) {
+  const int lane = threadIdx.x & 31, O = lt.O[l];
+  float tot = 0.f;
+  if (lane == 0) {
+    int next = 0;
+    tot = np_combine_leaves(g.lsum + g.loff[l], O, &next);
+  }
+  const float nrm = __fsqrt_rn(__shfl_sync(0xffffffffu, tot, 0));
+  const float* r = s_raw + lt.voff[l];
+  int last = -1, im = INT_MAX;
+  float m = INFINITY;
+  for (int i = lane; i < O; i += 32) {
+    const float v = __fdiv_rn(r[i], nrm);
+    if (v != 0.f) {
+      last = i;
+      if (v == v && (im == INT_MAX || v < m)) { m = v; im = i; }
+    }
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+    last = max(last, __shfl_xor_sync(0xffffffffu, last, o));
+    const float m2 = __shfl_xor_sync(0xffffffffu, m, o);
+    const int i2 = __shfl_xor_sync(0xffffffffu, im, o);
+    if (i2 != INT_MAX && (im == INT_MAX || m2 < m || (m2 == m && i2 < im))) { m = m2; im = i2; }
+  }
+  if (lane == 0) {
+    float cv = INFINITY;
+    int ci = -1;
+    if (last > 0) {
+      const float vl = __fdiv_rn(r[last], nrm);
+      if (vl == vl && m < vl) { cv = m; ci = im; }
+      else { cv = vl; ci = last; }
+    }
+    g.cval[l] = cv;
+    g.cidx[l] = ci;
+  }
+  __syncwarp();
+}
+
+// Pass 2 in one block.  Per pick (warp 0): np.argmin over the per-layer values (the first NaN, else the first minimum),
+// record (filter, nonzero count), count the zeros, then the stop test exactly as filter_prune evaluates it (float64
+// 100. * zeros / total < perc), after the pick: the reference starts from a rate of 0 and always prunes once.
+__global__ void __launch_bounds__(GR_THREADS) filter_greedy_kernel(const LayerTable lt, const float* __restrict__ raw,
+                                                                   const int* __restrict__ nz, long long zeros0,
+                                                                   long long total, double perc, int max_picks,
+                                                                   int2* __restrict__ picks, long long* __restrict__ result,
+                                                                   float* __restrict__ keepf, double* __restrict__ half) {
+  extern __shared__ __align__(16) unsigned char dsm[];
+  __shared__ GreedyShared g;
+  const int n = lt.voff[lt.nlayers], nl = lt.nlayers;
+  const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
+  float* s_raw = reinterpret_cast<float*>(dsm);
+  int* s_nz = reinterpret_cast<int*>(s_raw + n);
+  uint8_t* s_keep = reinterpret_cast<uint8_t*>(s_nz + n);
+  int bad = 0;
+  for (int i = tid; i < n; i += GR_THREADS) {
+    const float x = raw[i];
+    s_raw[i] = x;
+    s_nz[i] = nz[i];
+    s_keep[i] = 1;
+    bad |= !isfinite(x);
+  }
+  if (tid == 0) {
+    g.loff[0] = 0;
+    for (int l = 0; l < nl; ++l) g.loff[l + 1] = g.loff[l] + np_for_each_leaf(lt.O[l], [](int, int, int) {});
+  }
+  if (__syncthreads_or(bad)) {
+    if (tid == 0) {
+      result[0] = 0;
+      result[1] = zeros0;
+      result[2] = GR_NONFINITE;
+    }
+    return;
+  }
+  // leaf tables and sums, norms and candidates of every layer: one warp per layer
+  for (int l = wid; l < nl; l += GR_THREADS / 32) {
+    const int base = g.loff[l];
+    if (lane == 0)
+      np_for_each_leaf(lt.O[l], [&](int leaf, int st, int ln) {
+        g.lst[base + leaf] = st;
+        g.lln[base + leaf] = ln;
+      });
+    __syncwarp();
+    const float* r = s_raw + lt.voff[l];
+    for (int k = base; k < g.loff[l + 1]; ++k) {
+      const float s = warp_leaf_sumsq(r + g.lst[k], g.lln[k]);
+      if (lane == 0) g.lsum[k] = s;
+    }
+    __syncwarp();
+    greedy_refresh_layer(lt, l, s_raw, g);
+  }
+  __syncthreads();
+  if (wid == 0) {
+    long long zeros = zeros0;
+    int npick = 0, status = GR_BUDGET;
+    for (;;) {
+      float bv = INFINITY;
+      int bl = INT_MAX;
+      for (int l = lane; l < nl; l += 32) {  // ascending l: a later layer only wins with a NaN or a smaller value
+        const float v = g.cval[l];
+        if (bl == INT_MAX || (v != v && bv == bv) || (bv == bv && v < bv)) { bv = v; bl = l; }
+      }
+#pragma unroll
+      for (int o = 16; o > 0; o >>= 1) {
+        const float v2 = __shfl_xor_sync(0xffffffffu, bv, o);
+        const int l2 = __shfl_xor_sync(0xffffffffu, bl, o);
+        bool take;
+        if (l2 == INT_MAX) take = false;
+        else if (bl == INT_MAX) take = true;
+        else if ((v2 != v2) != (bv != bv)) take = v2 != v2;
+        else if (v2 != v2) take = l2 < bl;
+        else take = v2 < bv || (v2 == bv && l2 < bl);
+        if (take) { bv = v2; bl = l2; }
+      }
+      const int ci = g.cidx[bl];
+      if (ci < 0) {  // every layer reports (inf, inf): int(inf) raises in the reference
+        status = GR_NO_CANDIDATE;
+        break;
+      }
+      const int f = lt.voff[bl] + ci;
+      const int c = s_nz[f];
+      zeros += c;
+      __syncwarp();
+      if (lane == 0) {
+        picks[npick] = make_int2(f, c);
+        s_nz[f] = 0;
+        s_keep[f] = 0;
+      }
+      ++npick;
+      if (!(__ddiv_rn(__dmul_rn(100.0, (double)zeros), (double)total) < perc)) {
+        status = GR_DONE;
+        break;
+      }
+      if (npick >= max_picks) break;
+      if (bv != bv) {  // a NaN pick leaves every value as it was: the reference repeats it forever
+        status = GR_NAN_PICK;
+        break;
+      }
+      if (lane == 0) s_raw[f] = 0.f;
+      __syncwarp();
+      int leaf = -1;
+      for (int k0 = g.loff[bl]; k0 < g.loff[bl + 1] && leaf < 0; k0 += 32) {
+        const int k = k0 + lane;
+        const unsigned int hit = __ballot_sync(0xffffffffu, k < g.loff[bl + 1] && g.lst[k] <= ci &&
+                                                                ci < g.lst[k] + g.lln[k]);
+        if (hit) leaf = k0 + __ffs(hit) - 1;
+      }
+      const float s = warp_leaf_sumsq(s_raw + lt.voff[bl] + g.lst[leaf], g.lln[leaf]);
+      if (lane == 0) g.lsum[leaf] = s;
+      __syncwarp();
+      greedy_refresh_layer(lt, bl, s_raw, g);
+    }
+    if (lane == 0) {
+      result[0] = npick;
+      result[1] = zeros;
+      result[2] = status;
+    }
+  }
+  __syncthreads();
+  // keep flags as the 0 / 1 values the mask fill kernel compares against 0.5
+  for (int i = tid; i < n; i += GR_THREADS) keepf[i] = s_keep[i] ? 1.f : 0.f;
+  if (tid == 0) *half = 0.5;
+}
+
+}  // namespace
+
+static size_t greedy_ws_offset(int n, int part) {  // workspace: raw f32 [n] | nonzero counts i32 [n] | keep f32 [n] | 0.5
+  return (size_t)part * (((size_t)n * 4 + 15) / 16 * 16);
+}
+
+extern "C" size_t mc_workspace_bytes_filter_prune_greedy(int n_filters) {
+  return n_filters > 0 ? greedy_ws_offset(n_filters, 3) + 16 : 0;
+}
+
+extern "C" int mc_filter_prune_greedy(const float* const* h_w_ptrs, const int* h_O, const int* h_C, const int* h_kh,
+                                      const int* h_kw, int nlayers, int64_t zeros0, int64_t total_params, double perc,
+                                      int max_picks, int32_t* d_picks, int64_t* d_result, float* const* h_mask_ptrs,
+                                      void* d_ws, size_t ws_bytes, void* stream_) {
+  cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
+  MC_CHECK_ARG(h_w_ptrs && h_O && h_C && h_kh && h_kw && d_picks && d_result && d_ws,
+               "mc_filter_prune_greedy: null pointer");
+  MC_CHECK_ARG(nlayers > 0 && nlayers <= MAX_LAYERS, "mc_filter_prune_greedy: nlayers %d out of range", nlayers);
+  int taps[MAX_LAYERS];
+  for (int l = 0; l < nlayers; ++l) {
+    MC_CHECK_ARG(h_kh[l] == h_kw[l] && h_kh[l] >= 1 && h_kh[l] * h_kw[l] <= 49,
+                 "mc_filter_prune_greedy: layer %d kernel %dx%d unsupported (square, <=7x7)", l, h_kh[l], h_kw[l]);
+    MC_CHECK_ARG(h_w_ptrs[l] != nullptr, "mc_filter_prune_greedy: layer %d null weight", l);
+    MC_CHECK_ARG(!h_mask_ptrs || h_mask_ptrs[l] != nullptr, "mc_filter_prune_greedy: null mask %d", l);
+    taps[l] = h_kh[l] * h_kw[l];
+  }
+  LayerTable lt;
+  int rc = build_layers(&lt, h_w_ptrs, h_mask_ptrs, h_O, h_C, taps, nlayers, "mc_filter_prune_greedy");
+  if (rc) return rc;
+  const int n = lt.voff[nlayers];
+  if (n > GR_MAX_N)
+    return mc_set_error(MC_ERR_SHAPE, "mc_filter_prune_greedy: %d filters exceed the %d the greedy walk holds", n, GR_MAX_N);
+  MC_CHECK_ARG(max_picks >= 1 && max_picks <= n, "mc_filter_prune_greedy: max_picks %d out of range [1, %d]", max_picks, n);
+  MC_CHECK_ARG(total_params > 0 && zeros0 >= 0 && zeros0 <= total_params,
+               "mc_filter_prune_greedy: zeros0 / total_params out of range");
+  if (ws_bytes < mc_workspace_bytes_filter_prune_greedy(n))
+    return mc_set_error(MC_ERR_WS, "mc_filter_prune_greedy: workspace too small");
+  unsigned char* ws = reinterpret_cast<unsigned char*>(d_ws);
+  float* d_raw = reinterpret_cast<float*>(ws);
+  int* d_nz = reinterpret_cast<int*>(ws + greedy_ws_offset(n, 1));
+  float* d_keepf = reinterpret_cast<float*>(ws + greedy_ws_offset(n, 2));
+  double* d_half = reinterpret_cast<double*>(ws + greedy_ws_offset(n, 3));
+  static bool attr_set = false;
+  if (!attr_set) {
+    MC_CUDA(cudaFuncSetAttribute(filter_greedy_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GR_SMEM));
+    attr_set = true;
+  }
+  rc = launch_sumsq(lt, d_raw, stream);
+  if (rc) return rc;
+  filter_nonzero_kernel<<<(n + 7) / 8, 256, 0, stream>>>(lt, d_nz);
+  MC_LAUNCH_CHECK("filter_nonzero_kernel");
+  filter_greedy_kernel<<<1, GR_THREADS, (size_t)n * 9, stream>>>(
+      lt, d_raw, d_nz, (long long)zeros0, (long long)total_params, perc, max_picks, reinterpret_cast<int2*>(d_picks),
+      reinterpret_cast<long long*>(d_result), d_keepf, d_half);
+  MC_LAUNCH_CHECK("filter_greedy_kernel");
+  if (h_mask_ptrs) {
+    int blocks = n;
+    const int cap = mc_num_sms() * 16;
+    if (blocks > cap) blocks = cap;
+    filter_mask_fill_kernel<<<blocks, 256, 0, stream>>>(lt, d_keepf, d_half);
     MC_LAUNCH_CHECK("filter_mask_fill_kernel");
   }
   return 0;

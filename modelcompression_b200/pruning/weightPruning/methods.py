@@ -1,10 +1,10 @@
-"""Drop-in for src/pruning/weightPruning/methods.py of the reference: weight_prune (:9-26) and
-quick_filter_prune (:28-78), computed on the GPU by libmcb200 (no device->host copy of the weights).
+"""Drop-in for src/pruning/weightPruning/methods.py of the reference: weight_prune (:9-26), quick_filter_prune
+(:28-78), prune_one_filter (:81-126) and filter_prune (:129-142), computed on the GPU by libmcb200 (no device->host copy
+of the weights).
 
 Host-side logic kept here is the data-independent part of ``np.percentile``: the rank ``k`` and interpolation
 weight ``gamma`` of the 'linear' method, evaluated in the SAME dtype NumPy 2.x uses (float32 for the float32
 magnitude array of weight_prune, float64 for the float64 value array of quick_filter_prune; SURVEY.md §8a-5/6).
-``prune_one_filter`` / ``filter_prune`` (methods.py:81-142) are not on the hot path (SURVEY.md §2 #7).
 """
 from itertools import chain as _chain
 
@@ -12,6 +12,7 @@ import numpy as np
 import torch
 
 from ... import _lib
+from .utils import count_zeros
 
 
 def percentile_rank(n, pruning_perc, dtype):
@@ -358,11 +359,108 @@ def quick_filter_prune(model, pruning_perc, return_keep=False):
     return masks, keep_idx
 
 
+_GREEDY_DONE, _GREEDY_BUDGET, _GREEDY_NAN_PICK, _GREEDY_NO_CANDIDATE, _GREEDY_NONFINITE = range(5)
+
+
+def _greedy_prune(model, perc, max_picks, zeros0, total, want_masks):
+    """One mc_filter_prune_greedy call over the conv (4-D) weights.  Returns (masks or None, [(layer, filter, nonzero
+    weights)] in pick order, final zero count, status).  The picks come back in one device->host copy."""
+    lib = _lib.load()
+    plan, params, parr = _plan_and_tensors(model, conv_only=True)
+    if not params:
+        raise ValueError("filter pruning: the model has no 4-D (conv) parameters")
+    if len(params) > _lib.MC_MAX_SEGMENTS:
+        raise NotImplementedError("filter pruning: more than %d conv layers" % _lib.MC_MAX_SEGMENTS)
+    dev = params[0].device
+    n = sum(plan.O)
+    ws_bytes = lib.mc_workspace_bytes_filter_prune_greedy(n)
+    ws = _workspace(dev, ws_bytes)
+    out = torch.empty(6 + 2 * max_picks, dtype=torch.int32, device=dev)  # result int64 [3] | picks int32 [max_picks][2]
+    flat = mask_ptrs = None
+    if want_masks:
+        flat = torch.empty(plan.flat_len, dtype=torch.float32, device=dev)
+        mask_ptrs = (_lib.c_void_p * len(params))(*[flat.data_ptr() + 4 * o for o in plan.offs])
+    with _on_device(dev):
+        _lib.check(lib.mc_filter_prune_greedy(parr, plan.tables[0], plan.tables[1], plan.tables[2], plan.tables[3],
+                                              len(params), zeros0, total, float(perc), max_picks, out.data_ptr() + 24,
+                                              out.data_ptr(), mask_ptrs, ws.data_ptr(), ws_bytes, _lib.stream_ptr()),
+                   "mc_filter_prune_greedy")
+    host = out.cpu().numpy()
+    npick, zeros, status = (int(x) for x in host[:6].view(np.int64))
+    fc = host[6:6 + 2 * npick].reshape(-1, 2).astype(np.int64)
+    layer_of = np.searchsorted(np.cumsum(plan.O), fc[:, 0], side='right')
+    first = np.concatenate(([0], np.cumsum(plan.O)))[layer_of]
+    picks = list(zip(layer_of.tolist(), (fc[:, 0] - first).tolist(), fc[:, 1].tolist()))
+    masks = _mask_views(flat, plan) if want_masks else None
+    return masks, picks, zeros, status
+
+
+def _raise_for_status(status, what):
+    if status == _GREEDY_NONFINITE:
+        raise ValueError("%s: a conv weight gives a non-finite filter value (inf or NaN weights); nothing was pruned"
+                         % what)
+    if status == _GREEDY_NO_CANDIDATE:  # the reference raises OverflowError from int(inf) here
+        raise OverflowError("%s: no conv layer has a nonzero filter value left to prune" % what)
+
+
 def prune_one_filter(model, masks):
-    raise NotImplementedError("prune_one_filter (methods.py:81-126) is not on the B200 hot path: the reference's "
-                              "train path calls weight_prune / quick_filter_prune only (src/train.py:168-171)")
+    '''
+    methods.py:81-126.  Picks the filter with the smallest nonzero value v = mean(w^2) / ||mean(w^2) of its layer||_2
+    over all conv (4-D) parameters, read from the CURRENT weights (``masks`` is not consulted), and zeroes
+    ``masks[layer][filter]`` in place.  An empty ``masks`` is first filled with all-ones float32 masks on the parameters'
+    device.  Does not call set_masks.  Prints the reference's "Prune filter #f in layer #l" line and returns ``masks``.
+    Non-finite weights raise ValueError; when no layer has a nonzero filter left it raises OverflowError, as the
+    reference's int(inf) does.
+    '''
+    no_masks = not masks
+    if no_masks:
+        masks = []
+    else:
+        assert len(masks) == len(_prunable(model, conv_only=True)), "something wrong here"
+    built, picks, _, status = _greedy_prune(model, float('inf'), 1, 0, 1, want_masks=no_masks)
+    _raise_for_status(status, "prune_one_filter")
+    layer, filt, _ = picks[0]
+    if no_masks:
+        masks.extend(built)  # the picked filter is already zero in these
+    else:
+        masks[layer][filt] = 0.
+    print('Prune filter #{} in layer #{}'.format(filt, layer))
+    return masks
 
 
 def filter_prune(model, pruning_perc):
-    raise NotImplementedError("filter_prune (methods.py:129-142) is not on the B200 hot path: the reference's "
-                              "train path calls weight_prune / quick_filter_prune only (src/train.py:168-171)")
+    '''
+    Greedy filter pruning, one filter at a time (arXiv:1611.06440).  methods.py:129-142.
+
+    Repeats prune_one_filter until prune_rate(model) >= pruning_perc, starting from a rate of 0 (so at least one filter
+    is pruned whenever pruning_perc > 0; pruning_perc <= 0 returns [] and leaves the model alone).  A pruned filter's
+    surviving neighbours are only ever multiplied by 1.0, so the whole walk is one GPU call: each filter's value is
+    computed once and a pick re-normalises its own layer only.  Returns all-ones float32 masks with the picked filters
+    zeroed and applies them with model.set_masks (replacing earlier masks; weights zeroed earlier stay zero).  Prints
+    the reference's two lines per pick.  Where the reference never returns (a layer pruned empty, NaN weights, a target
+    above the reachable rate) or raises, this raises and leaves the model unchanged.
+    '''
+    if not (0. < pruning_perc):
+        return []
+    params = list(model.parameters())
+    total = sum(p.numel() for p in params)
+    prunable = [p.data for p in params if p.dim() != 1]
+    zeros0 = sum(count_zeros(prunable)) if prunable else 0
+    n = sum(_plan_and_tensors(model, conv_only=True)[0].O)
+    masks, picks, zeros, status = _greedy_prune(model, pruning_perc, n, zeros0, total, want_masks=True)
+    z = zeros0
+    for layer, filt, nz in picks:
+        z += nz
+        print('Prune filter #{} in layer #{}'.format(filt, layer))
+        print('{:.2f} pruned'.format(100. * z / total))
+    rate = 100. * zeros / total
+    _raise_for_status(status, "filter_prune (pruning rate %.4f%% after %d picks)" % (rate, len(picks)))
+    if status == _GREEDY_NAN_PICK:
+        raise RuntimeError("filter_prune: stopped at a pruning rate of %.4f%% < %s: a conv layer has no filter with a "
+                           "nonzero value left (all pruned or all-zero weights), the reference would loop forever"
+                           % (rate, pruning_perc))
+    if status == _GREEDY_BUDGET:
+        raise RuntimeError("filter_prune: every filter was pruned and the rate reached is only %.4f%% < %s"
+                           % (rate, pruning_perc))
+    model.set_masks(masks)
+    return masks

@@ -256,6 +256,24 @@ int mc_conv_fwd(const mc_conv_desc* desc, void* stream);
  * (launches on one stream are ordered); contents are meaningless between calls.                                  */
 size_t mc_workspace_bytes_conv_fwd(const mc_conv_desc* desc);
 
+/* A chain of 2..4 wide 3x3 layers in which member i+1 reads member i's output, as ONE launch of the CTA-pair kernel.
+ * Each member computes exactly what its own mc_conv_fwd call would (same plan, same arithmetic, bit-identical output);
+ * only the schedule changes: the (member, m-pair, n-tile) units are tickets in layer-major, m-major order, which the
+ * clusters claim with one atomic each, so the idle clusters of one member's partial last wave start the next member's
+ * first units, and the launches, drains and pipeline fills between the members disappear.  A unit of member i+1 starts
+ * once every unit of member i over its rows (3x3 halo included) is stored; a counter per (member, m-pair) in the
+ * workspace tracks that.  Returns an error WITHOUT launching unless: 2 <= n <= 4; every member takes the CTA-pair
+ * kernel under mc_conv_fwd's own rules with the TMA-store PNHWC epilogue and the same tile width, ring and activation;
+ * all members share B, H, W; no member asks for statistics; member i+1 reads member i's output allocation
+ * (d_in == previous d_out, Cin_ld == previous ldc) and no member reads or rewrites another member's output otherwise.
+ * Workspace: descs[0].d_ws / ws_bytes, 16-byte aligned, mc_workspace_bytes_conv_chain bytes, ZERO before the first
+ * launch; every launch leaves it zero again, except the status word (uint32 index 2), which becomes nonzero if a unit
+ * waited for its inputs longer than a second (never expected: a dependency bug).  d_ws of the other members is ignored. */
+int mc_conv_chain_fwd(const mc_conv_desc* descs, int n, void* stream);
+/* Workspace bytes of that chain, or 0 when mc_conv_chain_fwd would reject these descriptors (the same checks, no
+ * launch: callers use it to find the runs of layers the chain takes at a given batch size).                        */
+size_t mc_workspace_bytes_conv_chain(const mc_conv_desc* descs, int n);
+
 /* Which launch configuration the LAST mc_conv_fwd call of this host thread chose (tests / bench reporting):
  * info[0] = 1 CTA-pair kernel (tcgen05 cta_group::2, 256-row tiles, half of each weight tile per CTA), 0 single CTA
  * info[1] = tile width block_n      info[2] = resident CTAs per SM requested (1..3)

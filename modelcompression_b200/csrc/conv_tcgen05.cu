@@ -21,6 +21,7 @@
 #include <cuda.h>
 #include <stdio.h>
 #include <stdlib.h>
+#include <string.h>
 #include "common.cuh"
 #include "ptx_sm100.cuh"
 #include "tmap.cuh"
@@ -780,7 +781,8 @@ conv_gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __gri
 // unit's finisher: it adds the (at most three) earlier pieces and runs the epilogue.  The
 // earlier pieces were the FIRST thing their clusters did, so the finisher practically never waits.
 struct PairWork {
-  int unit;    // unit index (m-pair, n-tile)
+  int layer;   // entry of the layer table (chained launch; 0 otherwise)
+  int unit;    // unit index (m-pair, n-tile) inside the layer
   int g0, g1;  // K groups [g0, g1) of the unit
   int kind;    // 0 whole unit, 1 partial (dump to slot), 2 finisher (add n partials)
   int aux;     // kind 1: slot; kind 2: number of partial pieces to add
@@ -814,6 +816,7 @@ struct PairWorkIter {
     }
   }
   __device__ __forceinline__ bool next(PairWork& w) {
+    w.layer = 0;
     if (next_full < sk_first) {
       w.unit = next_full; w.g0 = 0; w.g1 = -1; w.kind = 0; w.aux = 0;  // g1 < 0: the whole K range
       next_full += step;
@@ -839,43 +842,160 @@ struct PairWorkIter {
   }
 };
 
+// ---------------------------------------------------------------------------------------------------------------
+// Layer table of the CTA-pair kernel.  One entry: today's launch (static schedule above, stream-K tail).  2..4 entries
+// (mc_conv_chain_fwd): a chain of 3x3 layers in which layer i+1 reads layer i's output, run as ONE persistent launch so
+// that the idle clusters of one layer's partial last wave start the next layer's first units and the layer boundaries
+// need no drain / launch / set-up / pipeline fill.  The entries share B, H, W, tile width, ring depth and epilogue.
+constexpr int MAX_CHAIN = 4;
+constexpr int WORK_SLOTS = 4;                           // work ring between the leader's producer and the other roles
+constexpr unsigned long long CHAIN_POLL_NS = 1000000000ull;  // bound of one readiness wait (then: status word, go on)
+enum { CHAIN_TICKET = 0, CHAIN_DONE = 1, CHAIN_STATUS = 2, CHAIN_COUNTERS = 4 };  // words of the chain workspace
+
+struct PairLayer {
+  CUtensorMap tmap_b, tmap_abox, tmap_out;
+  ConvKParams p;
+  int unit_end;  // tickets [unit_end of the previous entry, unit_end) are this layer's (m-pair, n-tile) units, m-major
+  int cnt_off;   // this layer's first readiness counter (one per m-pair) after CHAIN_COUNTERS
+};
+struct PairParams {
+  PairLayer layer[MAX_CHAIN];
+  int n_layers;
+  unsigned int* chain_ws;  // n_layers >= 2: ticket, clusters done, status, pad, then the readiness counters
+};
+
+// Work ring (chained launch): the leader CTA's producer lane claims a ticket, waits until the unit's inputs are
+// complete and publishes it into the ring of BOTH CTAs; the peer's producer, the MMA warp and the 8 epilogue warps take
+// their units from there (10 arrivals free a slot on the leader's empty barrier).  A ticket < 0 ends the launch.
+struct PairRing {
+  uint64_t* full;
+  uint64_t* empty;
+  int* val;
+  int slot;
+  uint32_t phase;
+};
+
+__device__ __forceinline__ void chain_decode(const PairParams& P, int t, PairWork& w) {
+  int l = 0;
+  while (l + 1 < P.n_layers && t >= P.layer[l].unit_end) ++l;
+  w.layer = l;
+  w.unit = t - (l > 0 ? P.layer[l - 1].unit_end : 0);
+  w.g0 = 0; w.g1 = -1; w.kind = 0; w.aux = 0;
+}
+
+__device__ __forceinline__ bool ring_take(const PairParams& P, PairRing& r, PairWork& w, bool whole_warp) {
+  ptx::mbar_wait_cluster(&r.full[r.slot], r.phase);
+  const int t = *reinterpret_cast<volatile int*>(&r.val[r.slot]);
+  if (whole_warp) __syncwarp();  // every lane has read the slot before it is handed back
+  if ((threadIdx.x & 31) == 0) ptx::mbar_arrive_leader(&r.empty[r.slot]);
+  if (++r.slot == WORK_SLOTS) { r.slot = 0; r.phase ^= 1u; }
+  if (t < 0) return false;
+  chain_decode(P, t, w);
+  return true;
+}
+
+// Readiness of a unit of layer l >= 1 at m-pair i: its activation boxes cover rows [256i - Wp - 1, 256i + 264 + Wp) of
+// layer l-1's output (3x3 halo around two 128-row tiles), i.e. the m-pairs of layer l-1 over those rows must have all
+// n_tiles units stored.  A counter is complete at n_tiles x 8 arrivals (every epilogue warp of both CTAs, per unit).
+__device__ __noinline__ void chain_wait_inputs(const PairParams& P, const PairWork& w) {
+  const PairLayer& prev = P.layer[w.layer - 1];
+  const int mp = w.unit / P.layer[w.layer].p.n_tiles;
+  int r0 = 256 * mp - prev.p.Wp - 1, r1 = 256 * mp + 264 + prev.p.Wp;
+  if (r0 < 0) r0 = 0;
+  if (r1 > prev.p.M_rows) r1 = prev.p.M_rows;
+  const unsigned int need = 8u * (unsigned int)prev.p.n_tiles;
+  const unsigned int* cnt = P.chain_ws + CHAIN_COUNTERS + prev.cnt_off;
+  const unsigned long long t0 = ptx::globaltimer();
+  for (int j = r0 / 256; j <= (r1 - 1) / 256; ++j) {
+    while (ptx::ld_acquire_gpu(cnt + j) < need) {
+      if (ptx::globaltimer() - t0 > CHAIN_POLL_NS) {  // never expected: report it and run on instead of hanging
+        atomicExch(P.chain_ws + CHAIN_STATUS, 1u);
+        return;
+      }
+    }
+  }
+}
+
+// Leader producer: claim the next ticket (increasing, one atomic), wait for its inputs, publish it to both CTAs.
+// Deadlock-free: a unit depends only on smaller tickets, tickets are claimed in order and only by running clusters,
+// and a cluster's producer claims its next ticket only after issuing every load of its previous one, so the smallest
+// unfinished ticket always has complete inputs and a pipeline that drains.
+__device__ __forceinline__ bool ring_claim(const PairParams& P, PairRing& r, PairWork& w) {
+  ptx::mbar_wait_cluster(&r.empty[r.slot], r.phase ^ 1u);
+  int t = (int)atomicAdd(P.chain_ws + CHAIN_TICKET, 1u);
+  if (t >= P.layer[P.n_layers - 1].unit_end) {
+    t = -1;
+  } else {
+    chain_decode(P, t, w);
+    if (w.layer > 0) chain_wait_inputs(P, w);
+    // the inputs were written by TMA stores (async proxy) of other SMs and published by their red.release; our
+    // ld.acquire made them visible to this thread's generic proxy, and this fence extends that to the TMA loads this
+    // thread issues next (PTX ISA, memory consistency model: proxies — a proxy fence is needed on BOTH sides)
+    ptx::fence_proxy_async_global();
+  }
+  for (uint32_t rk = 0; rk < 2; ++rk) {
+    ptx::st_cluster_u32(ptx::mapa_shared(&r.val[r.slot], rk), (uint32_t)t);
+    ptx::mbar_arrive_cluster(ptx::mapa_shared(&r.full[r.slot], rk));  // release.cluster: the value above first
+  }
+  if (++r.slot == WORK_SLOTS) { r.slot = 0; r.phase ^= 1u; }
+  return t >= 0;
+}
+
+// Writer side of the readiness protocol, per epilogue warp and unit (after the accumulator stage went back): the TMA
+// stores of this warp must be COMPLETE (wait_group, not .read), the async-proxy writes are then ordered before the
+// generic-proxy release by a proxy fence, and the release-add publishes them at GPU scope.
+__device__ __forceinline__ void chain_arrive(const PairParams& P, const PairWork& w, int lane) {
+  __threadfence();  // (direct stores of a last chunk narrower than 64 columns, by every lane)
+  __syncwarp();
+  if (lane == 0) {
+    ptx::bulk_wait_group_all();
+    ptx::fence_proxy_async_global();
+    const PairLayer& L = P.layer[w.layer];
+    ptx::red_release_gpu_add(P.chain_ws + CHAIN_COUNTERS + L.cnt_off + w.unit / L.p.n_tiles, 1u);
+  }
+}
+
 // Epilogue warps of the CTA-pair kernel: one pass per work item.  Whole units and finishers drain the accumulator
 // through scale/shift/leaky and store (a finisher first adds the partial accumulators of the unit's earlier K spans);
 // partial pieces park their raw fp32 accumulator in the workspace and count themselves in.
 template <int MODE, bool LEAKY>
-__device__ __forceinline__ void epilogue_loop_pair(const ConvKParams& p, uint32_t tmem_base, uint64_t* tmem_full_bar,
+__device__ __forceinline__ void epilogue_loop_pair(const PairParams& P, uint32_t tmem_base, uint64_t* tmem_full_bar,
                                                    uint64_t* tmem_empty_bar, float* s_ss, int cluster_id, int num_clusters,
-                                                   int pair_rank, uint8_t* s_out, const CUtensorMap* tm_out) {
+                                                   int pair_rank, uint8_t* s_out, PairRing ring) {
   const int warp_idx = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
   const int et = threadIdx.x - 64;   // 0..127
   const int quarter = warp_idx & 3;  // TMEM lane quarter this warp may access
-  const bool vec_ok = ((p.ldc | p.ch_off) & 7) == 0 && (MODE != MC_EPI_REORG2 || (p.N & 7) == 0);
+  const ConvKParams& p0 = P.layer[0].p;
+  const bool chain = P.n_layers > 1;
   int as = 0;
   uint32_t aphase = 0;
   int slab_buf = 0;
   float* stat_acc = nullptr;
   int stat_n0 = -1;
-  if (MODE == MC_EPI_PNHWC && p.tma_bufs > 0 && p.stat_sum != nullptr) {
-    stat_acc = reinterpret_cast<float*>(s_out + (size_t)4 * p.tma_bufs * 4096) + quarter * 512;
+  if (MODE == MC_EPI_PNHWC && p0.tma_bufs > 0 && p0.stat_sum != nullptr) {
+    stat_acc = reinterpret_cast<float*>(s_out + (size_t)4 * p0.tma_bufs * 4096) + quarter * 512;
     for (int c = lane; c < 512; c += 32) stat_acc[c] = 0.f;
     __syncwarp();
   }
-  const bool one_n_tile = p.n_tiles == 1;
+  const bool one_n_tile = !chain && p0.n_tiles == 1;
   if (one_n_tile) {
-    for (int i = et; i < p.block_n; i += 128) {
-      const bool ok = i < p.Npad;
-      s_ss[i] = ok ? __ldg(p.scale + i) : 0.f;
-      s_ss[256 + i] = ok ? __ldg(p.shift + i) : 0.f;
+    for (int i = et; i < p0.block_n; i += 128) {
+      const bool ok = i < p0.Npad;
+      s_ss[i] = ok ? __ldg(p0.scale + i) : 0.f;
+      s_ss[256 + i] = ok ? __ldg(p0.shift + i) : 0.f;
     }
     asm volatile("bar.sync 1, 128;" ::: "memory");
   }
   PairWorkIter it;
-  it.init(p, cluster_id, num_clusters);
+  it.init(p0, cluster_id, num_clusters);
   PairWork w;
   int ti = -1;
-  while (it.next(w)) {
+  while (chain ? ring_take(P, ring, w, true) : it.next(w)) {
     ++ti;
+    const ConvKParams& p = P.layer[w.layer].p;
+    const CUtensorMap* tm_out = &P.layer[w.layer].tmap_out;
+    const bool vec_ok = ((p.ldc | p.ch_off) & 7) == 0 && (MODE != MC_EPI_REORG2 || (p.N & 7) == 0);
     const int tile = w.unit;
     const int n0 = (tile % p.n_tiles) * p.block_n;
     const int m0 = (2 * (tile / p.n_tiles) + pair_rank) * BLOCK_M;
@@ -987,6 +1107,7 @@ __device__ __forceinline__ void epilogue_loop_pair(const ConvKParams& p, uint32_
                                            }
                                          }
                                        }, stat_acc);
+        if (chain) chain_arrive(P, w, lane);
         if (et == 0 && ti < 8) conv_stamp(p, 13 + 2 * ti);
         if (++as == ACC_STAGES) { as = 0; aphase ^= 1u; }
         continue;
@@ -1033,8 +1154,8 @@ __device__ __forceinline__ void epilogue_loop_pair(const ConvKParams& p, uint32_
     if (et == 0 && ti < 8) conv_stamp(p, 13 + 2 * ti);
     if (++as == ACC_STAGES) { as = 0; aphase ^= 1u; }
   }
-  if (stat_acc != nullptr && stat_n0 >= 0) flush_stats(p, stat_acc, stat_n0, lane);
-  if (MODE == MC_EPI_PNHWC && p.tma_bufs > 0 && lane == 0) ptx::bulk_wait_group_read<0>();  // slabs read before the CTA exits
+  if (stat_acc != nullptr && stat_n0 >= 0) flush_stats(p0, stat_acc, stat_n0, lane);
+  if (MODE == MC_EPI_PNHWC && p0.tma_bufs > 0 && lane == 0) ptx::bulk_wait_group_read<0>();  // slabs read before the CTA exits
 }
 
 // ---------------------------------------------------------------------------------------------------------------
@@ -1047,18 +1168,20 @@ __device__ __forceinline__ void epilogue_loop_pair(const ConvKParams& p, uint32_
 // is multicast to the empty / accumulator-full barriers of both CTAs; the epilogues of both CTAs hand the
 // accumulator stage back on the leader's barrier (8 arrivals).
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1)
-conv_gemm_tcgen05_pair_kernel(const __grid_constant__ CUtensorMap tmap_b, const __grid_constant__ CUtensorMap tmap_abox,
-                              const __grid_constant__ CUtensorMap tmap_out, const ConvKParams p) {
+conv_gemm_tcgen05_pair_kernel(const __grid_constant__ PairParams P) {
   extern __shared__ __align__(1024) uint8_t smem_raw[];
-  const uint32_t b_half_bytes = (uint32_t)(p.block_n / 2 * 128);
+  // every entry of the layer table shares the fields read here (tile width, ring depths, epilogue slabs)
+  const ConvKParams& p0 = P.layer[0].p;
+  const bool chain = P.n_layers > 1;
+  const uint32_t b_half_bytes = (uint32_t)(p0.block_n / 2 * 128);
   uint8_t* smem = smem_raw;
   {
     uint32_t a = ptx::smem_u32(smem);
     smem += (1024u - (a & 1023u)) & 1023u;
   }
   uint8_t* tiles = smem;
-  uint8_t* b_ring = tiles + (size_t)p.a_stages * A_BOX_STRIDE;
-  uint8_t* aux = b_ring + (size_t)p.stages * b_half_bytes;
+  uint8_t* b_ring = tiles + (size_t)p0.a_stages * A_BOX_STRIDE;
+  uint8_t* aux = b_ring + (size_t)p0.stages * b_half_bytes;
   uint64_t* full_bar = reinterpret_cast<uint64_t*>(aux);
   uint64_t* empty_bar = full_bar + MAX_STAGES;
   uint64_t* tmem_full_bar = empty_bar + MAX_STAGES;      // [ACC_STAGES]
@@ -1066,6 +1189,12 @@ conv_gemm_tcgen05_pair_kernel(const __grid_constant__ CUtensorMap tmap_b, const 
   uint64_t* afull_bar = tmem_empty_bar + ACC_STAGES;     // [MAX_A_STAGES]
   uint64_t* aempty_bar = afull_bar + MAX_A_STAGES;    // [MAX_A_STAGES]
   uint32_t* tmem_ptr_smem = reinterpret_cast<uint32_t*>(aempty_bar + MAX_A_STAGES);
+  PairRing ring;
+  ring.full = reinterpret_cast<uint64_t*>(aux + 256);  // [WORK_SLOTS]
+  ring.empty = ring.full + WORK_SLOTS;                 // [WORK_SLOTS]
+  ring.val = reinterpret_cast<int*>(ring.empty + WORK_SLOTS);
+  ring.slot = 0;
+  ring.phase = 0;
   float* s_ss = reinterpret_cast<float*>(aux + 512);
   uint8_t* s_out = aux + 5120;  // TMA-store slabs [4 warps][tma_bufs][4 KB], 1024-byte aligned
 
@@ -1073,13 +1202,15 @@ conv_gemm_tcgen05_pair_kernel(const __grid_constant__ CUtensorMap tmap_b, const 
   const int lane = threadIdx.x & 31;
   const int rank = (int)ptx::cluster_ctarank();
   const int cluster_id = blockIdx.x >> 1, num_clusters = gridDim.x >> 1;
-  if (threadIdx.x == 0) conv_stamp(p, 0);
+  if (threadIdx.x == 0) conv_stamp(p0, 0);
 
   if (warp_idx == 0 && lane == 0) {
-    ptx::prefetch_tensormap(&tmap_b);
-    ptx::prefetch_tensormap(&tmap_abox);
-    if (p.tma_bufs > 0) ptx::prefetch_tensormap(&tmap_out);
-    for (int s = 0; s < p.stages; ++s) {
+    for (int l = 0; l < P.n_layers; ++l) {
+      ptx::prefetch_tensormap(&P.layer[l].tmap_b);
+      ptx::prefetch_tensormap(&P.layer[l].tmap_abox);
+      if (p0.tma_bufs > 0) ptx::prefetch_tensormap(&P.layer[l].tmap_out);
+    }
+    for (int s = 0; s < p0.stages; ++s) {
       ptx::mbar_init(&full_bar[s], 1);
       ptx::mbar_init(&empty_bar[s], 1);
     }
@@ -1091,17 +1222,21 @@ conv_gemm_tcgen05_pair_kernel(const __grid_constant__ CUtensorMap tmap_b, const 
       ptx::mbar_init(&afull_bar[a], 1);
       ptx::mbar_init(&aempty_bar[a], 1);
     }
+    for (int s = 0; s < WORK_SLOTS; ++s) {
+      ptx::mbar_init(&ring.full[s], 1);
+      ptx::mbar_init(&ring.empty[s], 10);  // leader: MMA warp + 4 epilogue warps; peer: producer + 4 epilogue warps
+    }
     ptx::fence_barrier_init();
   }
   if (warp_idx == 1) {
-    ptx::tmem_alloc_pair(tmem_ptr_smem, (uint32_t)p.tmem_cols);
+    ptx::tmem_alloc_pair(tmem_ptr_smem, (uint32_t)p0.tmem_cols);
     ptx::tmem_relinquish_pair();
   }
   ptx::tc_fence_before();
   ptx::cluster_sync_all();  // barriers of BOTH CTAs initialised before any remote arrival / complete_tx
   ptx::tc_fence_after();
   const uint32_t tmem_base = *tmem_ptr_smem;
-  if (threadIdx.x == 0) conv_stamp(p, 1);
+  if (threadIdx.x == 0) conv_stamp(p0, 1);
 
   if (warp_idx == 0) {
     // ===================== TMA producer (one thread per CTA) =====================
@@ -1109,9 +1244,14 @@ conv_gemm_tcgen05_pair_kernel(const __grid_constant__ CUtensorMap tmap_b, const 
       int s = 0, sa = 0;
       uint32_t phase = 0, pha = 0;
       PairWorkIter it;
-      it.init(p, cluster_id, num_clusters);
+      it.init(p0, cluster_id, num_clusters);
       PairWork w;
-      while (it.next(w)) {
+      while (!chain ? it.next(w) : (rank == 0 ? ring_claim(P, ring, w) : ring_take(P, ring, w, false))) {
+        const PairLayer& L = P.layer[w.layer];
+        const ConvKParams& p = L.p;
+        // (chain, peer CTA) the leader acquired this unit's inputs; the mbarrier hand-over carries that to this
+        // thread, and the proxy fence to the TMA loads it issues (see ring_claim)
+        if (chain && rank != 0) ptx::fence_proxy_async_global();
         const int unit = w.unit;
         const int n0 = (unit % p.n_tiles) * p.block_n + rank * (p.block_n / 2);
         const int m0 = (2 * (unit / p.n_tiles) + rank) * BLOCK_M;
@@ -1120,19 +1260,19 @@ conv_gemm_tcgen05_pair_kernel(const __grid_constant__ CUtensorMap tmap_b, const 
           const int dy = g / p.kb_per_tap, cb = g - dy * p.kb_per_tap;
           ptx::mbar_wait(&aempty_bar[sa], pha ^ 1u);
           if (rank == 0) ptx::mbar_arrive_expect_tx(&afull_bar[sa], 2 * A_BOX_BYTES);
-          ptx::tma_load_2d_pair(tiles + (size_t)sa * A_BOX_STRIDE, &tmap_abox, &afull_bar[sa], cb * 64,
+          ptx::tma_load_2d_pair(tiles + (size_t)sa * A_BOX_STRIDE, &L.tmap_abox, &afull_bar[sa], cb * 64,
                                 m0 + (dy - 1) * p.Wp - 1);
           if (++sa == p.a_stages) { sa = 0; pha ^= 1u; }
           for (int dx = 0; dx < 3; ++dx) {
             const int kb = (dy * 3 + dx) * p.kb_per_tap + cb;
             ptx::mbar_wait(&empty_bar[s], phase ^ 1u);
             if (rank == 0) ptx::mbar_arrive_expect_tx(&full_bar[s], 2 * b_half_bytes);
-            ptx::tma_load_2d_pair(b_ring + (size_t)s * b_half_bytes, &tmap_b, &full_bar[s], kb * 64, n0);
+            ptx::tma_load_2d_pair(b_ring + (size_t)s * b_half_bytes, &L.tmap_b, &full_bar[s], kb * 64, n0);
             if (++s == p.stages) { s = 0; phase ^= 1u; }
           }
         }
       }
-      conv_stamp(p, 3);
+      conv_stamp(p0, 3);
     }
   } else if (warp_idx == 1) {
     // ===================== MMA issuer (warp 1 of the leader CTA; one elected lane issues) =====================
@@ -1140,17 +1280,20 @@ conv_gemm_tcgen05_pair_kernel(const __grid_constant__ CUtensorMap tmap_b, const 
       int s = 0, sa = 0, as = 0;
       uint32_t phase = 0, pha = 0, aphase = 0;
       PairWorkIter it;
-      it.init(p, cluster_id, num_clusters);
+      it.init(p0, cluster_id, num_clusters);
       PairWork w;
       int ti = -1;
-      while (it.next(w)) {
+      while (chain ? ring_take(P, ring, w, true) : it.next(w)) {
         ++ti;
+        const ConvKParams& p = P.layer[w.layer].p;
         ptx::mbar_wait(&tmem_empty_bar[as], aphase ^ 1u);
         ptx::tc_fence_after();
         const uint32_t tmem_acc = tmem_base + (uint32_t)(as * p.acc_stride);
-        const int gb = w.g0, ge = w.g1 < 0 ? 3 * p.kb_per_tap : w.g1;
+        const int kbt = p.kb_per_tap, lks = p.last_ksteps;
+        const uint32_t idesc = p.idesc;
+        const int gb = w.g0, ge = w.g1 < 0 ? 3 * kbt : w.g1;
         for (int g = gb; g < ge; ++g) {
-          const int nk = ((g % p.kb_per_tap) == p.kb_per_tap - 1) ? p.last_ksteps : 4;
+          const int nk = ((g % kbt) == kbt - 1) ? lks : 4;
           ptx::mbar_wait(&afull_bar[sa], pha);
           if (ti == 0 && g == gb && lane == 0) conv_stamp(p, 4);
           const uint32_t a_addr = ptx::smem_u32(tiles + (size_t)sa * A_BOX_STRIDE);
@@ -1163,16 +1306,16 @@ conv_gemm_tcgen05_pair_kernel(const __grid_constant__ CUtensorMap tmap_b, const 
 #pragma unroll
               for (int k = 0; k < 4; ++k)
                 if (k < nk)
-                  ptx::umma_bf16_ss_pair(tmem_acc, adesc + (uint64_t)(2 * k), bdesc + (uint64_t)(2 * k), p.idesc,
+                  ptx::umma_bf16_ss_pair(tmem_acc, adesc + (uint64_t)(2 * k), bdesc + (uint64_t)(2 * k), idesc,
                                          (g > gb || dx > 0 || k > 0) ? 1u : 0u);
               ptx::umma_commit_pair(&empty_bar[s]);
               if (dx == 2) ptx::umma_commit_pair(&aempty_bar[sa]);
               if (dx == 2 && g == ge - 1) ptx::umma_commit_pair(&tmem_full_bar[as]);
             }
             __syncwarp();
-            if (++s == p.stages) { s = 0; phase ^= 1u; }
+            if (++s == p0.stages) { s = 0; phase ^= 1u; }
           }
-          if (++sa == p.a_stages) { sa = 0; pha ^= 1u; }
+          if (++sa == p0.a_stages) { sa = 0; pha ^= 1u; }
         }
         if (lane == 0 && ti < 6) conv_stamp(p, 5 + ti);
         if (++as == ACC_STAGES) { as = 0; aphase ^= 1u; }
@@ -1180,21 +1323,35 @@ conv_gemm_tcgen05_pair_kernel(const __grid_constant__ CUtensorMap tmap_b, const 
     }
   } else {
     // ===================== epilogue: warps 2..5 of both CTAs =====================
-    if (p.epi_mode == MC_EPI_PNHWC) {
-      if (p.leaky) epilogue_loop_pair<MC_EPI_PNHWC, true>(p, tmem_base, tmem_full_bar, tmem_empty_bar, s_ss, cluster_id, num_clusters, rank, s_out, &tmap_out);
-      else epilogue_loop_pair<MC_EPI_PNHWC, false>(p, tmem_base, tmem_full_bar, tmem_empty_bar, s_ss, cluster_id, num_clusters, rank, s_out, &tmap_out);
-    } else if (p.epi_mode == MC_EPI_REORG2) {
-      if (p.leaky) epilogue_loop_pair<MC_EPI_REORG2, true>(p, tmem_base, tmem_full_bar, tmem_empty_bar, s_ss, cluster_id, num_clusters, rank, s_out, &tmap_out);
-      else epilogue_loop_pair<MC_EPI_REORG2, false>(p, tmem_base, tmem_full_bar, tmem_empty_bar, s_ss, cluster_id, num_clusters, rank, s_out, &tmap_out);
+    if (p0.epi_mode == MC_EPI_PNHWC) {
+      if (p0.leaky) epilogue_loop_pair<MC_EPI_PNHWC, true>(P, tmem_base, tmem_full_bar, tmem_empty_bar, s_ss, cluster_id, num_clusters, rank, s_out, ring);
+      else epilogue_loop_pair<MC_EPI_PNHWC, false>(P, tmem_base, tmem_full_bar, tmem_empty_bar, s_ss, cluster_id, num_clusters, rank, s_out, ring);
+    } else if (p0.epi_mode == MC_EPI_REORG2) {
+      if (p0.leaky) epilogue_loop_pair<MC_EPI_REORG2, true>(P, tmem_base, tmem_full_bar, tmem_empty_bar, s_ss, cluster_id, num_clusters, rank, s_out, ring);
+      else epilogue_loop_pair<MC_EPI_REORG2, false>(P, tmem_base, tmem_full_bar, tmem_empty_bar, s_ss, cluster_id, num_clusters, rank, s_out, ring);
     } else {
-      if (p.leaky) epilogue_loop_pair<MC_EPI_NCHW_F32, true>(p, tmem_base, tmem_full_bar, tmem_empty_bar, s_ss, cluster_id, num_clusters, rank, s_out, &tmap_out);
-      else epilogue_loop_pair<MC_EPI_NCHW_F32, false>(p, tmem_base, tmem_full_bar, tmem_empty_bar, s_ss, cluster_id, num_clusters, rank, s_out, &tmap_out);
+      if (p0.leaky) epilogue_loop_pair<MC_EPI_NCHW_F32, true>(P, tmem_base, tmem_full_bar, tmem_empty_bar, s_ss, cluster_id, num_clusters, rank, s_out, ring);
+      else epilogue_loop_pair<MC_EPI_NCHW_F32, false>(P, tmem_base, tmem_full_bar, tmem_empty_bar, s_ss, cluster_id, num_clusters, rank, s_out, ring);
     }
   }
 
   ptx::tc_fence_before();
   ptx::cluster_sync_all();  // the peer may still read this CTA's smem / signal its barriers until both are done
-  if (warp_idx == 1) ptx::tmem_dealloc_pair(tmem_base, (uint32_t)p.tmem_cols);
+  if (warp_idx == 1) ptx::tmem_dealloc_pair(tmem_base, (uint32_t)p0.tmem_cols);
+  if (threadIdx.x == 0) conv_stamp(p0, 30);
+  if (chain && rank == 0 && threadIdx.x == 0) {
+    // every unit of this cluster is stored and counted (cluster barrier above).  The LAST cluster out puts the tickets
+    // and counters back to zero, so every launch leaves the workspace as it found it (graph replays need no memset)
+    __threadfence();
+    if (atomicAdd(P.chain_ws + CHAIN_DONE, 1u) == (unsigned int)num_clusters - 1u) {
+      __threadfence();
+      const PairLayer& last = P.layer[P.n_layers - 1];
+      const int n_cnt = last.cnt_off + (last.p.m_tiles + 1) / 2;
+      for (int i = 0; i < n_cnt; ++i) P.chain_ws[CHAIN_COUNTERS + i] = 0u;
+      P.chain_ws[CHAIN_TICKET] = 0u;
+      P.chain_ws[CHAIN_DONE] = 0u;
+    }
+  }
 }
 
 // Tile-width heuristic.  One 64-wide k-block of a 128 x bn tile costs max(2*bn, 128+bn) SM cycles: 2*bn is the
@@ -1254,8 +1411,45 @@ extern "C" size_t mc_workspace_bytes_conv_fwd(const mc_conv_desc* d) {
   return (size_t)2048 + (size_t)clusters * 3 * 256 * 256 * sizeof(float);
 }
 
-extern "C" int mc_conv_fwd(const mc_conv_desc* d, void* stream_) {
-  cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
+// Clusters of the CTA-pair kernel that fit on the device at once (queried once)
+static int pair_max_clusters(int* out) {
+  static int max_clusters = -1;
+  if (max_clusters < 0) {
+    MC_CUDA(cudaFuncSetAttribute(conv_gemm_tcgen05_pair_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3(2 * (mc_num_sms() / 2));
+    cfg.blockDim = dim3(NUM_THREADS);
+    cfg.dynamicSmemBytes = 222 * 1024;
+    cudaLaunchAttribute at[1];
+    at[0].id = cudaLaunchAttributeClusterDimension;
+    at[0].val.clusterDim.x = 2; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
+    cfg.attrs = at;
+    cfg.numAttrs = 1;
+    int n = 0;
+    if (cudaOccupancyMaxActiveClusters(&n, conv_gemm_tcgen05_pair_kernel, &cfg) != cudaSuccess || n < 1) {
+      cudaGetLastError();
+      n = mc_num_sms() / 2;
+    }
+    max_clusters = n;
+  }
+  *out = max_clusters;
+  return 0;
+}
+
+// Everything mc_conv_fwd decides for one layer: kernel (CTA pair or single CTA), tile width, ring depth, CTAs per SM,
+// stream-K tail, tensor maps and kernel parameters.  mc_conv_chain_fwd plans its members with the same function, so a
+// chained layer computes exactly what its own mc_conv_fwd launch would.
+struct ConvPlan {
+  bool use_pair;
+  int ctas;        // single-CTA kernel: resident CTAs per SM
+  int grid;        // CTAs
+  int units;       // CTA pair: (m-pair, n-tile) units
+  size_t smem_bytes;
+  CUtensorMap tm_a, tm_b, tm_abox, tm_out;
+  ConvKParams p;
+};
+
+static int conv_plan(const mc_conv_desc* d, ConvPlan* L) {
   MC_CHECK_ARG(d != nullptr, "mc_conv_fwd: null descriptor");
   MC_CHECK_ARG(d->d_in && d->d_wpack && d->d_scale && d->d_shift && (d->d_out || d->epi_mode == MC_EPI_DECODE),
                "mc_conv_fwd: null pointer");
@@ -1510,25 +1704,9 @@ extern "C" int mc_conv_fwd(const mc_conv_desc* d, void* stream_) {
     p.acc_stride = ((block_n + 31) / 32) * 32;
     p.tmem_cols = 32;
     while (p.tmem_cols < ACC_STAGES * p.acc_stride) p.tmem_cols <<= 1;
-    static int max_clusters = -1;
-    if (max_clusters < 0) {
-      MC_CUDA(cudaFuncSetAttribute(conv_gemm_tcgen05_pair_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-      cudaLaunchConfig_t cfg = {};
-      cfg.gridDim = dim3(2 * (mc_num_sms() / 2));
-      cfg.blockDim = dim3(NUM_THREADS);
-      cfg.dynamicSmemBytes = 222 * 1024;
-      cudaLaunchAttribute at[1];
-      at[0].id = cudaLaunchAttributeClusterDimension;
-      at[0].val.clusterDim.x = 2; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
-      cfg.attrs = at;
-      cfg.numAttrs = 1;
-      int n = 0;
-      if (cudaOccupancyMaxActiveClusters(&n, conv_gemm_tcgen05_pair_kernel, &cfg) != cudaSuccess || n < 1) {
-        cudaGetLastError();
-        n = mc_num_sms() / 2;
-      }
-      max_clusters = n;
-    }
+    int max_clusters = 0;
+    int rc2 = pair_max_clusters(&max_clusters);
+    if (rc2) return rc2;
     const int m_pairs = (m_tiles + 1) / 2;
     const long long units = (long long)m_pairs * n_tiles;
     const int clusters = (int)(units < max_clusters ? units : max_clusters);
@@ -1557,9 +1735,48 @@ extern "C" int mc_conv_fwd(const mc_conv_desc* d, void* stream_) {
         p.sk_part = reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(d->d_ws) + 2048);
       }
     }
-    g_last_plan[0] = 1; g_last_plan[1] = block_n; g_last_plan[2] = 1; g_last_plan[3] = p.sk_units; g_last_plan[4] = 1;
-    g_last_plan[5] = stages; g_last_plan[6] = 2 * clusters; g_last_plan[7] = BLOCK_K;
-    conv_gemm_tcgen05_pair_kernel<<<2 * clusters, NUM_THREADS, smem_bytes, stream>>>(tm_b, tm_abox, tm_out, p);
+    L->use_pair = true;
+    L->ctas = 1;
+    L->grid = 2 * clusters;
+    L->units = (int)units;
+  } else {
+    const long long max_ctas = (long long)mc_num_sms() * ctas;
+    L->use_pair = false;
+    L->ctas = ctas;
+    L->grid = (int)(total_tiles < max_ctas ? total_tiles : max_ctas);
+    L->units = 0;
+  }
+  L->smem_bytes = smem_bytes;
+  L->tm_a = tm_a; L->tm_b = tm_b; L->tm_abox = tm_abox; L->tm_out = tm_out;
+  L->p = p;
+  return 0;
+}
+
+// one layer of the CTA-pair kernel's table from its plan
+static void pair_layer(const ConvPlan& L, PairLayer* e) {
+  e->tmap_b = L.tm_b;
+  e->tmap_abox = L.tm_abox;
+  e->tmap_out = L.tm_out;
+  e->p = L.p;
+  e->unit_end = L.units;
+  e->cnt_off = 0;
+}
+
+extern "C" int mc_conv_fwd(const mc_conv_desc* d, void* stream_) {
+  cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
+  ConvPlan L;
+  int rc = conv_plan(d, &L);
+  if (rc) return rc;
+  const ConvKParams& p = L.p;
+  if (L.use_pair) {
+    g_last_plan[0] = 1; g_last_plan[1] = p.block_n; g_last_plan[2] = 1; g_last_plan[3] = p.sk_units; g_last_plan[4] = 1;
+    g_last_plan[5] = p.stages; g_last_plan[6] = L.grid; g_last_plan[7] = p.block_k;
+    PairParams P;
+    memset(&P, 0, sizeof(P));
+    pair_layer(L, &P.layer[0]);
+    P.n_layers = 1;
+    P.chain_ws = nullptr;
+    conv_gemm_tcgen05_pair_kernel<<<L.grid, NUM_THREADS, L.smem_bytes, stream>>>(P);
     MC_LAUNCH_CHECK("conv_gemm_tcgen05_pair_kernel");
     return 0;
   }
@@ -1571,16 +1788,112 @@ extern "C" int mc_conv_fwd(const mc_conv_desc* d, void* stream_) {
     MC_CUDA(cudaFuncSetAttribute(conv_gemm_tcgen05_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, 112 * 1024));
     attr_set = true;
   }
-  const long long max_ctas = (long long)mc_num_sms() * ctas;
-  const int grid = (int)(total_tiles < max_ctas ? total_tiles : max_ctas);
-  g_last_plan[0] = 0; g_last_plan[1] = block_n; g_last_plan[2] = ctas; g_last_plan[3] = 0;
-  g_last_plan[4] = share_dx; g_last_plan[5] = stages; g_last_plan[6] = grid; g_last_plan[7] = BLOCK_K;
-  if (ctas >= 3)
-    conv_gemm_tcgen05_kernel<3><<<grid, NUM_THREADS, smem_bytes, stream>>>(tm_a, tm_b, tm_abox, tm_out, p);
-  else if (ctas == 2)
-    conv_gemm_tcgen05_kernel<2><<<grid, NUM_THREADS, smem_bytes, stream>>>(tm_a, tm_b, tm_abox, tm_out, p);
+  g_last_plan[0] = 0; g_last_plan[1] = p.block_n; g_last_plan[2] = L.ctas; g_last_plan[3] = 0;
+  g_last_plan[4] = p.share_dx; g_last_plan[5] = p.stages; g_last_plan[6] = L.grid; g_last_plan[7] = p.block_k;
+  if (L.ctas >= 3)
+    conv_gemm_tcgen05_kernel<3><<<L.grid, NUM_THREADS, L.smem_bytes, stream>>>(L.tm_a, L.tm_b, L.tm_abox, L.tm_out, p);
+  else if (L.ctas == 2)
+    conv_gemm_tcgen05_kernel<2><<<L.grid, NUM_THREADS, L.smem_bytes, stream>>>(L.tm_a, L.tm_b, L.tm_abox, L.tm_out, p);
   else
-    conv_gemm_tcgen05_kernel<1><<<grid, NUM_THREADS, smem_bytes, stream>>>(tm_a, tm_b, tm_abox, tm_out, p);
+    conv_gemm_tcgen05_kernel<1><<<L.grid, NUM_THREADS, L.smem_bytes, stream>>>(L.tm_a, L.tm_b, L.tm_abox, L.tm_out, p);
   MC_LAUNCH_CHECK("conv_gemm_tcgen05_kernel");
+  return 0;
+}
+
+// Words of the chain workspace: ticket, clusters done, status, pad, one readiness counter per (member, m-pair)
+static size_t chain_ws_words(const mc_conv_desc* descs, int n) {
+  size_t words = CHAIN_COUNTERS;
+  for (int i = 0; i < n; ++i) {
+    const long long rows = (long long)descs[i].B * (descs[i].H + 1) * (descs[i].W + 1);
+    words += (size_t)(((rows + BLOCK_M - 1) / BLOCK_M + 1) / 2);
+  }
+  return words;
+}
+
+// byte range [lo, hi) of the PNHWC rows a member reads (input) or writes (output)
+static bool ranges_overlap(const void* a, size_t na, const void* b, size_t nb) {
+  const uintptr_t a0 = (uintptr_t)a, b0 = (uintptr_t)b;
+  return a0 < b0 + nb && b0 < a0 + na;
+}
+
+// Plans every member (conv_plan, as mc_conv_fwd would) and checks that the members form a chain the kernel can run.
+static int chain_plan(const mc_conv_desc* descs, int n, ConvPlan* L) {
+  MC_CHECK_ARG(descs != nullptr, "mc_conv_chain_fwd: null descriptors");
+  MC_CHECK_ARG(n >= 2 && n <= MAX_CHAIN, "mc_conv_chain_fwd: %d members (2..%d)", n, MAX_CHAIN);
+  const mc_conv_desc& d0 = descs[0];
+  for (int i = 0; i < n; ++i) {
+    const mc_conv_desc& di = descs[i];
+    MC_CHECK_ARG(di.ksize == 3 && di.epi_mode == MC_EPI_PNHWC,
+                 "mc_conv_chain_fwd: member %d must be a 3x3 layer with the PNHWC epilogue", i);
+    MC_CHECK_ARG(di.d_stat_sum == nullptr && di.d_stat_sumsq == nullptr,
+                 "mc_conv_chain_fwd: member %d asks for batch statistics", i);
+    MC_CHECK_ARG(di.B == d0.B && di.H == d0.H && di.W == d0.W, "mc_conv_chain_fwd: member %d has another B, H or W", i);
+    mc_conv_desc one = di;
+    one.d_ws = nullptr;  // whole units only: the chain schedules the last waves itself
+    one.ws_bytes = 0;
+    const int rc = conv_plan(&one, &L[i]);
+    if (rc) return rc;
+    MC_CHECK_ARG(L[i].use_pair, "mc_conv_chain_fwd: member %d does not take the CTA-pair kernel", i);
+    MC_CHECK_ARG(L[i].p.tma_bufs > 0, "mc_conv_chain_fwd: member %d does not take the TMA-store epilogue", i);
+    MC_CHECK_ARG(L[i].p.block_n == L[0].p.block_n && L[i].p.stages == L[0].p.stages && L[i].p.leaky == L[0].p.leaky &&
+                     L[i].smem_bytes == L[0].smem_bytes,
+                 "mc_conv_chain_fwd: member %d has another tile width, ring or activation", i);
+    if (i > 0) {
+      MC_CHECK_ARG(di.d_in == descs[i - 1].d_out && di.Cin_ld == descs[i - 1].ldc,
+                   "mc_conv_chain_fwd: member %d does not read member %d's output allocation", i, i - 1);
+    }
+  }
+  // the only dependency the kernel tracks is member i -> i+1: no other member may read or rewrite what one writes
+  const size_t rows = (size_t)d0.B * (d0.H + 1) * (d0.W + 1);
+  for (int j = 0; j < n; ++j) {
+    const size_t out_bytes = rows * descs[j].ldc * 2;
+    for (int i = 0; i < n; ++i) {
+      if (i != j + 1)
+        MC_CHECK_ARG(!ranges_overlap(descs[i].d_in, rows * descs[i].Cin_ld * 2, descs[j].d_out, out_bytes),
+                     "mc_conv_chain_fwd: member %d reads member %d's output", i, j);
+      if (i != j)
+        MC_CHECK_ARG(!ranges_overlap(descs[i].d_out, rows * descs[i].ldc * 2, descs[j].d_out, out_bytes),
+                     "mc_conv_chain_fwd: members %d and %d write the same memory", i, j);
+    }
+  }
+  return 0;
+}
+
+extern "C" size_t mc_workspace_bytes_conv_chain(const mc_conv_desc* descs, int n) {
+  static thread_local ConvPlan L[MAX_CHAIN];  // (CUtensorMap-heavy: kept off the stack)
+  if (chain_plan(descs, n, L) != 0) return 0;
+  return chain_ws_words(descs, n) * sizeof(unsigned int);
+}
+
+extern "C" int mc_conv_chain_fwd(const mc_conv_desc* descs, int n, void* stream_) {
+  cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
+  static thread_local ConvPlan L[MAX_CHAIN];
+  int rc = chain_plan(descs, n, L);
+  if (rc) return rc;
+  const mc_conv_desc& d0 = descs[0];
+  const size_t need = chain_ws_words(descs, n) * sizeof(unsigned int);
+  MC_CHECK_ARG(d0.d_ws != nullptr && d0.ws_bytes >= need && ((uintptr_t)d0.d_ws & 15) == 0,
+               "mc_conv_chain_fwd: descs[0] needs a 16-byte aligned workspace of %zu bytes", need);
+
+  static thread_local PairParams P;
+  memset(&P, 0, sizeof(P));
+  int units = 0, cnt = 0;
+  for (int i = 0; i < n; ++i) {
+    pair_layer(L[i], &P.layer[i]);
+    units += L[i].units;
+    P.layer[i].unit_end = units;
+    P.layer[i].cnt_off = cnt;
+    cnt += (L[i].p.m_tiles + 1) / 2;
+  }
+  P.n_layers = n;
+  P.chain_ws = reinterpret_cast<unsigned int*>(d0.d_ws);
+  int max_clusters = 0;
+  rc = pair_max_clusters(&max_clusters);
+  if (rc) return rc;
+  const int clusters = units < max_clusters ? units : max_clusters;
+  g_last_plan[0] = 1; g_last_plan[1] = L[0].p.block_n; g_last_plan[2] = 1; g_last_plan[3] = 0; g_last_plan[4] = 1;
+  g_last_plan[5] = L[0].p.stages; g_last_plan[6] = 2 * clusters; g_last_plan[7] = 64;
+  conv_gemm_tcgen05_pair_kernel<<<2 * clusters, NUM_THREADS, L[0].smem_bytes, stream>>>(P);
+  MC_LAUNCH_CHECK("conv_gemm_tcgen05_pair_kernel");
   return 0;
 }

@@ -123,6 +123,24 @@ __device__ __forceinline__ void bulk_wait_group_read() {
   asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(N) : "memory");
 }
 
+// wait until ALL of this thread's bulk groups have completed (their global writes are performed)
+__device__ __forceinline__ void bulk_wait_group_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
+// orders this thread's generic-proxy accesses of global memory with its async-proxy (TMA) accesses
+__device__ __forceinline__ void fence_proxy_async_global() { asm volatile("fence.proxy.async.global;" ::: "memory"); }
+__device__ __forceinline__ void red_release_gpu_add(unsigned int* p, unsigned int v) {
+  asm volatile("red.release.gpu.global.add.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
+}
+__device__ __forceinline__ unsigned int ld_acquire_gpu(const unsigned int* p) {
+  unsigned int v;
+  asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
+  return v;
+}
+__device__ __forceinline__ unsigned long long globaltimer() {
+  unsigned long long t;
+  asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
+  return t;
+}
+
 // ---------------- tcgen05 / TMEM ----------------
 __device__ __forceinline__ void tmem_alloc(uint32_t* smem_dst, uint32_t ncols) {
   asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(smem_dst)),
@@ -182,6 +200,36 @@ __device__ __forceinline__ void tma_load_2d_pair(void* smem_dst, const void* tma
 __device__ __forceinline__ void mbar_arrive_leader(uint64_t* bar) {
   asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(smem_u32(bar) & kPeerBitMask)
                : "memory");
+}
+// shared::cluster address of this CTA's `p` in CTA `rank` of the cluster
+__device__ __forceinline__ uint32_t mapa_shared(const void* p, uint32_t rank) {
+  uint32_t r;
+  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(smem_u32(p)), "r"(rank));
+  return r;
+}
+__device__ __forceinline__ void st_cluster_u32(uint32_t cluster_addr, uint32_t v) {
+  asm volatile("st.shared::cluster.u32 [%0], %1;" ::"r"(cluster_addr), "r"(v) : "memory");
+}
+__device__ __forceinline__ void mbar_arrive_cluster(uint32_t cluster_addr) {
+  asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(cluster_addr) : "memory");
+}
+// wait for a phase that threads of the OTHER CTA of the cluster complete (acquire at cluster scope)
+__device__ __forceinline__ void mbar_wait_cluster(uint64_t* bar, uint32_t parity) {
+  uint32_t spins = 0;
+  for (;;) {
+    uint32_t ok;
+    asm volatile(
+        "{\n\t"
+        ".reg .pred P;\n\t"
+        "mbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 P, [%1], %2, %3;\n\t"
+        "selp.b32 %0, 1, 0, P;\n\t"
+        "}\n"
+        : "=r"(ok)
+        : "r"(smem_u32(bar)), "r"(parity), "r"(10000u)
+        : "memory");
+    if (ok) return;
+    if (++spins > (1u << 18)) __trap();
+  }
 }
 __device__ __forceinline__ void tmem_alloc_pair(uint32_t* smem_dst, uint32_t ncols) {
   asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(smem_dst)),

@@ -112,6 +112,9 @@ class CompiledDarknet(object):
         self.use_graph = True
         self.in_hw = None
         self._compile(model)
+        self._chain_runs = self._chain_runs_of(self.ops)
+        self._items = {}     # (B, H, W) -> launch list (ops, and one entry per chained run)
+        self._last_items = None
 
     # ------------------------------------------------------------------------------------------------ compile
     def _new_buf(self, H, W, ld, **kw):
@@ -234,6 +237,36 @@ class CompiledDarknet(object):
                 if block['type'] == 'route':
                     routed.update(int(i) if int(i) > 0 else int(i) + ind for i in block['layers'].split(','))
             self._fuse_thin_pairs(routed)
+
+    def _chain_runs_of(self, ops):
+        """Runs of 3x3 conv ops in which each reads the previous one's output (mc_conv_chain_fwd runs them as one launch;
+        which parts it takes depends on the batch size and is asked at run time, _launch_items).  An op between two
+        members may sit in a run when its input is produced before the run and no earlier member reads its output: it is
+        launched in front of the run (YOLOv2's reorg branch conv21 writes its slice of the concat buffer that the run's
+        last member reads).  self.ops keeps one entry per layer, in layer order."""
+        def chainable(op):
+            return op['kind'] == 'conv' and op['ksize'] == 3 and op['epi'] == _lib.MC_EPI_PNHWC
+
+        runs, i = [], 0
+        while i < len(ops):
+            if not chainable(ops[i]):
+                i += 1
+                continue
+            run, j, last = [ops[i]], i + 1, i
+            while j < len(ops) and len(run) < 4:
+                nxt = ops[j]
+                if chainable(nxt) and nxt['src'].buf_id == run[-1]['dst_buf'] and nxt['src'].ch_off == 0:
+                    run.append(nxt)
+                    last = j
+                elif nxt.get('src') is None or 'dst_buf' not in nxt or \
+                        nxt['src'].buf_id in {m['dst_buf'] for m in run} or \
+                        nxt['dst_buf'] in {m['src'].buf_id for m in run}:
+                    break
+                j += 1
+            if len(run) >= 2:
+                runs.append(run)
+            i = last + 1
+        return runs
 
     def _fuse_thin_pairs(self, routed):
         """thin 3x3 layer -> 1x1 layer with <= 8 outputs: the second layer is applied by the same thread to the bf16-rounded
@@ -636,13 +669,15 @@ class CompiledDarknet(object):
         return entry
 
     def _conv_workspace(self, nbytes):
-        """One scratch buffer for every conv launch of the plan (stream-K partial tiles of the CTA-pair kernel; launches
-        on a stream are ordered, and a captured graph keeps reading the same address)."""
+        """One scratch buffer for every conv launch of the plan (stream-K partial tiles of the CTA-pair kernel, and behind
+        them the tickets and counters of chained launches; launches on a stream are ordered, and a captured graph keeps
+        reading the same address).  64 KB more than asked: the chain's counters grow with the batch size, and a batch
+        size first seen after a graph capture must not need a larger buffer."""
         ws = getattr(self, '_ws', None)
         if ws is None or ws.numel() < nbytes:
             if ws is not None and self._graphs:
                 raise RuntimeError("internal: conv workspace grew after a CUDA graph captured its address")
-            ws = self._ws = torch.zeros(nbytes, dtype=torch.uint8, device=self.device)  # (counters start at zero)
+            ws = self._ws = torch.zeros(nbytes + 65536, dtype=torch.uint8, device=self.device)  # (counters start at zero)
         return ws
 
     def supports_detect(self, model):
@@ -652,6 +687,67 @@ class CompiledDarknet(object):
         n = self.ops[-1]['N']
         return n == model.num_anchors * (5 + model.num_classes) and self.ops[-1]['Npad'] <= 256 and \
             len(model.anchors) == 2 * model.num_anchors and model.num_anchors <= 16
+
+    def _conv_desc(self, op, bufs, B):
+        """mc_conv_desc of a conv op on this call's buffers (the head's output and decode are set by the caller)"""
+        s = op['src']
+        sb = self.bufs[s.buf_id]
+        d = _lib.mc_conv_desc()
+        d.d_in = bufs[s.buf_id].data_ptr() + 2 * s.ch_off
+        d.d_wpack = op['wpack'].data_ptr()
+        d.d_scale = op['scale'].data_ptr()
+        d.d_shift = op['shift'].data_ptr()
+        if op['epi'] != _lib.MC_EPI_NCHW_F32:
+            d.d_out = bufs[op['dst_buf']].data_ptr()
+        d.B, d.H, d.W = B, op['H'], op['W']
+        d.Cin, d.Cin_ld = op['Cin'], sb.ld
+        d.in_cols = sb.ld - s.ch_off  # the rest of the row: pad channels (zero) / a neighbouring slice (finite)
+        d.N, d.Npad = op['N'], op['Npad']
+        d.ksize, d.leaky, d.epi_mode = op['ksize'], op['leaky'], op['epi']
+        d.ldc, d.ch_off = op['ldc'], op['ch_off']
+        d.block_n = op.get('block_n', 0)
+        d.stages = op.get('stages', 0)
+        d.block_k = op.get('block_k', 0)
+        return d
+
+    def _launch_items(self, B, H, W, bufs):
+        """The launches of a forward at this input shape: self.ops, except that every maximal part of a run from
+        _chain_runs_of that mc_conv_chain_fwd accepts at this batch size (its members take the CTA-pair kernel) is ONE
+        entry of kind 'conv' named chain@<members>, launched in place of its first member."""
+        key = (B, H, W)
+        items = self._items.get(key)
+        if items is not None:
+            return items
+        lib = self.lib
+        first, skip = {}, set()
+        with torch.cuda.device(self.device):
+            for run in self._chain_runs:
+                i = 0
+                while i < len(run) - 1:
+                    for j in range(len(run), i + 1, -1):
+                        descs = (_lib.mc_conv_desc * (j - i))(*[self._conv_desc(m, bufs, B) for m in run[i:j]])
+                        nbytes = int(lib.mc_workspace_bytes_conv_chain(descs, j - i))
+                        if nbytes:
+                            break
+                    else:
+                        i += 1
+                        continue
+                    members = run[i:j]
+                    # the chain's words sit behind the region the stream-K tail of single launches uses
+                    ws_off = int(lib.mc_workspace_bytes_conv_fwd(ctypes.byref(descs[0])))
+                    ws_off = (ws_off + 255) // 256 * 256
+                    k0, k1 = self.ops.index(members[0]), self.ops.index(members[-1])
+                    ahead = [o for o in self.ops[k0 + 1:k1] if not any(o is m for m in members)]
+                    first[id(members[0])] = ahead + [dict(kind='conv', chain=members, ws_off=ws_off, ws_bytes=nbytes,
+                                                          name='chain@' + '+'.join(str(m['ind']) for m in members))]
+                    skip.update(id(o) for o in self.ops[k0 + 1:k1 + 1])
+                    i = j
+        items = []
+        for op in self.ops:
+            if id(op) not in skip:
+                items += first.get(id(op), [op])
+        self._items[key] = items
+        return items
 
     def _run_eager(self, x, events=None, detect=None, repeat=1):
         if x.dim() != 4:
@@ -676,7 +772,9 @@ class CompiledDarknet(object):
             stream = _lib.stream_ptr()
             out = None
             self._prev_op = None
-            for op in (o for o in self.ops for _ in range(repeat if events is not None else 1)):
+            items = self._launch_items(B, H, W, bufs)
+            self._last_items = items
+            for op in (o for o in items for _ in range(repeat if events is not None else 1)):
                 kind = op['kind']
                 first_rep = op is not getattr(self, '_prev_op', None)
                 self._prev_op = op
@@ -731,16 +829,15 @@ class CompiledDarknet(object):
                         raise NotImplementedError("maxpool on a channel slice")
                     _lib.check(lib.mc_maxpool2x2(bufs[s.buf_id].data_ptr(), bufs[op['dst_buf']].data_ptr(), B, s.H, s.W,
                                                  op['C'], sb.ld, self.bufs[op['dst_buf']].ld, stream), op['name'])
+                elif kind == 'conv' and 'chain' in op:
+                    members = op['chain']
+                    descs = (_lib.mc_conv_desc * len(members))(*[self._conv_desc(m, bufs, B) for m in members])
+                    ws = self._conv_workspace(op['ws_off'] + op['ws_bytes'])
+                    descs[0].d_ws, descs[0].ws_bytes = ws.data_ptr() + op['ws_off'], op['ws_bytes']
+                    _lib.check(lib.mc_conv_chain_fwd(descs, len(members), stream), op['name'])
                 elif kind == 'conv':
-                    s = op['src']
-                    d = _lib.mc_conv_desc()
-                    sb = self.bufs[s.buf_id]
-                    d.d_in = bufs[s.buf_id].data_ptr() + 2 * s.ch_off
-                    d.d_wpack = op['wpack'].data_ptr()
-                    d.d_scale = op['scale'].data_ptr()
-                    d.d_shift = op['shift'].data_ptr()
+                    d = self._conv_desc(op, bufs, B)
                     epi = op['epi']
-                    dec = None
                     if epi == _lib.MC_EPI_NCHW_F32 and detect is not None:
                         # region decode fused into the head's epilogue: dense slot table instead of the raw head
                         thr, only_obj, want_cls = detect
@@ -755,7 +852,7 @@ class CompiledDarknet(object):
                         dec.A, dec.nc, dec.conf_thresh, dec.only_objectness = A, nc, float(thr), 1 if only_obj else 0
                         for i, a in enumerate(self.detect_anchors):
                             dec.anchors[i] = float(a)
-                        epi = _lib.MC_EPI_DECODE
+                        d.epi_mode = _lib.MC_EPI_DECODE
                         out = (boxes, cls)
                         d.decode = ctypes.pointer(dec)
                         d.d_out = None
@@ -763,17 +860,6 @@ class CompiledDarknet(object):
                         out = torch.empty(B, op['N'], op['H'], op['W'], dtype=torch.float32, device=self.device)
                         bufs[op['dst_buf']] = out
                         d.d_out = out.data_ptr()
-                    else:
-                        d.d_out = bufs[op['dst_buf']].data_ptr()
-                    d.B, d.H, d.W = B, op['H'], op['W']
-                    d.Cin, d.Cin_ld = op['Cin'], sb.ld
-                    d.in_cols = sb.ld - s.ch_off  # the rest of the row: pad channels (zero) / a neighbouring slice (finite)
-                    d.N, d.Npad = op['N'], op['Npad']
-                    d.ksize, d.leaky, d.epi_mode = op['ksize'], op['leaky'], epi
-                    d.ldc, d.ch_off = op['ldc'], op['ch_off']
-                    d.block_n = op.get('block_n', 0)
-                    d.stages = op.get('stages', 0)
-                    d.block_k = op.get('block_k', 0)
                     if op.get('ws_bytes') is None:
                         op['ws_bytes'] = int(lib.mc_workspace_bytes_conv_fwd(ctypes.byref(d)))
                     if op['ws_bytes']:
@@ -794,8 +880,8 @@ class CompiledDarknet(object):
 
     @property
     def num_launches(self):
-        """kernel launches per forward."""
-        return len(self.ops)
+        """kernel launches per forward (of the last forward's input shape: which layers run chained depends on it)."""
+        return len(self._last_items if self._last_items is not None else self.ops)
 
     def block_activation(self, ind):
         """fp32 NCHW view (in the ORIGINAL channel space) of the output of models[ind] from the last run — for the

@@ -442,10 +442,19 @@ int mc_pack_conv_weights_dgrad(const float* d_w, const float* d_mask, int O, int
                                int Ko, void* stream);
 
 /* dW[O,C,k,k] (fp32, PyTorch layout) = mask * sum_p dZ[p, o] * A[p + off(tap), c]  on tcgen05 (both operands
- * MN-major from TMA); split over the pixel rows, partials in the workspace.  accumulate!=0 adds to d_dw.          */
+ * MN-major from TMA); split over the pixel rows, partials in the workspace.  accumulate!=0 adds the masked gradient
+ * to d_dw: dW = dW_old + mask * grad, so masked entries keep their old value (they are not zeroed).                */
 int mc_conv_wgrad(const void* d_a, int lda, int C, const void* d_dz, int ld_dz, int O, int B, int H, int W, int ksize,
                   const float* d_mask, float* d_dw, int accumulate, void* d_ws, size_t ws_bytes, void* stream);
 size_t mc_workspace_bytes_conv_wgrad(int B, int H, int W, int C, int O, int ksize);
+/* What mc_conv_wgrad does for this shape on the current device (no launch; tests / reporting):
+ * info[0] = nsplit (CTAs along the pixel rows)   info[1] = m_tiles (128 filters)   info[2] = n_tiles
+ * info[3] = block_n (input channels per tile)    info[4] = share3 (3x3: one CTA per filter row)
+ * info[5] = merge3 (the three dx taps as one N = 192 MMA)
+ * info[6] = split reduction: 1 rows<9>, 2 rows<1>, 3 small<1>, 4 small<4>, 5 small<8>
+ *           (wgrad_reduce_rows_kernel<TAPS> / wgrad_reduce_small_kernel<split groups>)
+ * info[7] = num_kb (64-row k-blocks of the whole reduction)                                                     */
+int mc_conv_wgrad_plan(int B, int H, int W, int C, int O, int ksize, int info[8]);
 
 /* Weight gradient of the first layer: x is the fp32 NCHW image [B,C,H,W], 3x3.  With a workspace of
  * mc_workspace_bytes_conv_wgrad_first() bytes (256-byte aligned; C*9 <= 32): the image is expanded to bf16 im2col rows

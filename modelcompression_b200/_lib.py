@@ -135,6 +135,7 @@ _SIGNATURES = {
     "mc_conv_wgrad": (c_int, [c_void_p, c_int, c_int, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p,
                               c_void_p, c_int, c_void_p, c_size_t, c_void_p]),
     "mc_workspace_bytes_conv_wgrad": (c_size_t, [c_int, c_int, c_int, c_int, c_int, c_int]),
+    "mc_conv_wgrad_plan": (c_int, [c_int, c_int, c_int, c_int, c_int, c_int, POINTER(c_int)]),
     "mc_conv_wgrad_first": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p,
                                     c_void_p, c_size_t, c_void_p]),
     "mc_workspace_bytes_conv_wgrad_first": (c_size_t, [c_int, c_int, c_int, c_int, c_int]),

@@ -15,7 +15,8 @@
 //
 // The reduction is very long (B*(H+1)*(W+1) rows: 2.8 M for conv2) and the output tiny for the early layers, so the row
 // range is split over CTAs; each CTA writes its partial tile [tap][o][c] to the workspace with plain vector stores and
-// wgrad_reduce_kernel sums the splits, applies the mask and emits the PyTorch layout [O, C, kh, kw].
+// a reduction kernel (wgrad_reduce_rows_kernel, or wgrad_reduce_small_kernel for small filter banks cut into many
+// splits; plan_wgrad picks it) sums the splits, applies the mask and emits the PyTorch layout [O, C, kh, kw].
 #include <cuda.h>
 #include <stdlib.h>
 #include "common.cuh"
@@ -223,27 +224,10 @@ conv_wgrad_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_dz, const __g
   if (warp_idx == 1) ptx::tmem_dealloc(tmem_base, (uint32_t)p.tmem_cols);
 }
 
-// dW[o][c][tap] = mask[o][c][tap] * sum_split ws[split][tap][o][c]   (PyTorch layout [O, C, kh, kw])
-__global__ void __launch_bounds__(256) wgrad_reduce_kernel(const float* __restrict__ ws, int nsplit, int ntaps, int Opad,
-                                                           int Cpad, int O, int C, const float* __restrict__ mask,
-                                                           float* __restrict__ dw, int accumulate) {
-  const long long total = (long long)O * C;
-  for (long long i = blockIdx.x * 256ll + threadIdx.x; i < total; i += (long long)gridDim.x * 256) {
-    const int o = (int)(i / C), c = (int)(i - (long long)o * C);
-    for (int t = 0; t < ntaps; ++t) {
-      float acc = 0.f;
-      for (int s = 0; s < nsplit; ++s) acc += ws[(((size_t)s * ntaps + t) * Opad + o) * Cpad + c];
-      const size_t di = (size_t)i * ntaps + t;
-      if (mask) acc *= mask[di];
-      dw[di] = accumulate ? dw[di] + acc : acc;
-    }
-  }
-}
-
 // Large filter banks, few splits: a warp owns 32 consecutive input channels of one filter for ALL taps.  Per tap the
 // lanes read one coalesced 128-byte run of every split; the taps * 32 results — which are contiguous in dW's [O, C, kh, kw]
-// layout — go through shared memory so that the mask read and the dW write are coalesced runs as well (the kernel above
-// writes 36-byte pieces 36 bytes apart and took 75 us for the 190 MB of the 1280 -> 1024 layer).
+// layout — go through shared memory so that the mask read and the dW write are coalesced runs as well (one thread per
+// (o, c) writing all taps wrote 36-byte pieces 36 bytes apart and took 75 us for the 190 MB of the 1280 -> 1024 layer).
 template <int TAPS>
 __global__ void __launch_bounds__(256) wgrad_reduce_rows_kernel(const float* __restrict__ ws, int nsplit, int Opad, int Cpad,
                                                                 int O, int C, const float* __restrict__ mask,
@@ -333,8 +317,11 @@ __global__ void __launch_bounds__(256) wgrad_reduce_small_kernel(const float* __
   }
 }
 
+// Reduction kernel of the split partial tiles (the numbering is the one mc_conv_wgrad_plan reports).
+enum WgradReduce { RED_ROWS9 = 1, RED_ROWS1 = 2, RED_SMALL1 = 3, RED_SMALL4 = 4, RED_SMALL8 = 5 };
+
 struct WgradPlan {
-  int block_n, nb64, n_tiles, m_tiles, ntaps, num_kb, nsplit, stages, tmem_cols, Opad, Cpad, share3, merge3;
+  int block_n, nb64, n_tiles, m_tiles, ntaps, num_kb, nsplit, stages, tmem_cols, Opad, Cpad, share3, merge3, reduce;
   size_t smem_bytes, ws_bytes;
 };
 
@@ -383,6 +370,11 @@ int plan_wgrad(WgradPlan* pl, int B, int H, int W, int C, int O, int ksize) {
   while (tc < (pl->merge3 ? 192 : (pl->share3 ? 3 : 1) * pl->block_n)) tc <<= 1;
   pl->tmem_cols = tc;
   pl->ws_bytes = (size_t)nsplit * pl->ntaps * pl->Opad * pl->Cpad * sizeof(float);
+  // few outputs, many splits: parallel over taps and split groups; otherwise a warp per 32 channels of a filter
+  if ((long long)O * C < 65536 && nsplit > 1)
+    pl->reduce = nsplit >= 32 ? RED_SMALL8 : nsplit >= 8 ? RED_SMALL4 : RED_SMALL1;
+  else
+    pl->reduce = pl->ntaps == 9 ? RED_ROWS9 : RED_ROWS1;
   return 0;
 }
 
@@ -393,6 +385,24 @@ extern "C" size_t mc_workspace_bytes_conv_wgrad(int B, int H, int W, int C, int 
   if (B <= 0 || H <= 0 || W <= 0 || C <= 0 || O <= 0 || (ksize != 1 && ksize != 3)) return 0;
   if (plan_wgrad(&pl, B, H, W, C, O, ksize)) return 0;
   return pl.ws_bytes;
+}
+
+extern "C" int mc_conv_wgrad_plan(int B, int H, int W, int C, int O, int ksize, int info[8]) {
+  MC_CHECK_ARG(info != nullptr, "mc_conv_wgrad_plan: null info");
+  MC_CHECK_ARG(ksize == 1 || ksize == 3, "mc_conv_wgrad_plan: ksize must be 1 or 3 (got %d)", ksize);
+  MC_CHECK_ARG(B > 0 && H > 0 && W > 0 && C > 0 && O > 0, "mc_conv_wgrad_plan: bad dims");
+  WgradPlan pl;
+  const int rc = plan_wgrad(&pl, B, H, W, C, O, ksize);
+  if (rc) return rc;
+  info[0] = pl.nsplit;
+  info[1] = pl.m_tiles;
+  info[2] = pl.n_tiles;
+  info[3] = pl.block_n;
+  info[4] = pl.share3;
+  info[5] = pl.merge3;
+  info[6] = pl.reduce;
+  info[7] = pl.num_kb;
+  return 0;
 }
 
 extern "C" int mc_conv_wgrad(const void* d_a, int lda, int C, const void* d_dz, int ld_dz, int O, int B, int H, int W,
@@ -450,37 +460,27 @@ extern "C" int mc_conv_wgrad(const void* d_a, int lda, int C, const void* d_dz, 
   const int grid = pl.m_tiles * pl.n_tiles * (pl.share3 ? 3 : pl.ntaps) * pl.nsplit;
   conv_wgrad_tcgen05_kernel<<<grid, NUM_THREADS, pl.smem_bytes, stream>>>(tm_dz, tm_a, p);
   MC_LAUNCH_CHECK("conv_wgrad_tcgen05_kernel");
-  long long tot = (long long)O * C;
-  if (tot < 65536 && pl.nsplit > 1) {
-    // few outputs, many splits: parallel over taps and split groups
-    const long long items = (long long)pl.ntaps * O * ((C + 31) / 32);
-    if (pl.nsplit >= 32) {
-      wgrad_reduce_small_kernel<8><<<(unsigned)items, 256, 0, stream>>>(p.ws, pl.nsplit, pl.ntaps, pl.Opad, pl.Cpad, O, C,
-                                                                        d_mask, d_dw, accumulate);
-    } else if (pl.nsplit >= 8) {
-      wgrad_reduce_small_kernel<4><<<(unsigned)((items + 1) / 2), 256, 0, stream>>>(p.ws, pl.nsplit, pl.ntaps, pl.Opad,
-                                                                                    pl.Cpad, O, C, d_mask, d_dw, accumulate);
-    } else {
-      wgrad_reduce_small_kernel<1><<<(unsigned)((items + 7) / 8), 256, 0, stream>>>(p.ws, pl.nsplit, pl.ntaps, pl.Opad,
-                                                                                    pl.Cpad, O, C, d_mask, d_dw, accumulate);
-    }
-    MC_LAUNCH_CHECK("wgrad_reduce_small_kernel");
-    return 0;
-  }
-  if (pl.ntaps == 9 || pl.ntaps == 1) {
+  if (pl.reduce == RED_ROWS9 || pl.reduce == RED_ROWS1) {
     const long long items = (long long)O * ((C + 31) / 32);
     const unsigned g = (unsigned)((items + 7) / 8);
-    if (pl.ntaps == 9)
+    if (pl.reduce == RED_ROWS9)
       wgrad_reduce_rows_kernel<9><<<g, 256, 0, stream>>>(p.ws, pl.nsplit, pl.Opad, pl.Cpad, O, C, d_mask, d_dw, accumulate);
     else
       wgrad_reduce_rows_kernel<1><<<g, 256, 0, stream>>>(p.ws, pl.nsplit, pl.Opad, pl.Cpad, O, C, d_mask, d_dw, accumulate);
     MC_LAUNCH_CHECK("wgrad_reduce_rows_kernel");
     return 0;
   }
-  int rgrid = (int)((tot + 255) / 256);
-  if (rgrid > mc_num_sms() * 8) rgrid = mc_num_sms() * 8;
-  wgrad_reduce_kernel<<<rgrid, 256, 0, stream>>>(p.ws, pl.nsplit, pl.ntaps, pl.Opad, pl.Cpad, O, C, d_mask, d_dw,
-                                                 accumulate);
-  MC_LAUNCH_CHECK("wgrad_reduce_kernel");
+  const long long items = (long long)pl.ntaps * O * ((C + 31) / 32);
+  if (pl.reduce == RED_SMALL8) {
+    wgrad_reduce_small_kernel<8><<<(unsigned)items, 256, 0, stream>>>(p.ws, pl.nsplit, pl.ntaps, pl.Opad, pl.Cpad, O, C,
+                                                                      d_mask, d_dw, accumulate);
+  } else if (pl.reduce == RED_SMALL4) {
+    wgrad_reduce_small_kernel<4><<<(unsigned)((items + 1) / 2), 256, 0, stream>>>(p.ws, pl.nsplit, pl.ntaps, pl.Opad,
+                                                                                  pl.Cpad, O, C, d_mask, d_dw, accumulate);
+  } else {
+    wgrad_reduce_small_kernel<1><<<(unsigned)((items + 7) / 8), 256, 0, stream>>>(p.ws, pl.nsplit, pl.ntaps, pl.Opad,
+                                                                                  pl.Cpad, O, C, d_mask, d_dw, accumulate);
+  }
+  MC_LAUNCH_CHECK("wgrad_reduce_small_kernel");
   return 0;
 }

@@ -92,28 +92,20 @@ int mc_masked_residual(const float* const* h_w_ptrs, const float* const* h_mask_
 
 /* Step 1 (methods.py:43-44 / 64-65): d_values[off_l + o] = (sum_{c,h,w} w^2) / (C*kh*kw) in float32, with
  * NumPy's exact summation order (sequential over c, then h, then w for kh*kw>1; pairwise over c for 1x1).
- * Step 2 (methods.py:46-51): v /= sqrt(pairwise_sum(v^2)); v /= max(v), per layer, float32.
- * off_l = sum of O of the previous layers.                                                           */
+ * Step 2 (methods.py:46-51): v /= sqrt(pairwise_sum(v^2)); v /= max(v), per layer, float32 (up to 51,200 filters
+ * per layer).  off_l = sum of O of the previous layers.                                             */
 int mc_filter_values(const float* const* h_w_ptrs, const int* h_O, const int* h_C, const int* h_kh,
                      const int* h_kw, int nlayers, float* d_values, void* stream);
 
-/* Step 3 (methods.py:55): float64 np.percentile(values, perc), method 'linear':
- *   *d_thr = _lerp(sorted[k], sorted[min(k+1,n-1)], gamma) in float64.  n <= 65536.                 */
-int mc_filter_threshold(const float* d_values, int n, int64_t k, double gamma, double* d_thr,
-                        void* d_ws, size_t ws_bytes, void* stream);
-size_t mc_workspace_bytes_filter_threshold(int n);
-
-/* Step 4 (methods.py:75): d_keep[off_l+o] = !( (double)v < *d_thr ); full-shape masks (fp32 1/0 per weight)
- * are written when h_mask_ptrs != NULL.                                                              */
-int mc_filter_masks(const float* d_values, const double* d_thr, const int* h_O, const int* h_per_filter,
-                    int nlayers, float* const* h_mask_ptrs, uint8_t* d_keep, void* stream);
-
-/* The whole of quick_filter_prune (steps 1-4 above) in one call: d_values [sum O] float32, *d_thr float64,
- * d_keep [sum O] (may be NULL), full-shape masks (h_mask_ptrs may be NULL).  ONE cooperative launch: persistent blocks
- * take filter groups from an atomic queue (3x3 layers through a cp.async shared-memory ring), the block that completes
- * a layer normalises it, the block that completes the last layer selects the float64 percentile (bitwise binary
- * search on the bit patterns) and publishes threshold + keep flags, then every block fills masks.  (More than 28,416
- * filters: three launches.)  d_ws: mc_workspace_bytes_filter_prune() bytes, any content.                          */
+/* The whole of quick_filter_prune in one call.  Step 1 and 2 as above; step 3 (methods.py:55): *d_thr = float64
+ * np.percentile(values, perc), method 'linear': _lerp(sorted[k], sorted[min(k+1,n-1)], gamma); step 4 (methods.py:75):
+ * d_keep[off_l + o] = !((double)v < *d_thr) and full-shape masks (fp32 1/0 per weight).  d_values [sum O] float32,
+ * d_keep [sum O] (may be NULL), h_mask_ptrs may be NULL.  ONE cooperative launch: persistent blocks take filter groups
+ * from an atomic queue (3x3 layers through a cp.async shared-memory ring); the block that completes the last group
+ * normalises every layer, selects the percentile (counting rounds on the top byte of the bit patterns, then radix
+ * passes) and publishes threshold + keep flags while the other blocks pre-fill their masks; every block then fixes up
+ * its masks.  (More than 26,368 filters: three launches, up to 51,200.)  d_ws: mc_workspace_bytes_filter_prune()
+ * bytes, any content.                                                                                                 */
 int mc_filter_prune(const float* const* h_w_ptrs, const int* h_O, const int* h_C, const int* h_kh, const int* h_kw,
                     int nlayers, int64_t k, double gamma, float* d_values, double* d_thr,
                     float* const* h_mask_ptrs, uint8_t* d_keep, void* d_ws, size_t ws_bytes, void* stream);

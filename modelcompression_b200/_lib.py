@@ -61,10 +61,6 @@ _SIGNATURES = {
                                    c_void_p]),
     "mc_filter_values": (c_int, [POINTER(c_void_p), POINTER(c_int), POINTER(c_int), POINTER(c_int), POINTER(c_int),
                                  c_int, c_void_p, c_void_p]),
-    "mc_filter_threshold": (c_int, [c_void_p, c_int, c_int64, c_double, c_void_p, c_void_p, c_size_t, c_void_p]),
-    "mc_workspace_bytes_filter_threshold": (c_size_t, [c_int]),
-    "mc_filter_masks": (c_int, [c_void_p, c_void_p, POINTER(c_int), POINTER(c_int), c_int, POINTER(c_void_p),
-                                c_void_p, c_void_p]),
     "mc_filter_prune": (c_int, [POINTER(c_void_p), POINTER(c_int), POINTER(c_int), POINTER(c_int), POINTER(c_int), c_int,
                                 c_int64, c_double, c_void_p, c_void_p, POINTER(c_void_p), c_void_p, c_void_p, c_size_t,
                                 c_void_p]),

@@ -34,90 +34,106 @@ struct LayerTable {
   int ntiled;
 };
 
-// NumPy pairwise sum of f(a[i]) for i in [0,n), a contiguous.  SQUARE: element is a[i]*a[i] rounded to fp32 first.
-template <bool SQUARE>
-__device__ float np_pairwise(const float* __restrict__ a, int n) {
-  auto el = [&](int i) -> float {
-    const float x = a[i];
-    return SQUARE ? __fmul_rn(x, x) : x;
-  };
-  if (n < 8) {
-    float res = 0.f;
-    for (int i = 0; i < n; ++i) res = __fadd_rn(res, el(i));
-    return res;
-  } else if (n <= 128) {
-    float r0 = el(0), r1 = el(1), r2 = el(2), r3 = el(3), r4 = el(4), r5 = el(5), r6 = el(6), r7 = el(7);
-    int i = 8;
-    for (; i < n - (n % 8); i += 8) {
-      r0 = __fadd_rn(r0, el(i + 0));
-      r1 = __fadd_rn(r1, el(i + 1));
-      r2 = __fadd_rn(r2, el(i + 2));
-      r3 = __fadd_rn(r3, el(i + 3));
-      r4 = __fadd_rn(r4, el(i + 4));
-      r5 = __fadd_rn(r5, el(i + 5));
-      r6 = __fadd_rn(r6, el(i + 6));
-      r7 = __fadd_rn(r7, el(i + 7));
-    }
-    float res = __fadd_rn(__fadd_rn(__fadd_rn(r0, r1), __fadd_rn(r2, r3)),
-                          __fadd_rn(__fadd_rn(r4, r5), __fadd_rn(r6, r7)));
-    for (; i < n; ++i) res = __fadd_rn(res, el(i));
-    return res;
-  } else {
-    int n2 = n / 2;
-    n2 -= n2 % 8;
-    return __fadd_rn(np_pairwise<SQUARE>(a, n2), np_pairwise<SQUARE>(a + n2, n - n2));
-  }
-}
-
-// ---- exact lane-parallel version of NumPy's pairwise sum -----------------------------------------------------
-// The recursion splits [0,n) into leaves of <= 128 elements (in order); a leaf is summed with 8 strided accumulators
-// (or sequentially when shorter than 8).  Leaves are independent, so lane L of a warp sums leaf L (L+32, ...), and
-// lane 0 then combines the leaf sums by replaying the recursion.  Same operations, same order per value => bit-exact.
-template <bool SQUARE>
-__device__ __forceinline__ float np_leaf_sum(const float* __restrict__ a, int n) {  // n <= 128
-  return np_pairwise<SQUARE>(a, n);
-}
-
-// walk the recursion; call f(leaf_index, start, len) for every leaf, in order.  Returns the number of leaves.
-template <typename F>
-__device__ __forceinline__ int np_for_each_leaf(int n, F f) {
-  int stack_start[24], stack_len[24];
-  int sp = 0, leaf = 0;
-  stack_start[0] = 0;
-  stack_len[0] = n;
-  sp = 1;
-  while (sp > 0) {
-    --sp;
-    const int st = stack_start[sp], ln = stack_len[sp];
-    if (ln <= 128) {
-      f(leaf, st, ln);
-      ++leaf;
-    } else {
+// ---- NumPy's pairwise sum of x^2, without recursion ---------------------------------------------------------------
+// NumPy's recursion over [0, n), walked in order with an explicit stack: a node longer than 128 is its left half
+// [0, n2) plus its right half, n2 = n/2 rounded down to a multiple of 8; a leaf is the current [st, st + ln).
+// next(s) adds the current leaf's sum s in the recursion's order and moves to the next leaf; it returns false after the
+// last leaf, and total then holds the sum.  Every leaf of an n > 128 walk is at least 64 long.
+struct NpWalk {
+  static constexpr int DEPTH = 25;  // levels of the recursion for any int n
+  int rln[DEPTH];                   // per open level: length of the right half, 0 once the walk is inside it
+  float lsum[DEPTH];                // ... and the sum of its left half
+  int sp = 0, st = 0, ln;
+  float total = 0.f;
+  __device__ explicit NpWalk(int n) : ln(n) { descend(); }
+  __device__ void descend() {
+    while (ln > 128) {
       int n2 = ln / 2;
       n2 -= n2 % 8;
-      // push right first so the left half is visited first (in-order)
-      stack_start[sp] = st + n2;
-      stack_len[sp] = ln - n2;
-      ++sp;
-      stack_start[sp] = st;
-      stack_len[sp] = n2;
-      ++sp;
+      rln[sp++] = ln - n2;
+      ln = n2;
     }
   }
-  return leaf;
+  __device__ bool next(float s) {
+    while (sp > 0 && rln[sp - 1] == 0) s = __fadd_rn(lsum[--sp], s);  // right halves complete: (left + right)
+    if (sp == 0) {
+      total = s;
+      return false;
+    }
+    lsum[sp - 1] = s;  // a left half is complete: its right half starts where the leaf ends
+    st += ln;
+    ln = rln[sp - 1];
+    rln[sp - 1] = 0;
+    descend();
+    return true;
+  }
+};
+
+// Leaf sums ls[0, ...) of a pairwise sum over n elements, combined in the recursion's order.
+__device__ float np_combine_leaves(const float* ls, int n) {
+  NpWalk w(n);
+  for (int i = 0; w.next(ls[i]); ++i) {}
+  return w.total;
 }
 
-// combine leaf sums in recursion order (replays the split; leaves are consumed in order)
-__device__ float np_combine_leaves(const float* __restrict__ leaf_sums, int n, int* next_leaf) {
-  if (n <= 128) return leaf_sums[(*next_leaf)++];
-  int n2 = n / 2;
-  n2 -= n2 % 8;
-  const float l = np_combine_leaves(leaf_sums, n2, next_leaf);
-  const float r = np_combine_leaves(leaf_sums, n - n2, next_leaf);
-  return __fadd_rn(l, r);
+// NumPy's pairwise sum of a[i]^2 over one leaf (n <= 128) by an 8-lane group: lane j = lane & 7 runs accumulator j, the
+// xor-1/2/4 butterfly performs ((r0+r1)+(r2+r3))+((r4+r5)+(r6+r7)) (fp add is commutative), then the sequential tail.
+// All 32 lanes call it, each group with its own leaf (n = 0: none); the result is valid in every lane of the group.
+__device__ __forceinline__ float group_leaf_sumsq(const float* a, int n) {
+  const int j = threadIdx.x & 7;
+  const int body = n - (n % 8);
+  float r = 0.f;
+  if (n >= 8) {
+    float x = a[j];
+    r = __fmul_rn(x, x);
+    for (int i = 8; i < body; i += 8) {
+      x = a[i + j];
+      r = __fadd_rn(r, __fmul_rn(x, x));
+    }
+  }
+  float t = __fadd_rn(r, __shfl_xor_sync(0xffffffffu, r, 1));
+  t = __fadd_rn(t, __shfl_xor_sync(0xffffffffu, t, 2));
+  t = __fadd_rn(t, __shfl_xor_sync(0xffffffffu, t, 4));
+  float sum = n >= 8 ? t : 0.f;
+  for (int i = n >= 8 ? body : 0; i < n; ++i) sum = __fadd_rn(sum, __fmul_rn(a[i], a[i]));
+  return sum;
 }
 
-constexpr int MAX_LEAVES = 128;  // leaves are >= 57 long once n > 128
+// NumPy's pairwise sum of a[i]^2 over [0, n) by one warp, bit-exact: one walk hands out the leaves four at a time
+// (group q of 8 lanes sums the q-th), a second walk combines their sums in the recursion's order.  Result in every lane.
+// n = 128 * L with L = 2^k <= 128 (and n <= 128) skips the walks: the recursion halves exactly, so the leaves are
+// [128 i, 128 i + 128) and their sums combine as a balanced tree, within a group of four by shuffles and across the
+// groups by lane (group b sits in lane b).
+__device__ float warp_pairwise_sumsq(const float* a, int n) {
+  const int lane = threadIdx.x & 31, lq = lane >> 3;
+  const int L = n <= 128 ? 1 : n / 128;
+  if (n <= 128 || (n % 128 == 0 && (L & (L - 1)) == 0 && L <= 128)) {
+    float mine = 0.f;
+    for (int b = 0; 4 * b < L; ++b) {
+      const int leaf = 4 * b + lq;
+      float t = group_leaf_sumsq(a + 128 * leaf, leaf < L ? (n < 128 ? n : 128) : 0);
+      if (L >= 2) t = __fadd_rn(t, __shfl_xor_sync(0xffffffffu, t, 8));
+      if (L >= 4) t = __fadd_rn(t, __shfl_xor_sync(0xffffffffu, t, 16));
+      if (lane == b) mine = t;
+    }
+    for (int o = 1; o < L / 4; o <<= 1) mine = __fadd_rn(mine, __shfl_xor_sync(0xffffffffu, mine, o));
+    __syncwarp();
+    return __shfl_sync(0xffffffffu, mine, 0);
+  }
+  NpWalk leaves(n), sums(n);
+  for (bool more = true; more;) {  // every lane walks the same leaves: the loop is warp-uniform
+    int st = 0, ln = 0, cnt = 0;
+    for (; cnt < 4 && more; ++cnt) {
+      if (cnt == lq) { st = leaves.st; ln = leaves.ln; }
+      more = leaves.next(0.f);
+    }
+    const float s = group_leaf_sumsq(a + st, ln);
+    for (int q = 0; q < cnt; ++q) sums.next(__shfl_sync(0xffffffffu, s, 8 * q));
+  }
+  __syncwarp();  // every lane's reads of a are done before the caller overwrites it
+  return sums.total;
+}
+
 constexpr int ROW_MAX = 2048;     // 1x1 rows up to this many channels are staged in shared memory (warp path)
 
 // Raw per-filter sums.  taps>1: one thread per (filter, tap) runs the sequential-in-c chain (loads are issued 32 deep
@@ -127,7 +143,7 @@ constexpr int SS_THREADS = 288;  // multiple of 9 and of 32
 
 template <int NT>
 __device__ void sumsq_generic_block(const LayerTable& lt, int gblk, float* __restrict__ values, float* s_tap,
-                                    float (*s_leaf)[MAX_LEAVES]) {
+                                    float* s_rows /*[NT / 32][ROW_MAX]*/) {
   const int gt = gblk * NT + threadIdx.x;  // global thread slot (blocks never straddle layers)
   int l = 0;
   while (l + 1 < lt.nlayers && gt >= lt.toff[l + 1]) ++l;
@@ -135,72 +151,24 @@ __device__ void sumsq_generic_block(const LayerTable& lt, int gblk, float* __res
   const int taps = lt.taps[l], C = lt.C[l], O = lt.O[l];
   const float* __restrict__ w = lt.w[l];
   if (taps == 1) {
-    // one WARP per filter.  The row (C floats, contiguous) is staged in shared memory with ONE round of coalesced
-    // loads; the leaves of NumPy's pairwise recursion are then summed four at a time, lane = (leaf, accumulator):
-    // a leaf of n >= 8 elements is 8 strided chains r[j] += a[i+j], combined ((r0+r1)+(r2+r3))+((r4+r5)+(r6+r7)) —
-    // the xor-butterfly does exactly these additions (fp add is commutative) — plus a sequential tail.
-    const int o = local >> 5, lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
+    // one WARP per filter.  A row (C floats, contiguous) of up to ROW_MAX channels is first staged in shared memory
+    // with ONE round of coalesced loads; a wider row is summed straight from global memory.
+    const int o = local >> 5, lane = threadIdx.x & 31;
     if (o >= O) return;  // whole warp
     const float* a = w + (long long)o * C;
-    float* ls = s_leaf[wib];                                    // [MAX_LEAVES] leaf sums
-    int* linfo = reinterpret_cast<int*>(s_leaf[NT / 32]) + wib * 2 * MAX_LEAVES;  // (start, len) per leaf
-    float* srow = reinterpret_cast<float*>(s_leaf[NT / 32]) + (NT / 32) * 2 * MAX_LEAVES + wib * ROW_MAX;
     if (C <= ROW_MAX) {
+      float* srow = s_rows + (threadIdx.x >> 5) * ROW_MAX;
       if ((C & 3) == 0) {
         const float4* a4 = reinterpret_cast<const float4*>(a);
         for (int i = lane; i < C / 4; i += 32) reinterpret_cast<float4*>(srow)[i] = ld_stream_f4(a4 + i);
       } else {
         for (int i = lane; i < C; i += 32) srow[i] = a[i];
       }
-      int nleaves = 0;
-      if (lane == 0) {
-        nleaves = np_for_each_leaf(C, [&](int leaf, int st, int ln) {
-          linfo[2 * leaf] = st;
-          linfo[2 * leaf + 1] = ln;
-        });
-      }
-      nleaves = __shfl_sync(0xffffffffu, nleaves, 0);
       __syncwarp();
-      const int lq = lane >> 3, j = lane & 7;
-      for (int g0 = 0; g0 < nleaves; g0 += 4) {
-        const int leaf = g0 + lq;
-        const bool have = leaf < nleaves;
-        const int st = have ? linfo[2 * leaf] : 0, ln = have ? linfo[2 * leaf + 1] : 0;
-        float res = 0.f;
-        if (ln >= 8) {
-          float x = srow[st + j];
-          float r = __fmul_rn(x, x);
-          const int body = ln - (ln % 8);
-          for (int i = 8; i < body; i += 8) {
-            x = srow[st + i + j];
-            r = __fadd_rn(r, __fmul_rn(x, x));
-          }
-          res = r;
-        }
-        // all 32 lanes take part in the butterfly (leaves shorter than 8 ignore its result)
-        float t = __fadd_rn(res, __shfl_xor_sync(0xffffffffu, res, 1));
-        t = __fadd_rn(t, __shfl_xor_sync(0xffffffffu, t, 2));
-        t = __fadd_rn(t, __shfl_xor_sync(0xffffffffu, t, 4));
-        if (have && j == 0) {
-          float sum;
-          int i;
-          if (ln >= 8) { sum = t; i = ln - (ln % 8); } else { sum = 0.f; i = 0; }
-          for (; i < ln; ++i) {
-            const float x = srow[st + i];
-            sum = __fadd_rn(sum, __fmul_rn(x, x));
-          }
-          ls[leaf] = sum;
-        }
-      }
-      __syncwarp();
-      if (lane == 0) {
-        int next = 0;
-        const float sres = np_combine_leaves(ls, C, &next);
-        values[lt.voff[l] + o] = __fdiv_rn(sres, (float)C);
-      }
-    } else if (lane == 0) {
-      values[lt.voff[l] + o] = __fdiv_rn(np_pairwise<true>(a, C), (float)C);
+      a = srow;
     }
+    const float s = warp_pairwise_sumsq(a, C);
+    if (lane == 0) values[lt.voff[l] + o] = __fdiv_rn(s, (float)C);
     return;
   }
   // blocks hold whole filters: fpb filters x taps threads, the remaining threads of the block idle
@@ -337,47 +305,55 @@ __global__ void __launch_bounds__(SS_THREADS) filter_sumsq_kernel(const LayerTab
     if (item >= first_wave) item = first_wave + (n_tiled - 1 - item);
     sumsq_tiled_block<TL_F, TL_STAGES>(lt, item, values, reinterpret_cast<float4*>(dsm), s_tap);
   } else {
-    sumsq_generic_block<SS_THREADS>(lt, (int)blockIdx.x - n_tiled, values, s_tap, reinterpret_cast<float(*)[MAX_LEAVES]>(dsm));
+    sumsq_generic_block<SS_THREADS>(lt, (int)blockIdx.x - n_tiled, values, s_tap, reinterpret_cast<float*>(dsm));
   }
 }
-constexpr size_t SUMSQ_SMEM = TL_STAGES * TL_TILE4 * sizeof(float4);  // 113,664 B (the generic path needs 4.6 KB of it)
+constexpr size_t SUMSQ_SMEM = TL_STAGES * TL_TILE4 * sizeof(float4);  // 113,664 B
+static_assert((size_t)(SS_THREADS / 32) * ROW_MAX * sizeof(float) <= SUMSQ_SMEM, "1x1 rows must fit the ring");
 
-// One block per layer: v /= sqrt(pairwise(v^2)); v /= max(v).  v is staged in shared memory so the serial pairwise
-// recursion of thread 0 runs at shared-memory latency.
-constexpr int NORM_SMEM = 8192;
-__global__ void __launch_bounds__(256) filter_norm_kernel(const LayerTable lt, float* __restrict__ values) {
-  __shared__ float s_v[NORM_SMEM];
-  __shared__ float s_norm;
-  __shared__ float s_red[256];
-  const int l = blockIdx.x;
-  const int O = lt.O[l];
-  float* v = values + lt.voff[l];
-  const bool staged = O <= NORM_SMEM;
-  if (staged)
-    for (int o = threadIdx.x; o < O; o += 256) s_v[o] = v[o];
-  __syncthreads();
-  if (threadIdx.x == 0) s_norm = __fsqrt_rn(np_pairwise<true>(staged ? s_v : v, O));
-  __syncthreads();
-  const float nrm = s_norm;
-  float mx = -INFINITY;
-  for (int o = threadIdx.x; o < O; o += 256) {
-    const float x = __fdiv_rn(staged ? s_v[o] : v[o], nrm);
-    if (staged) s_v[o] = x; else v[o] = x;
-    mx = fmaxf(mx, x);
-  }
-  s_red[threadIdx.x] = mx;
-  __syncthreads();
-  for (int s = 128; s > 0; s >>= 1) {
-    if (threadIdx.x < s) s_red[threadIdx.x] = fmaxf(s_red[threadIdx.x], s_red[threadIdx.x + s]);
+// ---- normalise, select, keep, fill: the steps after the sums, shared by the one-launch and three-launch paths ----------
+// methods.py:46-51 for one layer's values v[0, O) by NT threads: a warp (NT = 32) or the whole block.  v /= sqrt(sum of
+// v^2 in NumPy's pairwise order, run by the first warp), then v /= max(v).  The max of values >= 0 is the max of their
+// bit patterns, and a NaN's pattern (sign cleared) beats every number's, so a NaN wins as in np.max.  s_red: NT / 32 + 1
+// words (block only).  Returns whether the layer holds a NaN, uniform over the NT threads.
+template <int NT>
+__device__ bool normalise_layer(float* v, int O, unsigned int* s_red) {
+  constexpr int WARPS = NT / 32;
+  const int t = threadIdx.x % NT, lane = threadIdx.x & 31;
+  float nrm;
+  if constexpr (WARPS == 1) {
+    nrm = __fsqrt_rn(warp_pairwise_sumsq(v, O));
+  } else {
+    if (t < 32) {
+      const float s = warp_pairwise_sumsq(v, O);
+      if (t == 0) s_red[WARPS] = __float_as_uint(__fsqrt_rn(s));
+    }
     __syncthreads();
+    nrm = __uint_as_float(s_red[WARPS]);
   }
-  mx = s_red[0];
-  for (int o = threadIdx.x; o < O; o += 256) v[o] = __fdiv_rn(staged ? s_v[o] : v[o], mx);
+  unsigned int mb = 0u;
+  for (int i = t; i < O; i += NT) {
+    const float x = __fdiv_rn(v[i], nrm);
+    v[i] = x;
+    mb = max(mb, __float_as_uint(x) & 0x7fffffffu);
+  }
+  mb = __reduce_max_sync(0xffffffffu, mb);
+  if constexpr (WARPS > 1) {
+    if (lane == 0) s_red[t >> 5] = mb;
+    __syncthreads();
+    mb = __reduce_max_sync(0xffffffffu, lane < WARPS ? s_red[lane] : 0u);
+  }
+  const float mx = __uint_as_float(mb);
+  int nan = 0;
+  for (int i = t; i < O; i += NT) {
+    const float x = __fdiv_rn(v[i], mx);
+    v[i] = x;
+    nan |= x != x;
+  }
+  if constexpr (WARPS == 1) return __any_sync(0xffffffffu, nan) != 0;
+  else return __syncthreads_or(nan) != 0;
 }
 
-// Single-block radix select of TWO ranks at once over n non-negative floats (8 bits per pass, 4 passes), then NumPy's
-// float64 _lerp.  Each pass keeps one 256-bin histogram per rank (elements matching that rank's prefix); warp 0 / warp 1
-// locate the bins with shuffle prefix sums.
 __device__ __forceinline__ void warp_find_bin(const unsigned int* hist, unsigned int rank, unsigned int* out_bin,
                                               unsigned int* out_rem) {
   const int lane = threadIdx.x & 31;
@@ -405,410 +381,14 @@ __device__ __forceinline__ void warp_find_bin(const unsigned int* hist, unsigned
   }
 }
 
-__global__ void __launch_bounds__(1024) filter_threshold_kernel(const float* __restrict__ v, int n, long long k,
-                                                                double gamma, double* __restrict__ thr) {
-  __shared__ unsigned int s_hist[2][256];
-  __shared__ unsigned int s_bin[2], s_rem[2];
-  __shared__ int s_nan;
-  if (threadIdx.x == 0) s_nan = 0;
-  __syncthreads();
-  for (int i = threadIdx.x; i < n; i += blockDim.x)
-    if (v[i] != v[i]) s_nan = 1;  // np.percentile returns nan if any value is nan (an all-zero layer gives 0/0)
-  __syncthreads();
-  if (s_nan) {
-    if (threadIdx.x == 0) *thr = __longlong_as_double(0x7ff8000000000000LL);
-    return;
-  }
-  const long long k1 = (k + 1 < n) ? k + 1 : (long long)n - 1;
-  unsigned int rank[2] = {(unsigned int)k, (unsigned int)k1};
-  unsigned int prefix[2] = {0, 0}, mask = 0;
-  for (int shift = 24; shift >= 0; shift -= 8) {
-    for (int i = threadIdx.x; i < 512; i += blockDim.x) (&s_hist[0][0])[i] = 0;
-    __syncthreads();
-    for (int i = threadIdx.x; i < n; i += blockDim.x) {
-      const unsigned int key = __float_as_uint(v[i]);
-      const unsigned int d = (key >> shift) & 255u;
-      if ((key & mask) == prefix[0]) atomicAdd(&s_hist[0][d], 1u);
-      if ((key & mask) == prefix[1]) atomicAdd(&s_hist[1][d], 1u);
-    }
-    __syncthreads();
-    const int wid = threadIdx.x >> 5;
-    if (wid < 2) warp_find_bin(s_hist[wid], rank[wid], &s_bin[wid], &s_rem[wid]);
-    __syncthreads();
-    prefix[0] |= s_bin[0] << shift;
-    prefix[1] |= s_bin[1] << shift;
-    rank[0] = s_rem[0];
-    rank[1] = s_rem[1];
-    mask |= 255u << shift;
-    __syncthreads();
-  }
-  if (threadIdx.x == 0) {
-    const double a = (double)__uint_as_float(prefix[0]);
-    const double b = (double)__uint_as_float(prefix[1]);
-    const double diff = __dsub_rn(b, a);
-    double r = __dadd_rn(a, __dmul_rn(diff, gamma));
-    if (gamma >= 0.5) r = __dsub_rn(b, __dmul_rn(diff, __dsub_rn(1.0, gamma)));
-    *thr = r;
-  }
-}
 
-// ---- finish: per-layer normalisation, then (last block to arrive) the float64 percentile and the keep flags -------
-// Order statistics by bitwise binary search on the fp32 bit pattern (values are >= 0, so the pattern is monotone):
-// 31 rounds of "count keys below prefix|bit", both ranks at once, keys in shared memory — ~4 us for 10,461 values,
-// where a shared-memory radix histogram serialises on the few distinct high digits of values that all lie in (0,1].
-constexpr int FIN_THREADS = 1024;
-// Leaves of NumPy's pairwise recursion over one layer's values: at most 512 for the <= 51,200 values the kernel takes
-// (mc_filter_prune rejects more).  Every layer goes through the lane-parallel sum: thread 0 running the recursion itself
-// overflowed the 1 KB device stack on a layer of 27,000 filters.
-constexpr int FIN_MAX_LEAVES = 512;
-
-__device__ void block_count2(unsigned int c0, unsigned int c1, unsigned int* s_red /*[64]*/, unsigned int* out0,
-                             unsigned int* out1) {
-  for (int o = 16; o > 0; o >>= 1) {
-    c0 += __shfl_xor_sync(0xffffffffu, c0, o);
-    c1 += __shfl_xor_sync(0xffffffffu, c1, o);
-  }
-  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-  if (lane == 0) { s_red[wid] = c0; s_red[32 + wid] = c1; }
-  __syncthreads();
-  if (wid == 0) {
-    unsigned int a = s_red[lane], b = s_red[32 + lane];  // FIN_THREADS / 32 == 32 warps
-    for (int o = 16; o > 0; o >>= 1) {
-      a += __shfl_xor_sync(0xffffffffu, a, o);
-      b += __shfl_xor_sync(0xffffffffu, b, o);
-    }
-    if (lane == 0) { s_red[0] = a; s_red[32] = b; }
-  }
-  __syncthreads();
-  *out0 = s_red[0];
-  *out1 = s_red[32];
-  __syncthreads();
-}
-
-__global__ void __launch_bounds__(FIN_THREADS) filter_finish_kernel(const LayerTable lt, float* __restrict__ values,
-                                                                    long long k, double gamma, double* __restrict__ thr,
-                                                                    uint8_t* __restrict__ keep,
-                                                                    unsigned int* __restrict__ ticket) {
-  extern __shared__ __align__(16) unsigned char dsm[];
-  float* s_v = reinterpret_cast<float*>(dsm);  // max(O_l, n) floats
-  __shared__ float s_norm;
-  __shared__ float s_leaf[FIN_MAX_LEAVES];
-  __shared__ unsigned int s_red[64];
-  __shared__ unsigned int s_last;
-  const int l = blockIdx.x;
-  const int O = lt.O[l];
-  float* v = values + lt.voff[l];
-  unsigned long long* dbg = reinterpret_cast<unsigned long long*>(ticket) + 1;  // diagnostics: phase stamps of the last block
-  auto stamp = [&](int i) {
-    if (threadIdx.x == 0) { unsigned long long t; asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t)); dbg[i] = t; }
-  };
-  unsigned long long t_begin = 0;
-  if (threadIdx.x == 0) asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t_begin));
-  // ---- v /= sqrt(pairwise(v^2)); v /= max(v)   (methods.py:46-51)
-  for (int o = threadIdx.x; o < O; o += FIN_THREADS) s_v[o] = v[o];
-  __syncthreads();
-  if (threadIdx.x < 32) {  // lane-parallel replay of NumPy's pairwise recursion (leaves are independent)
-    const int lane = threadIdx.x;
-    np_for_each_leaf(O, [&](int leaf, int st, int ln) {
-      if ((leaf & 31) == lane) s_leaf[leaf] = np_leaf_sum<true>(s_v + st, ln);
-    });
-    __syncwarp();
-    if (lane == 0) {
-      int next = 0;
-      s_norm = __fsqrt_rn(np_combine_leaves(s_leaf, O, &next));
-    }
-  }
-  __syncthreads();
-  const float nrm = s_norm;
-  float mx = -INFINITY;
-  for (int o = threadIdx.x; o < O; o += FIN_THREADS) {
-    const float x = __fdiv_rn(s_v[o], nrm);
-    s_v[o] = x;
-    mx = fmaxf(mx, x);
-  }
-  {
-    unsigned int a, b;  // max of non-negative floats == max of their bit patterns; NaN (0/0) handled below
-    block_count2(0u, 0u, s_red, &a, &b);  // barrier only
-    for (int o = 16; o > 0; o >>= 1) mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o));
-    if ((threadIdx.x & 31) == 0) s_red[threadIdx.x >> 5] = __float_as_uint(mx);
-    __syncthreads();
-    if (threadIdx.x == 0) {
-      float m2 = -INFINITY;
-      for (int w2 = 0; w2 < FIN_THREADS / 32; ++w2) m2 = fmaxf(m2, __uint_as_float(s_red[w2]));
-      s_norm = m2;
-    }
-    __syncthreads();
-  }
-  mx = s_norm;
-  for (int o = threadIdx.x; o < O; o += FIN_THREADS) v[o] = __fdiv_rn(s_v[o], mx);
-  // ---- last block to finish computes the threshold over all layers
-  __threadfence();
-  __syncthreads();
-  if (threadIdx.x == 0) s_last = (atomicAdd(ticket, 1u) == gridDim.x - 1) ? 1u : 0u;
-  __syncthreads();
-  if (!s_last) return;
-  __threadfence();
-  if (threadIdx.x == 0) dbg[0] = t_begin;
-  stamp(1);
-  const int n = lt.voff[lt.nlayers];
-  unsigned int* s_k = reinterpret_cast<unsigned int*>(dsm);
-  unsigned int nan = 0;
-  for (int i = threadIdx.x; i < n; i += FIN_THREADS) {
-    const float x = __ldcg(values + i);
-    s_k[i] = __float_as_uint(x);
-    nan |= (x != x);
-  }
-  __syncthreads();
-  unsigned int nn, dummy;
-  block_count2(nan, 0u, s_red, &nn, &dummy);
-  if (nn) {  // np.percentile returns nan if any value is nan (an all-zero layer gives 0/0): nothing is < nan
-    if (threadIdx.x == 0) *thr = __longlong_as_double(0x7ff8000000000000LL);
-    if (keep)
-      for (int i = threadIdx.x; i < n; i += FIN_THREADS) keep[i] = 1;
-    return;
-  }
-  stamp(2);
-  const unsigned int r0 = (unsigned int)k, r1 = (unsigned int)((k + 1 < n) ? k + 1 : (long long)n - 1);
-  unsigned int p0 = 0, p1 = 0;
-  // The rounds run on ONE SM, so what they cost is warp-instructions issued (4 per clock), not latency: only the
-  // first SEL_THREADS threads take part (the others leave), keys sit in registers (n <= KPT*SEL_THREADS, else shared
-  // memory), the two ranks share one compare while their prefixes coincide, and the cross-warp sum is: redux -> one
-  // slot per warp -> ONE named barrier -> every warp adds the slots itself (slots alternate by round parity).
-  constexpr int SEL_THREADS = 512, SEL_WARPS = SEL_THREADS / 32, KPT = 24;
-  __shared__ unsigned int s_part[2][2][SEL_WARPS];
-  __syncthreads();  // s_k complete, NaN decision taken by everyone
-  if (threadIdx.x >= SEL_THREADS) return;
-  const bool in_regs = n <= KPT * SEL_THREADS;
-  unsigned int kreg[KPT];
-#pragma unroll
-  for (int u = 0; u < KPT; ++u) {
-    const int i = u * SEL_THREADS + threadIdx.x;
-    kreg[u] = (in_regs && i < n) ? s_k[i] : 0xffffffffu;  // padding never counts as "below"
-  }
-  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-  for (int bit = 30, r = 0; bit >= 0; --bit, ++r) {  // keys < 2^31
-    const unsigned int c0 = p0 | (1u << bit), c1 = p1 | (1u << bit);
-    const bool split = p0 != p1;  // block-uniform
-    unsigned int n0 = 0, n1 = 0;
-    if (in_regs) {
-#pragma unroll
-      for (int u = 0; u < KPT; ++u) n0 += kreg[u] < c0;
-      if (split) {
-#pragma unroll
-        for (int u = 0; u < KPT; ++u) n1 += kreg[u] < c1;
-      }
-    } else {
-      for (int i = threadIdx.x; i < n; i += SEL_THREADS) {
-        const unsigned int key = s_k[i];
-        n0 += key < c0;
-        n1 += key < c1;
-      }
-    }
-    n0 = __reduce_add_sync(0xffffffffu, n0);
-    if (split || !in_regs) n1 = __reduce_add_sync(0xffffffffu, n1);
-    if (lane == 0) {
-      s_part[r & 1][0][wid] = n0;
-      s_part[r & 1][1][wid] = n1;
-    }
-    asm volatile("bar.sync 1, %0;" ::"n"(SEL_THREADS) : "memory");
-    const unsigned int t0 = __reduce_add_sync(0xffffffffu, lane < SEL_WARPS ? s_part[r & 1][0][lane] : 0u);
-    unsigned int t1 = t0;
-    if (split || !in_regs) t1 = __reduce_add_sync(0xffffffffu, lane < SEL_WARPS ? s_part[r & 1][1][lane] : 0u);
-    if (t0 <= r0) p0 = c0;  // at most r0 keys below the candidate: the r0-th smallest is >= candidate
-    if (t1 <= r1) p1 = c1;
-  }
-  double t;
-  {
-    const double a = (double)__uint_as_float(p0);
-    const double b = (double)__uint_as_float(p1);
-    const double diff = __dsub_rn(b, a);
-    t = __dadd_rn(a, __dmul_rn(diff, gamma));
-    if (gamma >= 0.5) t = __dsub_rn(b, __dmul_rn(diff, __dsub_rn(1.0, gamma)));
-  }
-  stamp(3);
-  if (threadIdx.x == 0) *thr = t;
-  if (keep)
-    for (int i = threadIdx.x; i < n; i += SEL_THREADS) keep[i] = ((double)__uint_as_float(s_k[i]) < t) ? 0 : 1;
-  stamp(4);
-}
-
-__global__ void filter_keep_kernel(const float* __restrict__ v, int n, const double* __restrict__ thr,
-                                   uint8_t* __restrict__ keep) {
-  const double t = *thr;
-  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x)
-    keep[i] = ((double)v[i] < t) ? 0 : 1;
-}
-
-// one block per filter (grid-stride): constant fill of `per` floats, 128-bit stores on the aligned body
-__global__ void __launch_bounds__(256) filter_mask_fill_kernel(const LayerTable lt, const float* __restrict__ v,
-                                                               const double* __restrict__ thr) {
-  const double t = *thr;
-  const int nfilters = lt.voff[lt.nlayers];
-  for (int f = blockIdx.x; f < nfilters; f += gridDim.x) {
-    int l = 0;
-    while (l + 1 < lt.nlayers && f >= lt.voff[l + 1]) ++l;
-    const int o = f - lt.voff[l];
-    const int per = lt.C[l] * lt.taps[l];
-    const float val = ((double)v[f] < t) ? 0.f : 1.f;
-    float* m = lt.mask[l] + (long long)o * per;
-    // scalar head up to 16-byte alignment
-    int head = (int)(((16 - (reinterpret_cast<uintptr_t>(m) & 15)) & 15) >> 2);
-    if (head > per) head = per;
-    if ((int)threadIdx.x < head) m[threadIdx.x] = val;
-    const int body4 = (per - head) >> 2;
-    float4* m4 = reinterpret_cast<float4*>(m + head);
-    const float4 v4 = make_float4(val, val, val, val);
-    for (int i = threadIdx.x; i < body4; i += 256) st_stream_f4(m4 + i, v4);
-    const int tail0 = head + body4 * 4;
-    if ((int)threadIdx.x < per - tail0) m[tail0 + threadIdx.x] = val;
-  }
-}
-
-// ---- the whole of quick_filter_prune in ONE cooperative launch ------------------------------------------------------
-// Persistent blocks (2 per SM, all co-resident) take work items from an atomic queue: groups of FU_F filters of the 3x3
-// layers through a 6-stage cp.async ring, and the blocks of the generic path (1x1 layers) slotted in behind the long
-// items so that their latency-bound work does not form the tail.  Raw per-filter sums go to a scratch array.  When the
-// queue is empty EVERY block waits for the last item, pulls all raw sums (42 KB for Darknet-19) from L2 into shared
-// memory and redundantly runs the small serial part itself — per-layer normalisation in NumPy's pairwise order, then a
-// two-rank radix select for np.percentile — so nothing is exchanged between blocks after the sums and no block waits
-// for another one's result; it then writes its slice of the normalised values / keep flags and fills its share of the
-// masks.  Against three launches this removes two full drains + ramps of the grid and the single-block finish kernel
-// (~30 us of pure latency between the two bandwidth passes).
-constexpr int FU_THREADS = 160;  // 16 filters x 9 taps = 144 chain threads, rounded up to whole warps
-constexpr int FU_F = 16;
-constexpr int FU_STAGES = 6;
-constexpr size_t FU_SMEM = (size_t)FU_STAGES * FU_F * TL_ROW4 * sizeof(float4);  // 113,664 B: two blocks per SM
-constexpr int FU_AUX_BYTES = 8192;                                                // leaf table / histograms
-constexpr int FU_MAX_N = (int)((FU_SMEM - FU_AUX_BYTES) / sizeof(float));         // 26,368 filters
-static_assert((size_t)(FU_THREADS / 32) * MAX_LEAVES * 4 <= (size_t)FU_AUX_BYTES, "leaf sums must fit the aux region");
-
-struct FusedState {
-  unsigned int next_item;  // work queue
-  unsigned int pad0[31];
-  unsigned int items_done;
-  unsigned int pad1[31];
-  unsigned int flag;  // polled by idle blocks: its own 128-byte line
-  unsigned int pad2[31];
-  unsigned long long stamp[8];  // diagnostics (globaltimer ns): block 0 start, last block out of work, last block past the
-                                // wait, last block with thr, last block done
-};
-__device__ __forceinline__ void fused_stamp(FusedState* st, int i, bool max_over_blocks) {
-  unsigned long long t;
-  asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-  if (max_over_blocks) atomicMax(&st->stamp[i], t);
-  else st->stamp[i] = t;
-}
-
-__device__ __forceinline__ unsigned int ld_acquire_u32(const unsigned int* p) {
-  unsigned int v;
-  asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-  return v;
-}
-
-// All raw sums -> normalised values in shared memory (methods.py:43-51 for every layer), by one block.
-// s_val [n]; aux: leaf table (start, len) + leaf sums.  Returns true (block-uniform) if any value is NaN.
-template <int NT>
-__device__ bool fused_normalise_all(const LayerTable& lt, const float* __restrict__ raw, float* s_val, unsigned char* aux) {
-  const int n = lt.voff[lt.nlayers], nl = lt.nlayers;
-  const int tid = threadIdx.x;
-  float* s_lsum = reinterpret_cast<float*>(aux);  // [NT / 32][MAX_LEAVES] leaf sums, one row per warp
-  for (int i0 = 0; i0 < n; i0 += 16 * NT) {  // 16 independent L2 loads in flight per thread
-    float x[16];
-#pragma unroll
-    for (int u = 0; u < 16; ++u) {
-      const int i = i0 + u * NT + tid;
-      x[u] = i < n ? __ldcg(raw + i) : 0.f;
-    }
-#pragma unroll
-    for (int u = 0; u < 16; ++u) {
-      const int i = i0 + u * NT + tid;
-      if (i < n) s_val[i] = x[u];
-    }
-  }
-  __syncthreads();
-  // One warp per layer, start to finish (no block barrier inside).  ||v||: O <= 128 is one leaf of NumPy's pairwise
-  // recursion, O = 128 * 2^k splits into 2^k leaves of 128 combined as a balanced tree (the recursion halves exactly);
-  // a leaf is 8 strided accumulator chains combined ((r0+r1)+(r2+r3))+((r4+r5)+(r6+r7)) plus a sequential tail — lane =
-  // (leaf, accumulator), the xor-butterfly performs exactly those additions.  Any other O: lane 0 runs the recursion.
-  // Then x = v / ||v||, max(x) (a NaN wins, as np.max propagates it), v = x / max.
-  unsigned int nan = 0;
-  {
-    const int lane = tid & 31, wid = tid >> 5;
-    float* ls = s_lsum + wid * MAX_LEAVES;
-    for (int l = wid; l < nl; l += NT / 32) {
-      const int O = lt.O[l];
-      float* vv = s_val + lt.voff[l];
-      const int nleaf = O <= 128 ? 1 : O / 128;
-      const bool fast = O <= 128 || ((O % 128) == 0 && (nleaf & (nleaf - 1)) == 0 && nleaf <= MAX_LEAVES);
-      float nrm = 0.f;
-      if (fast) {
-        const int lq = lane >> 3, j = lane & 7;
-        for (int g0 = 0; g0 < nleaf; g0 += 4) {
-          const int leaf = g0 + lq;
-          const bool have = leaf < nleaf;
-          const int st = leaf * 128, ln = have ? (O <= 128 ? O : 128) : 0;
-          float r = 0.f;
-          if (ln >= 8) {
-            float x = vv[st + j];
-            r = __fmul_rn(x, x);
-            const int body = ln - (ln % 8);
-            for (int i = 8; i < body; i += 8) {
-              x = vv[st + i + j];
-              r = __fadd_rn(r, __fmul_rn(x, x));
-            }
-          }
-          float t = __fadd_rn(r, __shfl_xor_sync(0xffffffffu, r, 1));
-          t = __fadd_rn(t, __shfl_xor_sync(0xffffffffu, t, 2));
-          t = __fadd_rn(t, __shfl_xor_sync(0xffffffffu, t, 4));
-          if (have && j == 0) {
-            float sum;
-            int i;
-            if (ln >= 8) { sum = t; i = ln - (ln % 8); } else { sum = 0.f; i = 0; }
-            for (; i < ln; ++i) {
-              const float x = vv[st + i];
-              sum = __fadd_rn(sum, __fmul_rn(x, x));
-            }
-            ls[leaf] = sum;
-          }
-        }
-        __syncwarp();
-        for (int w2 = 1; w2 < nleaf; w2 <<= 1) {  // balanced tree: (L0+L1), (L2+L3), ... then pairs of those, ...
-          for (int i = lane * 2 * w2; i + w2 < nleaf; i += 64 * w2) ls[i] = __fadd_rn(ls[i], ls[i + w2]);
-          __syncwarp();
-        }
-        nrm = __fsqrt_rn(ls[0]);
-      } else {
-        if (lane == 0) ls[0] = __fsqrt_rn(np_pairwise<true>(vv, O));
-        __syncwarp();
-        nrm = ls[0];
-      }
-      __syncwarp();
-      unsigned int mb = 0u;
-      for (int i = lane; i < O; i += 32) {
-        const float x = __fdiv_rn(vv[i], nrm);
-        vv[i] = x;
-        mb = max(mb, __float_as_uint(x) & 0x7fffffffu);
-      }
-#pragma unroll
-      for (int o = 16; o > 0; o >>= 1) mb = max(mb, __shfl_xor_sync(0xffffffffu, mb, o));
-      const float mx = __uint_as_float(mb);
-      for (int i = lane; i < O; i += 32) {
-        const float v = __fdiv_rn(vv[i], mx);
-        vv[i] = v;
-        nan |= (v != v);
-      }
-    }
-  }
-  return __syncthreads_or((int)nan) != 0;
-}
-
-// np.percentile over the n normalised values in shared memory: the order statistics k and k+1 (both at once), then
+// np.percentile over the n normalised values in shared memory, by the NT threads of the block: the order statistics k and k+1 (both at once), then
 // NumPy's float64 _lerp.  The values of a layer crowd into a handful of exponents, so the top byte of the bit patterns
 // is resolved by 7 rounds of counting "keys below prefix|bit" (a shared-memory histogram would serialise 32-way on
 // those few bins: measured 10 us for that pass alone); the three lower bytes, which are well spread, by 8-bit radix
 // passes with shared-memory atomics (one histogram per rank).  Every thread returns the threshold.
 template <int NT>
-__device__ double fused_select(const float* s_val, int n, long long k, double gamma, unsigned int* s_hist /*[2][256]*/,
+__device__ double select_percentile(const float* s_val, int n, long long k, double gamma, unsigned int* s_hist /*[2][256]*/,
                                unsigned int* s_bin /*[4]*/) {
   const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
   constexpr int WARPS = NT / 32;
@@ -886,6 +466,147 @@ __device__ double fused_select(const float* s_val, int n, long long k, double ga
   return r;
 }
 
+// methods.py:75: a filter is pruned when its value is below the float64 threshold (nothing is below a NaN threshold).
+__device__ __forceinline__ bool kept(float v, double thr) { return !((double)v < thr); }
+
+// One filter's mask (per floats at m) set to val by the NT threads of a block: scalar head up to 16-byte alignment,
+// 128-bit streaming stores, scalar tail.
+template <int NT>
+__device__ void fill_filter(float* m, int per, float val) {
+  const int tid = threadIdx.x;
+  int head = (int)(((16 - (reinterpret_cast<uintptr_t>(m) & 15)) & 15) >> 2);
+  if (head > per) head = per;
+  if (tid < head) m[tid] = val;
+  const int body4 = (per - head) >> 2;
+  float4* m4 = reinterpret_cast<float4*>(m + head);
+  const float4 v4 = make_float4(val, val, val, val);
+  for (int i = tid; i < body4; i += NT) st_stream_f4(m4 + i, v4);
+  const int tail0 = head + body4 * 4;
+  if (tid < per - tail0) m[tail0 + tid] = val;
+}
+
+// ---- three launches (sums, finish, mask fill): more filters than the fused kernel holds, and the values alone -------
+// One block per layer normalises it.  With k >= 0 the last block to finish then selects the float64 percentile over all
+// n values and writes the threshold and the keep flags; with k < 0 it stops at the values (mc_filter_values).
+constexpr int FIN_THREADS = 1024;
+constexpr size_t FIN_MAX_SMEM = 200 * 1024;  // max(O_l, n) floats: up to 51,200 filters
+
+__global__ void __launch_bounds__(FIN_THREADS) filter_finish_kernel(const LayerTable lt, float* __restrict__ values,
+                                                                    long long k, double gamma, double* __restrict__ thr,
+                                                                    uint8_t* __restrict__ keep,
+                                                                    unsigned int* __restrict__ ticket) {
+  extern __shared__ __align__(16) unsigned char dsm[];
+  float* s_v = reinterpret_cast<float*>(dsm);  // max(O_l, n) floats
+  __shared__ unsigned int s_red[FIN_THREADS / 32 + 1];
+  __shared__ unsigned int s_hist[512], s_bin[4];
+  __shared__ unsigned int s_last;
+  const int O = lt.O[blockIdx.x];
+  float* v = values + lt.voff[blockIdx.x];
+  for (int o = threadIdx.x; o < O; o += FIN_THREADS) s_v[o] = v[o];
+  __syncthreads();
+  normalise_layer<FIN_THREADS>(s_v, O, s_red);
+  for (int o = threadIdx.x; o < O; o += FIN_THREADS) v[o] = s_v[o];
+  if (k < 0) return;
+  __threadfence();
+  __syncthreads();
+  if (threadIdx.x == 0) s_last = (atomicAdd(ticket, 1u) == gridDim.x - 1) ? 1u : 0u;
+  __syncthreads();
+  if (!s_last) return;
+  __threadfence();
+  const int n = lt.voff[lt.nlayers];
+  int nan = 0;
+  for (int i = threadIdx.x; i < n; i += FIN_THREADS) {
+    const float x = __ldcg(values + i);
+    s_v[i] = x;
+    nan |= x != x;
+  }
+  // np.percentile returns nan if any value is nan (an all-zero layer gives 0/0): nothing is < nan
+  const double t = __syncthreads_or(nan) ? __longlong_as_double(0x7ff8000000000000LL)
+                                         : select_percentile<FIN_THREADS>(s_v, n, k, gamma, s_hist, s_bin);
+  if (threadIdx.x == 0) *thr = t;
+  if (keep)
+    for (int i = threadIdx.x; i < n; i += FIN_THREADS) keep[i] = kept(s_v[i], t) ? 1 : 0;
+}
+
+// one block per filter (grid-stride)
+__global__ void __launch_bounds__(256) filter_mask_fill_kernel(const LayerTable lt, const float* __restrict__ v,
+                                                               const double* __restrict__ thr) {
+  const double t = *thr;
+  const int nfilters = lt.voff[lt.nlayers];
+  for (int f = blockIdx.x; f < nfilters; f += gridDim.x) {
+    int l = 0;
+    while (l + 1 < lt.nlayers && f >= lt.voff[l + 1]) ++l;
+    const int per = lt.C[l] * lt.taps[l];
+    fill_filter<256>(lt.mask[l] + (long long)(f - lt.voff[l]) * per, per, kept(v[f], t) ? 1.f : 0.f);
+  }
+}
+
+// ---- the whole of quick_filter_prune in ONE cooperative launch ------------------------------------------------------
+// Persistent blocks (2 per SM, all co-resident) take work items from an atomic queue: groups of FU_F filters of the 3x3
+// layers through a 6-stage cp.async ring, and the blocks of the generic path (1x1 layers) slotted in behind the long
+// items so that their latency-bound work does not form the tail.  Raw per-filter sums go to a scratch array.  The block
+// that completes the last item (the finisher) pulls all raw sums (42 KB for Darknet-19) from L2 into shared memory, runs
+// the serial part alone — per-layer normalisation in NumPy's pairwise order, then the two-rank select for
+// np.percentile — writes the values and keep flags and publishes the threshold through a flag.  The other blocks fill
+// their masks with the provisional value meanwhile and rewrite the filters that differ once the flag is up.  Against
+// three launches this removes two full drains + ramps of the grid (~30 us of pure latency between the two bandwidth
+// passes).
+constexpr int FU_THREADS = 160;  // 16 filters x 9 taps = 144 chain threads, rounded up to whole warps
+constexpr int FU_F = 16;
+constexpr int FU_STAGES = 6;
+constexpr size_t FU_SMEM = (size_t)FU_STAGES * FU_F * TL_ROW4 * sizeof(float4);  // 113,664 B: two blocks per SM
+constexpr int FU_AUX_BYTES = 8192;                                                // behind the values: histograms
+constexpr int FU_MAX_N = (int)((FU_SMEM - FU_AUX_BYTES) / sizeof(float));         // 26,368 filters
+static_assert((size_t)(FU_THREADS / 32) * ROW_MAX * sizeof(float) <= FU_SMEM, "1x1 rows must fit the ring");
+
+struct FusedState {
+  unsigned int next_item;  // work queue
+  unsigned int pad0[31];
+  unsigned int items_done;
+  unsigned int pad1[31];
+  unsigned int flag;  // polled by idle blocks: its own 128-byte line
+  unsigned int pad2[31];
+  unsigned long long stamp[8];  // diagnostics (globaltimer ns): block 0 start, last block out of work, last block past the
+                                // wait, last block with thr, last block done
+};
+__device__ __forceinline__ void fused_stamp(FusedState* st, int i, bool max_over_blocks) {
+  unsigned long long t;
+  asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
+  if (max_over_blocks) atomicMax(&st->stamp[i], t);
+  else st->stamp[i] = t;
+}
+
+__device__ __forceinline__ unsigned int ld_acquire_u32(const unsigned int* p) {
+  unsigned int v;
+  asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
+  return v;
+}
+
+// All raw sums -> normalised values s_val [n] in shared memory (methods.py:43-51 for every layer), by one block: one
+// warp per layer.  Returns true (block-uniform) if any value is NaN.
+template <int NT>
+__device__ bool fused_normalise_all(const LayerTable& lt, const float* __restrict__ raw, float* s_val) {
+  const int n = lt.voff[lt.nlayers];
+  const int tid = threadIdx.x;
+  for (int i0 = 0; i0 < n; i0 += 16 * NT) {  // 16 independent L2 loads in flight per thread
+    float x[16];
+#pragma unroll
+    for (int u = 0; u < 16; ++u) {
+      const int i = i0 + u * NT + tid;
+      x[u] = i < n ? __ldcg(raw + i) : 0.f;
+    }
+#pragma unroll
+    for (int u = 0; u < 16; ++u) {
+      const int i = i0 + u * NT + tid;
+      if (i < n) s_val[i] = x[u];
+    }
+  }
+  __syncthreads();
+  int nan = 0;
+  for (int l = tid >> 5; l < lt.nlayers; l += NT / 32) nan |= normalise_layer<32>(s_val + lt.voff[l], lt.O[l], nullptr);
+  return __syncthreads_or(nan) != 0;
+}
+
 __global__ void __launch_bounds__(FU_THREADS, 2)
 filter_prune_fused_kernel(const LayerTable lt, float* __restrict__ raw, float* __restrict__ values, int n_tiled, int n_big,
                           int n_items, long long k, double gamma, double* __restrict__ thr, uint8_t* __restrict__ keep,
@@ -914,7 +635,7 @@ filter_prune_fused_kernel(const LayerTable lt, float* __restrict__ raw, float* _
     if (item < n_tiled)
       sumsq_tiled_block<FU_F, FU_STAGES>(lt, item, raw, reinterpret_cast<float4*>(dsm), s_tap);
     else
-      sumsq_generic_block<FU_THREADS>(lt, item - n_tiled, raw, s_tap, reinterpret_cast<float(*)[MAX_LEAVES]>(dsm));
+      sumsq_generic_block<FU_THREADS>(lt, item - n_tiled, raw, s_tap, reinterpret_cast<float*>(dsm));
     __threadfence();  // this block's sums are visible device-wide before it counts the item in
     __syncthreads();
     if (tid == 0) s_last = (atomicAdd(&st->items_done, 1u) == (unsigned int)n_items - 1u) ? 1u : 0u;
@@ -927,15 +648,15 @@ filter_prune_fused_kernel(const LayerTable lt, float* __restrict__ raw, float* _
     __threadfence();
     if (tid == 0) fused_stamp(st, 2, false);
     float* s_val = reinterpret_cast<float*>(dsm);
-    unsigned char* aux = dsm + (FU_SMEM - FU_AUX_BYTES);
-    const bool any_nan = fused_normalise_all<FU_THREADS>(lt, raw, s_val, aux);
+    const bool any_nan = fused_normalise_all<FU_THREADS>(lt, raw, s_val);
     if (tid == 0) fused_stamp(st, 5, false);
     double t;
     if (any_nan) t = __longlong_as_double(0x7ff8000000000000LL);  // np.percentile returns nan: nothing is < nan
-    else t = fused_select<FU_THREADS>(s_val, n, k, gamma, reinterpret_cast<unsigned int*>(aux), s_bin);
+    else t = select_percentile<FU_THREADS>(s_val, n, k, gamma,
+                                           reinterpret_cast<unsigned int*>(dsm + (FU_SMEM - FU_AUX_BYTES)), s_bin);
     for (int i = tid; i < n; i += FU_THREADS) {
       values[i] = s_val[i];
-      if (keep) keep[i] = ((double)s_val[i] < t) ? 0 : 1;
+      if (keep) keep[i] = kept(s_val[i], t) ? 1 : 0;
     }
     if (tid == 0) *thr = t;
     __threadfence();
@@ -962,21 +683,11 @@ filter_prune_fused_kernel(const LayerTable lt, float* __restrict__ raw, float* _
       while (l + 1 < lt.nlayers && f >= lt.voff[l + 1]) ++l;
       float val = prov;
       if (pass) {
-        val = ((double)__ldcg(values + f) < t) ? 0.f : 1.f;
+        val = kept(__ldcg(values + f), t) ? 1.f : 0.f;
         if (!i_finished && val == prov) continue;  // already written by the provisional pass
       }
-      const int o = f - lt.voff[l];
       const int per = lt.C[l] * lt.taps[l];
-      float* m = lt.mask[l] + (long long)o * per;
-      int head = (int)(((16 - (reinterpret_cast<uintptr_t>(m) & 15)) & 15) >> 2);  // scalar head up to 16-byte alignment
-      if (head > per) head = per;
-      if (tid < head) m[tid] = val;
-      const int body4 = (per - head) >> 2;
-      float4* m4 = reinterpret_cast<float4*>(m + head);
-      const float4 v4 = make_float4(val, val, val, val);
-      for (int i = tid; i < body4; i += FU_THREADS) st_stream_f4(m4 + i, v4);
-      const int tail0 = head + body4 * 4;
-      if (tid < per - tail0) m[tail0 + tid] = val;
+      fill_filter<FU_THREADS>(lt.mask[l] + (long long)(f - lt.voff[l]) * per, per, val);
     }
   };
   if (!i_finished) fill_filters(0);
@@ -1001,7 +712,7 @@ int build_layers(LayerTable* lt, const float* const* w, float* const* masks, con
   lt->toff[0] = 0;
   for (int l = 0; l < nlayers; ++l) {
     if (O[l] <= 0 || C[l] <= 0 || taps[l] <= 0) return mc_set_error(MC_ERR_ARG, "%s: layer %d has bad dims", who, l);
-    lt->w[l] = w ? w[l] : nullptr;
+    lt->w[l] = w[l];
     lt->mask[l] = masks ? masks[l] : nullptr;
     lt->O[l] = O[l];
     lt->C[l] = C[l];
@@ -1013,7 +724,7 @@ int build_layers(LayerTable* lt, const float* const* w, float* const* masks, con
     const long long thr = (taps[l] == 1) ? O[l] : (long long)O[l] * taps[l];
     // per-layer thread slots rounded up to whole blocks; for taps>1 a block must hold whole filters
     long long slots;
-    if (w && taps[l] == 9 && (C[l] % TL_C) == 0 && (O[l] % tl_f) == 0) slots = 0;  // tiled path
+    if (taps[l] == 9 && (C[l] % TL_C) == 0 && (O[l] % tl_f) == 0) slots = 0;  // tiled path
     else if (taps[l] == 1) slots = ((thr * 32 + nt - 1) / nt) * nt;  // one warp per filter
     else {
       const int fpb = nt / taps[l];  // filters per block
@@ -1024,7 +735,7 @@ int build_layers(LayerTable* lt, const float* const* w, float* const* masks, con
   // tiled layers, largest C first (insertion sort; nlayers <= 64)
   lt->ntiled = 0;
   for (int l = 0; l < nlayers; ++l) {
-    if (!(w && taps[l] == 9 && (C[l] % TL_C) == 0 && (O[l] % tl_f) == 0)) continue;
+    if (!(taps[l] == 9 && (C[l] % TL_C) == 0 && (O[l] % tl_f) == 0)) continue;
     int pos = lt->ntiled++;
     while (pos > 0 && C[lt->torder[pos - 1]] < C[l]) {
       lt->torder[pos] = lt->torder[pos - 1];
@@ -1049,9 +760,6 @@ int build_layers(LayerTable* lt, const float* const* w, float* const* masks, con
   return 0;
 }
 
-}  // namespace
-
-namespace {
 int launch_sumsq(const LayerTable& lt, float* d_values, cudaStream_t stream) {
   static bool attr_set = false;
   if (!attr_set) {
@@ -1064,6 +772,33 @@ int launch_sumsq(const LayerTable& lt, float* d_values, cudaStream_t stream) {
   if (n_tiled + n_generic == 0) return 0;
   filter_sumsq_kernel<<<n_tiled + n_generic, SS_THREADS, SUMSQ_SMEM, stream>>>(lt, d_values, n_tiled, first_wave);
   MC_LAUNCH_CHECK("filter_sumsq_kernel");
+  return 0;
+}
+
+// filter_finish_kernel over the n values of lt: k < 0 normalises them only, k >= 0 also selects (d_ticket zeroed).
+int launch_finish(const LayerTable& lt, float* d_values, long long k, double gamma, double* d_thr, uint8_t* d_keep,
+                  unsigned int* d_ticket, cudaStream_t stream, const char* who) {
+  const int n = lt.voff[lt.nlayers];
+  int staged = k >= 0 ? n : 0;
+  for (int l = 0; l < lt.nlayers; ++l) staged = lt.O[l] > staged ? lt.O[l] : staged;
+  const size_t smem = (size_t)staged * sizeof(float);
+  if (smem > FIN_MAX_SMEM) return mc_set_error(MC_ERR_SHAPE, "%s: %d filters exceed the single-block finish", who, staged);
+  static size_t attr = 0;
+  if (smem > attr) {
+    MC_CUDA(cudaFuncSetAttribute(filter_finish_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    attr = smem;
+  }
+  filter_finish_kernel<<<lt.nlayers, FIN_THREADS, smem, stream>>>(lt, d_values, k, gamma, d_thr, d_keep, d_ticket);
+  MC_LAUNCH_CHECK("filter_finish_kernel");
+  return 0;
+}
+
+int launch_mask_fill(const LayerTable& lt, const float* d_v, const double* d_thr, cudaStream_t stream) {
+  int blocks = lt.voff[lt.nlayers];
+  const int cap = mc_num_sms() * 16;
+  if (blocks > cap) blocks = cap;
+  filter_mask_fill_kernel<<<blocks, 256, 0, stream>>>(lt, d_v, d_thr);
+  MC_LAUNCH_CHECK("filter_mask_fill_kernel");
   return 0;
 }
 }  // namespace
@@ -1085,58 +820,11 @@ extern "C" int mc_filter_values(const float* const* h_w_ptrs, const int* h_O, co
   if (rc) return rc;
   rc = launch_sumsq(lt, d_values, stream);
   if (rc) return rc;
-  filter_norm_kernel<<<nlayers, 256, 0, stream>>>(lt, d_values);
-  MC_LAUNCH_CHECK("filter_norm_kernel");
-  return 0;
-}
-
-extern "C" size_t mc_workspace_bytes_filter_threshold(int n) {
-  (void)n;
-  return 0;
-}
-
-extern "C" int mc_filter_threshold(const float* d_values, int n, int64_t k, double gamma, double* d_thr, void* d_ws,
-                                   size_t ws_bytes, void* stream_) {
-  (void)d_ws;
-  (void)ws_bytes;
-  cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
-  MC_CHECK_ARG(d_values && d_thr && n > 0, "mc_filter_threshold: bad argument");
-  MC_CHECK_ARG(k >= 0 && k < n, "mc_filter_threshold: rank out of range");
-  MC_CHECK_ARG(gamma >= 0.0 && gamma < 1.0, "mc_filter_threshold: gamma must be in [0,1)");
-  filter_threshold_kernel<<<1, 1024, 0, stream>>>(d_values, n, (long long)k, gamma, d_thr);
-  MC_LAUNCH_CHECK("filter_threshold_kernel");
-  return 0;
-}
-
-extern "C" int mc_filter_masks(const float* d_values, const double* d_thr, const int* h_O, const int* h_per_filter,
-                               int nlayers, float* const* h_mask_ptrs, uint8_t* d_keep, void* stream_) {
-  cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
-  MC_CHECK_ARG(d_values && d_thr && h_O && h_per_filter, "mc_filter_masks: null pointer");
-  MC_CHECK_ARG(h_mask_ptrs || d_keep, "mc_filter_masks: nothing to do");
-  int ones[MAX_LAYERS];
-  for (int l = 0; l < nlayers && l < MAX_LAYERS; ++l) ones[l] = 1;
-  LayerTable lt;
-  // per-filter element count goes into C, taps = 1
-  int rc = build_layers(&lt, nullptr, h_mask_ptrs, h_O, h_per_filter, ones, nlayers, "mc_filter_masks");
-  if (rc) return rc;
-  const int n = lt.voff[nlayers];
-  if (d_keep) {
-    filter_keep_kernel<<<(n + 255) / 256, 256, 0, stream>>>(d_values, n, d_thr, d_keep);
-    MC_LAUNCH_CHECK("filter_keep_kernel");
-  }
-  if (h_mask_ptrs) {
-    for (int l = 0; l < nlayers; ++l) MC_CHECK_ARG(h_mask_ptrs[l] != nullptr, "mc_filter_masks: null mask %d", l);
-    int blocks = lt.voff[nlayers];
-    const int cap = mc_num_sms() * 16;
-    if (blocks > cap) blocks = cap;
-    filter_mask_fill_kernel<<<blocks, 256, 0, stream>>>(lt, d_values, d_thr);
-    MC_LAUNCH_CHECK("filter_mask_fill_kernel");
-  }
-  return 0;
+  return launch_finish(lt, d_values, -1, 0.0, nullptr, nullptr, nullptr, stream, "mc_filter_values");
 }
 
 /* The whole of quick_filter_prune in one call: ONE cooperative launch (filter_prune_fused_kernel); models with more
- * filters than the single-block select holds take the three-launch path.  See include/mcb200.h. */
+ * filters than its finisher block holds take the three-launch path.  See include/mcb200.h. */
 extern "C" size_t mc_workspace_bytes_filter_prune(void) { return 2048 + (size_t)FU_MAX_N * sizeof(float); }
 static_assert(sizeof(FusedState) <= 2048, "FusedState must fit the head of the filter-prune workspace");
 
@@ -1148,25 +836,25 @@ extern "C" int mc_filter_prune(const float* const* h_w_ptrs, const int* h_O, con
   MC_CHECK_ARG(nlayers > 0 && nlayers <= MAX_LAYERS, "mc_filter_prune: nlayers out of range");
   if (ws_bytes < mc_workspace_bytes_filter_prune()) return mc_set_error(MC_ERR_WS, "mc_filter_prune: workspace too small");
   int taps[MAX_LAYERS];
-  int max_o = 0;
+  long long n_all = 0;
   for (int l = 0; l < nlayers; ++l) {
     MC_CHECK_ARG(h_kh[l] == h_kw[l] && h_kh[l] >= 1 && h_kh[l] * h_kw[l] <= 49,
                  "mc_filter_prune: layer %d kernel %dx%d unsupported (square, <=7x7)", l, h_kh[l], h_kw[l]);
     MC_CHECK_ARG(h_w_ptrs[l] != nullptr, "mc_filter_prune: layer %d null weight", l);
     MC_CHECK_ARG(!h_mask_ptrs || h_mask_ptrs[l] != nullptr, "mc_filter_prune: null mask %d", l);
     taps[l] = h_kh[l] * h_kw[l];
-    if (h_O[l] > max_o) max_o = h_O[l];
+    n_all += h_O[l];
   }
+  // the fused kernel's work items are smaller than the three-launch path's: the table is built for the path taken
+  const bool fused = n_all <= FU_MAX_N;
   LayerTable lt;
-  int rc = build_layers(&lt, h_w_ptrs, h_mask_ptrs, h_O, h_C, taps, nlayers, "mc_filter_prune");
+  int rc = build_layers(&lt, h_w_ptrs, h_mask_ptrs, h_O, h_C, taps, nlayers, "mc_filter_prune",
+                        fused ? FU_THREADS : SS_THREADS, fused ? FU_F : TL_F);
   if (rc) return rc;
   const int n = lt.voff[nlayers];
   MC_CHECK_ARG(k >= 0 && k < n, "mc_filter_prune: rank out of range");
   MC_CHECK_ARG(gamma >= 0.0 && gamma < 1.0, "mc_filter_prune: gamma must be in [0,1)");
-  if (n <= FU_MAX_N) {
-    LayerTable lf;
-    rc = build_layers(&lf, h_w_ptrs, h_mask_ptrs, h_O, h_C, taps, nlayers, "mc_filter_prune", FU_THREADS, FU_F);
-    if (rc) return rc;
+  if (fused) {
     static int max_blocks = -1;
     if (max_blocks < 0) {
       MC_CUDA(cudaFuncSetAttribute(filter_prune_fused_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)FU_SMEM));
@@ -1175,10 +863,10 @@ extern "C" int mc_filter_prune(const float* const* h_w_ptrs, const int* h_O, con
       if (per_sm < 1) return mc_set_error(MC_ERR_SHAPE, "mc_filter_prune: fused kernel does not fit an SM");
       max_blocks = per_sm * mc_num_sms();
     }
-    int n_tiled = lf.tblk[lf.ntiled];
-    int n_items = n_tiled + lf.toff[lf.nlayers] / FU_THREADS;
+    int n_tiled = lt.tblk[lt.ntiled];
+    int n_items = n_tiled + lt.toff[lt.nlayers] / FU_THREADS;
     int n_big = 0;  // tiled items of the layers with >= 1024 input channels (torder is sorted by descending C)
-    for (int i2 = 0; i2 < lf.ntiled && h_C[lf.torder[i2]] >= 1024; ++i2) n_big = lf.tblk[i2 + 1];
+    for (int i2 = 0; i2 < lt.ntiled && h_C[lt.torder[i2]] >= 1024; ++i2) n_big = lt.tblk[i2 + 1];
     int grid = n_items < max_blocks ? n_items : max_blocks;
     if (grid < 1) grid = 1;
     MC_CUDA(cudaMemsetAsync(d_ws, 0, sizeof(FusedState), stream));
@@ -1186,33 +874,17 @@ extern "C" int mc_filter_prune(const float* const* h_w_ptrs, const int* h_O, con
     FusedState* stp = reinterpret_cast<FusedState*>(d_ws);
     float* d_raw = reinterpret_cast<float*>(reinterpret_cast<unsigned char*>(d_ws) + 2048);  // raw sums [n]
     int fill = h_mask_ptrs ? 1 : 0;
-    void* args[] = {&lf, &d_raw, &d_values, &n_tiled, &n_big, &n_items, &kk, &gamma, &d_thr, &d_keep, &stp, &fill};
+    void* args[] = {&lt, &d_raw, &d_values, &n_tiled, &n_big, &n_items, &kk, &gamma, &d_thr, &d_keep, &stp, &fill};
     MC_CUDA(cudaLaunchCooperativeKernel(reinterpret_cast<void*>(filter_prune_fused_kernel), dim3((unsigned)grid),
                                         dim3(FU_THREADS), args, FU_SMEM, stream));
     return 0;
   }
-  const size_t fin_smem = (size_t)(n > max_o ? n : max_o) * sizeof(float);
-  if (fin_smem > 200 * 1024) return mc_set_error(MC_ERR_SHAPE, "mc_filter_prune: %d filters exceed the single-block select", n);
-  static size_t fin_attr = 0;
-  if (fin_smem > fin_attr) {
-    MC_CUDA(cudaFuncSetAttribute(filter_finish_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fin_smem));
-    fin_attr = fin_smem;
-  }
-  MC_CUDA(cudaMemsetAsync(d_ws, 0, 8, stream));
+  MC_CUDA(cudaMemsetAsync(d_ws, 0, sizeof(unsigned int), stream));
   rc = launch_sumsq(lt, d_values, stream);
-  if (rc) return rc;
-  filter_finish_kernel<<<nlayers, FIN_THREADS, fin_smem, stream>>>(lt, d_values, (long long)k, gamma, d_thr, d_keep,
-                                                                   reinterpret_cast<unsigned int*>(d_ws));
-  MC_LAUNCH_CHECK("filter_finish_kernel");
-  if (h_mask_ptrs) {
-    // the fill kernel addresses layer l's filter o at mask[l] + o*per: per-filter element count in C, taps = 1
-    int blocks = n;
-    const int cap = mc_num_sms() * 16;
-    if (blocks > cap) blocks = cap;
-    filter_mask_fill_kernel<<<blocks, 256, 0, stream>>>(lt, d_values, d_thr);
-    MC_LAUNCH_CHECK("filter_mask_fill_kernel");
-  }
-  return 0;
+  if (!rc) rc = launch_finish(lt, d_values, (long long)k, gamma, d_thr, d_keep, reinterpret_cast<unsigned int*>(d_ws),
+                              stream, "mc_filter_prune");
+  if (!rc && h_mask_ptrs) rc = launch_mask_fill(lt, d_values, d_thr, stream);
+  return rc;
 }
 
 // ---- greedy filter pruning: prune_one_filter / filter_prune (methods.py:81-142, arXiv:1611.06440) ----------------------
@@ -1255,28 +927,6 @@ constexpr int GR_MAX_N = 20480;  // filters staged in shared memory: raw value, 
 constexpr int GR_MAX_LEAVES = GR_MAX_N / 56 + 2 * MAX_LAYERS;
 constexpr size_t GR_SMEM = (size_t)GR_MAX_N * 9;
 
-// NumPy's pairwise sum of a[i]^2 over one leaf (n <= 128) by a warp: lane j & 7 runs accumulator j, the xor butterfly
-// performs ((r0+r1)+(r2+r3))+((r4+r5)+(r6+r7)), then the sequential tail.  The result is valid in every lane.
-__device__ __forceinline__ float warp_leaf_sumsq(const float* a, int n) {
-  const int j = threadIdx.x & 7;
-  const int body = n - (n % 8);
-  float r = 0.f;
-  if (n >= 8) {
-    float x = a[j];
-    r = __fmul_rn(x, x);
-    for (int i = 8; i < body; i += 8) {
-      x = a[i + j];
-      r = __fadd_rn(r, __fmul_rn(x, x));
-    }
-  }
-  float t = __fadd_rn(r, __shfl_xor_sync(0xffffffffu, r, 1));
-  t = __fadd_rn(t, __shfl_xor_sync(0xffffffffu, t, 2));
-  t = __fadd_rn(t, __shfl_xor_sync(0xffffffffu, t, 4));
-  float sum = n >= 8 ? t : 0.f;
-  for (int i = n >= 8 ? body : 0; i < n; ++i) sum = __fadd_rn(sum, __fmul_rn(a[i], a[i]));
-  return sum;
-}
-
 enum { GR_DONE = 0, GR_BUDGET = 1, GR_NAN_PICK = 2, GR_NO_CANDIDATE = 3, GR_NONFINITE = 4 };
 
 struct GreedyShared {
@@ -1293,12 +943,7 @@ struct GreedyShared {
 // or index 0 as the last one, reports (inf, inf).
 __device__ void greedy_refresh_layer(const LayerTable& lt, int l, const float* s_raw, GreedyShared& g) {
   const int lane = threadIdx.x & 31, O = lt.O[l];
-  float tot = 0.f;
-  if (lane == 0) {
-    int next = 0;
-    tot = np_combine_leaves(g.lsum + g.loff[l], O, &next);
-  }
-  const float nrm = __fsqrt_rn(__shfl_sync(0xffffffffu, tot, 0));
+  const float nrm = __fsqrt_rn(np_combine_leaves(g.lsum + g.loff[l], O));
   const float* r = s_raw + lt.voff[l];
   int last = -1, im = INT_MAX;
   float m = INFINITY;
@@ -1355,7 +1000,11 @@ __global__ void __launch_bounds__(GR_THREADS) filter_greedy_kernel(const LayerTa
   }
   if (tid == 0) {
     g.loff[0] = 0;
-    for (int l = 0; l < nl; ++l) g.loff[l + 1] = g.loff[l] + np_for_each_leaf(lt.O[l], [](int, int, int) {});
+    for (int l = 0; l < nl; ++l) {
+      int leaves = 1;
+      for (NpWalk w(lt.O[l]); w.next(0.f);) ++leaves;
+      g.loff[l + 1] = g.loff[l] + leaves;
+    }
   }
   if (__syncthreads_or(bad)) {
     if (tid == 0) {
@@ -1368,16 +1017,21 @@ __global__ void __launch_bounds__(GR_THREADS) filter_greedy_kernel(const LayerTa
   // leaf tables and sums, norms and candidates of every layer: one warp per layer
   for (int l = wid; l < nl; l += GR_THREADS / 32) {
     const int base = g.loff[l];
-    if (lane == 0)
-      np_for_each_leaf(lt.O[l], [&](int leaf, int st, int ln) {
-        g.lst[base + leaf] = st;
-        g.lln[base + leaf] = ln;
-      });
+    if (lane == 0) {
+      NpWalk w(lt.O[l]);
+      for (int k = base;; ++k) {
+        g.lst[k] = w.st;
+        g.lln[k] = w.ln;
+        if (!w.next(0.f)) break;
+      }
+    }
     __syncwarp();
     const float* r = s_raw + lt.voff[l];
-    for (int k = base; k < g.loff[l + 1]; ++k) {
-      const float s = warp_leaf_sumsq(r + g.lst[k], g.lln[k]);
-      if (lane == 0) g.lsum[k] = s;
+    for (int k0 = base; k0 < g.loff[l + 1]; k0 += 4) {  // four leaves at a time
+      const int k = k0 + (lane >> 3);
+      const bool have = k < g.loff[l + 1];
+      const float s = group_leaf_sumsq(r + (have ? g.lst[k] : 0), have ? g.lln[k] : 0);
+      if (have && (lane & 7) == 0) g.lsum[k] = s;
     }
     __syncwarp();
     greedy_refresh_layer(lt, l, s_raw, g);
@@ -1438,7 +1092,7 @@ __global__ void __launch_bounds__(GR_THREADS) filter_greedy_kernel(const LayerTa
                                                                 ci < g.lst[k] + g.lln[k]);
         if (hit) leaf = k0 + __ffs(hit) - 1;
       }
-      const float s = warp_leaf_sumsq(s_raw + lt.voff[bl] + g.lst[leaf], g.lln[leaf]);
+      const float s = group_leaf_sumsq(s_raw + lt.voff[bl] + g.lst[leaf], g.lln[leaf]);
       if (lane == 0) g.lsum[leaf] = s;
       __syncwarp();
       greedy_refresh_layer(lt, bl, s_raw, g);
@@ -1510,12 +1164,5 @@ extern "C" int mc_filter_prune_greedy(const float* const* h_w_ptrs, const int* h
       lt, d_raw, d_nz, (long long)zeros0, (long long)total_params, perc, max_picks, reinterpret_cast<int2*>(d_picks),
       reinterpret_cast<long long*>(d_result), d_keepf, d_half);
   MC_LAUNCH_CHECK("filter_greedy_kernel");
-  if (h_mask_ptrs) {
-    int blocks = n;
-    const int cap = mc_num_sms() * 16;
-    if (blocks > cap) blocks = cap;
-    filter_mask_fill_kernel<<<blocks, 256, 0, stream>>>(lt, d_keepf, d_half);
-    MC_LAUNCH_CHECK("filter_mask_fill_kernel");
-  }
-  return 0;
+  return h_mask_ptrs ? launch_mask_fill(lt, d_keepf, d_half, stream) : 0;
 }

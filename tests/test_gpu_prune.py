@@ -220,7 +220,9 @@ def test_filter_values_bit_exact(darknet):
 
 
 def test_filter_prune_odd_shapes():
-    # pairwise-sum corner cases (C < 8, C % 8 != 0, C > 128 with odd halves) and a 5x5 kernel
+    # pairwise-sum corner cases (C < 8, C % 8 != 0, C > 128 with odd halves), a 5x5 kernel, a 1x1 row wider than the
+    # 2,048 channels staged in shared memory, and a layer of 3,000 filters (not 128 * 2^k: an uneven recursion)
+    from modelcompression_b200.pruning.weightPruning.methods import filter_values
     torch.manual_seed(3)
 
     class Net(torch.nn.Module):
@@ -232,9 +234,13 @@ def test_filter_prune_odd_shapes():
             self.d = torch.nn.Conv2d(1001, 4, 1)
             self.e = torch.nn.Conv2d(6, 10, 5)
             self.f = torch.nn.Conv2d(300, 40, 3)
+            self.g = torch.nn.Conv2d(2500, 6, 1)
+            self.h = torch.nn.Conv2d(8, 3000, 1)
 
     net = Net().to(DEV)
     cw = [p.detach().cpu().numpy() for p in net.parameters() if p.dim() == 4]
+    v = filter_values([p.data for p in net.parameters() if p.dim() == 4]).cpu().numpy()
+    assert np.array_equal(v, np.concatenate([prune_oracle.filter_values_np(w) for w in cw]))
     for perc in (10., 47.3, 90.):
         masks, keep = mc.quick_filter_prune(net, perc, return_keep=True)
         _, _, keep_o, masks_o = prune_oracle.quick_filter_prune_np(cw, perc)

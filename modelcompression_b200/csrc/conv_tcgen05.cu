@@ -12,11 +12,13 @@
 // M tile = 128 rows (UMMA M=128, cta_group::1), N tile = block_n (16..256), K block = 64 bf16 = one
 // 128-byte swizzle row (or 32 bf16 / 64-byte swizzle for <= 32 input channels).  Warp roles: warp0 = TMA producer,
 // warp1 = TMEM owner + MMA issuer (warp-uniform loop, one elected lane issues), warps 2..5 = epilogue (TMEM -> regs ->
-// scale/shift/leaky -> bf16/fp32 stores, staged through shared memory for 32..96-wide PNHWC tiles).
-// Two kernels share this file:
+// scale/shift/leaky -> bf16/fp32 stores, through TMA-store slabs for PNHWC tiles >= 64 wide).
+// Two kernels share this file, and with it the shared-memory carve-up and barrier set-up, the shared-activation-box
+// mainloop (produce_box_groups / mma_box_unit) and the per-tile epilogue (epi_tile_begin / epilogue_tile):
 //   conv_gemm_tcgen05_kernel<MINB>   persistent, 1..3 CTAs per SM (MINB = register budget), every layer shape;
 //   conv_gemm_tcgen05_pair_kernel    cluster of 2 CTAs, tcgen05 cta_group::2: 256-row tiles, each CTA loads half of every
-//                                    weight tile — the wide 3x3 layers (block_n >= 192, >= 36 k-blocks).
+//                                    weight tile — the wide 3x3 layers (block_n >= 192, >= 36 k-blocks), with a
+//                                    stream-K tail and the chained launch of several layers (mc_conv_chain_fwd).
 // mc_conv_fwd picks kernel, tile width, ring depth and CTAs per SM (mc_conv_last_plan reports the choice).
 #include <cuda.h>
 #include <stdio.h>
@@ -37,6 +39,7 @@ constexpr int A_BOX_BYTES = A_BOX_ROWS * 128;   // 17,408 B landed by TMA
 constexpr int A_BOX_STRIDE = 18 * 1024;         // ring pitch (1024-byte aligned for the 128-byte swizzle)
 constexpr int ACC_STAGES = 2;  // accumulator stages in TMEM: the MMA issuer runs this many tiles ahead of the epilogue
 constexpr int NUM_THREADS = 192;
+constexpr int WORK_SLOTS = 4;  // work ring of the CTA-pair kernel's chained launch (see PairRing)
 
 struct ConvKParams {
   int M_rows;      // B*(H+1)*(W+1)
@@ -79,7 +82,7 @@ struct ConvKParams {
   unsigned long long* dbg;  // mc_debug_conv_trace: globaltimer stamps, 32 slots per CTA (nullptr: no tracing)
 };
 
-// Timeline stamps of the single-CTA kernel (slot layout in tools/trace_conv.py)
+// Timeline stamps of both kernels (slot layout in tools/trace_conv.py)
 __device__ __forceinline__ void conv_stamp(const ConvKParams& p, int slot) {
   if (p.dbg != nullptr && slot < 32) {
     unsigned long long t;
@@ -87,6 +90,210 @@ __device__ __forceinline__ void conv_stamp(const ConvKParams& p, int slot) {
     p.dbg[(size_t)blockIdx.x * 32 + slot] = t;
   }
 }
+
+// ---------------------------------------------------------------------------------------------------------------
+// Shared memory and its barriers.  PAIR: the CTA-pair kernel, which always shares the activation box, loads half of
+// every B tile per CTA and adds the work ring of its chained launch.
+struct ConvSmem {
+  uint8_t* tiles;     // shared box: [a_stages x activation box] then b_ring; else [stages x (A tile | B tile)]
+  uint8_t* b_ring;    // shared box: [stages x B tile]
+  uint64_t* full_bar;        // [MAX_STAGES]  B tile (or A | B stage) landed
+  uint64_t* empty_bar;       // [MAX_STAGES]  its MMAs retired
+  uint64_t* tmem_full_bar;   // [ACC_STAGES]  accumulator complete
+  uint64_t* tmem_empty_bar;  // [ACC_STAGES]  accumulator drained by the epilogue
+  uint64_t* afull_bar;       // [MAX_A_STAGES] activation box landed
+  uint64_t* aempty_bar;      // [MAX_A_STAGES] its three taps retired
+  uint32_t* tmem_ptr;
+  uint64_t* work_full;       // (PAIR) [WORK_SLOTS] work ring, see PairRing
+  uint64_t* work_empty;      // (PAIR) [WORK_SLOTS]
+  int* work_val;             // (PAIR) [WORK_SLOTS]
+  float* s_ss;    // [2 acc stages][scale|shift][256]
+  uint8_t* s_out;  // staged epilogue: [4 warps][32 rows][out_pitch]; TMA-store slabs [4 warps][tma_bufs][4 KB]
+                   // (1024-byte aligned: swizzle pattern), then the batch-statistics accumulators; decode: logits
+};
+
+// box_stride: pitch of the activation-box ring; b_bytes: one B tile (of this CTA); stage_bytes: one A | B stage of the
+// ring without a shared box.  The host reserves 5 KB for aux (barriers, scale/shift) plus 1 KB of alignment slack.
+template <bool PAIR>
+__device__ __forceinline__ ConvSmem carve_smem(uint8_t* smem, const ConvKParams& p, uint32_t box_stride,
+                                               uint32_t b_bytes, uint32_t stage_bytes) {
+  {  // dynamic smem base is only guaranteed 16B aligned: align up to 1024 (host adds 1 KB of slack)
+    uint32_t a = ptx::smem_u32(smem);
+    smem += (1024u - (a & 1023u)) & 1023u;
+  }
+  ConvSmem m;
+  m.tiles = smem;
+  m.b_ring = smem + (size_t)p.a_stages * box_stride;
+  uint8_t* aux = (PAIR || p.share_dx) ? m.b_ring + (size_t)p.stages * b_bytes : smem + (size_t)p.stages * stage_bytes;
+  m.full_bar = reinterpret_cast<uint64_t*>(aux);
+  m.empty_bar = m.full_bar + MAX_STAGES;
+  m.tmem_full_bar = m.empty_bar + MAX_STAGES;
+  m.tmem_empty_bar = m.tmem_full_bar + ACC_STAGES;
+  m.afull_bar = m.tmem_empty_bar + ACC_STAGES;
+  m.aempty_bar = m.afull_bar + MAX_A_STAGES;
+  m.tmem_ptr = reinterpret_cast<uint32_t*>(m.aempty_bar + MAX_A_STAGES);
+  m.work_full = reinterpret_cast<uint64_t*>(aux + 256);
+  m.work_empty = m.work_full + WORK_SLOTS;
+  m.work_val = reinterpret_cast<int*>(m.work_empty + WORK_SLOTS);
+  m.s_ss = reinterpret_cast<float*>(aux + 512);
+  m.s_out = aux + 5120;
+  return m;
+}
+
+// Barrier initialisation (thread 0) and TMEM allocation (warp 1), published to the block — PAIR: to both CTAs of the
+// cluster, whose barriers must be initialised before any remote arrival / complete_tx.  Returns the TMEM base.
+template <bool PAIR>
+__device__ __forceinline__ uint32_t block_setup(const ConvSmem& m, const ConvKParams& p) {
+  if (threadIdx.x == 0) {
+    for (int s = 0; s < p.stages; ++s) {
+      ptx::mbar_init(&m.full_bar[s], 1);
+      ptx::mbar_init(&m.empty_bar[s], 1);
+    }
+    for (int a = 0; a < ACC_STAGES; ++a) {
+      ptx::mbar_init(&m.tmem_full_bar[a], 1);
+      ptx::mbar_init(&m.tmem_empty_bar[a], PAIR ? 8 : 4);  // one arrive per epilogue warp (PAIR: of each CTA)
+    }
+    for (int a = 0; a < MAX_A_STAGES; ++a) {
+      ptx::mbar_init(&m.afull_bar[a], 1);
+      ptx::mbar_init(&m.aempty_bar[a], 1);
+    }
+    if (PAIR) {
+      for (int s = 0; s < WORK_SLOTS; ++s) {
+        ptx::mbar_init(&m.work_full[s], 1);
+        ptx::mbar_init(&m.work_empty[s], 10);  // leader: MMA warp + 4 epilogue warps; peer: producer + 4 epilogue warps
+      }
+    }
+    ptx::fence_barrier_init();
+  }
+  if ((threadIdx.x >> 5) == 1) {
+    if (PAIR) {
+      ptx::tmem_alloc_pair(m.tmem_ptr, (uint32_t)p.tmem_cols);
+      ptx::tmem_relinquish_pair();
+    } else {
+      ptx::tmem_alloc(m.tmem_ptr, (uint32_t)p.tmem_cols);
+      ptx::tmem_relinquish();
+    }
+  }
+  ptx::tc_fence_before();
+  if (PAIR) ptx::cluster_sync_all();
+  else __syncthreads();
+  ptx::tc_fence_after();
+  return *m.tmem_ptr;
+}
+
+// ---------------------------------------------------------------------------------------------------------------
+// Shared-activation-box mainloop (3x3 layers).  K group g = (filter row dy, channel block cb) of a tile: one 136-row
+// activation box serves the three dx taps, which read it at row offsets 0, 1, 2, so the activations cross
+// L2 -> smem 3 times per tile instead of 9; the B tile of every tap comes through its own ring.
+
+// Ring positions and phases: B tiles (s), activation boxes (sa), accumulator stages (as)
+struct Pipe {
+  int stages, a_stages;
+  int s = 0, sa = 0, as = 0;
+  uint32_t phase = 0, pha = 0, aphase = 0;
+  __device__ __forceinline__ Pipe(int stages_, int a_stages_) : stages(stages_), a_stages(a_stages_) {}
+  __device__ __forceinline__ void next_b() { if (++s == stages) { s = 0; phase ^= 1u; } }
+  __device__ __forceinline__ void next_box() { if (++sa == a_stages) { sa = 0; pha ^= 1u; } }
+  __device__ __forceinline__ void next_acc() { if (++as == ACC_STAGES) { as = 0; aphase ^= 1u; } }
+};
+
+// Producer (one thread) of K groups [g0, g1) of the tile at rows m0, B rows n0.  box_bytes: one box (136 rows of one
+// k-block row); b_bytes: one B tile of this CTA.  PAIR: every CTA loads its own box and its half of the B tile, and the
+// leader's barriers count the bytes of both CTAs.
+template <bool PAIR>
+__device__ __forceinline__ void produce_box_groups(const ConvKParams& p, const ConvSmem& m, const CUtensorMap* tm_abox,
+                                                   const CUtensorMap* tm_b, int m0, int n0, int g0, int g1,
+                                                   uint32_t box_stride, uint32_t box_bytes, uint32_t b_bytes,
+                                                   bool leader, Pipe& pp) {
+  const int block_k = PAIR ? 64 : p.block_k;
+  for (int g = g0; g < g1; ++g) {
+    const int dy = g / p.kb_per_tap, cb = g - dy * p.kb_per_tap;
+    ptx::mbar_wait(&m.aempty_bar[pp.sa], pp.pha ^ 1u);
+    if (leader) ptx::mbar_arrive_expect_tx(&m.afull_bar[pp.sa], PAIR ? 2 * box_bytes : box_bytes);
+    uint8_t* box = m.tiles + (size_t)pp.sa * box_stride;
+    const int box_row = m0 + (dy - 1) * p.Wp - 1;
+    if (PAIR) ptx::tma_load_2d_pair(box, tm_abox, &m.afull_bar[pp.sa], cb * block_k, box_row);
+    else ptx::tma_load_2d(box, tm_abox, &m.afull_bar[pp.sa], cb * block_k, box_row);
+    pp.next_box();
+    for (int dx = 0; dx < 3; ++dx) {
+      const int kb = (dy * 3 + dx) * p.kb_per_tap + cb;
+      ptx::mbar_wait(&m.empty_bar[pp.s], pp.phase ^ 1u);
+      if (leader) ptx::mbar_arrive_expect_tx(&m.full_bar[pp.s], PAIR ? 2 * b_bytes : b_bytes);
+      uint8_t* b_dst = m.b_ring + (size_t)pp.s * b_bytes;
+      if (PAIR) ptx::tma_load_2d_pair(b_dst, tm_b, &m.full_bar[pp.s], kb * block_k, n0);
+      else ptx::tma_load_2d(b_dst, tm_b, &m.full_bar[pp.s], kb * block_k, n0);
+      pp.next_b();
+    }
+  }
+}
+
+template <bool PAIR>
+__device__ __forceinline__ void umma_commit_both(uint64_t* bar) {  // PAIR: on this barrier in both CTAs
+  if (PAIR) ptx::umma_commit_pair(bar);
+  else ptx::umma_commit(bar);
+}
+
+// MMA issue of one tile, K groups [g0, g1), into the next accumulator stage (ti: tiles this CTA issued before, for
+// tracing).  The WHOLE warp walks the loop (warp-uniform control flow and operands, so descriptors live in uniform
+// registers) and one elected lane issues the tcgen05 instructions.  With the loop inside `if (lane == 0)` the compiler
+// wraps every UTCHMMA in a vote/R2UR.BROADCAST loop (~25 instructions), and that single thread's issue rate — not the
+// tensor pipe — bounds the k-block time.
+template <bool PAIR>
+__device__ __forceinline__ void mma_box_unit(const ConvKParams& p, const ConvSmem& m, uint32_t tmem_base, int g0,
+                                             int g1, uint32_t box_stride, uint32_t b_bytes, Pipe& pp, int ti) {
+  const int lane = threadIdx.x & 31;
+  ptx::mbar_wait(&m.tmem_empty_bar[pp.as], pp.aphase ^ 1u);  // the epilogue has drained this accumulator stage
+  ptx::tc_fence_after();
+  const uint32_t tmem_acc = tmem_base + (uint32_t)(pp.as * p.acc_stride);
+  const bool k64 = PAIR || p.block_k == 64;
+  // (copied out of the parameters once: the asm statements below clobber memory, which would reload them per MMA)
+  const int kbt = p.kb_per_tap, lks = p.last_ksteps;
+  const uint32_t idesc = p.idesc;
+  for (int g = g0; g < g1; ++g) {
+    // K steps beyond the layer's real channels multiply TMA zero fill by zero weights: not issued
+    const int nk = (g % kbt == kbt - 1) ? lks : (k64 ? 4 : 2);
+    ptx::mbar_wait(&m.afull_bar[pp.sa], pp.pha);
+    if (ti == 0 && g == g0 && lane == 0) conv_stamp(p, 4);
+    const uint32_t a_addr = ptx::smem_u32(m.tiles + (size_t)pp.sa * box_stride);
+    for (int dx = 0; dx < 3; ++dx) {
+      ptx::mbar_wait(&m.full_bar[pp.s], pp.phase);
+      ptx::tc_fence_after();
+      const uint32_t b_addr = ptx::smem_u32(m.b_ring + (size_t)pp.s * b_bytes);
+      // the window of tap dx starts dx rows (dx * 128 B) into the box.  The start is then not aligned to the
+      // 1024-byte swizzle pattern; measured on B200: the tensor core applies the 128-byte swizzle to the absolute
+      // shared-memory address (as TMA did when it wrote the box), so the descriptor's base-offset field must stay
+      // 0 — setting it to dx (or 8-dx) reads garbage (tools/debug_share.py)
+      // (32-wide k-blocks: the same holds for the 64-byte swizzle — rows of 64 B, window dx starts dx * 64 B in)
+      const uint64_t adesc = k64 ? ptx::make_sw128_kmajor_desc(a_addr + (uint32_t)dx * 128u)
+                                 : ptx::make_sw64_kmajor_desc(a_addr + (uint32_t)dx * 64u);
+      const uint64_t bdesc = k64 ? ptx::make_sw128_kmajor_desc(b_addr) : ptx::make_sw64_kmajor_desc(b_addr);
+      if (ptx::elect_one()) {
+        // (compile-time trip count with a per-step predicate: this issue loop is on the critical path, a
+        //  run-time trip count costs the narrow-Cin layers ~4 us each)
+#pragma unroll
+        for (int k = 0; k < 4; ++k) {
+          // advance 16 bf16 = 32 B along K inside the swizzle row: +2 in the (addr>>4) field
+          const uint32_t acc = (g > g0 || dx > 0 || k > 0) ? 1u : 0u;
+          if (k < nk) {
+            if (PAIR) ptx::umma_bf16_ss_pair(tmem_acc, adesc + (uint64_t)(2 * k), bdesc + (uint64_t)(2 * k), idesc, acc);
+            else ptx::umma_bf16_ss(tmem_acc, adesc + (uint64_t)(2 * k), bdesc + (uint64_t)(2 * k), idesc, acc);
+          }
+        }
+        umma_commit_both<PAIR>(&m.empty_bar[pp.s]);
+        if (dx == 2) umma_commit_both<PAIR>(&m.aempty_bar[pp.sa]);  // the box may be refilled once its three taps retire
+        if (dx == 2 && g == g1 - 1) umma_commit_both<PAIR>(&m.tmem_full_bar[pp.as]);
+      }
+      __syncwarp();
+      pp.next_b();
+    }
+    pp.next_box();
+  }
+  if (lane == 0 && ti < 6) conv_stamp(p, 5 + ti);
+  pp.next_acc();
+}
+
+// ---------------------------------------------------------------------------------------------------------------
+// Epilogue of one accumulator tile (warps 2..5: warp w owns TMEM lanes / tile rows 32*(w & 3) .. +31).
 
 // 16 accumulator columns of one row: y = acc*scale + shift (-> leaky) ; rows outside the image become 0.
 template <bool LEAKY>
@@ -106,6 +313,16 @@ __device__ __forceinline__ void scale_act16(const uint32_t (&r)[16], const float
     if (LEAKY) v[j] = fmaxf(v[j], 0.1f * v[j]);
     v[j] = interior ? v[j] : 0.f;
   }
+}
+
+// 8 fp32 -> 8 bf16 (round to nearest even) in one 16-byte word
+__device__ __forceinline__ uint4 pack8_bf16(const float* v) {
+  const __nv_bfloat162 h0 = __floats2bfloat162_rn(v[0], v[1]);
+  const __nv_bfloat162 h1 = __floats2bfloat162_rn(v[2], v[3]);
+  const __nv_bfloat162 h2 = __floats2bfloat162_rn(v[4], v[5]);
+  const __nv_bfloat162 h3 = __floats2bfloat162_rn(v[6], v[7]);
+  return make_uint4(*reinterpret_cast<const uint32_t*>(&h0), *reinterpret_cast<const uint32_t*>(&h1),
+                    *reinterpret_cast<const uint32_t*>(&h2), *reinterpret_cast<const uint32_t*>(&h3));
 }
 
 template <int MODE>
@@ -130,16 +347,7 @@ __device__ __forceinline__ void store16(const ConvKParams& p, const float (&v)[1
         float w[8];
 #pragma unroll
         for (int j = 0; j < 8; ++j) w[j] = (full || n + j < p.N) ? v[g * 8 + j] : 0.f;
-        __nv_bfloat162 h0 = __floats2bfloat162_rn(w[0], w[1]);
-        __nv_bfloat162 h1 = __floats2bfloat162_rn(w[2], w[3]);
-        __nv_bfloat162 h2 = __floats2bfloat162_rn(w[4], w[5]);
-        __nv_bfloat162 h3 = __floats2bfloat162_rn(w[6], w[7]);
-        uint4 pk;
-        pk.x = *reinterpret_cast<uint32_t*>(&h0);
-        pk.y = *reinterpret_cast<uint32_t*>(&h1);
-        pk.z = *reinterpret_cast<uint32_t*>(&h2);
-        pk.w = *reinterpret_cast<uint32_t*>(&h3);
-        *reinterpret_cast<uint4*>(out_bf + n) = pk;
+        *reinterpret_cast<uint4*>(out_bf + n) = pack8_bf16(w);
       } else {
 #pragma unroll
         for (int j = 0; j < 8; ++j)
@@ -152,36 +360,15 @@ __device__ __forceinline__ void store16(const ConvKParams& p, const float (&v)[1
 // 16 fp32 -> 16 bf16 -> two 16-byte shared-memory stores
 __device__ __forceinline__ void pack16_to_smem(const float (&v)[16], uint8_t* dst) {
 #pragma unroll
-  for (int g = 0; g < 2; ++g) {
-    __nv_bfloat162 h0 = __floats2bfloat162_rn(v[g * 8 + 0], v[g * 8 + 1]);
-    __nv_bfloat162 h1 = __floats2bfloat162_rn(v[g * 8 + 2], v[g * 8 + 3]);
-    __nv_bfloat162 h2 = __floats2bfloat162_rn(v[g * 8 + 4], v[g * 8 + 5]);
-    __nv_bfloat162 h3 = __floats2bfloat162_rn(v[g * 8 + 6], v[g * 8 + 7]);
-    uint4 pk;
-    pk.x = *reinterpret_cast<uint32_t*>(&h0);
-    pk.y = *reinterpret_cast<uint32_t*>(&h1);
-    pk.z = *reinterpret_cast<uint32_t*>(&h2);
-    pk.w = *reinterpret_cast<uint32_t*>(&h3);
-    *reinterpret_cast<uint4*>(dst + g * 16) = pk;
-  }
+  for (int g = 0; g < 2; ++g) *reinterpret_cast<uint4*>(dst + g * 16) = pack8_bf16(v + g * 8);
 }
 
 // 16 fp32 -> 16 bf16 -> the two 16-byte chunks (index chunk, chunk + 1) of this lane's 128-byte row of a TMA store
 // slab.  The slab has the tensor map's 128-byte swizzle: chunk j of row r sits at chunk position j ^ (r & 7).
 __device__ __forceinline__ void pack16_to_slab(const float (&v)[16], uint8_t* row, int chunk, int lane) {
 #pragma unroll
-  for (int g = 0; g < 2; ++g) {
-    __nv_bfloat162 h0 = __floats2bfloat162_rn(v[g * 8 + 0], v[g * 8 + 1]);
-    __nv_bfloat162 h1 = __floats2bfloat162_rn(v[g * 8 + 2], v[g * 8 + 3]);
-    __nv_bfloat162 h2 = __floats2bfloat162_rn(v[g * 8 + 4], v[g * 8 + 5]);
-    __nv_bfloat162 h3 = __floats2bfloat162_rn(v[g * 8 + 6], v[g * 8 + 7]);
-    uint4 pk;
-    pk.x = *reinterpret_cast<uint32_t*>(&h0);
-    pk.y = *reinterpret_cast<uint32_t*>(&h1);
-    pk.z = *reinterpret_cast<uint32_t*>(&h2);
-    pk.w = *reinterpret_cast<uint32_t*>(&h3);
-    *reinterpret_cast<uint4*>(row + (((chunk + g) ^ (lane & 7)) << 4)) = pk;
-  }
+  for (int g = 0; g < 2; ++g)
+    *reinterpret_cast<uint4*>(row + (((chunk + g) ^ (lane & 7)) << 4)) = pack8_bf16(v + g * 8);
 }
 
 // Batch statistics from a finished 32-row x 64-column slab: lane L owns columns 2L, 2L+1 (one 4-byte word per row: the
@@ -215,20 +402,144 @@ __device__ __forceinline__ void flush_stats(const ConvKParams& p, float* acc, in
   __syncwarp();
 }
 
+// scale/shift of columns [n0, n0 + block_n) -> dst[i] / dst[256 + i], zeros beyond Npad (the 128 epilogue threads)
+__device__ __forceinline__ void stage_scale_shift(const ConvKParams& p, float* dst, int n0) {
+  for (int i = (int)threadIdx.x - 64; i < p.block_n; i += 128) {
+    const bool ok = (n0 + i) < p.Npad;
+    dst[i] = ok ? __ldg(p.scale + n0 + i) : 0.f;
+    dst[256 + i] = ok ? __ldg(p.shift + n0 + i) : 0.f;
+  }
+}
+
+// this warp has finished reading the accumulator stage: hand it back to the MMA issuer (PAIR: on the leader CTA's
+// barrier, where the MMA issuer waits for the epilogues of both CTAs)
+template <bool PAIR>
+__device__ __forceinline__ void release_acc_stage(uint64_t* empty_bar) {
+  ptx::tc_fence_before();
+  __syncwarp();
+  if ((threadIdx.x & 31) == 0) {
+    if (PAIR) ptx::mbar_arrive_leader(empty_bar);
+    else ptx::mbar_arrive(empty_bar);
+  }
+}
+
+// Start of an epilogue loop.  Batch statistics: zero this warp's accumulators behind the TMA-store slabs (returned;
+// flushed whenever the N tile changes and at the end).  One N tile: every tile of the launch uses the same
+// scale/shift slice, staged once (a narrow layer's epilogue is otherwise a chain of global-load latency + barrier per
+// 128 rows).
+template <int MODE>
+__device__ __forceinline__ float* epilogue_begin(const ConvKParams& p, const ConvSmem& m, bool one_n_tile) {
+  float* stat_acc = nullptr;
+  if (MODE == MC_EPI_PNHWC && p.tma_bufs > 0 && p.stat_sum != nullptr) {
+    stat_acc = reinterpret_cast<float*>(m.s_out + (size_t)4 * p.tma_bufs * 4096) + ((threadIdx.x >> 5) & 3) * 512;
+    for (int c = threadIdx.x & 31; c < 512; c += 32) stat_acc[c] = 0.f;
+    __syncwarp();
+  }
+  if (one_n_tile) {
+    stage_scale_shift(p, m.s_ss, 0);
+    asm volatile("bar.sync 1, 128;" ::: "memory");
+  }
+  return stat_acc;
+}
+
+template <int MODE>
+__device__ __forceinline__ void epilogue_end(const ConvKParams& p, float* stat_acc, int stat_n0) {
+  const int lane = threadIdx.x & 31;
+  if (stat_acc != nullptr && stat_n0 >= 0) flush_stats(p, stat_acc, stat_n0, lane);
+  if (MODE == MC_EPI_PNHWC && p.tma_bufs > 0 && lane == 0) ptx::bulk_wait_group_read<0>();  // slabs read before the CTA exits
+}
+
+// One accumulator tile as this thread sees it: its row, its pixel and where its outputs go
+struct EpiTile {
+  const float* sc;   // scale of the tile's columns in shared memory; the shift follows at sc + 256
+  uint32_t taddr;    // TMEM address of this warp's 32 lanes in the accumulator stage
+  int n0, row0;      // first column; first row of this warp's 32
+  int x, y, b;       // this thread's pixel (x >= W or y >= H: pad row)
+  bool in_buf, interior, do_store;
+  long long out_row_base;
+};
+
+// Start of one tile in the epilogue: stage its scale/shift (unless staged once for the launch), decode the row ->
+// (b, y, x) by magic-number division, address the output for the store mode and wait for the accumulator stage `as`.
+// ti: tiles this CTA's epilogue did before (tracing).
+template <int MODE>
+__device__ __forceinline__ EpiTile epi_tile_begin(const ConvKParams& p, const ConvSmem& m, uint32_t tmem_base,
+                                                  bool one_n_tile, int m0, int n0, int as, uint32_t aphase, int ti) {
+  const int quarter = (threadIdx.x >> 5) & 3;  // TMEM lane quarter this warp may access
+  EpiTile t;
+  float* sc = m.s_ss + (one_n_tile ? 0 : as * 512);
+  if (!one_n_tile) stage_scale_shift(p, sc, n0);
+  t.sc = sc;
+  t.n0 = n0;
+  t.row0 = m0 + quarter * 32;
+  const int row = t.row0 + (threadIdx.x & 31);
+  const int q = (int)(__umulhi((unsigned int)row, p.wp_mul) >> p.wp_shr);  // row / Wp
+  t.x = row - q * p.Wp;
+  t.b = (int)(__umulhi((unsigned int)q, p.hp_mul) >> p.hp_shr);            // (row / Wp) / Hp
+  t.y = q - t.b * p.Hp;
+  t.in_buf = row < p.M_rows;
+  t.interior = t.in_buf && (t.x < p.W) && (t.y < p.H);
+  if (MODE == MC_EPI_PNHWC) {
+    t.out_row_base = (long long)row * p.ldc + p.ch_off;
+    t.do_store = t.in_buf;  // pad rows are written as zeros to keep the layout invariant
+  } else if (MODE == MC_EPI_REORG2) {
+    const int Wo = p.W / 2 + 1, Ho = p.H / 2 + 1;
+    const long long orow = ((long long)t.b * Ho + (t.y >> 1)) * Wo + (t.x >> 1);
+    t.out_row_base = orow * p.ldc + p.ch_off + ((t.y & 1) * 2 + (t.x & 1)) * p.N;
+    t.do_store = t.interior;
+  } else {  // MC_EPI_NCHW_F32 (+ n*H*W); MC_EPI_DECODE addresses its outputs itself
+    t.out_row_base = ((long long)t.b * p.N * p.H + t.y) * p.W + t.x;
+    t.do_store = t.interior;
+  }
+  if (!one_n_tile) asm volatile("bar.sync 1, 128;" ::: "memory");  // scale/shift of this tile visible to the 4 warps
+
+  ptx::mbar_wait(&m.tmem_full_bar[as], aphase);
+  ptx::tc_fence_after();
+  if (threadIdx.x == 64 && ti < 8) conv_stamp(p, 12 + 2 * ti);
+  t.taddr = tmem_base + ((uint32_t)(quarter * 32) << 16) + (uint32_t)(as * p.acc_stride);
+  return t;
+}
+
+// Direct stores of accumulator columns [c_begin, block_n), 32 at a time: a thread writes its own row.  add(r, col)
+// runs on the raw accumulator first (a stream-K finisher adds the partial accumulators there; otherwise a no-op).
+template <int MODE, bool LEAKY, typename AddFn>
+__device__ __forceinline__ void store_cols_direct(const ConvKParams& p, const EpiTile& t, int c_begin, bool vec_ok,
+                                                  AddFn& add) {
+  const float* sc = t.sc;
+  const float* sh = t.sc + 256;
+  for (int c0 = c_begin; c0 < p.block_n; c0 += 32) {
+    uint32_t r0[16], r1[16];
+    const bool two = c0 + 16 < p.block_n;
+    ptx::tmem_ld_32x32b_x16(t.taddr + (uint32_t)c0, r0);
+    if (two) ptx::tmem_ld_32x32b_x16(t.taddr + (uint32_t)(c0 + 16), r1);
+    ptx::tmem_ld_wait();
+    if (!t.do_store) continue;
+    add(r0, c0);
+    if (two) add(r1, c0 + 16);
+    float v[16];
+    scale_act16<LEAKY>(r0, sc + c0, sh + c0, t.interior, v);
+    store16<MODE>(p, v, t.n0 + c0, t.out_row_base, vec_ok);
+    if (two) {
+      scale_act16<LEAKY>(r1, sc + c0 + 16, sh + c0 + 16, t.interior, v);
+      store16<MODE>(p, v, t.n0 + c0 + 16, t.out_row_base, vec_ok);
+    }
+  }
+}
+
 // PNHWC epilogue of one accumulator tile through TMA stores.  A warp owns 32 rows; every whole 64-column chunk of the
 // tile is converted into the warp's 4 KB slab (32 rows x 128 B, swizzled like the tensor map of the output) and leaves
 // as ONE bulk tensor store — 128-byte rows, issued by one lane, asynchronous — instead of 16-byte pieces one row pitch
 // apart per thread (measured: ~38 cycles per output column and tile, 4..7.6 us for a 208..256-wide tile, which
 // throttles short-K layers and is exposed after the last tile of every CTA).  With two slabs per warp the conversion of
 // chunk i+1 overlaps the store of chunk i.  The tile's last block_n % 64 columns take direct stores; rows and columns
-// outside the output tensor are clipped by TMA.  add(r, col) lets a stream-K finisher add partial accumulators.
-template <bool LEAKY, bool PAIR, bool WIDE_LD, typename AddFn>
-__device__ __forceinline__ void epilogue_tile_tma(const ConvKParams& p, const CUtensorMap* tm_out, uint32_t taddr_row,
-                                                  const float* sc, const float* sh, bool interior, bool in_buf,
-                                                  int row0, int n0, long long out_row_base, bool vec_ok, uint8_t* slab,
-                                                  int& buf, uint64_t* empty_bar, AddFn add, float* stat_acc = nullptr) {
+// outside the output tensor are clipped by TMA.
+template <bool LEAKY, bool WIDE_LD, typename AddFn>
+__device__ __forceinline__ void epilogue_tile_tma(const ConvKParams& p, const CUtensorMap* tm_out, const EpiTile& t,
+                                                  bool vec_ok, uint8_t* slab, int& buf, AddFn& add, float* stat_acc) {
   const int lane = threadIdx.x & 31;
-  int cols_valid = ((p.N - n0 + 7) >> 3) << 3;  // whole 8-groups up to the last one holding a real channel
+  const float* sc = t.sc;
+  const float* sh = t.sc + 256;
+  int cols_valid = ((p.N - t.n0 + 7) >> 3) << 3;  // whole 8-groups up to the last one holding a real channel
   if (cols_valid > p.block_n) cols_valid = p.block_n;
   const int full_cols = p.block_n & ~63;
   for (int cc = 0; cc < full_cols && cc < cols_valid; cc += 64) {
@@ -243,159 +554,86 @@ __device__ __forceinline__ void epilogue_tile_tma(const ConvKParams& p, const CU
       // all 64 columns of the chunk in flight before the one wait (register budget of the 1-CTA-per-SM variants)
       uint32_t r[4][16];
 #pragma unroll
-      for (int q = 0; q < 4; ++q) ptx::tmem_ld_32x32b_x16(taddr_row + (uint32_t)(cc + 16 * q), r[q]);
+      for (int q = 0; q < 4; ++q) ptx::tmem_ld_32x32b_x16(t.taddr + (uint32_t)(cc + 16 * q), r[q]);
       ptx::tmem_ld_wait();
 #pragma unroll
       for (int q = 0; q < 4; ++q) {
         add(r[q], cc + 16 * q);
         float v[16];
-        scale_act16<LEAKY>(r[q], sc + cc + 16 * q, sh + cc + 16 * q, interior, v);
+        scale_act16<LEAKY>(r[q], sc + cc + 16 * q, sh + cc + 16 * q, t.interior, v);
         pack16_to_slab(v, mine, 2 * q, lane);
       }
     } else {
 #pragma unroll
       for (int h = 0; h < 2; ++h) {
         uint32_t r0[16], r1[16];
-        ptx::tmem_ld_32x32b_x16(taddr_row + (uint32_t)(cc + 32 * h), r0);
-        ptx::tmem_ld_32x32b_x16(taddr_row + (uint32_t)(cc + 32 * h + 16), r1);
+        ptx::tmem_ld_32x32b_x16(t.taddr + (uint32_t)(cc + 32 * h), r0);
+        ptx::tmem_ld_32x32b_x16(t.taddr + (uint32_t)(cc + 32 * h + 16), r1);
         ptx::tmem_ld_wait();
         add(r0, cc + 32 * h);
         add(r1, cc + 32 * h + 16);
         float v[16];
-        scale_act16<LEAKY>(r0, sc + cc + 32 * h, sh + cc + 32 * h, interior, v);
+        scale_act16<LEAKY>(r0, sc + cc + 32 * h, sh + cc + 32 * h, t.interior, v);
         pack16_to_slab(v, mine, 4 * h, lane);
-        scale_act16<LEAKY>(r1, sc + cc + 32 * h + 16, sh + cc + 32 * h + 16, interior, v);
+        scale_act16<LEAKY>(r1, sc + cc + 32 * h + 16, sh + cc + 32 * h + 16, t.interior, v);
         pack16_to_slab(v, mine, 4 * h + 2, lane);
       }
     }
     ptx::fence_proxy_async_smem();  // this lane's slab writes -> visible to the TMA (async proxy)
     __syncwarp();
     if (lane == 0) {
-      ptx::tma_store_2d(tm_out, sb, n0 + cc, row0);
+      ptx::tma_store_2d(tm_out, sb, t.n0 + cc, t.row0);
       ptx::bulk_commit_group();
     }
     if (stat_acc != nullptr) slab_stats(sb, stat_acc, cc, lane);
     if (p.tma_bufs >= 2) buf ^= 1;
   }
-  for (int c0 = full_cols; c0 < p.block_n; c0 += 32) {
-    uint32_t r0[16], r1[16];
-    const bool two = c0 + 16 < p.block_n;
-    ptx::tmem_ld_32x32b_x16(taddr_row + (uint32_t)c0, r0);
-    if (two) ptx::tmem_ld_32x32b_x16(taddr_row + (uint32_t)(c0 + 16), r1);
-    ptx::tmem_ld_wait();
-    if (!in_buf) continue;
-    add(r0, c0);
-    if (two) add(r1, c0 + 16);
-    float v[16];
-    scale_act16<LEAKY>(r0, sc + c0, sh + c0, interior, v);
-    store16<MC_EPI_PNHWC>(p, v, n0 + c0, out_row_base, vec_ok);
-    if (two) {
-      scale_act16<LEAKY>(r1, sc + c0 + 16, sh + c0 + 16, interior, v);
-      store16<MC_EPI_PNHWC>(p, v, n0 + c0 + 16, out_row_base, vec_ok);
-    }
-  }
-  // this warp has finished reading the accumulator stage: hand it back to the MMA issuer
-  ptx::tc_fence_before();
-  __syncwarp();
-  if (lane == 0) {
-    if (PAIR) ptx::mbar_arrive_leader(empty_bar);
-    else ptx::mbar_arrive(empty_bar);
-  }
+  store_cols_direct<MC_EPI_PNHWC, LEAKY>(p, t, full_cols, vec_ok, add);
 }
 
-// Epilogue warps (threads 64..191): per tile, stage the tile's scale/shift in shared memory (double-buffered with
-// the accumulator stage, one named barrier per tile), then drain the accumulator 32 columns at a time.
-// PAIR (CTA-pair kernel): `tile` counts (m-tile pair, n-tile) units of the cluster, this CTA owns m-tile 2*pair + rank,
-// and the accumulator stage is handed back on the LEADER CTA's barrier (the MMA issuer waits for both epilogues).
-template <int MODE, bool LEAKY, bool PAIR = false, bool WIDE_LD = false>
-__device__ __forceinline__ void epilogue_loop(const ConvKParams& p, uint32_t tmem_base, uint64_t* tmem_full_bar,
-                                              uint64_t* tmem_empty_bar, float* s_ss, uint8_t* s_out = nullptr,
-                                              const CUtensorMap* tm_out = nullptr,
-                                              int tile0 = -1, int tile_step = 0, int total_units = 0, int pair_rank = 0) {
-  const int warp_idx = threadIdx.x >> 5;
+// Scale/shift/leaky and store of one accumulator tile in both kernels — TMA stores (PNHWC, p.tma_bufs > 0) or direct
+// stores — then the stage goes back to the MMA issuer.  add(r, col): see store_cols_direct.  slab_buf, stat_acc and
+// stat_n0 are the warp's TMA-store slab and batch-statistics state across tiles.
+template <int MODE, bool LEAKY, bool PAIR, bool WIDE_LD, typename AddFn>
+__device__ __forceinline__ void epilogue_tile(const ConvKParams& p, const CUtensorMap* tm_out, const ConvSmem& m,
+                                              const EpiTile& t, bool vec_ok, uint64_t* empty_bar, int& slab_buf,
+                                              float* stat_acc, int& stat_n0, AddFn add) {
+  if (MODE == MC_EPI_PNHWC && p.tma_bufs > 0) {
+    if (stat_acc != nullptr && t.n0 != stat_n0) {
+      if (stat_n0 >= 0) flush_stats(p, stat_acc, stat_n0, threadIdx.x & 31);
+      stat_n0 = t.n0;
+    }
+    uint8_t* slab = m.s_out + (size_t)((threadIdx.x >> 5) & 3) * p.tma_bufs * 4096;
+    epilogue_tile_tma<LEAKY, WIDE_LD>(p, tm_out, t, vec_ok, slab, slab_buf, add, stat_acc);
+  } else {
+    store_cols_direct<MODE, LEAKY>(p, t, 0, vec_ok, add);
+  }
+  release_acc_stage<PAIR>(empty_bar);
+}
+
+// Epilogue warps (threads 64..191) of the single-CTA kernel: tiles blockIdx.x, + gridDim.x, ...  Besides the TMA-store
+// and direct paths of epilogue_tile, PNHWC tiles without TMA stores take the staged store where the planner gave them a
+// staging buffer (p.out_pitch > 0), and the head takes the decode.
+template <int MODE, bool LEAKY, bool WIDE_LD = false>
+__device__ __forceinline__ void epilogue_loop(const ConvKParams& p, const ConvSmem& m, uint32_t tmem_base,
+                                              const CUtensorMap* tm_out) {
   const int lane = threadIdx.x & 31;
-  const int et = threadIdx.x - 64;   // 0..127
-  const int quarter = warp_idx & 3;  // TMEM lane quarter this warp may access
-  const int total_tiles = PAIR ? total_units : p.m_tiles * p.n_tiles;
-  if (!PAIR) { tile0 = blockIdx.x; tile_step = gridDim.x; }
+  const int quarter = (threadIdx.x >> 5) & 3;
+  const int total_tiles = p.m_tiles * p.n_tiles;
   const bool vec_ok = ((p.ldc | p.ch_off) & 7) == 0 && (MODE != MC_EPI_REORG2 || (p.N & 7) == 0);
+  const bool one_n_tile = p.n_tiles == 1;
+  float* stat_acc = epilogue_begin<MODE>(p, m, one_n_tile);
+  int stat_n0 = -1;
+  int slab_buf = 0;  // (TMA-store epilogue) slab of this warp the next chunk goes to
   int as = 0;
   uint32_t aphase = 0;
-  int slab_buf = 0;  // (TMA-store epilogue) slab of this warp the next chunk goes to
-  // (batch statistics) this warp's accumulators behind the slabs; flushed whenever the N tile changes and at the end
-  float* stat_acc = nullptr;
-  int stat_n0 = -1;
-  if (MODE == MC_EPI_PNHWC && p.tma_bufs > 0 && p.stat_sum != nullptr) {
-    stat_acc = reinterpret_cast<float*>(s_out + (size_t)4 * p.tma_bufs * 4096) + quarter * 512;
-    for (int c = lane; c < 512; c += 32) stat_acc[c] = 0.f;
-    __syncwarp();
-  }
-  // one N tile: every tile of the launch uses the same scale/shift slice, staged once (a narrow layer's epilogue is
-  // otherwise a chain of global-load latency + barrier per 128 rows)
-  const bool one_n_tile = p.n_tiles == 1;
-  if (one_n_tile) {
-    for (int i = et; i < p.block_n; i += 128) {
-      const bool ok = i < p.Npad;
-      s_ss[i] = ok ? __ldg(p.scale + i) : 0.f;
-      s_ss[256 + i] = ok ? __ldg(p.shift + i) : 0.f;
-    }
-    asm volatile("bar.sync 1, 128;" ::: "memory");
-  }
   int ti = 0;  // (tracing) tiles done by this CTA
-  for (int tile = tile0; tile < total_tiles; tile += tile_step, ++ti) {
+  for (int tile = blockIdx.x; tile < total_tiles; tile += gridDim.x, ++ti) {
     const int n0 = (tile % p.n_tiles) * p.block_n;
-    const int m0 = (PAIR ? 2 * (tile / p.n_tiles) + pair_rank : tile / p.n_tiles) * BLOCK_M;
-    float* sc = s_ss + (one_n_tile ? 0 : as * 512);
-    float* sh = sc + 256;
-    if (!one_n_tile) {
-      for (int i = et; i < p.block_n; i += 128) {
-        const bool ok = (n0 + i) < p.Npad;
-        sc[i] = ok ? __ldg(p.scale + n0 + i) : 0.f;
-        sh[i] = ok ? __ldg(p.shift + n0 + i) : 0.f;
-      }
-    }
-    const int row = m0 + quarter * 32 + lane;
-    const int t = (int)(__umulhi((unsigned int)row, p.wp_mul) >> p.wp_shr);  // row / Wp (magic-number division)
-    const int x = row - t * p.Wp;
-    const int b = (int)(__umulhi((unsigned int)t, p.hp_mul) >> p.hp_shr);    // t / Hp
-    const int y = t - b * p.Hp;
-    const bool in_buf = row < p.M_rows;
-    const bool interior = in_buf && (x < p.W) && (y < p.H);
-    long long out_row_base = 0;
-    bool do_store = false;
-    if (MODE == MC_EPI_PNHWC) {
-      out_row_base = (long long)row * p.ldc + p.ch_off;
-      do_store = in_buf;  // pad rows are written as zeros to keep the layout invariant
-    } else if (MODE == MC_EPI_REORG2) {
-      const int Wo = p.W / 2 + 1, Ho = p.H / 2 + 1;
-      const long long orow = ((long long)b * Ho + (y >> 1)) * Wo + (x >> 1);
-      out_row_base = orow * p.ldc + p.ch_off + ((y & 1) * 2 + (x & 1)) * p.N;
-      do_store = interior;
-    } else {  // MC_EPI_NCHW_F32
-      out_row_base = ((long long)b * p.N * p.H + y) * p.W + x;  // + n*H*W
-      do_store = interior;
-    }
-    if (!one_n_tile) asm volatile("bar.sync 1, 128;" ::: "memory");  // scale/shift of this tile visible to the 4 epilogue warps
+    const int m0 = (tile / p.n_tiles) * BLOCK_M;
+    const EpiTile t = epi_tile_begin<MODE>(p, m, tmem_base, one_n_tile, m0, n0, as, aphase, ti);
 
-    ptx::mbar_wait(&tmem_full_bar[as], aphase);
-    ptx::tc_fence_after();
-    if (!PAIR && et == 0 && ti < 8) conv_stamp(p, 12 + 2 * ti);
-    const uint32_t taddr_row = tmem_base + ((uint32_t)(quarter * 32) << 16) + (uint32_t)(as * p.acc_stride);
-
-    if (MODE == MC_EPI_PNHWC && p.tma_bufs > 0) {
-      if (stat_acc != nullptr && n0 != stat_n0) {
-        if (stat_n0 >= 0) flush_stats(p, stat_acc, stat_n0, lane);
-        stat_n0 = n0;
-      }
-      epilogue_tile_tma<LEAKY, PAIR, WIDE_LD>(p, tm_out, taddr_row, sc, sh, interior, in_buf, m0 + quarter * 32, n0, out_row_base,
-                                     vec_ok, s_out + (size_t)quarter * p.tma_bufs * 4096, slab_buf, &tmem_empty_bar[as],
-                                     [](uint32_t (&)[16], int) {}, stat_acc);
-      if (!PAIR && et == 0 && ti < 8) conv_stamp(p, 13 + 2 * ti);
-      if (++as == ACC_STAGES) { as = 0; aphase ^= 1u; }
-      continue;
-    }
-
-    if (MODE == MC_EPI_PNHWC && s_out != nullptr) {
+    if (MODE == MC_EPI_PNHWC && p.tma_bufs == 0 && p.out_pitch > 0) {
       // Staged store: a thread owns one output ROW, so direct stores are 16-byte pieces one row pitch apart (32 half-
       // filled sectors per warp instruction: measured ~38 cycles per output column and tile).  Instead the warp parks
       // its 32 rows x block_n bf16 in shared memory (pitch +16 B: conflict-free), hands the TMEM stage back at once,
@@ -403,9 +641,8 @@ __device__ __forceinline__ void epilogue_loop(const ConvKParams& p, uint32_t tme
       // Tiles wider than the staging buffer (64 columns) go through it in 64-column chunks.
       const int pitch = p.out_pitch;
       const int chunk = p.out_chunk;
-      uint8_t* wbuf = s_out + (size_t)quarter * 32 * pitch;
+      uint8_t* wbuf = m.s_out + (size_t)quarter * 32 * pitch;
       uint8_t* mine = wbuf + (size_t)lane * pitch;
-      const int row0 = m0 + quarter * 32;
       int cols_left = ((p.N - n0 + 7) >> 3) << 3;  // whole 8-groups up to the last one holding a real channel
       if (cols_left > p.block_n) cols_left = p.block_n;
       for (int cc = 0; cc < p.block_n; cc += chunk) {
@@ -413,27 +650,19 @@ __device__ __forceinline__ void epilogue_loop(const ConvKParams& p, uint32_t tme
         for (int c0 = 0; c0 < cw; c0 += 32) {
           uint32_t r0[16], r1[16];
           const bool two = c0 + 16 < cw;
-          ptx::tmem_ld_32x32b_x16(taddr_row + (uint32_t)(cc + c0), r0);
-          if (two) ptx::tmem_ld_32x32b_x16(taddr_row + (uint32_t)(cc + c0 + 16), r1);
+          ptx::tmem_ld_32x32b_x16(t.taddr + (uint32_t)(cc + c0), r0);
+          if (two) ptx::tmem_ld_32x32b_x16(t.taddr + (uint32_t)(cc + c0 + 16), r1);
           ptx::tmem_ld_wait();
           float v[16];
-          scale_act16<LEAKY>(r0, sc + cc + c0, sh + cc + c0, interior, v);
+          scale_act16<LEAKY>(r0, t.sc + cc + c0, t.sc + 256 + cc + c0, t.interior, v);
           pack16_to_smem(v, mine + c0 * 2);
           if (two) {
-            scale_act16<LEAKY>(r1, sc + cc + c0 + 16, sh + cc + c0 + 16, interior, v);
+            scale_act16<LEAKY>(r1, t.sc + cc + c0 + 16, t.sc + 256 + cc + c0 + 16, t.interior, v);
             pack16_to_smem(v, mine + (c0 + 16) * 2);
           }
         }
-        if (cc + chunk >= p.block_n) {  // last chunk read: hand the TMEM stage back before the copy-out
-          ptx::tc_fence_before();
-          __syncwarp();
-          if (lane == 0) {
-            if (PAIR) ptx::mbar_arrive_leader(&tmem_empty_bar[as]);
-            else ptx::mbar_arrive(&tmem_empty_bar[as]);
-          }
-        } else {
-          __syncwarp();
-        }
+        if (cc + chunk >= p.block_n) release_acc_stage<false>(&m.tmem_empty_bar[as]);  // before the copy-out
+        else __syncwarp();
         int cols_w = cols_left - cc;
         if (cols_w > cw) cols_w = cw;
         if (cols_w > 0) {
@@ -442,8 +671,8 @@ __device__ __forceinline__ void epilogue_loop(const ConvKParams& p, uint32_t tme
           const int dr = 32 / cpr, dc = 32 - dr * cpr;
           __nv_bfloat16* obase = reinterpret_cast<__nv_bfloat16*>(p.out) + p.ch_off + n0 + cc;
           while (r < 32) {
-            if (row0 + r < p.M_rows)
-              *reinterpret_cast<uint4*>(obase + (long long)(row0 + r) * p.ldc + c * 8) =
+            if (t.row0 + r < p.M_rows)
+              *reinterpret_cast<uint4*>(obase + (long long)(t.row0 + r) * p.ldc + c * 8) =
                   *reinterpret_cast<const uint4*>(wbuf + (size_t)r * pitch + c * 16);
             r += dr; c += dc;
             if (c >= cpr) { c -= cpr; ++r; }
@@ -451,31 +680,25 @@ __device__ __forceinline__ void epilogue_loop(const ConvKParams& p, uint32_t tme
         }
         __syncwarp();  // wbuf is rewritten by the next chunk / tile
       }
-      if (!PAIR && et == 0 && ti < 8) conv_stamp(p, 13 + 2 * ti);
-      if (++as == ACC_STAGES) { as = 0; aphase ^= 1u; }
-      continue;
-    }
-
-    if (MODE == MC_EPI_DECODE) {
+    } else if (MODE == MC_EPI_DECODE) {
       // Region decode in the epilogue (get_region_boxes, src/nets2_utils.py:158-205).  The thread owns pixel (b, y, x):
       // its A*(5+nc) logits (= acc*scale + shift, the head's bias) are parked in the warp's shared-memory rows (row
       // pitch block_n+1 floats: lanes hit different banks), the TMEM stage goes back to the MMA issuer at once, and the
       // thread then decodes its A anchors from shared memory with the arithmetic of decode_math.cuh.
       const int pitch_f = p.block_n + 1;
-      float* mine = reinterpret_cast<float*>(s_out) + (size_t)(quarter * 32 + lane) * pitch_f;
+      float* mine = reinterpret_cast<float*>(m.s_out) + (size_t)(quarter * 32 + lane) * pitch_f;
       for (int c0 = 0; c0 < p.block_n; c0 += 16) {
         uint32_t r0[16];
-        ptx::tmem_ld_32x32b_x16(taddr_row + (uint32_t)c0, r0);
+        ptx::tmem_ld_32x32b_x16(t.taddr + (uint32_t)c0, r0);
         ptx::tmem_ld_wait();
         float v[16];
-        scale_act16<LEAKY>(r0, sc + c0, sh + c0, true, v);
+        scale_act16<LEAKY>(r0, t.sc + c0, t.sc + 256 + c0, true, v);
 #pragma unroll
         for (int j = 0; j < 16; ++j) mine[c0 + j] = v[j];
       }
-      ptx::tc_fence_before();
-      __syncwarp();
-      if (lane == 0) ptx::mbar_arrive(&tmem_empty_bar[as]);
-      if (interior) {
+      release_acc_stage<false>(&m.tmem_empty_bar[as]);
+      if (t.interior) {
+        const int x = t.x, y = t.y, b = t.b;
         const int A = p.dec_A, nc = p.dec_nc, F = 5 + p.dec_nc;
         const long long P = (long long)p.H * p.W * A;
         const long long slot0 = (long long)(y * p.W + x) * A;
@@ -499,37 +722,14 @@ __device__ __forceinline__ void epilogue_loop(const ConvKParams& p, uint32_t tme
         }
       }
       __syncwarp();  // the rows are rewritten by the next tile
-      if (++as == ACC_STAGES) { as = 0; aphase ^= 1u; }
-      continue;
+    } else {
+      epilogue_tile<MODE, LEAKY, false, WIDE_LD>(p, tm_out, m, t, vec_ok, &m.tmem_empty_bar[as], slab_buf, stat_acc,
+                                                 stat_n0, [](uint32_t (&)[16], int) {});
     }
-
-    for (int c0 = 0; c0 < p.block_n; c0 += 32) {
-      uint32_t r0[16], r1[16];
-      const bool two = c0 + 16 < p.block_n;
-      ptx::tmem_ld_32x32b_x16(taddr_row + (uint32_t)c0, r0);
-      if (two) ptx::tmem_ld_32x32b_x16(taddr_row + (uint32_t)(c0 + 16), r1);
-      ptx::tmem_ld_wait();
-      if (!do_store) continue;
-      float v[16];
-      scale_act16<LEAKY>(r0, sc + c0, sh + c0, interior, v);
-      store16<MODE>(p, v, n0 + c0, out_row_base, vec_ok);
-      if (two) {
-        scale_act16<LEAKY>(r1, sc + c0 + 16, sh + c0 + 16, interior, v);
-        store16<MODE>(p, v, n0 + c0 + 16, out_row_base, vec_ok);
-      }
-    }
-    // this warp has finished reading the accumulator stage: hand it back to the MMA issuer
-    ptx::tc_fence_before();
-    __syncwarp();
-    if (lane == 0) {
-      if (PAIR) ptx::mbar_arrive_leader(&tmem_empty_bar[as]);
-      else ptx::mbar_arrive(&tmem_empty_bar[as]);
-    }
-    if (!PAIR && et == 0 && ti < 8) conv_stamp(p, 13 + 2 * ti);
+    if (MODE != MC_EPI_DECODE && threadIdx.x == 64 && ti < 8) conv_stamp(p, 13 + 2 * ti);
     if (++as == ACC_STAGES) { as = 0; aphase ^= 1u; }
   }
-  if (stat_acc != nullptr && stat_n0 >= 0) flush_stats(p, stat_acc, stat_n0, lane);
-  if (MODE == MC_EPI_PNHWC && p.tma_bufs > 0 && lane == 0) ptx::bulk_wait_group_read<0>();  // slabs read before the CTA exits
+  epilogue_end<MODE>(p, stat_acc, stat_n0);
 }
 
 // Persistent: grid = min(#tiles, #SMs); CTA c works on tiles c, c+grid, ...  The smem ring runs across tiles, and the
@@ -544,188 +744,86 @@ conv_gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __gri
                          const __grid_constant__ CUtensorMap tmap_abox, const __grid_constant__ CUtensorMap tmap_out,
                          const ConvKParams p) {
   extern __shared__ __align__(1024) uint8_t smem_raw[];
-  // carve-up: [stages x (A 16KB | B block_n*128)] | barriers | tmem ptr | scale/shift staging (4 KB)
   const uint32_t a_tile_bytes = (uint32_t)(BLOCK_M * p.block_k * 2);
   const uint32_t b_tile_bytes = (uint32_t)(p.block_n * p.block_k * 2);
   const uint32_t stage_bytes = a_tile_bytes + b_tile_bytes;
-  uint8_t* smem = smem_raw;
-  {  // dynamic smem base is only guaranteed 16B aligned: align up to 1024 (host adds 1 KB of slack)
-    uint32_t a = ptx::smem_u32(smem);
-    smem += (1024u - (a & 1023u)) & 1023u;
-  }
-  uint8_t* tiles = smem;
-  // share_dx: [a_stages x A box (18 KB pitch)] [stages x B tile]; else [stages x (A | B)]
   // shared activation box: 136 rows of one k-block row (128 B with 64-wide k-blocks / 128-byte swizzle, 64 B with 32-wide
   // k-blocks / 64-byte swizzle); ring pitch 18 KB / 9 KB keeps every box 1024-byte aligned
-  const uint32_t a_row_bytes = (uint32_t)p.block_k * 2u;
-  const uint32_t a_box_bytes = (uint32_t)A_BOX_ROWS * a_row_bytes;
-  const uint32_t a_box_stride = p.block_k == 64 ? (uint32_t)A_BOX_STRIDE : (uint32_t)A_BOX_STRIDE / 2u;
-  uint8_t* b_ring = tiles + (size_t)p.a_stages * a_box_stride;
-  uint8_t* aux = p.share_dx ? b_ring + (size_t)p.stages * b_tile_bytes : tiles + (size_t)p.stages * stage_bytes;
-  uint64_t* full_bar = reinterpret_cast<uint64_t*>(aux);
-  uint64_t* empty_bar = full_bar + MAX_STAGES;
-  uint64_t* tmem_full_bar = empty_bar + MAX_STAGES;      // [ACC_STAGES]
-  uint64_t* tmem_empty_bar = tmem_full_bar + ACC_STAGES; // [ACC_STAGES]
-  uint64_t* afull_bar = tmem_empty_bar + ACC_STAGES;     // [MAX_A_STAGES]
-  uint64_t* aempty_bar = afull_bar + MAX_A_STAGES;    // [MAX_A_STAGES]
-  uint32_t* tmem_ptr_smem = reinterpret_cast<uint32_t*>(aempty_bar + MAX_A_STAGES);
-  float* s_ss = reinterpret_cast<float*>(aux + 512);  // [2 acc stages][scale|shift][256]
-  uint8_t* s_out = aux + 5120;                        // staged epilogue: [4 warps][32 rows][out_pitch]; TMA-store slabs
-                                                      // [4 warps][tma_bufs][4 KB] (1024-byte aligned: swizzle pattern)
+  const uint32_t box_bytes = (uint32_t)A_BOX_ROWS * (uint32_t)p.block_k * 2u;
+  const uint32_t box_stride = p.block_k == 64 ? (uint32_t)A_BOX_STRIDE : (uint32_t)A_BOX_STRIDE / 2u;
+  const ConvSmem m = carve_smem<false>(smem_raw, p, box_stride, b_tile_bytes, stage_bytes);
 
   const int warp_idx = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
   const int total_tiles = p.m_tiles * p.n_tiles;
-  if (threadIdx.x == 0) conv_stamp(p, 0);
-
-  if (warp_idx == 0 && lane == 0) {
+  if (threadIdx.x == 0) {
+    conv_stamp(p, 0);
     ptx::prefetch_tensormap(&tmap_a);
     ptx::prefetch_tensormap(&tmap_b);
-    for (int s = 0; s < p.stages; ++s) {
-      ptx::mbar_init(&full_bar[s], 1);
-      ptx::mbar_init(&empty_bar[s], 1);
-    }
-    for (int a = 0; a < ACC_STAGES; ++a) {
-      ptx::mbar_init(&tmem_full_bar[a], 1);
-      ptx::mbar_init(&tmem_empty_bar[a], 4);  // one arrive per epilogue warp
-    }
-    for (int a = 0; a < MAX_A_STAGES; ++a) {
-      ptx::mbar_init(&afull_bar[a], 1);
-      ptx::mbar_init(&aempty_bar[a], 1);
-    }
     ptx::prefetch_tensormap(&tmap_abox);
     if (p.tma_bufs > 0) ptx::prefetch_tensormap(&tmap_out);
-    ptx::fence_barrier_init();
   }
-  if (warp_idx == 1) {
-    ptx::tmem_alloc(tmem_ptr_smem, (uint32_t)p.tmem_cols);
-    ptx::tmem_relinquish();
-  }
-  ptx::tc_fence_before();
-  __syncthreads();
-  ptx::tc_fence_after();
-  const uint32_t tmem_base = *tmem_ptr_smem;
+  const uint32_t tmem_base = block_setup<false>(m, p);
   if (threadIdx.x == 0) conv_stamp(p, 1);
 
   if (warp_idx == 0) {
     // ===================== TMA producer (one thread) =====================
-    if (lane == 0 && p.share_dx) {
-      // A: one 136-row box per (filter row dy, channel block) — the three dx taps read it at row offsets 0, 1, 2, so
-      // the activations cross L2 -> smem 3 times per tile instead of 9.  B: one tile per tap, its own ring.
-      int s = 0, sa = 0;
-      uint32_t phase = 0, pha = 0;
-      for (int tile = blockIdx.x; tile < total_tiles; tile += gridDim.x) {
-        const int n0 = (tile % p.n_tiles) * p.block_n;
-        const int m0 = (tile / p.n_tiles) * BLOCK_M;
-        for (int g = 0; g < 3 * p.kb_per_tap; ++g) {
-          const int dy = g / p.kb_per_tap, cb = g - dy * p.kb_per_tap;
-          ptx::mbar_wait(&aempty_bar[sa], pha ^ 1u);
-          ptx::mbar_arrive_expect_tx(&afull_bar[sa], a_box_bytes);
-          ptx::tma_load_2d(tiles + (size_t)sa * a_box_stride, &tmap_abox, &afull_bar[sa], cb * p.block_k,
-                           m0 + (dy - 1) * p.Wp - 1);
-          if (++sa == p.a_stages) { sa = 0; pha ^= 1u; }
-          for (int dx = 0; dx < 3; ++dx) {
-            const int kb = (dy * 3 + dx) * p.kb_per_tap + cb;
-            ptx::mbar_wait(&empty_bar[s], phase ^ 1u);
-            ptx::mbar_arrive_expect_tx(&full_bar[s], b_tile_bytes);
-            ptx::tma_load_2d(b_ring + (size_t)s * b_tile_bytes, &tmap_b, &full_bar[s], kb * p.block_k, n0);
+    if (lane == 0) {
+      if (p.share_dx) {
+        Pipe pp(p.stages, p.a_stages);
+        for (int tile = blockIdx.x; tile < total_tiles; tile += gridDim.x) {
+          const int n0 = (tile % p.n_tiles) * p.block_n;
+          const int m0 = (tile / p.n_tiles) * BLOCK_M;
+          produce_box_groups<false>(p, m, &tmap_abox, &tmap_b, m0, n0, 0, 3 * p.kb_per_tap, box_stride, box_bytes,
+                                    b_tile_bytes, true, pp);
+        }
+      } else {
+        int s = 0;
+        uint32_t phase = 0;
+        for (int tile = blockIdx.x; tile < total_tiles; tile += gridDim.x) {
+          const int n0 = (tile % p.n_tiles) * p.block_n;
+          const int m0 = (tile / p.n_tiles) * BLOCK_M;
+          for (int kb = 0; kb < p.num_kb; ++kb) {
+            const int tap = kb / p.kb_per_tap;
+            const int cb = kb - tap * p.kb_per_tap;
+            int row_off = 0;
+            if (p.ksize == 3) row_off = (tap / 3 - 1) * p.Wp + (tap % 3 - 1);
+            ptx::mbar_wait(&m.empty_bar[s], phase ^ 1u);
+            uint8_t* a_dst = m.tiles + (size_t)s * stage_bytes;
+            uint8_t* b_dst = a_dst + a_tile_bytes;
+            ptx::mbar_arrive_expect_tx(&m.full_bar[s], stage_bytes);
+            ptx::tma_load_2d(a_dst, &tmap_a, &m.full_bar[s], cb * p.block_k, m0 + row_off);
+            ptx::tma_load_2d(b_dst, &tmap_b, &m.full_bar[s], kb * p.block_k, n0);
             if (++s == p.stages) { s = 0; phase ^= 1u; }
           }
-        }
-      }
-      conv_stamp(p, 3);
-    } else if (lane == 0) {
-      int s = 0;
-      uint32_t phase = 0;
-      for (int tile = blockIdx.x; tile < total_tiles; tile += gridDim.x) {
-        const int n0 = (tile % p.n_tiles) * p.block_n;
-        const int m0 = (tile / p.n_tiles) * BLOCK_M;
-        for (int kb = 0; kb < p.num_kb; ++kb) {
-          const int tap = kb / p.kb_per_tap;
-          const int cb = kb - tap * p.kb_per_tap;
-          int row_off = 0;
-          if (p.ksize == 3) row_off = (tap / 3 - 1) * p.Wp + (tap % 3 - 1);
-          ptx::mbar_wait(&empty_bar[s], phase ^ 1u);
-          uint8_t* a_dst = tiles + (size_t)s * stage_bytes;
-          uint8_t* b_dst = a_dst + a_tile_bytes;
-          ptx::mbar_arrive_expect_tx(&full_bar[s], stage_bytes);
-          ptx::tma_load_2d(a_dst, &tmap_a, &full_bar[s], cb * p.block_k, m0 + row_off);
-          ptx::tma_load_2d(b_dst, &tmap_b, &full_bar[s], kb * p.block_k, n0);
-          if (++s == p.stages) { s = 0; phase ^= 1u; }
         }
       }
       conv_stamp(p, 3);
     }
   } else if (warp_idx == 1) {
-    // ===================== MMA issuer =====================
-    // The WHOLE warp walks the loop (warp-uniform control flow and operands, so descriptors live in uniform
-    // registers) and one elected lane issues the tcgen05 instructions.  With the loop inside `if (lane == 0)` the
-    // compiler wraps every UTCHMMA in a vote/R2UR.BROADCAST loop (~25 instructions), and that single thread's issue
-    // rate — not the tensor pipe — bounds the k-block time.
+    // ===================== MMA issuer (whole warp, one elected lane issues: see mma_box_unit) =====================
     if (p.share_dx) {
-      int s = 0, sa = 0, as = 0;
-      uint32_t phase = 0, pha = 0, aphase = 0;
+      Pipe pp(p.stages, p.a_stages);
       int ti = 0;
-      for (int tile = blockIdx.x; tile < total_tiles; tile += gridDim.x, ++ti) {
-        ptx::mbar_wait(&tmem_empty_bar[as], aphase ^ 1u);
-        ptx::tc_fence_after();
-        const uint32_t tmem_acc = tmem_base + (uint32_t)(as * p.acc_stride);
-        for (int g = 0; g < 3 * p.kb_per_tap; ++g) {
-          const int dy = g / p.kb_per_tap, cb = g - dy * p.kb_per_tap;
-          // K steps beyond the layer's real channels multiply TMA zero fill by zero weights: not issued
-          const int nk = (cb == p.kb_per_tap - 1) ? p.last_ksteps : (int)(a_row_bytes >> 5);
-          ptx::mbar_wait(&afull_bar[sa], pha);
-          if (ti == 0 && g == 0 && lane == 0) conv_stamp(p, 4);
-          const uint32_t a_addr = ptx::smem_u32(tiles + (size_t)sa * a_box_stride);
-          for (int dx = 0; dx < 3; ++dx) {
-            ptx::mbar_wait(&full_bar[s], phase);
-            ptx::tc_fence_after();
-            const uint32_t b_addr = ptx::smem_u32(b_ring + (size_t)s * b_tile_bytes);
-            // the window of tap dx starts dx rows (dx * 128 B) into the box.  The start is then not aligned to the
-            // 1024-byte swizzle pattern; measured on B200: the tensor core applies the 128-byte swizzle to the absolute
-            // shared-memory address (as TMA did when it wrote the box), so the descriptor's base-offset field must stay
-            // 0 — setting it to dx (or 8-dx) reads garbage (tools/debug_share.py)
-            // (32-wide k-blocks: the same holds for the 64-byte swizzle — rows of 64 B, window dx starts dx * 64 B in)
-            const bool k64 = p.block_k == 64;
-            const uint64_t adesc = k64 ? ptx::make_sw128_kmajor_desc(a_addr + (uint32_t)dx * 128u)
-                                       : ptx::make_sw64_kmajor_desc(a_addr + (uint32_t)dx * 64u);
-            const uint64_t bdesc = k64 ? ptx::make_sw128_kmajor_desc(b_addr) : ptx::make_sw64_kmajor_desc(b_addr);
-            if (ptx::elect_one()) {
-              // (compile-time trip count with a per-step predicate: this issue loop is on the critical path, a
-              //  run-time trip count costs the narrow-Cin layers ~4 us each)
-#pragma unroll
-              for (int k = 0; k < 4; ++k)
-                if (k < nk)
-                  ptx::umma_bf16_ss(tmem_acc, adesc + (uint64_t)(2 * k), bdesc + (uint64_t)(2 * k), p.idesc,
-                                    (g > 0 || dx > 0 || k > 0) ? 1u : 0u);
-              ptx::umma_commit(&empty_bar[s]);
-              if (dx == 2) ptx::umma_commit(&aempty_bar[sa]);  // the box may be refilled once its three taps retire
-              if (dx == 2 && g == 3 * p.kb_per_tap - 1) ptx::umma_commit(&tmem_full_bar[as]);
-            }
-            __syncwarp();
-            if (++s == p.stages) { s = 0; phase ^= 1u; }
-          }
-          if (++sa == p.a_stages) { sa = 0; pha ^= 1u; }
-        }
-        if (lane == 0 && ti < 6) conv_stamp(p, 5 + ti);
-        if (++as == ACC_STAGES) { as = 0; aphase ^= 1u; }
-      }
+      for (int tile = blockIdx.x; tile < total_tiles; tile += gridDim.x, ++ti)
+        mma_box_unit<false>(p, m, tmem_base, 0, 3 * p.kb_per_tap, box_stride, b_tile_bytes, pp, ti);
     } else {
+      // one A | B stage per k-block, the A tile already shifted to the tap
       int s = 0;
       uint32_t phase = 0;
       int as = 0;
       uint32_t aphase = 0;
       int ti = 0;
       for (int tile = blockIdx.x; tile < total_tiles; tile += gridDim.x, ++ti) {
-        ptx::mbar_wait(&tmem_empty_bar[as], aphase ^ 1u);  // epilogue has drained this accumulator stage
+        ptx::mbar_wait(&m.tmem_empty_bar[as], aphase ^ 1u);  // epilogue has drained this accumulator stage
         ptx::tc_fence_after();
         const uint32_t tmem_acc = tmem_base + (uint32_t)(as * p.acc_stride);
         int cb_i = 0;  // channel block inside the tap
         for (int kb = 0; kb < p.num_kb; ++kb) {
-          ptx::mbar_wait(&full_bar[s], phase);
+          ptx::mbar_wait(&m.full_bar[s], phase);
           ptx::tc_fence_after();
           if (ti == 0 && kb == 0 && lane == 0) conv_stamp(p, 4);
-          const uint32_t a_addr = ptx::smem_u32(tiles + (size_t)s * stage_bytes);
+          const uint32_t a_addr = ptx::smem_u32(m.tiles + (size_t)s * stage_bytes);
           const bool k64 = p.block_k == 64;
           const uint64_t adesc = k64 ? ptx::make_sw128_kmajor_desc(a_addr) : ptx::make_sw64_kmajor_desc(a_addr);
           const uint64_t bdesc = k64 ? ptx::make_sw128_kmajor_desc(a_addr + a_tile_bytes)
@@ -740,8 +838,8 @@ conv_gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __gri
                 ptx::umma_bf16_ss(tmem_acc, adesc + (uint64_t)(2 * k), bdesc + (uint64_t)(2 * k), p.idesc,
                                   (kb > 0 || k > 0) ? 1u : 0u);
             }
-            ptx::umma_commit(&empty_bar[s]);  // frees the smem slot when these MMAs retire
-            if (kb == p.num_kb - 1) ptx::umma_commit(&tmem_full_bar[as]);  // accumulator complete
+            ptx::umma_commit(&m.empty_bar[s]);  // frees the smem slot when these MMAs retire
+            if (kb == p.num_kb - 1) ptx::umma_commit(&m.tmem_full_bar[as]);  // accumulator complete
           }
           __syncwarp();
           if (++s == p.stages) { s = 0; phase ^= 1u; }
@@ -753,17 +851,16 @@ conv_gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __gri
   } else {
     // ===================== epilogue: warps 2..5 =====================
     if (p.epi_mode == MC_EPI_PNHWC) {
-      uint8_t* so = (p.out_pitch || p.tma_bufs) ? s_out : nullptr;
-      if (p.leaky) epilogue_loop<MC_EPI_PNHWC, true, false, MINB == 1>(p, tmem_base, tmem_full_bar, tmem_empty_bar, s_ss, so, &tmap_out);
-      else epilogue_loop<MC_EPI_PNHWC, false, false, MINB == 1>(p, tmem_base, tmem_full_bar, tmem_empty_bar, s_ss, so, &tmap_out);
+      if (p.leaky) epilogue_loop<MC_EPI_PNHWC, true, MINB == 1>(p, m, tmem_base, &tmap_out);
+      else epilogue_loop<MC_EPI_PNHWC, false, MINB == 1>(p, m, tmem_base, &tmap_out);
     } else if (p.epi_mode == MC_EPI_REORG2) {
-      if (p.leaky) epilogue_loop<MC_EPI_REORG2, true>(p, tmem_base, tmem_full_bar, tmem_empty_bar, s_ss);
-      else epilogue_loop<MC_EPI_REORG2, false>(p, tmem_base, tmem_full_bar, tmem_empty_bar, s_ss);
+      if (p.leaky) epilogue_loop<MC_EPI_REORG2, true>(p, m, tmem_base, &tmap_out);
+      else epilogue_loop<MC_EPI_REORG2, false>(p, m, tmem_base, &tmap_out);
     } else if (p.epi_mode == MC_EPI_DECODE) {
-      epilogue_loop<MC_EPI_DECODE, false>(p, tmem_base, tmem_full_bar, tmem_empty_bar, s_ss, s_out);
+      epilogue_loop<MC_EPI_DECODE, false>(p, m, tmem_base, &tmap_out);
     } else {
-      if (p.leaky) epilogue_loop<MC_EPI_NCHW_F32, true>(p, tmem_base, tmem_full_bar, tmem_empty_bar, s_ss);
-      else epilogue_loop<MC_EPI_NCHW_F32, false>(p, tmem_base, tmem_full_bar, tmem_empty_bar, s_ss);
+      if (p.leaky) epilogue_loop<MC_EPI_NCHW_F32, true>(p, m, tmem_base, &tmap_out);
+      else epilogue_loop<MC_EPI_NCHW_F32, false>(p, m, tmem_base, &tmap_out);
     }
   }
 
@@ -848,7 +945,6 @@ struct PairWorkIter {
 // that the idle clusters of one layer's partial last wave start the next layer's first units and the layer boundaries
 // need no drain / launch / set-up / pipeline fill.  The entries share B, H, W, tile width, ring depth and epilogue.
 constexpr int MAX_CHAIN = 4;
-constexpr int WORK_SLOTS = 4;                           // work ring between the leader's producer and the other roles
 constexpr unsigned long long CHAIN_POLL_NS = 1000000000ull;  // bound of one readiness wait (then: status word, go on)
 enum { CHAIN_TICKET = 0, CHAIN_DONE = 1, CHAIN_STATUS = 2, CHAIN_COUNTERS = 4 };  // words of the chain workspace
 
@@ -955,38 +1051,22 @@ __device__ __forceinline__ void chain_arrive(const PairParams& P, const PairWork
   }
 }
 
-// Epilogue warps of the CTA-pair kernel: one pass per work item.  Whole units and finishers drain the accumulator
-// through scale/shift/leaky and store (a finisher first adds the partial accumulators of the unit's earlier K spans);
-// partial pieces park their raw fp32 accumulator in the workspace and count themselves in.
+// Epilogue warps of the CTA-pair kernel: one pass per work item, this CTA's 128 rows of the 256-row unit.  Whole units
+// and finishers run epilogue_tile (a finisher first waits for the partial accumulators of the unit's earlier K spans and
+// adds them there); partial pieces park their raw fp32 accumulator in the workspace and count themselves in.
 template <int MODE, bool LEAKY>
-__device__ __forceinline__ void epilogue_loop_pair(const PairParams& P, uint32_t tmem_base, uint64_t* tmem_full_bar,
-                                                   uint64_t* tmem_empty_bar, float* s_ss, int cluster_id, int num_clusters,
-                                                   int pair_rank, uint8_t* s_out, PairRing ring) {
-  const int warp_idx = threadIdx.x >> 5;
+__device__ __forceinline__ void epilogue_loop_pair(const PairParams& P, const ConvSmem& m, uint32_t tmem_base,
+                                                   int cluster_id, int num_clusters, int pair_rank, PairRing ring) {
   const int lane = threadIdx.x & 31;
-  const int et = threadIdx.x - 64;   // 0..127
-  const int quarter = warp_idx & 3;  // TMEM lane quarter this warp may access
+  const int quarter = (threadIdx.x >> 5) & 3;
   const ConvKParams& p0 = P.layer[0].p;
   const bool chain = P.n_layers > 1;
+  const bool one_n_tile = !chain && p0.n_tiles == 1;
+  float* stat_acc = epilogue_begin<MODE>(p0, m, one_n_tile);
+  int stat_n0 = -1;
+  int slab_buf = 0;
   int as = 0;
   uint32_t aphase = 0;
-  int slab_buf = 0;
-  float* stat_acc = nullptr;
-  int stat_n0 = -1;
-  if (MODE == MC_EPI_PNHWC && p0.tma_bufs > 0 && p0.stat_sum != nullptr) {
-    stat_acc = reinterpret_cast<float*>(s_out + (size_t)4 * p0.tma_bufs * 4096) + quarter * 512;
-    for (int c = lane; c < 512; c += 32) stat_acc[c] = 0.f;
-    __syncwarp();
-  }
-  const bool one_n_tile = !chain && p0.n_tiles == 1;
-  if (one_n_tile) {
-    for (int i = et; i < p0.block_n; i += 128) {
-      const bool ok = i < p0.Npad;
-      s_ss[i] = ok ? __ldg(p0.scale + i) : 0.f;
-      s_ss[256 + i] = ok ? __ldg(p0.shift + i) : 0.f;
-    }
-    asm volatile("bar.sync 1, 128;" ::: "memory");
-  }
   PairWorkIter it;
   it.init(p0, cluster_id, num_clusters);
   PairWork w;
@@ -994,48 +1074,11 @@ __device__ __forceinline__ void epilogue_loop_pair(const PairParams& P, uint32_t
   while (chain ? ring_take(P, ring, w, true) : it.next(w)) {
     ++ti;
     const ConvKParams& p = P.layer[w.layer].p;
-    const CUtensorMap* tm_out = &P.layer[w.layer].tmap_out;
     const bool vec_ok = ((p.ldc | p.ch_off) & 7) == 0 && (MODE != MC_EPI_REORG2 || (p.N & 7) == 0);
-    const int tile = w.unit;
-    const int n0 = (tile % p.n_tiles) * p.block_n;
-    const int m0 = (2 * (tile / p.n_tiles) + pair_rank) * BLOCK_M;
-    float* sc = s_ss + (one_n_tile ? 0 : as * 512);
-    float* sh = sc + 256;
-    if (!one_n_tile) {
-      for (int i = et; i < p.block_n; i += 128) {
-        const bool ok = (n0 + i) < p.Npad;
-        sc[i] = ok ? __ldg(p.scale + n0 + i) : 0.f;
-        sh[i] = ok ? __ldg(p.shift + n0 + i) : 0.f;
-      }
-    }
-    const int row = m0 + quarter * 32 + lane;
-    const int t = (int)(__umulhi((unsigned int)row, p.wp_mul) >> p.wp_shr);  // row / Wp (magic-number division)
-    const int x = row - t * p.Wp;
-    const int b = (int)(__umulhi((unsigned int)t, p.hp_mul) >> p.hp_shr);    // t / Hp
-    const int y = t - b * p.Hp;
-    const bool in_buf = row < p.M_rows;
-    const bool interior = in_buf && (x < p.W) && (y < p.H);
-    long long out_row_base = 0;
-    bool do_store = false;
-    if (MODE == MC_EPI_PNHWC) {
-      out_row_base = (long long)row * p.ldc + p.ch_off;
-      do_store = in_buf;  // pad rows are written as zeros to keep the layout invariant
-    } else if (MODE == MC_EPI_REORG2) {
-      const int Wo = p.W / 2 + 1, Ho = p.H / 2 + 1;
-      const long long orow = ((long long)b * Ho + (y >> 1)) * Wo + (x >> 1);
-      out_row_base = orow * p.ldc + p.ch_off + ((y & 1) * 2 + (x & 1)) * p.N;
-      do_store = interior;
-    } else {  // MC_EPI_NCHW_F32
-      out_row_base = ((long long)b * p.N * p.H + y) * p.W + x;  // + n*H*W
-      do_store = interior;
-    }
-    if (!one_n_tile) asm volatile("bar.sync 1, 128;" ::: "memory");  // scale/shift of this tile visible to the 4 warps
-
-    ptx::mbar_wait(&tmem_full_bar[as], aphase);
-    ptx::tc_fence_after();
-    if (et == 0 && ti < 8) conv_stamp(p, 12 + 2 * ti);
-    const uint32_t taddr_row = tmem_base + ((uint32_t)(quarter * 32) << 16) + (uint32_t)(as * p.acc_stride);
-    const int u_sk = tile - p.sk_first;  // (stream-K pieces only)
+    const int n0 = (w.unit % p.n_tiles) * p.block_n;
+    const int m0 = (2 * (w.unit / p.n_tiles) + pair_rank) * BLOCK_M;
+    const EpiTile t = epi_tile_begin<MODE>(p, m, tmem_base, one_n_tile, m0, n0, as, aphase, ti);
+    const int u_sk = w.unit - p.sk_first;  // (stream-K pieces only)
     // partial tiles are stored [slot][column / 4][256 rows][4 floats]: a warp instruction (32 rows, one float4 each) is one
     // contiguous 512-byte segment, for the writers and for the finisher that reads them back with the same mapping
     const int prow = pair_rank * 128 + quarter * 32 + lane;
@@ -1049,8 +1092,8 @@ __device__ __forceinline__ void epilogue_loop_pair(const PairParams& P, uint32_t
       for (int c0 = 0; c0 < p.block_n; c0 += 32) {
         uint32_t r0[16], r1[16];
         const bool two = c0 + 16 < p.block_n;
-        ptx::tmem_ld_32x32b_x16(taddr_row + (uint32_t)c0, r0);
-        if (two) ptx::tmem_ld_32x32b_x16(taddr_row + (uint32_t)(c0 + 16), r1);
+        ptx::tmem_ld_32x32b_x16(t.taddr + (uint32_t)c0, r0);
+        if (two) ptx::tmem_ld_32x32b_x16(t.taddr + (uint32_t)(c0 + 16), r1);
         ptx::tmem_ld_wait();
 #pragma unroll
         for (int q = 0; q < 4; ++q)
@@ -1066,7 +1109,7 @@ __device__ __forceinline__ void epilogue_loop_pair(const PairParams& P, uint32_t
       __syncwarp();
       if (lane == 0) {
         atomicAdd(p.sk_count + u_sk, 1u);
-        ptx::mbar_arrive_leader(&tmem_empty_bar[as]);
+        ptx::mbar_arrive_leader(&m.tmem_empty_bar[as]);
       }
     } else {
       const int nparts = w.kind == 2 ? w.aux : 0;
@@ -1088,74 +1131,25 @@ __device__ __forceinline__ void epilogue_loop_pair(const PairParams& P, uint32_t
         __syncwarp();
         __threadfence();
       }
-      if (MODE == MC_EPI_PNHWC && p.tma_bufs > 0) {
-        if (stat_acc != nullptr && n0 != stat_n0) {
-          if (stat_n0 >= 0) flush_stats(p, stat_acc, stat_n0, lane);
-          stat_n0 = n0;
-        }
-        epilogue_tile_tma<LEAKY, true, true>(p, tm_out, taddr_row, sc, sh, interior, in_buf, m0 + quarter * 32, n0, out_row_base,
-                                       vec_ok, s_out + (size_t)quarter * p.tma_bufs * 4096, slab_buf, &tmem_empty_bar[as],
-                                       [&](uint32_t (&r)[16], int col) {
-                                         for (int s2 = 0; s2 < nparts; ++s2) {
-#pragma unroll
-                                           for (int q = 0; q < 4; ++q) {
-                                             const float4 a = __ldcg(reinterpret_cast<const float4*>(part_ptr(s2, col + 4 * q)));
-                                             r[4 * q] = __float_as_uint(__uint_as_float(r[4 * q]) + a.x);
-                                             r[4 * q + 1] = __float_as_uint(__uint_as_float(r[4 * q + 1]) + a.y);
-                                             r[4 * q + 2] = __float_as_uint(__uint_as_float(r[4 * q + 2]) + a.z);
-                                             r[4 * q + 3] = __float_as_uint(__uint_as_float(r[4 * q + 3]) + a.w);
-                                           }
-                                         }
-                                       }, stat_acc);
-        if (chain) chain_arrive(P, w, lane);
-        if (et == 0 && ti < 8) conv_stamp(p, 13 + 2 * ti);
-        if (++as == ACC_STAGES) { as = 0; aphase ^= 1u; }
-        continue;
-      }
-      for (int c0 = 0; c0 < p.block_n; c0 += 32) {
-        uint32_t r0[16], r1[16];
-        const bool two = c0 + 16 < p.block_n;
-        ptx::tmem_ld_32x32b_x16(taddr_row + (uint32_t)c0, r0);
-        if (two) ptx::tmem_ld_32x32b_x16(taddr_row + (uint32_t)(c0 + 16), r1);
-        ptx::tmem_ld_wait();
-        if (!do_store) continue;
+      epilogue_tile<MODE, LEAKY, true, true>(p, &P.layer[w.layer].tmap_out, m, t, vec_ok, &m.tmem_empty_bar[as],
+                                             slab_buf, stat_acc, stat_n0, [&](uint32_t (&r)[16], int col) {
         for (int s2 = 0; s2 < nparts; ++s2) {
 #pragma unroll
           for (int q = 0; q < 4; ++q) {
-            const float4 a = __ldcg(reinterpret_cast<const float4*>(part_ptr(s2, c0 + 4 * q)));
-            r0[4 * q] = __float_as_uint(__uint_as_float(r0[4 * q]) + a.x);
-            r0[4 * q + 1] = __float_as_uint(__uint_as_float(r0[4 * q + 1]) + a.y);
-            r0[4 * q + 2] = __float_as_uint(__uint_as_float(r0[4 * q + 2]) + a.z);
-            r0[4 * q + 3] = __float_as_uint(__uint_as_float(r0[4 * q + 3]) + a.w);
-          }
-          if (two) {
-#pragma unroll
-            for (int q = 0; q < 4; ++q) {
-              const float4 a = __ldcg(reinterpret_cast<const float4*>(part_ptr(s2, c0 + 16 + 4 * q)));
-              r1[4 * q] = __float_as_uint(__uint_as_float(r1[4 * q]) + a.x);
-              r1[4 * q + 1] = __float_as_uint(__uint_as_float(r1[4 * q + 1]) + a.y);
-              r1[4 * q + 2] = __float_as_uint(__uint_as_float(r1[4 * q + 2]) + a.z);
-              r1[4 * q + 3] = __float_as_uint(__uint_as_float(r1[4 * q + 3]) + a.w);
-            }
+            const float4 a = __ldcg(reinterpret_cast<const float4*>(part_ptr(s2, col + 4 * q)));
+            r[4 * q] = __float_as_uint(__uint_as_float(r[4 * q]) + a.x);
+            r[4 * q + 1] = __float_as_uint(__uint_as_float(r[4 * q + 1]) + a.y);
+            r[4 * q + 2] = __float_as_uint(__uint_as_float(r[4 * q + 2]) + a.z);
+            r[4 * q + 3] = __float_as_uint(__uint_as_float(r[4 * q + 3]) + a.w);
           }
         }
-        float v[16];
-        scale_act16<LEAKY>(r0, sc + c0, sh + c0, interior, v);
-        store16<MODE>(p, v, n0 + c0, out_row_base, vec_ok);
-        if (two) {
-          scale_act16<LEAKY>(r1, sc + c0 + 16, sh + c0 + 16, interior, v);
-          store16<MODE>(p, v, n0 + c0 + 16, out_row_base, vec_ok);
-        }
-      }
-      ptx::tc_fence_before();
-      __syncwarp();
-      if (lane == 0) ptx::mbar_arrive_leader(&tmem_empty_bar[as]);
+      });
+      if (chain) chain_arrive(P, w, lane);
     }
-    if (et == 0 && ti < 8) conv_stamp(p, 13 + 2 * ti);
+    if (threadIdx.x == 64 && ti < 8) conv_stamp(p, 13 + 2 * ti);
     if (++as == ACC_STAGES) { as = 0; aphase ^= 1u; }
   }
-  if (stat_acc != nullptr && stat_n0 >= 0) flush_stats(p0, stat_acc, stat_n0, lane);
-  if (MODE == MC_EPI_PNHWC && p0.tma_bufs > 0 && lane == 0) ptx::bulk_wait_group_read<0>();  // slabs read before the CTA exits
+  epilogue_end<MODE>(p0, stat_acc, stat_n0);
 }
 
 // ---------------------------------------------------------------------------------------------------------------
@@ -1174,75 +1168,33 @@ conv_gemm_tcgen05_pair_kernel(const __grid_constant__ PairParams P) {
   const ConvKParams& p0 = P.layer[0].p;
   const bool chain = P.n_layers > 1;
   const uint32_t b_half_bytes = (uint32_t)(p0.block_n / 2 * 128);
-  uint8_t* smem = smem_raw;
-  {
-    uint32_t a = ptx::smem_u32(smem);
-    smem += (1024u - (a & 1023u)) & 1023u;
-  }
-  uint8_t* tiles = smem;
-  uint8_t* b_ring = tiles + (size_t)p0.a_stages * A_BOX_STRIDE;
-  uint8_t* aux = b_ring + (size_t)p0.stages * b_half_bytes;
-  uint64_t* full_bar = reinterpret_cast<uint64_t*>(aux);
-  uint64_t* empty_bar = full_bar + MAX_STAGES;
-  uint64_t* tmem_full_bar = empty_bar + MAX_STAGES;      // [ACC_STAGES]
-  uint64_t* tmem_empty_bar = tmem_full_bar + ACC_STAGES; // [ACC_STAGES]
-  uint64_t* afull_bar = tmem_empty_bar + ACC_STAGES;     // [MAX_A_STAGES]
-  uint64_t* aempty_bar = afull_bar + MAX_A_STAGES;    // [MAX_A_STAGES]
-  uint32_t* tmem_ptr_smem = reinterpret_cast<uint32_t*>(aempty_bar + MAX_A_STAGES);
+  const ConvSmem m = carve_smem<true>(smem_raw, p0, A_BOX_STRIDE, b_half_bytes, 0);
   PairRing ring;
-  ring.full = reinterpret_cast<uint64_t*>(aux + 256);  // [WORK_SLOTS]
-  ring.empty = ring.full + WORK_SLOTS;                 // [WORK_SLOTS]
-  ring.val = reinterpret_cast<int*>(ring.empty + WORK_SLOTS);
+  ring.full = m.work_full;
+  ring.empty = m.work_empty;
+  ring.val = m.work_val;
   ring.slot = 0;
   ring.phase = 0;
-  float* s_ss = reinterpret_cast<float*>(aux + 512);
-  uint8_t* s_out = aux + 5120;  // TMA-store slabs [4 warps][tma_bufs][4 KB], 1024-byte aligned
 
   const int warp_idx = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
   const int rank = (int)ptx::cluster_ctarank();
   const int cluster_id = blockIdx.x >> 1, num_clusters = gridDim.x >> 1;
-  if (threadIdx.x == 0) conv_stamp(p0, 0);
-
-  if (warp_idx == 0 && lane == 0) {
+  if (threadIdx.x == 0) {
+    conv_stamp(p0, 0);
     for (int l = 0; l < P.n_layers; ++l) {
       ptx::prefetch_tensormap(&P.layer[l].tmap_b);
       ptx::prefetch_tensormap(&P.layer[l].tmap_abox);
       if (p0.tma_bufs > 0) ptx::prefetch_tensormap(&P.layer[l].tmap_out);
     }
-    for (int s = 0; s < p0.stages; ++s) {
-      ptx::mbar_init(&full_bar[s], 1);
-      ptx::mbar_init(&empty_bar[s], 1);
-    }
-    for (int a = 0; a < ACC_STAGES; ++a) {
-      ptx::mbar_init(&tmem_full_bar[a], 1);
-      ptx::mbar_init(&tmem_empty_bar[a], 8);  // 4 epilogue warps of each CTA
-    }
-    for (int a = 0; a < MAX_A_STAGES; ++a) {
-      ptx::mbar_init(&afull_bar[a], 1);
-      ptx::mbar_init(&aempty_bar[a], 1);
-    }
-    for (int s = 0; s < WORK_SLOTS; ++s) {
-      ptx::mbar_init(&ring.full[s], 1);
-      ptx::mbar_init(&ring.empty[s], 10);  // leader: MMA warp + 4 epilogue warps; peer: producer + 4 epilogue warps
-    }
-    ptx::fence_barrier_init();
   }
-  if (warp_idx == 1) {
-    ptx::tmem_alloc_pair(tmem_ptr_smem, (uint32_t)p0.tmem_cols);
-    ptx::tmem_relinquish_pair();
-  }
-  ptx::tc_fence_before();
-  ptx::cluster_sync_all();  // barriers of BOTH CTAs initialised before any remote arrival / complete_tx
-  ptx::tc_fence_after();
-  const uint32_t tmem_base = *tmem_ptr_smem;
+  const uint32_t tmem_base = block_setup<true>(m, p0);
   if (threadIdx.x == 0) conv_stamp(p0, 1);
 
   if (warp_idx == 0) {
     // ===================== TMA producer (one thread per CTA) =====================
     if (lane == 0) {
-      int s = 0, sa = 0;
-      uint32_t phase = 0, pha = 0;
+      Pipe pp(p0.stages, p0.a_stages);
       PairWorkIter it;
       it.init(p0, cluster_id, num_clusters);
       PairWork w;
@@ -1252,33 +1204,17 @@ conv_gemm_tcgen05_pair_kernel(const __grid_constant__ PairParams P) {
         // (chain, peer CTA) the leader acquired this unit's inputs; the mbarrier hand-over carries that to this
         // thread, and the proxy fence to the TMA loads it issues (see ring_claim)
         if (chain && rank != 0) ptx::fence_proxy_async_global();
-        const int unit = w.unit;
-        const int n0 = (unit % p.n_tiles) * p.block_n + rank * (p.block_n / 2);
-        const int m0 = (2 * (unit / p.n_tiles) + rank) * BLOCK_M;
-        const int gb = w.g0, ge = w.g1 < 0 ? 3 * p.kb_per_tap : w.g1;
-        for (int g = gb; g < ge; ++g) {
-          const int dy = g / p.kb_per_tap, cb = g - dy * p.kb_per_tap;
-          ptx::mbar_wait(&aempty_bar[sa], pha ^ 1u);
-          if (rank == 0) ptx::mbar_arrive_expect_tx(&afull_bar[sa], 2 * A_BOX_BYTES);
-          ptx::tma_load_2d_pair(tiles + (size_t)sa * A_BOX_STRIDE, &L.tmap_abox, &afull_bar[sa], cb * 64,
-                                m0 + (dy - 1) * p.Wp - 1);
-          if (++sa == p.a_stages) { sa = 0; pha ^= 1u; }
-          for (int dx = 0; dx < 3; ++dx) {
-            const int kb = (dy * 3 + dx) * p.kb_per_tap + cb;
-            ptx::mbar_wait(&empty_bar[s], phase ^ 1u);
-            if (rank == 0) ptx::mbar_arrive_expect_tx(&full_bar[s], 2 * b_half_bytes);
-            ptx::tma_load_2d_pair(b_ring + (size_t)s * b_half_bytes, &L.tmap_b, &full_bar[s], kb * 64, n0);
-            if (++s == p.stages) { s = 0; phase ^= 1u; }
-          }
-        }
+        const int n0 = (w.unit % p.n_tiles) * p.block_n + rank * (p.block_n / 2);
+        const int m0 = (2 * (w.unit / p.n_tiles) + rank) * BLOCK_M;
+        produce_box_groups<true>(p, m, &L.tmap_abox, &L.tmap_b, m0, n0, w.g0, w.g1 < 0 ? 3 * p.kb_per_tap : w.g1,
+                                 A_BOX_STRIDE, A_BOX_BYTES, b_half_bytes, rank == 0, pp);
       }
       conv_stamp(p0, 3);
     }
   } else if (warp_idx == 1) {
     // ===================== MMA issuer (warp 1 of the leader CTA; one elected lane issues) =====================
     if (rank == 0) {
-      int s = 0, sa = 0, as = 0;
-      uint32_t phase = 0, pha = 0, aphase = 0;
+      Pipe pp(p0.stages, p0.a_stages);
       PairWorkIter it;
       it.init(p0, cluster_id, num_clusters);
       PairWork w;
@@ -1286,52 +1222,20 @@ conv_gemm_tcgen05_pair_kernel(const __grid_constant__ PairParams P) {
       while (chain ? ring_take(P, ring, w, true) : it.next(w)) {
         ++ti;
         const ConvKParams& p = P.layer[w.layer].p;
-        ptx::mbar_wait(&tmem_empty_bar[as], aphase ^ 1u);
-        ptx::tc_fence_after();
-        const uint32_t tmem_acc = tmem_base + (uint32_t)(as * p.acc_stride);
-        const int kbt = p.kb_per_tap, lks = p.last_ksteps;
-        const uint32_t idesc = p.idesc;
-        const int gb = w.g0, ge = w.g1 < 0 ? 3 * kbt : w.g1;
-        for (int g = gb; g < ge; ++g) {
-          const int nk = ((g % kbt) == kbt - 1) ? lks : 4;
-          ptx::mbar_wait(&afull_bar[sa], pha);
-          if (ti == 0 && g == gb && lane == 0) conv_stamp(p, 4);
-          const uint32_t a_addr = ptx::smem_u32(tiles + (size_t)sa * A_BOX_STRIDE);
-          for (int dx = 0; dx < 3; ++dx) {
-            ptx::mbar_wait(&full_bar[s], phase);
-            ptx::tc_fence_after();
-            const uint64_t adesc = ptx::make_sw128_kmajor_desc(a_addr + (uint32_t)dx * 128u);
-            const uint64_t bdesc = ptx::make_sw128_kmajor_desc(ptx::smem_u32(b_ring + (size_t)s * b_half_bytes));
-            if (ptx::elect_one()) {
-#pragma unroll
-              for (int k = 0; k < 4; ++k)
-                if (k < nk)
-                  ptx::umma_bf16_ss_pair(tmem_acc, adesc + (uint64_t)(2 * k), bdesc + (uint64_t)(2 * k), idesc,
-                                         (g > gb || dx > 0 || k > 0) ? 1u : 0u);
-              ptx::umma_commit_pair(&empty_bar[s]);
-              if (dx == 2) ptx::umma_commit_pair(&aempty_bar[sa]);
-              if (dx == 2 && g == ge - 1) ptx::umma_commit_pair(&tmem_full_bar[as]);
-            }
-            __syncwarp();
-            if (++s == p0.stages) { s = 0; phase ^= 1u; }
-          }
-          if (++sa == p0.a_stages) { sa = 0; pha ^= 1u; }
-        }
-        if (lane == 0 && ti < 6) conv_stamp(p, 5 + ti);
-        if (++as == ACC_STAGES) { as = 0; aphase ^= 1u; }
+        mma_box_unit<true>(p, m, tmem_base, w.g0, w.g1 < 0 ? 3 * p.kb_per_tap : w.g1, A_BOX_STRIDE, b_half_bytes, pp, ti);
       }
     }
   } else {
     // ===================== epilogue: warps 2..5 of both CTAs =====================
     if (p0.epi_mode == MC_EPI_PNHWC) {
-      if (p0.leaky) epilogue_loop_pair<MC_EPI_PNHWC, true>(P, tmem_base, tmem_full_bar, tmem_empty_bar, s_ss, cluster_id, num_clusters, rank, s_out, ring);
-      else epilogue_loop_pair<MC_EPI_PNHWC, false>(P, tmem_base, tmem_full_bar, tmem_empty_bar, s_ss, cluster_id, num_clusters, rank, s_out, ring);
+      if (p0.leaky) epilogue_loop_pair<MC_EPI_PNHWC, true>(P, m, tmem_base, cluster_id, num_clusters, rank, ring);
+      else epilogue_loop_pair<MC_EPI_PNHWC, false>(P, m, tmem_base, cluster_id, num_clusters, rank, ring);
     } else if (p0.epi_mode == MC_EPI_REORG2) {
-      if (p0.leaky) epilogue_loop_pair<MC_EPI_REORG2, true>(P, tmem_base, tmem_full_bar, tmem_empty_bar, s_ss, cluster_id, num_clusters, rank, s_out, ring);
-      else epilogue_loop_pair<MC_EPI_REORG2, false>(P, tmem_base, tmem_full_bar, tmem_empty_bar, s_ss, cluster_id, num_clusters, rank, s_out, ring);
+      if (p0.leaky) epilogue_loop_pair<MC_EPI_REORG2, true>(P, m, tmem_base, cluster_id, num_clusters, rank, ring);
+      else epilogue_loop_pair<MC_EPI_REORG2, false>(P, m, tmem_base, cluster_id, num_clusters, rank, ring);
     } else {
-      if (p0.leaky) epilogue_loop_pair<MC_EPI_NCHW_F32, true>(P, tmem_base, tmem_full_bar, tmem_empty_bar, s_ss, cluster_id, num_clusters, rank, s_out, ring);
-      else epilogue_loop_pair<MC_EPI_NCHW_F32, false>(P, tmem_base, tmem_full_bar, tmem_empty_bar, s_ss, cluster_id, num_clusters, rank, s_out, ring);
+      if (p0.leaky) epilogue_loop_pair<MC_EPI_NCHW_F32, true>(P, m, tmem_base, cluster_id, num_clusters, rank, ring);
+      else epilogue_loop_pair<MC_EPI_NCHW_F32, false>(P, m, tmem_base, cluster_id, num_clusters, rank, ring);
     }
   }
 
@@ -1389,8 +1293,8 @@ int pick_block_n(int Npad, int m_tiles, int num_kb, int num_sms, bool share_dx) 
 static thread_local int g_last_plan[8] = {0, 0, 0, 0, 0, 0, 0, 0};
 static unsigned long long* g_conv_dbg = nullptr;
 
-// Debug: timeline stamps of the single-CTA conv GEMM kernel (32 x uint64 per CTA, globaltimer ns) into d_buf, which
-// must hold 32 * 8 * grid bytes; NULL switches tracing off again.  tools/trace_conv.py prints the timelines.
+// Debug: timeline stamps of the conv GEMM kernels (32 x uint64 per CTA, globaltimer ns) into d_buf, which must hold
+// 32 * 8 * grid bytes; NULL switches tracing off again.  tools/trace_conv.py and tools/trace_chain.py print the timelines.
 extern "C" int mc_debug_conv_trace(void* d_buf) {
   g_conv_dbg = reinterpret_cast<unsigned long long*>(d_buf);
   return 0;

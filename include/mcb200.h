@@ -365,6 +365,11 @@ int mc_pack_pnhwc(const float* d_in, void* d_out, int B, int H, int W, int C, in
  * mc_conv_wgrad.  All activations / gradients are PNHWC bf16, per-channel statistics and weight gradients fp32.
  * -------------------------------------------------------------------------------------------- */
 
+/* The BatchNorm / pool passes below move 8 channels per 16-byte access, for any C up to 2048 (a ragged last group
+ * of C % 8 channels is handled; columns past C are never written).  They return an argument error unless
+ * C <= 2048, every pitch (ld*) and ch_off is a multiple of 8, every tensor pointer is 16-byte aligned and
+ * B*(H+1)*(W+1) (rows for mc_col_stats) is below 2^31.  Pitches of round_up(C, 8) and torch allocations meet this.    */
+
 /* d_sum[c] = sum over rows of z[row, ch_off+c]; d_sumsq[c] likewise of z^2 (may be NULL).  Pad rows are zero.       */
 int mc_col_stats(const void* d_z, int64_t rows, int C, int ld, int ch_off, float* d_sum, float* d_sumsq, void* stream);
 
@@ -394,7 +399,8 @@ int mc_maxpool2x2_backward(const void* d_a_full, int ld_a, const void* d_dpooled
  * the pool (nn.BatchNorm2d / nn.LeakyReLU / nn.MaxPool2d of src/nets.py:802-821 and their autograd backward): the
  * forward writes pooled = maxpool(bf16(act(z*scale + shift))) straight from z; the backward recomputes the window
  * from z, routes d_pooled to the first maximum and produces dbeta / dgamma / dz like mc_bn_backward — the un-pooled
- * activation and its gradient never exist.  Needs C = 8 * 2^k (mc_bn_pool_supported), even H and W.                */
+ * activation and its gradient never exist.  Needs C = 8 * 2^k <= 2048 (mc_bn_pool_supported), even H and W, and the
+ * pitch / alignment / row-count conditions above.                                                                   */
 int mc_bn_pool_supported(int C);
 int mc_bn_apply_pool(const void* d_z, int ld_z, int B, int H, int W, int C, const float* d_scale, const float* d_shift,
                      int leaky, void* d_pooled, int ld_p, void* stream);

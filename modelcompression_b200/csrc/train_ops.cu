@@ -11,51 +11,7 @@
 namespace {
 
 constexpr int TB = 256;
-
-__device__ __forceinline__ bool interior_row(long long row, int H, int W, int* b, int* y, int* x) {
-  const int xx = (int)(row % (W + 1));
-  const long long t = row / (W + 1);
-  const int yy = (int)(t % (H + 1));
-  *b = (int)(t / (H + 1));
-  *y = yy;
-  *x = xx;
-  return xx < W && yy < H;
-}
-
-// ---- column sums: sum[c] += z[row,c], sumsq[c] += z[row,c]^2 over all rows (pad rows are zero) -----------------------
-// block = 256 threads = 32 channel-octets x 8 row lanes; grid.x strides rows, grid.y strides channel groups of 256.
-__global__ void __launch_bounds__(TB) col_stats_kernel(const __nv_bfloat16* __restrict__ z, long long rows, int C, int ld,
-                                                       int ch_off, float* __restrict__ sum, float* __restrict__ sumsq) {
-  __shared__ float s_a[8][256], s_b[8][256];
-  const int cg = threadIdx.x & 31, rl = threadIdx.x >> 5;
-  const int c0 = blockIdx.y * 256 + cg * 8;
-  float a[8], b[8];
-#pragma unroll
-  for (int j = 0; j < 8; ++j) a[j] = b[j] = 0.f;
-  if (c0 < C) {
-    for (long long r = (long long)blockIdx.x * 8 + rl; r < rows; r += (long long)gridDim.x * 8) {
-      const uint4 q = *reinterpret_cast<const uint4*>(z + r * ld + ch_off + c0);
-      const __nv_bfloat162* h = reinterpret_cast<const __nv_bfloat162*>(&q);
-#pragma unroll
-      for (int j = 0; j < 4; ++j) {
-        const float2 f = __bfloat1622float2(h[j]);
-        a[2 * j] += f.x; b[2 * j] += f.x * f.x;
-        a[2 * j + 1] += f.y; b[2 * j + 1] += f.y * f.y;
-      }
-    }
-  }
-#pragma unroll
-  for (int j = 0; j < 8; ++j) { s_a[rl][cg * 8 + j] = a[j]; s_b[rl][cg * 8 + j] = b[j]; }
-  __syncthreads();
-  const int c = blockIdx.y * 256 + threadIdx.x;
-  if (c < C) {
-    float ta = 0.f, tb = 0.f;
-#pragma unroll
-    for (int k = 0; k < 8; ++k) { ta += s_a[k][threadIdx.x]; tb += s_b[k][threadIdx.x]; }
-    atomicAdd(&sum[c], ta);
-    if (sumsq) atomicAdd(&sumsq[c], tb);
-  }
-}
+constexpr int MAX_C = 8 * TB;  // one channel octet per thread of a block
 
 // ---- BN finalize: batch mean / biased var -> (scale, shift, mean, invstd); running stats update --------------------
 __global__ void bn_finalize_kernel(const float* __restrict__ sum, const float* __restrict__ sumsq, int C, double count,
@@ -81,162 +37,41 @@ __global__ void bn_finalize_kernel(const float* __restrict__ sum, const float* _
   }
 }
 
-// ---- BN apply (+leaky): out = act(z*scale+shift), pads zero; optional reorg / channel-slice store ------------------
-__global__ void __launch_bounds__(TB) bn_apply_kernel(const __nv_bfloat16* __restrict__ z, int ld_z, int B, int H, int W,
-                                                      int C, const float* __restrict__ scale,
-                                                      const float* __restrict__ shift, int leaky,
-                                                      __nv_bfloat16* __restrict__ out, int ld_out, int ch_off, int reorg) {
-  const int C8 = (C + 7) / 8;
-  const long long rows = (long long)B * (H + 1) * (W + 1);
-  const long long total = rows * C8;
-  for (long long i = blockIdx.x * (long long)TB + threadIdx.x; i < total; i += (long long)gridDim.x * TB) {
-    const long long row = i / C8;
-    const int c0 = (int)(i - row * C8) * 8;
-    int b, y, x;
-    const bool in = interior_row(row, H, W, &b, &y, &x);
-    __align__(16) __nv_bfloat16 o[8];
-    if (in) {
-      const uint4 q = *reinterpret_cast<const uint4*>(z + row * ld_z + c0);
-      const __nv_bfloat16* h = reinterpret_cast<const __nv_bfloat16*>(&q);
+// ---- 8 channels ("an octet") = one 16-byte access per thread ----------------------------------------------------
+// Octet mapping of every pass below: a block has O8 * floor(TB / O8) threads (O8 = ceil(C / 8) octets per row; TB for
+// every power of two), and thread t keeps octet t % O8 for the whole launch while it walks rows (pooled pixels for the
+// pool passes) row0, row0 + stride, ...  Its per-channel constants and accumulators live in registers, consecutive
+// threads touch consecutive 16-byte pieces of a row, and the threads that share an octet sit O8 apart in the block.
+struct OctetWalk {
+  int c0;                         // first channel of the thread's octet
+  unsigned int row0, stride;
+};
+__device__ __forceinline__ OctetWalk octet_walk(int O8) {
+  const unsigned int rows_per_block = blockDim.x / O8, q = threadIdx.x / O8;
+  return {(int)(threadIdx.x - q * O8) * 8, blockIdx.x * rows_per_block + q, gridDim.x * rows_per_block};
+}
+inline int octet_threads(int O8) { return O8 * (TB / O8); }
+
+// A ragged last octet (C % 8 != 0, the WHOLE = false instantiations): per-channel vectors read as 0 past C, stores
+// only below C (the columns past C may belong to a neighbouring concat slice), and accesses that are not 16-byte
+// aligned (Reorg quadrants q*C) go element by element.  n = C - c0 channels are left in the octet.
+template <bool WHOLE>
+__device__ __forceinline__ void load_ch(const float* __restrict__ p, int c0, int C, float (&v)[8]) {
 #pragma unroll
-      for (int j = 0; j < 8; ++j) {
-        float v = 0.f;
-        if (c0 + j < C) {
-          v = fmaf(__bfloat162float(h[j]), scale[c0 + j], shift[c0 + j]);
-          if (leaky) v = fmaxf(v, 0.1f * v);
-        }
-        o[j] = __float2bfloat16_rn(v);
-      }
-    } else {
+  for (int j = 0; j < 8; ++j) v[j] = (WHOLE || c0 + j < C) ? p[c0 + j] : 0.f;
+}
+template <bool WHOLE>
+__device__ __forceinline__ uint4 load8(const __nv_bfloat16* p, bool aligned, int n) {
+  if constexpr (!WHOLE) {
+    if (!aligned) {
+      unsigned int h[8];
 #pragma unroll
-      for (int j = 0; j < 8; ++j) o[j] = __float2bfloat16_rn(0.f);
-    }
-    if (!reorg) {
-      __nv_bfloat16* dst = out + row * ld_out + ch_off + c0;
-      if (c0 + 8 <= C && ((ld_out | ch_off) & 7) == 0) *reinterpret_cast<uint4*>(dst) = *reinterpret_cast<const uint4*>(o);
-      else
-        for (int j = 0; j < 8 && c0 + j < C; ++j) dst[j] = o[j];
-    } else if (in) {
-      const int Wo = W / 2 + 1, Ho = H / 2 + 1;
-      const long long orow = ((long long)b * Ho + (y >> 1)) * Wo + (x >> 1);
-      __nv_bfloat16* dst = out + orow * ld_out + ch_off + ((y & 1) * 2 + (x & 1)) * C + c0;
-      for (int j = 0; j < 8 && c0 + j < C; ++j) dst[j] = o[j];
+      for (int j = 0; j < 8; ++j) h[j] = j < n ? __bfloat16_as_ushort(p[j]) : 0u;
+      return make_uint4(h[0] | h[1] << 16, h[2] | h[3] << 16, h[4] | h[5] << 16, h[6] | h[7] << 16);
     }
   }
+  return *reinterpret_cast<const uint4*>(p);
 }
-
-// ---- BN + leaky backward -----------------------------------------------------------------------------------------
-// da is read through (ld_da, ch_off, reorg) so a concat slice / reorg'd tensor needs no un-shuffling copy.
-__device__ __forceinline__ const __nv_bfloat16* da_ptr(const __nv_bfloat16* da, long long row, int b, int y, int x, int H,
-                                                       int W, int C, int ld_da, int ch_off, int reorg) {
-  if (!reorg) return da + row * ld_da + ch_off;
-  const int Wo = W / 2 + 1, Ho = H / 2 + 1;
-  const long long orow = ((long long)b * Ho + (y >> 1)) * Wo + (x >> 1);
-  return da + orow * ld_da + ch_off + ((y & 1) * 2 + (x & 1)) * C;
-}
-
-// pass 1: dbeta[c] = sum g, dgamma[c] = sum g*xhat with g = da * leaky'(zhat), xhat = (z-mean)*invstd
-__global__ void __launch_bounds__(TB) bn_bwd_reduce_kernel(const __nv_bfloat16* __restrict__ z, int ld_z,
-                                                           const __nv_bfloat16* __restrict__ da, int ld_da, int ch_off,
-                                                           int reorg, int B, int H, int W, int C,
-                                                           const float* __restrict__ mean, const float* __restrict__ invstd,
-                                                           const float* __restrict__ gamma, const float* __restrict__ beta,
-                                                           int leaky, float* __restrict__ dbeta, float* __restrict__ dgamma) {
-  __shared__ float s_a[TB], s_b[TB];
-  // block handles channel c = blockIdx.y*32 + (tid&31) over a strided set of rows; 8 row lanes per block
-  const int c = blockIdx.y * 32 + (threadIdx.x & 31);
-  const int rl = threadIdx.x >> 5;
-  const long long rows = (long long)B * (H + 1) * (W + 1);
-  float sa = 0.f, sb = 0.f;
-  if (c < C) {
-    const float m = mean[c], is = invstd[c], g0 = gamma ? gamma[c] : 1.f, b0 = beta ? beta[c] : 0.f;
-    for (long long r = (long long)blockIdx.x * 8 + rl; r < rows; r += (long long)gridDim.x * 8) {
-      int b, y, x;
-      if (!interior_row(r, H, W, &b, &y, &x)) continue;
-      const float xh = (__bfloat162float(z[r * ld_z + c]) - m) * is;
-      float g = __bfloat162float(da_ptr(da, r, b, y, x, H, W, C, ld_da, ch_off, reorg)[c]);
-      if (leaky && (g0 * xh + b0) <= 0.f) g *= 0.1f;
-      sa += g;
-      sb += g * xh;
-    }
-  }
-  s_a[threadIdx.x] = sa;
-  s_b[threadIdx.x] = sb;
-  __syncthreads();
-  if (rl == 0 && c < C) {
-    for (int k = 1; k < 8; ++k) { sa += s_a[k * 32 + threadIdx.x]; sb += s_b[k * 32 + threadIdx.x]; }
-    atomicAdd(&dbeta[c], sa);
-    atomicAdd(&dgamma[c], sb);
-  }
-}
-
-// pass 2: dz = gamma*invstd*(g - dbeta/N - xhat*dgamma/N) at interior pixels, 0 at pads.  With bn == 0 (no BatchNorm:
-// the head) dz = g.
-__global__ void __launch_bounds__(TB) bn_bwd_apply_kernel(const __nv_bfloat16* __restrict__ z, int ld_z,
-                                                          const __nv_bfloat16* __restrict__ da, int ld_da, int ch_off,
-                                                          int reorg, int B, int H, int W, int C,
-                                                          const float* __restrict__ mean, const float* __restrict__ invstd,
-                                                          const float* __restrict__ gamma, const float* __restrict__ beta,
-                                                          int leaky, const float* __restrict__ dbeta,
-                                                          const float* __restrict__ dgamma, float inv_count,
-                                                          __nv_bfloat16* __restrict__ dz, int ld_dz) {
-  const long long rows = (long long)B * (H + 1) * (W + 1);
-  const long long total = rows * C;
-  for (long long i = blockIdx.x * (long long)TB + threadIdx.x; i < total; i += (long long)gridDim.x * TB) {
-    const long long row = i / C;
-    const int c = (int)(i - row * C);
-    int b, y, x;
-    float v = 0.f;
-    if (interior_row(row, H, W, &b, &y, &x)) {
-      const float xh = (__bfloat162float(z[row * ld_z + c]) - mean[c]) * invstd[c];
-      float g = __bfloat162float(da_ptr(da, row, b, y, x, H, W, C, ld_da, ch_off, reorg)[c]);
-      if (leaky && (gamma[c] * xh + beta[c]) <= 0.f) g *= 0.1f;
-      v = gamma[c] * invstd[c] * (g - dbeta[c] * inv_count - xh * dgamma[c] * inv_count);
-    }
-    dz[row * ld_dz + c] = __float2bfloat16_rn(v);
-  }
-}
-
-// ---- max-pool 2x2/2 backward: gradient goes to the first maximum of each window (PyTorch scan order) ---------------
-__global__ void __launch_bounds__(TB) maxpool_bwd_kernel(const __nv_bfloat16* __restrict__ a_full, int ld_a,
-                                                         const __nv_bfloat16* __restrict__ d_pooled, int ld_dp, int B,
-                                                         int H, int W, int C, __nv_bfloat16* __restrict__ d_full,
-                                                         int ld_df, int accumulate) {
-  const long long rows = (long long)B * (H + 1) * (W + 1);
-  const long long total = rows * C;
-  const int Ho = H / 2, Wo = W / 2;
-  for (long long i = blockIdx.x * (long long)TB + threadIdx.x; i < total; i += (long long)gridDim.x * TB) {
-    const long long row = i / C;
-    const int c = (int)(i - row * C);
-    int b, y, x;
-    float v = 0.f;
-    if (interior_row(row, H, W, &b, &y, &x)) {
-      const int wy = y >> 1, wx = x >> 1;
-      const long long r00 = ((long long)b * (H + 1) + 2 * wy) * (W + 1) + 2 * wx;
-      const float v00 = __bfloat162float(a_full[r00 * ld_a + c]);
-      const float v01 = __bfloat162float(a_full[(r00 + 1) * ld_a + c]);
-      const float v10 = __bfloat162float(a_full[(r00 + W + 1) * ld_a + c]);
-      const float v11 = __bfloat162float(a_full[(r00 + W + 2) * ld_a + c]);
-      int arg = 0;
-      float best = v00;
-      if (v01 > best) { best = v01; arg = 1; }
-      if (v10 > best) { best = v10; arg = 2; }
-      if (v11 > best) { best = v11; arg = 3; }
-      if (arg == ((y & 1) * 2 + (x & 1))) {
-        const long long prow = ((long long)b * (Ho + 1) + wy) * (Wo + 1) + wx;
-        v = __bfloat162float(d_pooled[prow * ld_dp + c]);
-      }
-    }
-    __nv_bfloat16* dst = d_full + row * ld_df + c;
-    if (accumulate) v += __bfloat162float(*dst);
-    *dst = __float2bfloat16_rn(v);
-  }
-}
-
-// ---- vectorised versions (8 channels = one 16-byte access per thread) -----------------------------------------
-// Work item i = row * O8 + octet (O8 = C/8 octets per row).  The launch uses a thread count that is a multiple of O8,
-// so a thread meets the same octet on every grid-stride step: its per-channel constants / accumulators live in
-// registers, and consecutive threads touch consecutive 16-byte pieces of a row.
 __device__ __forceinline__ void unpack8(const uint4& q, float (&f)[8]) {
   const __nv_bfloat162* h = reinterpret_cast<const __nv_bfloat162*>(&q);
 #pragma unroll
@@ -253,6 +88,36 @@ __device__ __forceinline__ uint4 pack8(const float (&f)[8]) {
   for (int j = 0; j < 4; ++j) h[j] = __floats2bfloat162_rn(f[2 * j], f[2 * j + 1]);
   return q;
 }
+template <bool WHOLE>
+__device__ __forceinline__ void store8(__nv_bfloat16* p, bool aligned, int n, const float (&f)[8]) {
+  if constexpr (!WHOLE) {
+    if (!aligned || n < 8) {
+#pragma unroll
+      for (int j = 0; j < 8; ++j)
+        if (j < n) p[j] = __float2bfloat16_rn(f[j]);
+      return;
+    }
+  }
+  *reinterpret_cast<uint4*>(p) = pack8(f);
+}
+
+// sum[c] += the block's partials a[c] (sumsq[c] += b[c] unless sumsq is NULL): one atomic per channel and block, the
+// threads of a channel added in thread order.  Channels >= C (a ragged last octet) are dropped.
+__device__ __forceinline__ void block_col_sums(const float (&a)[8], const float (&b)[8], int O8, int C,
+                                               float* __restrict__ sum, float* __restrict__ sumsq) {
+  __shared__ float s_a[TB][9], s_b[TB][9];  // padded rows: conflict-free column sums
+#pragma unroll
+  for (int j = 0; j < 8; ++j) { s_a[threadIdx.x][j] = a[j]; s_b[threadIdx.x][j] = b[j]; }
+  __syncthreads();
+  for (int c = threadIdx.x; c < C; c += blockDim.x) {
+    const int o = c >> 3, j = c & 7;
+    float ta = 0.f, tb = 0.f;
+    for (int t = o; t < (int)blockDim.x; t += O8) { ta += s_a[t][j]; tb += s_b[t][j]; }
+    atomicAdd(&sum[c], ta);
+    if (sumsq) atomicAdd(&sumsq[c], tb);
+  }
+}
+
 // Division by a run-time constant without the ~30-instruction integer divide (these kernels issue three per 16 bytes
 // and were instruction-bound): q = umulhi(n, mul) >> shr, exact for n < 2^31 and d >= 2 (mul = ceil(2^(31+ceil_log2 d) / d)).
 struct FastDiv {
@@ -282,130 +147,138 @@ __device__ __forceinline__ bool row_coords(unsigned int row, const FastDiv& Wp, 
   *x = (int)xx;
   return (int)xx < W && (int)yy < H;
 }
-__device__ __forceinline__ const uint4* da_vec(const __nv_bfloat16* da, unsigned int row, int b, int y, int x, int H,
-                                               int W, int C, int ld_da, int ch_off, int reorg, int c0) {
-  if (!reorg) return reinterpret_cast<const uint4*>(da + (long long)row * ld_da + ch_off + c0);
+
+// Element offset of row (b, y, x) of an activation in a buffer addressed through (ld, ch_off), or through the Reorg(2)
+// shuffle into a (H/2, W/2) buffer at channel ch_off + ((y&1)*2 + (x&1))*C (interior rows only), so that a concat slice
+// or a reorg'd tensor is written / read in place.
+__device__ __forceinline__ long long act_offset(unsigned int row, int b, int y, int x, int H, int W, int C, int ld,
+                                                int ch_off, int reorg) {
+  if (!reorg) return (long long)row * ld + ch_off;
   const int Wo = W / 2 + 1, Ho = H / 2 + 1;
   const long long orow = ((long long)b * Ho + (y >> 1)) * Wo + (x >> 1);
-  return reinterpret_cast<const uint4*>(da + orow * ld_da + ch_off + ((y & 1) * 2 + (x & 1)) * C + c0);
+  return orow * ld + ch_off + ((y & 1) * 2 + (x & 1)) * C;
 }
 
-__global__ void __launch_bounds__(TB, 3) bn_bwd_reduce_vec_kernel(const __nv_bfloat16* __restrict__ z, int ld_z,
-                                                               const __nv_bfloat16* __restrict__ da, int ld_da, int ch_off,
-                                                               int reorg, int B, int H, int W, int C, int O8,
-                                                               const float* __restrict__ mean, const float* __restrict__ invstd,
-                                                               const float* __restrict__ gamma, const float* __restrict__ beta,
-                                                               int leaky, float* __restrict__ dbeta, float* __restrict__ dgamma,
-                                                               int o8_shift, FastDiv fWp, FastDiv fHp) {
-  __shared__ float s_a[TB][9], s_b[TB][9];  // padded rows: conflict-free column sums
+// ---- column sums: sum[c] += z[row, ch_off+c], sumsq[c] += z[row, ch_off+c]^2 over all rows (pad rows are zero) -----
+__global__ void __launch_bounds__(TB) col_stats_vec_kernel(const __nv_bfloat16* __restrict__ z, unsigned int rows, int C,
+                                                           int O8, int ld, int ch_off, float* __restrict__ sum,
+                                                           float* __restrict__ sumsq) {
+  const OctetWalk w = octet_walk(O8);
+  const __nv_bfloat16* zc = z + ch_off + w.c0;
+  float a[8], b[8];
+#pragma unroll
+  for (int j = 0; j < 8; ++j) a[j] = b[j] = 0.f;
+  unsigned int r = w.row0;
+  // 4 independent 16-byte loads in flight per thread
+  for (; r + 3 * w.stride < rows; r += 4 * w.stride) {
+    uint4 q[4];
+#pragma unroll
+    for (int u = 0; u < 4; ++u) q[u] = *reinterpret_cast<const uint4*>(zc + (long long)(r + u * w.stride) * ld);
+#pragma unroll
+    for (int u = 0; u < 4; ++u) {
+      float f[8];
+      unpack8(q[u], f);
+#pragma unroll
+      for (int j = 0; j < 8; ++j) { a[j] += f[j]; b[j] = fmaf(f[j], f[j], b[j]); }
+    }
+  }
+  for (; r < rows; r += w.stride) {
+    float f[8];
+    unpack8(*reinterpret_cast<const uint4*>(zc + (long long)r * ld), f);
+#pragma unroll
+    for (int j = 0; j < 8; ++j) { a[j] += f[j]; b[j] = fmaf(f[j], f[j], b[j]); }
+  }
+  block_col_sums(a, b, O8, C, sum, sumsq);
+}
+
+// ---- BN apply (+leaky): out = act(z*scale+shift), pads zero; optional reorg / channel-slice store ------------------
+template <bool WHOLE>
+__global__ void __launch_bounds__(TB) bn_apply_vec_kernel(const __nv_bfloat16* __restrict__ z, int ld_z, int B, int H, int W,
+                                                          int C, int O8, const float* __restrict__ scale,
+                                                          const float* __restrict__ shift, int leaky,
+                                                          __nv_bfloat16* __restrict__ out, int ld_out, int ch_off, int reorg,
+                                                          FastDiv fWp, FastDiv fHp) {
+  const OctetWalk w = octet_walk(O8);
   const unsigned int rows = (unsigned int)B * (H + 1) * (W + 1);
-  const unsigned int total = rows * (unsigned int)O8;  // host guarantees < 2^32
-  const unsigned int nthreads = gridDim.x * TB;        // multiple of O8
-  unsigned int i = blockIdx.x * TB + threadIdx.x;
-  const int oc = (int)(i & (unsigned int)(O8 - 1)), c0 = oc * 8;  // O8 is a power of two on this path
-  float m[8], is[8], g0[8], b0[8], sa[8], sb[8];
+  float sc[8], sh[8];
+  load_ch<WHOLE>(scale, w.c0, C, sc);
+  load_ch<WHOLE>(shift, w.c0, C, sh);
+  for (unsigned int row = w.row0; row < rows; row += w.stride) {
+    int b, y, x;
+    const bool in = row_coords(row, fWp, fHp, H, W, &b, &y, &x);
+    float o[8];
+    if (in) {
+      float f[8];
+      unpack8(*reinterpret_cast<const uint4*>(z + (long long)row * ld_z + w.c0), f);
+#pragma unroll
+      for (int j = 0; j < 8; ++j) {
+        const float v = fmaf(f[j], sc[j], sh[j]);
+        o[j] = leaky ? fmaxf(v, 0.1f * v) : v;
+      }
+    } else {
+#pragma unroll
+      for (int j = 0; j < 8; ++j) o[j] = 0.f;
+    }
+    if (!reorg || in) store8<WHOLE>(out + act_offset(row, b, y, x, H, W, C, ld_out, ch_off, reorg) + w.c0, !reorg, C - w.c0, o);
+  }
+}
+
+// ---- BN + leaky backward -----------------------------------------------------------------------------------------
+// APPLY = false: dbeta += sum g, dgamma += sum g*xhat.  APPLY = true: dz = gamma*invstd*(g - dbeta/N - xhat*dgamma/N)
+// at interior pixels, 0 at pads.  g = da * leaky'(gamma*xhat + beta), xhat = (z-mean)*invstd; da is read through
+// (ld_da, ch_off, reorg) so a concat slice / reorg'd gradient needs no un-shuffling copy.
+template <bool APPLY, bool WHOLE>
+__global__ void __launch_bounds__(TB, 3) bn_bwd_vec_kernel(const __nv_bfloat16* __restrict__ z, int ld_z,
+                                                           const __nv_bfloat16* __restrict__ da, int ld_da, int ch_off,
+                                                           int reorg, int B, int H, int W, int C, int O8,
+                                                           const float* __restrict__ mean, const float* __restrict__ invstd,
+                                                           const float* __restrict__ gamma, const float* __restrict__ beta,
+                                                           int leaky, float* __restrict__ dbeta, float* __restrict__ dgamma,
+                                                           float inv_count, __nv_bfloat16* __restrict__ dz, int ld_dz,
+                                                           FastDiv fWp, FastDiv fHp) {
+  OctetWalk w = octet_walk(O8);
+  asm("" : "+r"(w.c0));  // keep c0 in a register: rebuilt from threadIdx.x / O8 in the loop it cost a spill (ptxas -v)
+  const unsigned int rows = (unsigned int)B * (H + 1) * (W + 1);
+  const int n = C - w.c0;
+  float m[8], is[8], g0[8], b0[8], k1[8], kb[8], kg[8], sa[8], sb[8];
+  load_ch<WHOLE>(mean, w.c0, C, m);
+  load_ch<WHOLE>(invstd, w.c0, C, is);
+  load_ch<WHOLE>(gamma, w.c0, C, g0);
+  load_ch<WHOLE>(beta, w.c0, C, b0);
+  if (APPLY) {
+    load_ch<WHOLE>(dbeta, w.c0, C, kb);
+    load_ch<WHOLE>(dgamma, w.c0, C, kg);
+  }
 #pragma unroll
   for (int j = 0; j < 8; ++j) {
-    m[j] = mean[c0 + j]; is[j] = invstd[c0 + j]; g0[j] = gamma[c0 + j]; b0[j] = beta[c0 + j];
+    k1[j] = g0[j] * is[j];
+    kb[j] = APPLY ? kb[j] * inv_count : 0.f;
+    kg[j] = APPLY ? kg[j] * inv_count : 0.f;
     sa[j] = sb[j] = 0.f;
   }
   const uint4 zero4 = make_uint4(0u, 0u, 0u, 0u);
-  for (; i < total; i += 2 * nthreads) {  // two items per step: four independent 16-byte loads in flight
+  for (unsigned int row = w.row0; row < rows; row += 2 * w.stride) {  // two rows per step: four 16-byte loads in flight
     uint4 qz[2], qa[2];
-    bool in[2];
+    bool ok[2], in[2];
+    unsigned int r[2];
 #pragma unroll
     for (int u = 0; u < 2; ++u) {
-      const unsigned int it = i + u * nthreads;
+      r[u] = row + u * w.stride;
+      ok[u] = r[u] < rows;
       in[u] = false;
       qz[u] = qa[u] = zero4;
-      if (it < total) {
-        const unsigned int row = it >> o8_shift;
-        int b, y, x;
-        in[u] = row_coords(row, fWp, fHp, H, W, &b, &y, &x);
-        if (in[u]) {
-          qz[u] = *reinterpret_cast<const uint4*>(z + (long long)row * ld_z + c0);
-          qa[u] = *da_vec(da, row, b, y, x, H, W, C, ld_da, ch_off, reorg, c0);
-        }
-      }
-    }
-#pragma unroll
-    for (int u = 0; u < 2; ++u) {
-      if (!in[u]) continue;
-      float fz[8], fa[8];
-      unpack8(qz[u], fz);
-      unpack8(qa[u], fa);
-#pragma unroll
-      for (int j = 0; j < 8; ++j) {
-        const float xh = (fz[j] - m[j]) * is[j];
-        float g = fa[j];
-        if (leaky && (g0[j] * xh + b0[j]) <= 0.f) g *= 0.1f;
-        sa[j] += g;
-        sb[j] += g * xh;
-      }
-    }
-  }
-#pragma unroll
-  for (int j = 0; j < 8; ++j) { s_a[threadIdx.x][j] = sa[j]; s_b[threadIdx.x][j] = sb[j]; }
-  __syncthreads();
-  // threads with the same octet are O8 apart inside the block (TB % O8 == 0)
-  for (int w = threadIdx.x; w < O8 * 8; w += TB) {
-    const int o2 = w >> 3, j = w & 7;
-    float ta = 0.f, tb = 0.f;
-    const int first = (int)(((unsigned int)O8 + o2 - (blockIdx.x * TB) % (unsigned int)O8) % (unsigned int)O8);
-    for (int t = first; t < TB; t += O8) { ta += s_a[t][j]; tb += s_b[t][j]; }
-    atomicAdd(&dbeta[o2 * 8 + j], ta);
-    atomicAdd(&dgamma[o2 * 8 + j], tb);
-  }
-}
-
-__global__ void __launch_bounds__(TB, 3) bn_bwd_apply_vec_kernel(const __nv_bfloat16* __restrict__ z, int ld_z,
-                                                              const __nv_bfloat16* __restrict__ da, int ld_da, int ch_off,
-                                                              int reorg, int B, int H, int W, int C, int O8,
-                                                              const float* __restrict__ mean, const float* __restrict__ invstd,
-                                                              const float* __restrict__ gamma, const float* __restrict__ beta,
-                                                              int leaky, const float* __restrict__ dbeta,
-                                                              const float* __restrict__ dgamma, float inv_count,
-                                                              __nv_bfloat16* __restrict__ dz, int ld_dz, int o8_shift,
-                                                              FastDiv fWp, FastDiv fHp) {
-  const unsigned int rows = (unsigned int)B * (H + 1) * (W + 1);
-  const unsigned int total = rows * (unsigned int)O8;
-  const unsigned int nthreads = gridDim.x * TB;
-  unsigned int i = blockIdx.x * TB + threadIdx.x;
-  const int oc = (int)(i & (unsigned int)(O8 - 1)), c0 = oc * 8;  // O8 is a power of two on this path
-  float m[8], is[8], g0[8], b0[8], k1[8], kb[8], kg[8];
-#pragma unroll
-  for (int j = 0; j < 8; ++j) {
-    m[j] = mean[c0 + j]; is[j] = invstd[c0 + j]; g0[j] = gamma[c0 + j]; b0[j] = beta[c0 + j];
-    k1[j] = g0[j] * is[j];
-    kb[j] = dbeta[c0 + j] * inv_count;
-    kg[j] = dgamma[c0 + j] * inv_count;
-  }
-  const uint4 zero4 = make_uint4(0u, 0u, 0u, 0u);
-  for (; i < total; i += 2 * nthreads) {  // two items per step: four independent 16-byte loads in flight
-    uint4 qz[2], qa[2];
-    bool in[2], ok[2];
-    unsigned int rows2[2];
-#pragma unroll
-    for (int u = 0; u < 2; ++u) {
-      const unsigned int it = i + u * nthreads;
-      ok[u] = it < total;
-      in[u] = false;
-      qz[u] = qa[u] = zero4;
-      rows2[u] = 0;
       if (ok[u]) {
-        const unsigned int row = it >> o8_shift;
-        rows2[u] = row;
         int b, y, x;
-        in[u] = row_coords(row, fWp, fHp, H, W, &b, &y, &x);
+        in[u] = row_coords(r[u], fWp, fHp, H, W, &b, &y, &x);
         if (in[u]) {
-          qz[u] = *reinterpret_cast<const uint4*>(z + (long long)row * ld_z + c0);
-          qa[u] = *da_vec(da, row, b, y, x, H, W, C, ld_da, ch_off, reorg, c0);
+          qz[u] = *reinterpret_cast<const uint4*>(z + (long long)r[u] * ld_z + w.c0);
+          qa[u] = load8<WHOLE>(da + act_offset(r[u], b, y, x, H, W, C, ld_da, ch_off, reorg) + w.c0, !reorg, n);
         }
       }
     }
 #pragma unroll
     for (int u = 0; u < 2; ++u) {
-      if (!ok[u]) continue;
+      if (!(APPLY ? ok[u] : in[u])) continue;
       float out[8];
       if (in[u]) {
         float fz[8], fa[8];
@@ -416,28 +289,35 @@ __global__ void __launch_bounds__(TB, 3) bn_bwd_apply_vec_kernel(const __nv_bflo
           const float xh = (fz[j] - m[j]) * is[j];
           float g = fa[j];
           if (leaky && (g0[j] * xh + b0[j]) <= 0.f) g *= 0.1f;
-          out[j] = k1[j] * (g - kb[j] - xh * kg[j]);
+          if (APPLY) {
+            out[j] = k1[j] * (g - kb[j] - xh * kg[j]);
+          } else {
+            sa[j] += g;
+            sb[j] += g * xh;
+          }
         }
       } else {
 #pragma unroll
         for (int j = 0; j < 8; ++j) out[j] = 0.f;
       }
-      *reinterpret_cast<uint4*>(dz + (long long)rows2[u] * ld_dz + c0) = pack8(out);
+      if (APPLY) store8<WHOLE>(dz + (long long)r[u] * ld_dz + w.c0, true, n, out);
     }
   }
+  if (!APPLY) block_col_sums(sa, sb, O8, C, dbeta, dgamma);
 }
 
+// ---- max-pool 2x2/2 backward: gradient goes to the first maximum of each window (PyTorch scan order) ---------------
 // one thread = one pooled pixel x 8 channels: the 2x2 window is read once, the four gradients written once.  Pad
 // rows/columns of d_full are not touched (they are zero and stay zero).
+template <bool WHOLE>
 __global__ void __launch_bounds__(TB) maxpool_bwd_vec_kernel(const __nv_bfloat16* __restrict__ a_full, int ld_a,
                                                              const __nv_bfloat16* __restrict__ d_pooled, int ld_dp, int B,
-                                                             int H, int W, int O8, __nv_bfloat16* __restrict__ d_full,
+                                                             int H, int W, int C, int O8, __nv_bfloat16* __restrict__ d_full,
                                                              int ld_df, int accumulate) {
-  const int Ho = H / 2, Wo = W / 2;
-  const unsigned int total = (unsigned int)B * Ho * Wo * O8;
-  for (unsigned int i = blockIdx.x * TB + threadIdx.x; i < total; i += gridDim.x * TB) {
-    const unsigned int pix = i / (unsigned int)O8;
-    const int c0 = (int)(i - pix * (unsigned int)O8) * 8;
+  const OctetWalk w = octet_walk(O8);
+  const int Ho = H / 2, Wo = W / 2, c0 = w.c0;
+  const unsigned int pixels = (unsigned int)B * Ho * Wo;
+  for (unsigned int pix = w.row0; pix < pixels; pix += w.stride) {
     const unsigned int t = pix / (unsigned int)Wo;
     const int wx = (int)(pix - t * (unsigned int)Wo);
     const int b = (int)(t / (unsigned int)Ho), wy = (int)(t - (t / (unsigned int)Ho) * (unsigned int)Ho);
@@ -461,97 +341,14 @@ __global__ void __launch_bounds__(TB) maxpool_bwd_vec_kernel(const __nv_bfloat16
     }
 #pragma unroll
     for (int q = 0; q < 4; ++q) {
-      uint4* dst = reinterpret_cast<uint4*>(d_full + roff[q] * ld_df + c0);
+      __nv_bfloat16* dst = d_full + roff[q] * ld_df + c0;
       if (accumulate) {
         float old[8];
-        unpack8(*dst, old);
+        unpack8(*reinterpret_cast<const uint4*>(dst), old);
 #pragma unroll
         for (int j = 0; j < 8; ++j) o[q][j] += old[j];
       }
-      *dst = pack8(o[q]);
-    }
-  }
-}
-
-__global__ void __launch_bounds__(TB) col_stats_vec_kernel(const __nv_bfloat16* __restrict__ z, unsigned int rows, int O8,
-                                                           int ld, int ch_off, float* __restrict__ sum,
-                                                           float* __restrict__ sumsq, int o8_shift) {
-  __shared__ float s_a[TB][9], s_b[TB][9];
-  const unsigned int total = rows * (unsigned int)O8;
-  const unsigned int nthreads = gridDim.x * TB;  // multiple of O8
-  unsigned int i = blockIdx.x * TB + threadIdx.x;
-  const int c0 = (int)(i & (unsigned int)(O8 - 1)) * 8;  // O8 is a power of two on this path
-  float a[8], b[8];
-#pragma unroll
-  for (int j = 0; j < 8; ++j) a[j] = b[j] = 0.f;
-  // 4 independent 16-byte loads in flight per thread
-  for (; i + 3 * nthreads < total; i += 4 * nthreads) {
-    uint4 q[4];
-#pragma unroll
-    for (int u = 0; u < 4; ++u)
-      q[u] = *reinterpret_cast<const uint4*>(z + (long long)((i + u * nthreads) >> o8_shift) * ld + ch_off + c0);
-#pragma unroll
-    for (int u = 0; u < 4; ++u) {
-      float f[8];
-      unpack8(q[u], f);
-#pragma unroll
-      for (int j = 0; j < 8; ++j) { a[j] += f[j]; b[j] = fmaf(f[j], f[j], b[j]); }
-    }
-  }
-  for (; i < total; i += nthreads) {
-    float f[8];
-    unpack8(*reinterpret_cast<const uint4*>(z + (long long)(i >> o8_shift) * ld + ch_off + c0), f);
-#pragma unroll
-    for (int j = 0; j < 8; ++j) { a[j] += f[j]; b[j] = fmaf(f[j], f[j], b[j]); }
-  }
-#pragma unroll
-  for (int j = 0; j < 8; ++j) { s_a[threadIdx.x][j] = a[j]; s_b[threadIdx.x][j] = b[j]; }
-  __syncthreads();
-  for (int w = threadIdx.x; w < O8 * 8; w += TB) {
-    const int o2 = w >> 3, j = w & 7;
-    float ta = 0.f, tb = 0.f;
-    for (int t = o2; t < TB; t += O8) { ta += s_a[t][j]; tb += s_b[t][j]; }
-    atomicAdd(&sum[o2 * 8 + j], ta);
-    if (sumsq) atomicAdd(&sumsq[o2 * 8 + j], tb);
-  }
-}
-
-__global__ void __launch_bounds__(TB) bn_apply_vec_kernel(const __nv_bfloat16* __restrict__ z, int ld_z, int B, int H, int W,
-                                                          int C, int O8, const float* __restrict__ scale,
-                                                          const float* __restrict__ shift, int leaky,
-                                                          __nv_bfloat16* __restrict__ out, int ld_out, int ch_off, int reorg,
-                                                          int o8_shift, FastDiv fWp, FastDiv fHp) {
-  const unsigned int rows = (unsigned int)B * (H + 1) * (W + 1);
-  const unsigned int total = rows * (unsigned int)O8;
-  const unsigned int nthreads = gridDim.x * TB;
-  unsigned int i = blockIdx.x * TB + threadIdx.x;
-  const int c0 = (int)(i & (unsigned int)(O8 - 1)) * 8;  // O8 is a power of two on this path
-  float sc[8], sh[8];
-#pragma unroll
-  for (int j = 0; j < 8; ++j) { sc[j] = scale[c0 + j]; sh[j] = shift[c0 + j]; }
-  for (; i < total; i += nthreads) {
-    const unsigned int row = i >> o8_shift;
-    int b, y, x;
-    const bool in = row_coords(row, fWp, fHp, H, W, &b, &y, &x);
-    float o[8];
-    if (in) {
-      float f[8];
-      unpack8(*reinterpret_cast<const uint4*>(z + (long long)row * ld_z + c0), f);
-#pragma unroll
-      for (int j = 0; j < 8; ++j) {
-        const float v = fmaf(f[j], sc[j], sh[j]);
-        o[j] = leaky ? fmaxf(v, 0.1f * v) : v;
-      }
-    } else {
-#pragma unroll
-      for (int j = 0; j < 8; ++j) o[j] = 0.f;
-    }
-    if (!reorg) {
-      *reinterpret_cast<uint4*>(out + (long long)row * ld_out + ch_off + c0) = pack8(o);
-    } else if (in) {
-      const int Wo = W / 2 + 1, Ho = H / 2 + 1;
-      const long long orow = ((long long)b * Ho + (y >> 1)) * Wo + (x >> 1);
-      *reinterpret_cast<uint4*>(out + orow * ld_out + ch_off + ((y & 1) * 2 + (x & 1)) * C + c0) = pack8(o);
+      store8<WHOLE>(dst, true, C - c0, o[q]);
     }
   }
 }
@@ -562,7 +359,7 @@ __global__ void __launch_bounds__(TB) bn_apply_vec_kernel(const __nv_bfloat16* _
 // stored tensor would have had), routes the pooled gradient to the first maximum — nn.MaxPool2d's rule — and feeds the
 // BatchNorm reductions / dz directly.  Per pooled layer this moves 1.25 S (forward) + 3.5 S (backward) bytes instead
 // of 2 S + 1.25 S and 7.25 S (S = bytes of z): the four pooled layers of Darknet-19 hold 63 % of all activation bytes.
-// Work item = (pooled pixel, channel octet); a thread keeps its octet over the grid-stride loop like the kernels above.
+// A thread keeps its octet over the pooled pixels like the kernels above; C is a whole number of octets.
 __device__ __forceinline__ float bf16_round(float v) { return __bfloat162float(__float2bfloat16_rn(v)); }
 
 __device__ __forceinline__ void pool_item(unsigned int pix, const FastDiv& fWo, const FastDiv& fHo, int H, int W,
@@ -578,18 +375,17 @@ __device__ __forceinline__ void pool_item(unsigned int pix, const FastDiv& fWo, 
 __global__ void __launch_bounds__(TB) bn_apply_pool_vec_kernel(const __nv_bfloat16* __restrict__ z, int ld_z, int B, int H,
                                                                int W, int O8, const float* __restrict__ scale,
                                                                const float* __restrict__ shift, int leaky,
-                                                               __nv_bfloat16* __restrict__ pooled, int ld_p, int o8_shift,
-                                                               FastDiv fWo, FastDiv fHo) {
-  const unsigned int total = (unsigned int)B * fHo.d * fWo.d * (unsigned int)O8;
-  const unsigned int nthreads = gridDim.x * TB;
-  unsigned int i = blockIdx.x * TB + threadIdx.x;
-  const int c0 = (int)(i & (unsigned int)(O8 - 1)) * 8;
+                                                               __nv_bfloat16* __restrict__ pooled, int ld_p, FastDiv fWo,
+                                                               FastDiv fHo) {
+  const OctetWalk w = octet_walk(O8);
+  const int c0 = w.c0;
+  const unsigned int pixels = (unsigned int)B * fHo.d * fWo.d;
   float sc[8], sh[8];
 #pragma unroll
   for (int j = 0; j < 8; ++j) { sc[j] = scale[c0 + j]; sh[j] = shift[c0 + j]; }
-  for (; i < total; i += nthreads) {
+  for (unsigned int pix = w.row0; pix < pixels; pix += w.stride) {
     long long r00, prow;
-    pool_item(i >> o8_shift, fWo, fHo, H, W, &r00, &prow);
+    pool_item(pix, fWo, fHo, H, W, &r00, &prow);
     const long long roff[4] = {r00, r00 + 1, r00 + W + 1, r00 + W + 2};
     uint4 q[4];
 #pragma unroll
@@ -622,12 +418,10 @@ __global__ void __launch_bounds__(TB, 2) bn_pool_bwd_vec_kernel(const __nv_bfloa
                                                                 const float* __restrict__ invstd, int leaky,
                                                                 float* __restrict__ dbeta, float* __restrict__ dgamma,
                                                                 float inv_count, __nv_bfloat16* __restrict__ dz, int ld_dz,
-                                                                int o8_shift, FastDiv fWo, FastDiv fHo) {
-  __shared__ float s_a[APPLY ? 1 : TB][9], s_b[APPLY ? 1 : TB][9];
-  const unsigned int total = (unsigned int)B * fHo.d * fWo.d * (unsigned int)O8;
-  const unsigned int nthreads = gridDim.x * TB;  // multiple of O8
-  unsigned int i = blockIdx.x * TB + threadIdx.x;
-  const int c0 = (int)(i & (unsigned int)(O8 - 1)) * 8;
+                                                                FastDiv fWo, FastDiv fHo) {
+  const OctetWalk w = octet_walk(O8);
+  const int c0 = w.c0;
+  const unsigned int pixels = (unsigned int)B * fHo.d * fWo.d;
   float sc[8], sh[8], m[8], is[8], kb[8], kg[8], sa[8], sb[8];
 #pragma unroll
   for (int j = 0; j < 8; ++j) {
@@ -638,9 +432,9 @@ __global__ void __launch_bounds__(TB, 2) bn_pool_bwd_vec_kernel(const __nv_bfloa
     kg[j] = APPLY ? dgamma[c0 + j] * inv_count : 0.f;
   }
   const float slope = leaky ? 0.1f : 1.0f;
-  for (; i < total; i += nthreads) {
+  for (unsigned int pix = w.row0; pix < pixels; pix += w.stride) {
     long long r00, prow;
-    pool_item(i >> o8_shift, fWo, fHo, H, W, &r00, &prow);
+    pool_item(pix, fWo, fHo, H, W, &r00, &prow);
     const long long roff[4] = {r00, r00 + 1, r00 + W + 1, r00 + W + 2};
     uint4 q[4];
 #pragma unroll
@@ -685,40 +479,28 @@ __global__ void __launch_bounds__(TB, 2) bn_pool_bwd_vec_kernel(const __nv_bfloa
       }
     }
   }
-  if (!APPLY) {
-#pragma unroll
-    for (int j = 0; j < 8; ++j) { s_a[threadIdx.x][j] = sa[j]; s_b[threadIdx.x][j] = sb[j]; }
-    __syncthreads();
-    for (int w = threadIdx.x; w < O8 * 8; w += TB) {
-      const int o2 = w >> 3, j = w & 7;
-      float ta = 0.f, tb = 0.f;
-      const int first = (int)(((unsigned int)O8 + o2 - (blockIdx.x * TB) % (unsigned int)O8) % (unsigned int)O8);
-      for (int t = first; t < TB; t += O8) { ta += s_a[t][j]; tb += s_b[t][j]; }
-      atomicAdd(&dbeta[o2 * 8 + j], ta);
-      atomicAdd(&dgamma[o2 * 8 + j], tb);
-    }
-  }
+  if (!APPLY) block_col_sums(sa, sb, O8, O8 * 8, dbeta, dgamma);
 }
 
-// thread count that is a multiple of O8 (O8 must divide TB * k): returns blocks, or 0 if the vector path does not apply
-inline int ilog2(int v) {
-  int l = 0;
-  while ((1 << l) < v) ++l;
-  return l;
-}
-
-// items_per_thread > 1: kernels that end in per-block atomics (one per channel and block) want fewer, longer blocks on the
-// small layers — at 13x13x1024 the cap of 8 blocks per SM gave every thread 5 items and the grid 2.4 M atomics
-inline int vec_blocks(long long total, int O8, int items_per_thread = 1) {
-  if (O8 <= 0 || (TB % O8) != 0 || (O8 & (O8 - 1)) != 0 || total >= (1ll << 31)) return 0;
-  long long blocks = (total + (long long)TB * items_per_thread - 1) / ((long long)TB * items_per_thread);
+// Blocks of octet_threads(O8) threads for `rows` rows (pooled pixels).  items_per_thread > 1: kernels that end in
+// per-block atomics (one per channel and block) want fewer, longer blocks on the small layers — at 13x13x1024 the cap
+// of 8 blocks per SM gave every thread 5 items and the grid 2.4 M atomics
+inline int vec_blocks(long long rows, int O8, int items_per_thread = 1) {
+  const long long rows_per_block = TB / O8;
+  long long blocks = (rows + rows_per_block * items_per_thread - 1) / (rows_per_block * items_per_thread);
   const long long cap = (long long)mc_num_sms() * 8;
   if (items_per_thread > 1 && blocks < 2ll * mc_num_sms()) {
-    blocks = (total + TB - 1) / TB;
+    blocks = (rows + rows_per_block - 1) / rows_per_block;
     if (blocks > 2ll * mc_num_sms()) blocks = 2ll * mc_num_sms();
   }
   if (blocks > cap) blocks = cap;
   return (int)(blocks < 1 ? 1 : blocks);
+}
+
+// What the octet passes need (mcb200.h): at most MAX_C channels, pitches and channel offsets (or-ed together) multiples
+// of 8 and buffers (or-ed) 16-byte aligned so that an octet is one 16-byte access, row indices below 2^31.
+inline bool octets_ok(int C, long long rows, int pitches, uintptr_t ptrs) {
+  return C <= MAX_C && (pitches & 7) == 0 && (ptrs & 15) == 0 && rows < (1ll << 31);
 }
 
 inline int grid_for(long long total, int threads) {
@@ -737,23 +519,14 @@ extern "C" int mc_col_stats(const void* d_z, int64_t rows, int C, int ld, int ch
   MC_CHECK_ARG(d_z && d_sum && rows > 0 && C > 0, "mc_col_stats: bad argument");
   MC_CHECK_ARG((ld % 8) == 0 && (ch_off % 8) == 0 && ch_off + ((C + 7) / 8) * 8 <= ld,
                "mc_col_stats: ld/ch_off must be multiples of 8 and cover round_up(C,8) channels");
+  MC_CHECK_ARG(octets_ok(C, rows, ld | ch_off, (uintptr_t)d_z),
+               "mc_col_stats: needs C <= 2048, a 16-byte aligned d_z and rows < 2^31");
   MC_CUDA(cudaMemsetAsync(d_sum, 0, sizeof(float) * C, stream));
   if (d_sumsq) MC_CUDA(cudaMemsetAsync(d_sumsq, 0, sizeof(float) * C, stream));
-  if ((C % 8) == 0 && ((uintptr_t)d_z & 15) == 0) {
-    const int vb = vec_blocks(rows * (C / 8), C / 8);
-    if (vb > 0) {
-      col_stats_vec_kernel<<<vb, TB, 0, stream>>>((const __nv_bfloat16*)d_z, (unsigned int)rows, C / 8, ld, ch_off, d_sum,
-                                                  d_sumsq, ilog2(C / 8));
-      MC_LAUNCH_CHECK("col_stats_vec_kernel");
-      return 0;
-    }
-  }
-  long long gx = (rows + 8 * 64 - 1) / (8 * 64);
-  const long long cap = (long long)mc_num_sms() * 4;
-  if (gx > cap) gx = cap;
-  dim3 grid((unsigned)gx, (unsigned)((C + 255) / 256), 1);
-  col_stats_kernel<<<grid, TB, 0, stream>>>((const __nv_bfloat16*)d_z, rows, C, ld, ch_off, d_sum, d_sumsq);
-  MC_LAUNCH_CHECK("col_stats_kernel");
+  const int O8 = (C + 7) / 8;
+  col_stats_vec_kernel<<<vec_blocks(rows, O8), octet_threads(O8), 0, stream>>>((const __nv_bfloat16*)d_z, (unsigned int)rows,
+                                                                              C, O8, ld, ch_off, d_sum, d_sumsq);
+  MC_LAUNCH_CHECK("col_stats_vec_kernel");
   return 0;
 }
 
@@ -778,20 +551,16 @@ extern "C" int mc_bn_apply(const void* d_z, int ld_z, int B, int H, int W, int C
   MC_CHECK_ARG(d_z && d_scale && d_shift && d_out && B > 0 && H > 0 && W > 0 && C > 0, "mc_bn_apply: bad argument");
   MC_CHECK_ARG((ld_z % 8) == 0 && ld_z >= ((C + 7) / 8) * 8, "mc_bn_apply: ld_z must be a multiple of 8 covering C");
   if (reorg) MC_CHECK_ARG((H % 2) == 0 && (W % 2) == 0, "mc_bn_apply: reorg needs even H,W");
-  const long long total = (long long)B * (H + 1) * (W + 1) * ((C + 7) / 8);
-  if ((C % 8) == 0 && (ld_out % 8) == 0 && (ch_off % 8) == 0 && (((uintptr_t)d_z | (uintptr_t)d_out) & 15) == 0) {
-    const int vb = vec_blocks(total, C / 8);
-    if (vb > 0) {
-      bn_apply_vec_kernel<<<vb, TB, 0, stream>>>((const __nv_bfloat16*)d_z, ld_z, B, H, W, C, C / 8, d_scale, d_shift, leaky,
-                                                 (__nv_bfloat16*)d_out, ld_out, ch_off, reorg, ilog2(C / 8),
-                                                 make_fastdiv(W + 1), make_fastdiv(H + 1));
-      MC_LAUNCH_CHECK("bn_apply_vec_kernel");
-      return 0;
-    }
-  }
-  bn_apply_kernel<<<grid_for(total, TB), TB, 0, stream>>>((const __nv_bfloat16*)d_z, ld_z, B, H, W, C, d_scale, d_shift,
-                                                          leaky, (__nv_bfloat16*)d_out, ld_out, ch_off, reorg);
-  MC_LAUNCH_CHECK("bn_apply_kernel");
+  const long long rows = (long long)B * (H + 1) * (W + 1);
+  MC_CHECK_ARG(octets_ok(C, rows, ld_out | ch_off, (uintptr_t)d_z | (uintptr_t)d_out),
+               "mc_bn_apply: needs C <= 2048, ld_out and ch_off multiples of 8, 16-byte aligned buffers and "
+               "B*(H+1)*(W+1) < 2^31");
+  const int O8 = (C + 7) / 8;
+  auto* kernel = (C % 8) == 0 ? bn_apply_vec_kernel<true> : bn_apply_vec_kernel<false>;
+  kernel<<<vec_blocks(rows, O8), octet_threads(O8), 0, stream>>>((const __nv_bfloat16*)d_z, ld_z, B, H, W, C, O8, d_scale,
+                                                                d_shift, leaky, (__nv_bfloat16*)d_out, ld_out, ch_off,
+                                                                reorg, make_fastdiv(W + 1), make_fastdiv(H + 1));
+  MC_LAUNCH_CHECK("bn_apply_vec_kernel");
   return 0;
 }
 
@@ -803,41 +572,26 @@ extern "C" int mc_bn_backward(const void* d_z, int ld_z, const void* d_da, int l
   MC_CHECK_ARG(d_z && d_da && d_mean && d_invstd && d_gamma && d_beta && d_dbeta && d_dgamma && d_dz,
                "mc_bn_backward: null pointer");
   MC_CHECK_ARG(B > 0 && H > 0 && W > 0 && C > 0, "mc_bn_backward: bad dims");
+  const long long rows = (long long)B * (H + 1) * (W + 1);
+  MC_CHECK_ARG(octets_ok(C, rows, ld_z | ld_da | ld_dz | ch_off, (uintptr_t)d_z | (uintptr_t)d_da | (uintptr_t)d_dz),
+               "mc_bn_backward: needs C <= 2048, pitches and ch_off multiples of 8, 16-byte aligned buffers and "
+               "B*(H+1)*(W+1) < 2^31");
   MC_CUDA(cudaMemsetAsync(d_dbeta, 0, sizeof(float) * C, stream));
   MC_CUDA(cudaMemsetAsync(d_dgamma, 0, sizeof(float) * C, stream));
-  const long long rows = (long long)B * (H + 1) * (W + 1);
   const float inv_count = 1.0f / (float)((double)B * H * W);
-  // vector path: whole octets of channels, 16-byte aligned pieces everywhere
-  const bool vec_ok = (C % 8) == 0 && (ld_z % 8) == 0 && (ld_da % 8) == 0 && (ld_dz % 8) == 0 && (ch_off % 8) == 0 &&
-                      (((uintptr_t)d_z | (uintptr_t)d_da | (uintptr_t)d_dz) & 15) == 0;
-  const int vb = vec_ok ? vec_blocks(rows * (C / 8), C / 8) : 0;
-  if (vb > 0) {
-    const int vbr = vec_blocks(rows * (C / 8), C / 8, 16);
-    bn_bwd_reduce_vec_kernel<<<vbr, TB, 0, stream>>>((const __nv_bfloat16*)d_z, ld_z, (const __nv_bfloat16*)d_da, ld_da,
-                                                    ch_off, reorg, B, H, W, C, C / 8, d_mean, d_invstd, d_gamma, d_beta,
-                                                    leaky, d_dbeta, d_dgamma, ilog2(C / 8), make_fastdiv(W + 1),
-                                                    make_fastdiv(H + 1));
-    MC_LAUNCH_CHECK("bn_bwd_reduce_vec_kernel");
-    bn_bwd_apply_vec_kernel<<<vb, TB, 0, stream>>>((const __nv_bfloat16*)d_z, ld_z, (const __nv_bfloat16*)d_da, ld_da,
-                                                   ch_off, reorg, B, H, W, C, C / 8, d_mean, d_invstd, d_gamma, d_beta,
-                                                   leaky, d_dbeta, d_dgamma, inv_count, (__nv_bfloat16*)d_dz, ld_dz,
-                                                   ilog2(C / 8), make_fastdiv(W + 1), make_fastdiv(H + 1));
-    MC_LAUNCH_CHECK("bn_bwd_apply_vec_kernel");
-    return 0;
-  }
-  long long gx = (rows + 8 * 32 - 1) / (8 * 32);
-  const long long cap = (long long)mc_num_sms() * 8;
-  if (gx > cap) gx = cap;
-  dim3 grid((unsigned)gx, (unsigned)((C + 31) / 32), 1);
-  bn_bwd_reduce_kernel<<<grid, TB, 0, stream>>>((const __nv_bfloat16*)d_z, ld_z, (const __nv_bfloat16*)d_da, ld_da, ch_off,
-                                                reorg, B, H, W, C, d_mean, d_invstd, d_gamma, d_beta, leaky, d_dbeta,
-                                                d_dgamma);
-  MC_LAUNCH_CHECK("bn_bwd_reduce_kernel");
-  bn_bwd_apply_kernel<<<grid_for(rows * C, TB), TB, 0, stream>>>((const __nv_bfloat16*)d_z, ld_z, (const __nv_bfloat16*)d_da,
-                                                                 ld_da, ch_off, reorg, B, H, W, C, d_mean, d_invstd,
-                                                                 d_gamma, d_beta, leaky, d_dbeta, d_dgamma, inv_count,
-                                                                 (__nv_bfloat16*)d_dz, ld_dz);
-  MC_LAUNCH_CHECK("bn_bwd_apply_kernel");
+  const int O8 = (C + 7) / 8;
+  const bool whole = (C % 8) == 0;
+  auto* reduce = whole ? bn_bwd_vec_kernel<false, true> : bn_bwd_vec_kernel<false, false>;
+  auto* apply = whole ? bn_bwd_vec_kernel<true, true> : bn_bwd_vec_kernel<true, false>;
+  const FastDiv fWp = make_fastdiv(W + 1), fHp = make_fastdiv(H + 1);
+  reduce<<<vec_blocks(rows, O8, 16), octet_threads(O8), 0, stream>>>(
+      (const __nv_bfloat16*)d_z, ld_z, (const __nv_bfloat16*)d_da, ld_da, ch_off, reorg, B, H, W, C, O8, d_mean, d_invstd,
+      d_gamma, d_beta, leaky, d_dbeta, d_dgamma, inv_count, nullptr, ld_dz, fWp, fHp);
+  MC_LAUNCH_CHECK("bn_bwd_vec_kernel<reduce>");
+  apply<<<vec_blocks(rows, O8), octet_threads(O8), 0, stream>>>(
+      (const __nv_bfloat16*)d_z, ld_z, (const __nv_bfloat16*)d_da, ld_da, ch_off, reorg, B, H, W, C, O8, d_mean, d_invstd,
+      d_gamma, d_beta, leaky, d_dbeta, d_dgamma, inv_count, (__nv_bfloat16*)d_dz, ld_dz, fWp, fHp);
+  MC_LAUNCH_CHECK("bn_bwd_vec_kernel<apply>");
   return 0;
 }
 
@@ -846,21 +600,17 @@ extern "C" int mc_maxpool2x2_backward(const void* d_a_full, int ld_a, const void
   cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
   MC_CHECK_ARG(d_a_full && d_dpooled && d_dfull && B > 0 && H > 0 && W > 0 && C > 0, "mc_maxpool2x2_backward: bad argument");
   MC_CHECK_ARG((H % 2) == 0 && (W % 2) == 0, "mc_maxpool2x2_backward: H, W must be even");
-  if ((C % 8) == 0 && (ld_a % 8) == 0 && (ld_dp % 8) == 0 && (ld_df % 8) == 0 &&
-      (((uintptr_t)d_a_full | (uintptr_t)d_dpooled | (uintptr_t)d_dfull) & 15) == 0 &&
-      (long long)B * (H / 2) * (W / 2) * (C / 8) < (1ll << 32)) {
-    const long long tv = (long long)B * (H / 2) * (W / 2) * (C / 8);
-    maxpool_bwd_vec_kernel<<<grid_for(tv, TB), TB, 0, stream>>>((const __nv_bfloat16*)d_a_full, ld_a,
-                                                               (const __nv_bfloat16*)d_dpooled, ld_dp, B, H, W, C / 8,
-                                                               (__nv_bfloat16*)d_dfull, ld_df, accumulate);
-    MC_LAUNCH_CHECK("maxpool_bwd_vec_kernel");
-    return 0;
-  }
-  const long long total = (long long)B * (H + 1) * (W + 1) * C;
-  maxpool_bwd_kernel<<<grid_for(total, TB), TB, 0, stream>>>((const __nv_bfloat16*)d_a_full, ld_a,
-                                                             (const __nv_bfloat16*)d_dpooled, ld_dp, B, H, W, C,
-                                                             (__nv_bfloat16*)d_dfull, ld_df, accumulate);
-  MC_LAUNCH_CHECK("maxpool_bwd_kernel");
+  MC_CHECK_ARG(octets_ok(C, (long long)B * (H + 1) * (W + 1), ld_a | ld_dp | ld_df,
+                         (uintptr_t)d_a_full | (uintptr_t)d_dpooled | (uintptr_t)d_dfull),
+               "mc_maxpool2x2_backward: needs C <= 2048, pitches multiples of 8, 16-byte aligned buffers and "
+               "B*(H+1)*(W+1) < 2^31");
+  const int O8 = (C + 7) / 8;
+  const long long pixels = (long long)B * (H / 2) * (W / 2);
+  auto* kernel = (C % 8) == 0 ? maxpool_bwd_vec_kernel<true> : maxpool_bwd_vec_kernel<false>;
+  kernel<<<grid_for(pixels * O8, octet_threads(O8)), octet_threads(O8), 0, stream>>>(
+      (const __nv_bfloat16*)d_a_full, ld_a, (const __nv_bfloat16*)d_dpooled, ld_dp, B, H, W, C, O8,
+      (__nv_bfloat16*)d_dfull, ld_df, accumulate);
+  MC_LAUNCH_CHECK("maxpool_bwd_vec_kernel");
   return 0;
 }
 
@@ -874,15 +624,14 @@ extern "C" int mc_bn_apply_pool(const void* d_z, int ld_z, int B, int H, int W, 
   cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
   MC_CHECK_ARG(d_z && d_scale && d_shift && d_pooled && B > 0 && H > 0 && W > 0 && C > 0, "mc_bn_apply_pool: bad argument");
   MC_CHECK_ARG((H % 2) == 0 && (W % 2) == 0, "mc_bn_apply_pool: H, W must be even");
-  MC_CHECK_ARG(mc_bn_pool_supported(C) == 1 && (ld_z % 8) == 0 && (ld_p % 8) == 0 && ld_z >= C && ld_p >= C &&
-                   (((uintptr_t)d_z | (uintptr_t)d_pooled) & 15) == 0,
-               "mc_bn_apply_pool: needs C = 8 * 2^k <= 2048, pitches multiples of 8, 16-byte aligned buffers");
-  const long long total = (long long)B * (H / 2) * (W / 2) * (C / 8);
-  const int vb = vec_blocks(total, C / 8);
-  MC_CHECK_ARG(vb > 0, "mc_bn_apply_pool: too many work items");
-  bn_apply_pool_vec_kernel<<<vb, TB, 0, stream>>>((const __nv_bfloat16*)d_z, ld_z, B, H, W, C / 8, d_scale, d_shift, leaky,
-                                                  (__nv_bfloat16*)d_pooled, ld_p, ilog2(C / 8), make_fastdiv(W / 2),
-                                                  make_fastdiv(H / 2));
+  MC_CHECK_ARG(mc_bn_pool_supported(C) == 1 && ld_z >= C && ld_p >= C &&
+                   octets_ok(C, (long long)B * (H + 1) * (W + 1), ld_z | ld_p, (uintptr_t)d_z | (uintptr_t)d_pooled),
+               "mc_bn_apply_pool: needs C = 8 * 2^k <= 2048, pitches multiples of 8, 16-byte aligned buffers and "
+               "B*(H+1)*(W+1) < 2^31");
+  const int O8 = C / 8;
+  bn_apply_pool_vec_kernel<<<vec_blocks((long long)B * (H / 2) * (W / 2), O8), octet_threads(O8), 0, stream>>>(
+      (const __nv_bfloat16*)d_z, ld_z, B, H, W, O8, d_scale, d_shift, leaky, (__nv_bfloat16*)d_pooled, ld_p,
+      make_fastdiv(W / 2), make_fastdiv(H / 2));
   MC_LAUNCH_CHECK("bn_apply_pool_vec_kernel");
   return 0;
 }
@@ -895,23 +644,27 @@ extern "C" int mc_bn_pool_backward(const void* d_z, int ld_z, const void* d_dpoo
   MC_CHECK_ARG(d_z && d_dpooled && d_scale && d_shift && d_mean && d_invstd && d_gamma && d_beta && d_dbeta && d_dgamma && d_dz,
                "mc_bn_pool_backward: null pointer");
   MC_CHECK_ARG(B > 0 && H > 0 && W > 0 && C > 0 && (H % 2) == 0 && (W % 2) == 0, "mc_bn_pool_backward: bad dims");
-  MC_CHECK_ARG(mc_bn_pool_supported(C) == 1 && (ld_z % 8) == 0 && (ld_dp % 8) == 0 && (ld_dz % 8) == 0 &&
-                   (((uintptr_t)d_z | (uintptr_t)d_dpooled | (uintptr_t)d_dz) & 15) == 0,
-               "mc_bn_pool_backward: needs C = 8 * 2^k <= 2048, pitches multiples of 8, 16-byte aligned buffers");
+  MC_CHECK_ARG(mc_bn_pool_supported(C) == 1 &&
+                   octets_ok(C, (long long)B * (H + 1) * (W + 1), ld_z | ld_dp | ld_dz,
+                             (uintptr_t)d_z | (uintptr_t)d_dpooled | (uintptr_t)d_dz),
+               "mc_bn_pool_backward: needs C = 8 * 2^k <= 2048, pitches multiples of 8, 16-byte aligned buffers and "
+               "B*(H+1)*(W+1) < 2^31");
   MC_CUDA(cudaMemsetAsync(d_dbeta, 0, sizeof(float) * C, stream));
   MC_CUDA(cudaMemsetAsync(d_dgamma, 0, sizeof(float) * C, stream));
-  const long long total = (long long)B * (H / 2) * (W / 2) * (C / 8);
-  const int vb = vec_blocks(total, C / 8);
-  MC_CHECK_ARG(vb > 0, "mc_bn_pool_backward: too many work items");
+  const int O8 = C / 8;
+  const int vb = vec_blocks((long long)B * (H / 2) * (W / 2), O8);
   const float inv_count = 1.0f / (float)((double)B * H * W);
   const FastDiv fWo = make_fastdiv(W / 2), fHo = make_fastdiv(H / 2);
-  bn_pool_bwd_vec_kernel<false><<<vb, TB, 0, stream>>>((const __nv_bfloat16*)d_z, ld_z, (const __nv_bfloat16*)d_dpooled, ld_dp,
-                                                       B, H, W, C / 8, d_scale, d_shift, d_mean, d_invstd, leaky, d_dbeta,
-                                                       d_dgamma, inv_count, nullptr, ld_dz, ilog2(C / 8), fWo, fHo);
+  bn_pool_bwd_vec_kernel<false><<<vb, octet_threads(O8), 0, stream>>>((const __nv_bfloat16*)d_z, ld_z,
+                                                                      (const __nv_bfloat16*)d_dpooled, ld_dp, B, H, W, O8,
+                                                                      d_scale, d_shift, d_mean, d_invstd, leaky, d_dbeta,
+                                                                      d_dgamma, inv_count, nullptr, ld_dz, fWo, fHo);
   MC_LAUNCH_CHECK("bn_pool_bwd_vec_kernel<reduce>");
-  bn_pool_bwd_vec_kernel<true><<<vb, TB, 0, stream>>>((const __nv_bfloat16*)d_z, ld_z, (const __nv_bfloat16*)d_dpooled, ld_dp, B,
-                                                      H, W, C / 8, d_scale, d_shift, d_mean, d_invstd, leaky, d_dbeta, d_dgamma,
-                                                      inv_count, (__nv_bfloat16*)d_dz, ld_dz, ilog2(C / 8), fWo, fHo);
+  bn_pool_bwd_vec_kernel<true><<<vb, octet_threads(O8), 0, stream>>>((const __nv_bfloat16*)d_z, ld_z,
+                                                                     (const __nv_bfloat16*)d_dpooled, ld_dp, B, H, W, O8,
+                                                                     d_scale, d_shift, d_mean, d_invstd, leaky, d_dbeta,
+                                                                     d_dgamma, inv_count, (__nv_bfloat16*)d_dz, ld_dz, fWo,
+                                                                     fHo);
   MC_LAUNCH_CHECK("bn_pool_bwd_vec_kernel<apply>");
   return 0;
 }

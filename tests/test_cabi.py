@@ -91,3 +91,52 @@ def test_conv_desc_offsets_match_the_c_compiler(tmp_path):
     assert out[0] == ctypes.sizeof(_lib.mc_conv_desc)
     for f, off in zip(fields, out[1:]):
         assert getattr(_lib.mc_conv_desc, f).offset == off, f
+
+
+def test_bn_pool_pass_contract_without_gpu():
+    """The BatchNorm / pool passes (train_ops.cu) move 8 channels per 16-byte access: C > 2048, pitches or ch_off that
+    are not multiples of 8, pointers that are not 16-byte aligned and B*(H+1)*(W+1) >= 2^31 are argument errors,
+    reported before any CUDA call.  (Pointers are fake addresses: nothing may be launched.)"""
+    lib = _lib.load()
+    P, Q = 1 << 20, (1 << 20) + 2  # 16-byte aligned / misaligned device addresses
+    f = ctypes.c_void_p(P)
+
+    def col_stats(C=64, ld=64, ch_off=0, z=P, rows=100):
+        return lib.mc_col_stats(z, rows, C, ld, ch_off, f, f, None)
+
+    def bn_apply(C=64, ld_z=64, ld_out=64, ch_off=0, z=P, out=P, B=2, H=8, W=8):
+        return lib.mc_bn_apply(z, ld_z, B, H, W, C, f, f, 1, out, ld_out, ch_off, 0, None)
+
+    def bn_backward(C=64, ld_z=64, ld_da=64, ld_dz=64, ch_off=0, z=P, da=P, dz=P, B=2, H=8, W=8):
+        return lib.mc_bn_backward(z, ld_z, da, ld_da, ch_off, 0, B, H, W, C, f, f, f, f, 1, f, f, dz, ld_dz, None)
+
+    def pool_backward(C=64, ld_a=64, ld_dp=64, ld_df=64, a=P, dp=P, df=P, B=2, H=8, W=8):
+        return lib.mc_maxpool2x2_backward(a, ld_a, dp, ld_dp, B, H, W, C, df, ld_df, 0, None)
+
+    def bn_apply_pool(C=64, ld_z=64, ld_p=64, z=P, p=P, B=2, H=8, W=8):
+        return lib.mc_bn_apply_pool(z, ld_z, B, H, W, C, f, f, 1, p, ld_p, None)
+
+    def bn_pool_backward(C=64, ld_z=64, ld_dp=64, ld_dz=64, z=P, dp=P, dz=P, B=2, H=8, W=8):
+        return lib.mc_bn_pool_backward(z, ld_z, dp, ld_dp, B, H, W, C, f, f, f, f, f, f, 1, f, f, dz, ld_dz, None)
+
+    big = dict(B=1 << 13, H=511, W=511)  # 2^13 * 512 * 512 = 2^31 rows
+    cases = [
+        (col_stats, dict(C=2056, ld=2056)), (col_stats, dict(ld=68)), (col_stats, dict(ch_off=4, ld=72)),
+        (col_stats, dict(z=Q)), (col_stats, dict(rows=1 << 31)),
+        (bn_apply, dict(C=2056, ld_z=2056, ld_out=2056)), (bn_apply, dict(ld_out=68)), (bn_apply, dict(ch_off=4, ld_out=72)),
+        (bn_apply, dict(z=Q)), (bn_apply, dict(out=Q)), (bn_apply, big),
+        (bn_backward, dict(C=2056, ld_z=2056, ld_da=2056, ld_dz=2056)), (bn_backward, dict(ld_z=68)),
+        (bn_backward, dict(ld_da=68)), (bn_backward, dict(ld_dz=68)), (bn_backward, dict(ch_off=4, ld_da=72)),
+        (bn_backward, dict(z=Q)), (bn_backward, dict(da=Q)), (bn_backward, dict(dz=Q)), (bn_backward, big),
+        (pool_backward, dict(C=2056, ld_a=2056, ld_dp=2056, ld_df=2056)), (pool_backward, dict(ld_a=68)),
+        (pool_backward, dict(ld_dp=68)), (pool_backward, dict(ld_df=68)), (pool_backward, dict(a=Q)),
+        (pool_backward, dict(dp=Q)), (pool_backward, dict(df=Q)), (pool_backward, dict(B=1 << 13, H=510, W=511)),
+        (bn_apply_pool, dict(C=4096, ld_z=4096, ld_p=4096)), (bn_apply_pool, dict(ld_z=68)), (bn_apply_pool, dict(p=Q)),
+        (bn_apply_pool, dict(B=1 << 13, H=510, W=511)),
+        (bn_pool_backward, dict(C=4096, ld_z=4096, ld_dp=4096, ld_dz=4096)), (bn_pool_backward, dict(ld_dz=68)),
+        (bn_pool_backward, dict(dz=Q)), (bn_pool_backward, dict(B=1 << 13, H=510, W=511)),
+    ]
+    for fn, kw in cases:
+        rc = fn(**kw)
+        msg = lib.mc_last_error_string()
+        assert rc == -1 and msg.startswith(b'mc_'), "%s(%s): rc %d, %r" % (fn.__name__, kw, rc, msg)

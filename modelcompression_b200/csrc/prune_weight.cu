@@ -7,7 +7,12 @@
 //
 // Selection is exact: |w| >= 0, so its fp32 bit pattern is monotone as uint32 and order statistics can be found by
 // integer radix/histogram selection on the bit patterns (weight_prune_kernel below: one cooperative launch).
+//
+// Every pass over the weights, in the cooperative kernel and in the stand-alone kernels, is walk_chunks: a block takes
+// chunks of CHUNK elements of the segment table in grid-stride order, loads its 4*ITERS values per thread before the
+// first use and hands them to the pass's per-chunk body.
 #include <stdlib.h>
+#include <type_traits>
 #include <cooperative_groups.h>
 #include "common.cuh"
 
@@ -31,31 +36,149 @@ __device__ __forceinline__ int find_seg(const Chunks& ch, int nseg, long long ci
   return s;
 }
 
-// Visit every element of every segment: f(value, seg, index).  Vectorised when the segment base is 16B aligned.
-template <typename F>
-__device__ __forceinline__ void for_each_element(const SegTable& st, const Chunks& ch, F f) {
-  const long long nchunks = ch.cstart[st.nseg];
-  for (long long cid = blockIdx.x; cid < nchunks; cid += gridDim.x) {
-    const int s = find_seg(ch, st.nseg, cid);
-    const long long size = st.start[s + 1] - st.start[s];
-    const long long base = (cid - ch.cstart[s]) * CHUNK;
-    const float* p = st.ptr[s];
-    const bool aligned = (reinterpret_cast<uintptr_t>(p) & 15) == 0;
+// ---- the chunk walk ---------------------------------------------------------------------------------------------
+// Thread t holds elements base + (it * THREADS + t) * 4 + j of its chunk, j < 4: float4 q[it], bit it * 4 + j.
+struct Where {
+  const float* p;  // the segment's weights
+  float* out;      // the segment's mask
+  long long base, size, gstart;  // chunk offset in the segment, segment length, segment offset in the whole table
+  int s;
+  bool full;  // the whole chunk lies in the segment and every pointer the pass streams is 16-byte aligned
+};
+
+// OUT: the pass streams out[] too, so it must be aligned for the vector path
+template <bool OUT>
+__device__ __forceinline__ Where locate(const SegTable& st, const Chunks& ch, long long cid) {
+  Where w;
+  w.s = find_seg(ch, st.nseg, cid);
+  w.size = st.start[w.s + 1] - st.start[w.s];
+  w.gstart = st.start[w.s];
+  w.base = (cid - ch.cstart[w.s]) * CHUNK;
+  w.p = st.ptr[w.s];
+  w.out = st.out[w.s];
+  const bool aligned = ((reinterpret_cast<uintptr_t>(w.p) | (OUT ? reinterpret_cast<uintptr_t>(w.out) : 0)) & 15) == 0;
+  w.full = aligned && w.base + CHUNK <= w.size;
+  return w;
+}
+
+__device__ __forceinline__ long long elem(const Where& w, int it) {
+  return w.base + ((long long)it * THREADS + threadIdx.x) * 4;
+}
+
+__device__ __forceinline__ float part(const float4& v, int j) { return j == 0 ? v.x : j == 1 ? v.y : j == 2 ? v.z : v.w; }
+
+// bit it * 4 + j set when that element exists; a ragged chunk's loads read 0 past the end.  No element is read after
+// a pass wrote it, so the read-only path is safe for the weights that mask_pass / apply_masks_kernel overwrite.
+template <bool FULL>
+__device__ __forceinline__ unsigned int valid_bits(const Where& w) {
+  if constexpr (FULL) return 0xffffu;
+  unsigned int vm = 0;
 #pragma unroll
-    for (int it = 0; it < ITERS; ++it) {
-      const long long i = base + ((long long)it * THREADS + threadIdx.x) * 4;
-      if (aligned && i + 4 <= size) {
-        const float4 v = ld_stream_f4(reinterpret_cast<const float4*>(p + i));
-        f(v.x, s, i);
-        f(v.y, s, i + 1);
-        f(v.z, s, i + 2);
-        f(v.w, s, i + 3);
-      } else {
-        for (int j = 0; j < 4; ++j)
-          if (i + j < size) f(p[i + j], s, i + j);
-      }
+  for (int it = 0; it < ITERS; ++it) {
+    const long long r = w.size - elem(w, it);
+    vm |= (r >= 4 ? 15u : r > 0 ? (1u << r) - 1u : 0u) << (it * 4);
+  }
+  return vm;
+}
+
+template <bool FULL>
+__device__ __forceinline__ float4 load4(const float* src, const Where& w, int it) {
+  const long long i = elem(w, it);
+  if constexpr (FULL) {
+    return ld_stream_f4(reinterpret_cast<const float4*>(src + i));
+  } else {
+    float v[4];
+#pragma unroll
+    for (int j = 0; j < 4; ++j) v[j] = i + j < w.size ? __ldg(src + i + j) : 0.f;
+    return make_float4(v[0], v[1], v[2], v[3]);
+  }
+}
+
+template <bool FULL>
+__device__ __forceinline__ void load_chunk(const float* src, const Where& w, float4 (&q)[ITERS]) {
+#pragma unroll
+  for (int it = 0; it < ITERS; ++it) q[it] = load4<FULL>(src, w, it);
+}
+
+template <bool FULL>
+__device__ __forceinline__ void store4(float* dst, const Where& w, int it, const float4& v) {
+  const long long i = elem(w, it);
+  if constexpr (FULL) {
+    st_stream_f4(reinterpret_cast<float4*>(dst + i), v);
+  } else {
+#pragma unroll
+    for (int j = 0; j < 4; ++j)
+      if (i + j < w.size) dst[i + j] = part(v, j);
+  }
+}
+
+// f(value, bit) for every element of the chunk
+template <bool FULL, typename F>
+__device__ __forceinline__ void for_each_valid(const Where& w, const float4 (&q)[ITERS], F f) {
+  const unsigned int vm = valid_bits<FULL>(w);
+#pragma unroll
+  for (int b = 0; b < 4 * ITERS; ++b)
+    if (vm & (1u << b)) f(part(q[b >> 2], b & 3), b);
+}
+
+// Visit every chunk of the table: body(where, q, full) with full a std::integral_constant<bool, FULL>, so the
+// instantiation for whole aligned chunks holds no per-element test.  PREFETCH issues the loads of the block's next
+// chunk before the body of the current one runs, so every warp keeps 2 KB in flight while it computes (the fast pass
+// is latency-bound at ~40 % of the HBM rate without it); it holds 16 more values in registers, which the stand-alone
+// passes (<= 32 registers for 8 resident blocks per SM) cannot spare.
+template <bool PREFETCH, bool OUT, typename Body>
+__device__ __forceinline__ void walk_chunks(const SegTable& st, const Chunks& ch, Body body) {
+  const long long nchunks = ch.cstart[st.nseg];
+  long long cid = blockIdx.x;
+  Where nxt;
+  float4 qn[ITERS];
+  auto fetch = [&](long long c) {
+    nxt = locate<OUT>(st, ch, c);
+    if (nxt.full) load_chunk<true>(nxt.p, nxt, qn);
+  };
+  if (PREFETCH && cid < nchunks) fetch(cid);
+  for (; cid < nchunks; cid += gridDim.x) {
+    Where w;
+    float4 q[ITERS];
+    if (PREFETCH) {
+      w = nxt;
+#pragma unroll
+      for (int it = 0; it < ITERS; ++it) q[it] = qn[it];
+      if (cid + gridDim.x < nchunks) fetch(cid + gridDim.x);
+    } else {
+      w = locate<OUT>(st, ch, cid);
+      if (w.full) load_chunk<true>(w.p, w, q);
+    }
+    if (w.full) {
+      body(w, q, std::true_type());
+    } else {
+      load_chunk<false>(w.p, w, q);
+      body(w, q, std::false_type());
     }
   }
+}
+
+__device__ __forceinline__ float4 gt4(const float4& v, float thr) {
+  return make_float4(fabsf(v.x) > thr ? 1.f : 0.f, fabsf(v.y) > thr ? 1.f : 0.f, fabsf(v.z) > thr ? 1.f : 0.f,
+                     fabsf(v.w) > thr ? 1.f : 0.f);
+}
+
+__device__ __forceinline__ float4 mul4(const float4& a, const float4& b) {
+  return make_float4(__fmul_rn(a.x, b.x), __fmul_rn(a.y, b.y), __fmul_rn(a.z, b.z), __fmul_rn(a.w, b.w));
+}
+
+// mask = |w| > thr, and / or w *= mask
+template <bool WRITE_MASK, bool APPLY>
+__device__ __forceinline__ void mask_pass(const SegTable& st, const Chunks& ch, float thr) {
+  walk_chunks<false, WRITE_MASK>(st, ch, [&](const Where& w, const float4 (&q)[ITERS], auto full) {
+    constexpr bool FULL = decltype(full)::value;
+#pragma unroll
+    for (int it = 0; it < ITERS; ++it) {
+      const float4 m = gt4(q[it], thr);
+      if (WRITE_MASK) store4<FULL>(w.out, w, it, m);
+      if (APPLY) store4<FULL>(const_cast<float*>(w.p), w, it, mul4(q[it], m));
+    }
+  });
 }
 
 // ---------------------------------------------------------------------------------------------------------------
@@ -67,22 +190,27 @@ __device__ __forceinline__ void for_each_element(const SegTable& st, const Chunk
 //   P  ONE pass over W: count keys < lo, append (key, element index) of the keys in [lo, hi] (~5 % of n) to the
 //      candidate list (and bin them for the first histogram level), and write the PROVISIONAL mask |w| > mid —
 //      final for everything outside the bracket.
-//   R  exact rank inside the candidates: 10-bit histogram levels on (key - lo), all from L2.
+//   R  exact rank inside the candidates: 10-bit histogram levels on (key - lo), all from L2; then the successor
+//      key and the threshold (select_key_b, select_finish).
 //   F  fix-up: the candidates on which (|w| > mid) and (|w| > thr) disagree (~0.5 % of n) are rewritten.
 //
 // HBM traffic on this path: read W once + write the masks once = 8n bytes (SURVEY.md §8d charges 12n).
 // If the bracket missed (k outside, non-finite values present, candidate list overflow) the same kernel falls through
-// to the EXACT path: 12-bit histogram of all keys -> compact the selected bin -> 10-bit levels -> full mask pass.  The
-// result is always the exact order statistic; only the time differs.
+// to the EXACT path: 12-bit histogram of all keys -> compact the selected bin (keys only) -> 10-bit levels -> the
+// same successor and threshold steps over all of W -> full mask pass.  The result is always the exact order
+// statistic; only the time differs.
 constexpr int SAMPLE = 4096;
 constexpr int SAMPLE_LOG2 = 12;
 constexpr int LVL_BITS = 10;
 constexpr int LVL_BINS = 1 << LVL_BITS;
 constexpr int MAX_LVLS = 4;     // keys are < 2^31: 10+10+10+1
 constexpr int NWARPS = THREADS / 32;
-constexpr int STG = 256;        // staged candidates per warp in the fast pass
-constexpr int STG_X = 640;      // ... in the exact-path compaction (a warp-iteration appends at most 32*4*ITERS = 512)
-constexpr int SMEM_WORDS = 2 * NWARPS * STG_X;  // 40 KB, carved differently per phase
+constexpr int STG = 256;        // staged (key, index) pairs per warp; 2 * STG keys when no index is kept
+constexpr int HOLD_WORDS = NWARPS * ITERS * 32 * 4;  // every lane's chunk values, for the candidate sink
+constexpr int STAGE_WORDS = 2 * NWARPS * STG;
+// 40 KB, carved differently per phase.  The candidate passes need 36 KB; the 40 KB footprint is kept so that the
+// occupancy, hence the grid and the candidate slice of each block, stay as measured.
+constexpr int SMEM_WORDS = 10 * 1024;
 constexpr int MAXB = 2048;      // max blocks of the cooperative grid (148 SMs x <= 8 resident blocks, with headroom)
 
 // Global atomics are avoided on purpose: atomics to one 128-byte line serialise in L2 at ~5 ns each (measured: 600 K
@@ -177,57 +305,40 @@ __device__ __forceinline__ unsigned int sample_key(const SegTable& st, long long
   return absbits(st.ptr[s][g - st.start[s]]);
 }
 
-// The whole grid ranks the sample by counting (S^2 = 16.7 M compares, ~100 per thread): block b compares its 256 keys
-// (key group b % 16) against slice b / 16 of the sample and adds the counts with global atomics.  A radix select in
-// one block (8 warps, dependent shuffle/atomic chains) costs 30-50 us; this costs ~5.
+// The whole grid ranks the sample by counting (S^2 = 16.7 M compares, ~100 per thread): a unit compares the 256 keys
+// of one key group against one of nslices = max(1, grid / 16) slices of the sample and adds the counts with global
+// atomics; blocks loop over the 16 * nslices units (one unit each unless the grid has fewer than 16 blocks).  A radix
+// select in one block (8 warps, dependent shuffle/atomic chains) costs 30-50 us; this costs ~5.
+// s_slice holds one slice: up to the whole sample.
 __device__ void sample_rank_count(const SegTable& st, long long n, SelState* state, unsigned int* s_slice) {
   constexpr int GROUPS = SAMPLE / THREADS;  // 16
-  const int nslices = (int)gridDim.x / GROUPS;
-  if (nslices == 0) {  // tiny grid: every block handles whole key groups against the full sample
-    for (int grp = blockIdx.x; grp < GROUPS; grp += gridDim.x) {
-      const int i = grp * THREADS + threadIdx.x;
-      const unsigned int ki = sample_key(st, n, i);
-      state->sample[i] = ki;
-      unsigned int lt = 0, le = 0;
-      for (int j0 = 0; j0 < SAMPLE; j0 += THREADS) {
-        __syncthreads();
-        s_slice[threadIdx.x] = sample_key(st, n, j0 + threadIdx.x);
-        __syncthreads();
-        for (int j = 0; j < THREADS; ++j) {
-          const unsigned int kj = s_slice[j];
-          lt += kj < ki;
-          le += kj <= ki;
-        }
-      }
-      state->rank_lt[i] = lt;
-      state->rank_le[i] = le;
+  const int nslices = gridDim.x >= GROUPS ? (int)gridDim.x / GROUPS : 1;
+  const int len = (SAMPLE + nslices - 1) / nslices;
+  for (int unit = blockIdx.x; unit < GROUPS * nslices; unit += gridDim.x) {
+    const int grp = unit % GROUPS, slice = unit / GROUPS;
+    const int j0 = slice * len;
+    const int jn = (j0 + len < SAMPLE ? j0 + len : SAMPLE) - j0;
+    const int i = grp * THREADS + threadIdx.x;
+    const unsigned int ki = sample_key(st, n, i);
+    __syncthreads();  // the previous unit's slice is read
+    for (int j = threadIdx.x; j < jn; j += THREADS) s_slice[j] = sample_key(st, n, j0 + j);
+    if (slice == 0) state->sample[i] = ki;
+    __syncthreads();
+    unsigned int lt = 0, le = 0;
+    int j = 0;
+    for (; j + 4 <= jn; j += 4) {
+      const uint4 kq = *reinterpret_cast<const uint4*>(s_slice + j);
+      lt += (kq.x < ki) + (kq.y < ki) + (kq.z < ki) + (kq.w < ki);
+      le += (kq.x <= ki) + (kq.y <= ki) + (kq.z <= ki) + (kq.w <= ki);
     }
-    return;
+    for (; j < jn; ++j) {
+      const unsigned int kj = s_slice[j];
+      lt += kj < ki;
+      le += kj <= ki;
+    }
+    if (lt) atomicAdd(&state->rank_lt[i], lt);
+    if (le) atomicAdd(&state->rank_le[i], le);
   }
-  const int grp = blockIdx.x % GROUPS, slice = blockIdx.x / GROUPS;
-  if (slice >= nslices) return;
-  const int len = (SAMPLE + nslices - 1) / nslices;  // <= THREADS because nslices >= 1 ... guarded below
-  const int j0 = slice * len;
-  const int jn = (j0 + len < SAMPLE ? j0 + len : SAMPLE) - j0;
-  const int i = grp * THREADS + threadIdx.x;
-  const unsigned int ki = sample_key(st, n, i);
-  for (int j = threadIdx.x; j < jn; j += THREADS) s_slice[j] = sample_key(st, n, j0 + j);
-  if (slice == 0) state->sample[i] = ki;
-  __syncthreads();
-  unsigned int lt = 0, le = 0;
-  int j = 0;
-  for (; j + 4 <= jn; j += 4) {
-    const uint4 kq = *reinterpret_cast<const uint4*>(s_slice + j);
-    lt += (kq.x < ki) + (kq.y < ki) + (kq.z < ki) + (kq.w < ki);
-    le += (kq.x <= ki) + (kq.y <= ki) + (kq.z <= ki) + (kq.w <= ki);
-  }
-  for (; j < jn; ++j) {
-    const unsigned int kj = s_slice[j];
-    lt += kj < ki;
-    le += kj <= ki;
-  }
-  if (lt) atomicAdd(&state->rank_lt[i], lt);
-  if (le) atomicAdd(&state->rank_le[i], le);
 }
 
 // after the grid barrier: every block finds the sample keys holding three ranks (rank_lt <= r < rank_le)
@@ -329,278 +440,190 @@ __device__ unsigned int resolve_rank(cg::grid_group& grid, unsigned int* ghist /
   return lo + prefix;
 }
 
-// ---- P: the one pass of the fast path.  ~12 instructions per element: the per-element work is three float compares
-// (|w| against the pivots), the mask select and two predicated bit-sets; candidate keys are recovered afterwards
-// from a per-lane copy of the 16 values in shared memory, only for the ~5 % that are candidates.
-template <bool WRITE_MASK>
-__device__ __forceinline__ void fast_pass(const SegTable& st, const Chunks& ch, SelState* state, unsigned int lo,
-                                          unsigned int mid, unsigned int hi, unsigned int* __restrict__ cand_key,
-                                          unsigned int* __restrict__ cand_idx, unsigned int cap, unsigned int* s_mem) {
-  __shared__ unsigned int s_cnt;         // candidates appended by this block
-  __shared__ unsigned int s_below[NWARPS];
-  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-  // smem: [NWARPS][ITERS][32] float4 value copies | [NWARPS][STG] keys | [NWARPS][STG] indices | [LVL_BINS] level-0 bins
-  float4* vals = reinterpret_cast<float4*>(s_mem) + wid * (ITERS * 32);
-  unsigned int* wkeys = s_mem + NWARPS * ITERS * 32 * 4 + wid * STG;
-  unsigned int* widx = wkeys + NWARPS * STG;
-  unsigned int* s_lvl = s_mem + NWARPS * ITERS * 32 * 4 + 2 * NWARPS * STG;
-  static_assert(NWARPS * ITERS * 32 * 4 + 2 * NWARPS * STG + LVL_BINS <= SMEM_WORDS, "fast_pass smem carve-up");
-  const float lo_f = __uint_as_float(lo), mid_f = __uint_as_float(mid), hi_f = __uint_as_float(hi);
-  const int shiftA = level0_shift(hi - lo);
-  for (int i = threadIdx.x; i < LVL_BINS; i += THREADS) s_lvl[i] = 0;
-  if (threadIdx.x == 0) s_cnt = 0;
-  __syncthreads();
-  unsigned int wcnt = 0;  // warp-uniform
-  unsigned int below = 0;
-  float nanacc = 0.f;  // becomes NaN iff a NaN or Inf was seen (x*0)
-  auto flush = [&]() {  // warp-wide
+// ---- the candidate sink ---------------------------------------------------------------------------------------
+// Appends the chunk elements a pass selects to the block's private slice of the candidate list: per-warp staging in
+// shared memory, flushed in bursts; a warp-iteration with more than the staging holds (e.g. thousands of equal keys)
+// goes straight to the slice.  Appends beyond `cap` are dropped and reported as overflow.  IDX keeps each key's global
+// element index beside it (the fast pass's fix-up needs it); without it the staging holds twice as many keys.
+template <bool IDX>
+struct CandSink {
+  static constexpr unsigned int STAGE = IDX ? STG : 2 * STG;
+  float* held;          // this lane's chunk values in shared memory (hold())
+  unsigned int* wkeys;  // this warp's staging
+  unsigned int* widx;
+  unsigned int* keys;   // the block's slice
+  unsigned int* idx;
+  unsigned int cap;
+  unsigned int* cnt;    // shared: elements appended by the block (zeroed and synchronised by the caller)
+  unsigned int wcnt;    // staged by this warp (warp-uniform)
+
+  // smem: [HOLD_WORDS] chunk values | [STAGE_WORDS] staging
+  __device__ CandSink(unsigned int* smem, unsigned int* keys_, unsigned int* idx_, unsigned int cap_,
+                      unsigned int* cnt_)
+      : held(reinterpret_cast<float*>(smem) + (threadIdx.x >> 5) * (ITERS * 32 * 4) + (threadIdx.x & 31) * 4),
+        wkeys(smem + HOLD_WORDS + (threadIdx.x >> 5) * STAGE), widx(wkeys + NWARPS * STG), keys(keys_), idx(idx_),
+        cap(cap_), cnt(cnt_), wcnt(0) {}
+
+  // keep the chunk's values where append() can read any of them by bit (only the ~5 % selected are read back)
+  __device__ __forceinline__ void hold(const float4 (&q)[ITERS]) {
+#pragma unroll
+    for (int it = 0; it < ITERS; ++it)
+      reinterpret_cast<float4*>(held)[it * 32] = q[it];
+  }
+
+  __device__ __forceinline__ void flush() {  // warp-wide
+    const int lane = threadIdx.x & 31;
     unsigned int base = 0;
-    if (lane == 0 && wcnt) base = atomicAdd(&s_cnt, wcnt);
+    if (lane == 0 && wcnt) base = atomicAdd(cnt, wcnt);
     base = __shfl_sync(0xffffffffu, base, 0);
     __syncwarp();
     for (unsigned int i = lane; i < wcnt; i += 32)
       if (base + i < cap) {
-        cand_key[base + i] = wkeys[i];
-        cand_idx[base + i] = widx[i];
+        keys[base + i] = wkeys[i];
+        if (IDX) idx[base + i] = widx[i];
       }
     __syncwarp();
     wcnt = 0;
-  };
-  const long long nchunks = ch.cstart[st.nseg];
-  // software pipeline: the loads of chunk i+1 are issued before chunk i is processed, so every warp keeps 2 KB in
-  // flight while it computes (without this the pass is latency-bound at ~40 % of the HBM rate)
-  struct Where {
-    const float* p;
-    float* mk;
-    long long base, size, gstart;
-    bool full;
-  };
-  auto locate = [&](long long cid) {
-    Where w;
-    const int s = find_seg(ch, st.nseg, cid);
-    w.size = st.start[s + 1] - st.start[s];
-    w.gstart = st.start[s];
-    w.base = (cid - ch.cstart[s]) * CHUNK;
-    w.p = st.ptr[s];
-    w.mk = st.out[s];
-    const bool aligned = ((reinterpret_cast<uintptr_t>(w.p) | (WRITE_MASK ? reinterpret_cast<uintptr_t>(w.mk) : 0)) & 15) == 0;
-    w.full = aligned && w.base + CHUNK <= w.size;
-    return w;
-  };
-  float4 qn[ITERS];
-  Where nxt;
-  long long cid = blockIdx.x;
-  if (cid < nchunks) {
-    nxt = locate(cid);
-    if (nxt.full) {
-#pragma unroll
-      for (int it = 0; it < ITERS; ++it)
-        qn[it] = ld_stream_f4(reinterpret_cast<const float4*>(nxt.p + nxt.base + ((long long)it * THREADS + threadIdx.x) * 4));
-    }
   }
-  for (; cid < nchunks; cid += gridDim.x) {
-    const Where cur = nxt;
-    float4 q[ITERS];
-#pragma unroll
-    for (int it = 0; it < ITERS; ++it) q[it] = qn[it];
-    if (cid + gridDim.x < nchunks) {
-      nxt = locate(cid + gridDim.x);
-      if (nxt.full) {
-#pragma unroll
-        for (int it = 0; it < ITERS; ++it)
-          qn[it] = ld_stream_f4(reinterpret_cast<const float4*>(nxt.p + nxt.base + ((long long)it * THREADS + threadIdx.x) * 4));
-      }
-    }
-    const long long size = cur.size, base = cur.base;
-    const float* p = cur.p;
-    float* mk = cur.mk;
-    if (!cur.full) {
-      // ragged chunk (segment tail / unaligned tensor): scalar, candidates appended one by one
-      for (long long i = base + threadIdx.x; i < size && i < base + CHUNK; i += THREADS) {
-        const float v = p[i];
-        const float a = fabsf(v);
-        nanacc = fmaf(v, 0.f, nanacc);
-        if (WRITE_MASK) mk[i] = a > mid_f ? 1.f : 0.f;
-        if (a < lo_f) ++below;
-        else if (a <= hi_f) {
-          const unsigned int key = __float_as_uint(a);
-          const unsigned int pos = atomicAdd(&s_cnt, 1u);
-          if (pos < cap) {
-            cand_key[pos] = key;
-            cand_idx[pos] = (unsigned int)(cur.gstart + i);
-          }
-          atomicAdd(&s_lvl[(key - lo) >> shiftA], 1u);
-        }
-      }
-      continue;
-    }
-    unsigned int hits = 0, ge = 0;
-#pragma unroll
-    for (int it = 0; it < ITERS; ++it) {
-      const float v[4] = {q[it].x, q[it].y, q[it].z, q[it].w};
-      float m4[4];
-#pragma unroll
-      for (int j = 0; j < 4; ++j) {
-        const float a = fabsf(v[j]);
-        nanacc = fmaf(v[j], 0.f, nanacc);
-        m4[j] = a > mid_f ? 1.f : 0.f;
-        const bool p1 = a >= lo_f;
-        if (p1) ge |= 1u << (it * 4 + j);
-        if (p1 && a <= hi_f) hits |= 1u << (it * 4 + j);
-      }
-      if (WRITE_MASK)
-        st_stream_f4(reinterpret_cast<float4*>(mk + base + ((long long)it * THREADS + threadIdx.x) * 4),
-                     make_float4(m4[0], m4[1], m4[2], m4[3]));
-      vals[it * 32 + lane] = q[it];
-    }
-    below += 4 * ITERS - __popc(ge);
-    const unsigned int cnt = __popc(hits);
-    unsigned int incl = cnt;
+
+  // Warp-wide: append the held elements whose bit is set in `hits`; idx0 is the global index of this lane's bit 0.
+  // on_key(key) runs once per appended key.
+  template <typename F>
+  __device__ __forceinline__ void append(unsigned int hits, unsigned int idx0, F on_key) {
+    const int lane = threadIdx.x & 31;
+    const unsigned int n = __popc(hits);
+    unsigned int incl = n;
 #pragma unroll
     for (int o = 1; o < 32; o <<= 1) {
       const unsigned int t = __shfl_up_sync(0xffffffffu, incl, o);
       if (lane >= o) incl += t;
     }
     const unsigned int tot = __shfl_sync(0xffffffffu, incl, 31);
-    if (tot == 0) continue;  // warp-uniform
-    if (wcnt + tot > STG) flush();
-    const bool direct = tot > STG;  // burst (e.g. thousands of equal keys): straight to the global list
+    if (tot == 0) return;  // warp-uniform
+    if (wcnt + tot > STAGE) flush();
+    const bool direct = tot > STAGE;
     unsigned int gbase = 0;
     if (direct) {
-      if (lane == 0) gbase = atomicAdd(&s_cnt, tot);
+      if (lane == 0) gbase = atomicAdd(cnt, tot);
       gbase = __shfl_sync(0xffffffffu, gbase, 0);
     }
-    unsigned int pos = (direct ? gbase : wcnt) + (incl - cnt);
-    const unsigned int idx0 = (unsigned int)(cur.gstart + base) + threadIdx.x * 4;
-    const float* myvals = reinterpret_cast<const float*>(vals);
+    unsigned int pos = (direct ? gbase : wcnt) + (incl - n);
     while (hits) {
       const int j = __ffs(hits) - 1;
       hits &= hits - 1;
-      const unsigned int key = absbits(myvals[((j >> 2) * 32 + lane) * 4 + (j & 3)]);
-      const unsigned int idx = idx0 + (unsigned int)(j >> 2) * (THREADS * 4) + (unsigned int)(j & 3);
+      const unsigned int key = absbits(held[(j >> 2) * 32 * 4 + (j & 3)]);
+      const unsigned int ix = idx0 + (unsigned int)(j >> 2) * (THREADS * 4) + (unsigned int)(j & 3);
       if (direct) {
         if (pos < cap) {
-          cand_key[pos] = key;
-          cand_idx[pos] = idx;
+          keys[pos] = key;
+          if (IDX) idx[pos] = ix;
         }
       } else {
         wkeys[pos] = key;
-        widx[pos] = idx;
+        if (IDX) widx[pos] = ix;
       }
       ++pos;
-      atomicAdd(&s_lvl[(key - lo) >> shiftA], 1u);
+      on_key(key);
     }
     if (!direct) wcnt += tot;
   }
-  flush();
+
+  // block-wide, after the last append: flush every warp and publish the block's count (with a block barrier)
+  __device__ __forceinline__ void finish(unsigned int* blk_cnt, unsigned int* overflow) {
+    flush();
+    __syncthreads();
+    if (threadIdx.x == 0) {
+      const unsigned int c = *cnt;
+      *blk_cnt = c < cap ? c : cap;
+      if (c > cap) *overflow = 1u;
+    }
+  }
+};
+
+// ---- P: the one pass of the fast path.  ~12 instructions per element: the per-element work is three float compares
+// (|w| against the pivots), the mask select and two predicated bit-sets; candidate keys are recovered afterwards
+// from the held values, only for the ~5 % that are candidates.
+template <bool WRITE_MASK>
+__device__ __forceinline__ void fast_pass(const SegTable& st, const Chunks& ch, SelState* state, unsigned int lo,
+                                          unsigned int mid, unsigned int hi, unsigned int* __restrict__ cand_key,
+                                          unsigned int* __restrict__ cand_idx, unsigned int cap, unsigned int* s_mem) {
+  __shared__ unsigned int s_cnt;  // candidates appended by this block
+  __shared__ unsigned int s_below[NWARPS];
+  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+  // smem: held values | staging | [LVL_BINS] level-0 bins
+  unsigned int* s_lvl = s_mem + HOLD_WORDS + STAGE_WORDS;
+  static_assert(HOLD_WORDS + STAGE_WORDS + LVL_BINS <= SMEM_WORDS, "fast_pass smem carve-up");
+  const float lo_f = __uint_as_float(lo), mid_f = __uint_as_float(mid), hi_f = __uint_as_float(hi);
+  const int shiftA = level0_shift(hi - lo);
+  for (int i = threadIdx.x; i < LVL_BINS; i += THREADS) s_lvl[i] = 0;
+  if (threadIdx.x == 0) s_cnt = 0;
+  __syncthreads();
+  CandSink<true> sink(s_mem, cand_key, cand_idx, cap, &s_cnt);
+  unsigned int below = 0;
+  float nanacc = 0.f;  // becomes NaN iff a NaN or Inf was seen (x*0)
+  walk_chunks<true, WRITE_MASK>(st, ch, [&](const Where& w, const float4 (&q)[ITERS], auto full) {
+    constexpr bool FULL = decltype(full)::value;
+    unsigned int hits = 0, ge = 0;
+#pragma unroll
+    for (int it = 0; it < ITERS; ++it) {
+      float m4[4];
+#pragma unroll
+      for (int j = 0; j < 4; ++j) {
+        const float v = part(q[it], j);
+        const float a = fabsf(v);
+        nanacc = fmaf(v, 0.f, nanacc);
+        m4[j] = a > mid_f ? 1.f : 0.f;
+        const bool p1 = a >= lo_f;
+        if (p1) ge |= 1u << (it * 4 + j);
+        if (p1 && a <= hi_f) hits |= 1u << (it * 4 + j);
+      }
+      if (WRITE_MASK) store4<FULL>(w.out, w, it, make_float4(m4[0], m4[1], m4[2], m4[3]));
+    }
+    sink.hold(q);
+    const unsigned int vm = valid_bits<FULL>(w);
+    below += __popc(vm) - __popc(ge & vm);
+    sink.append(hits & vm, (unsigned int)(w.gstart + w.base) + threadIdx.x * 4,
+                [&](unsigned int key) { atomicAdd(&s_lvl[(key - lo) >> shiftA], 1u); });
+  });
   for (int o = 16; o > 0; o >>= 1) below += __shfl_xor_sync(0xffffffffu, below, o);
   if (lane == 0) s_below[wid] = below;
   if (nanacc != nanacc) state->has_nan = 1u;  // rare; every writer stores the same value
-  __syncthreads();
   // publish this block's results (read by everyone after the grid barrier)
+  sink.finish(&state->blk_cnt[0][blockIdx.x], &state->overflow);
   for (int i = threadIdx.x; i < LVL_BINS; i += THREADS)
     if (s_lvl[i]) atomicAdd(&state->lvl_hist[0][0][i], s_lvl[i]);
   if (threadIdx.x == 0) {
     unsigned long long tot = 0;
     for (int w = 0; w < NWARPS; ++w) tot += s_below[w];
     state->blk_below[blockIdx.x] = tot;
-    const unsigned int c = s_cnt;
-    state->blk_cnt[0][blockIdx.x] = c < cap ? c : cap;
-    if (c > cap) state->overflow = 1u;
   }
 }
 
-// Streaming passes of the exact path.
-//   MODE 1: stage the keys in [lo, hi] (one 12-bit bin) and append them to the candidate list
-//   MODE 2: 4096-bin histogram of key >> 19 into s_mem (flushed by the caller); records NaNs
-template <int MODE>
-__device__ __forceinline__ void exact_pass(const SegTable& st, const Chunks& ch, SelState* state, unsigned int lo,
-                                           unsigned int hi, unsigned int* __restrict__ cand_key, unsigned int cand_cap,
-                                           unsigned int* s_mem) {
-  __shared__ unsigned int s_cnt;
-  if (threadIdx.x == 0) s_cnt = 0;
-  __syncthreads();
-  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-  unsigned int* wkeys = s_mem + wid * STG_X;
-  unsigned int wcnt = 0;  // warp-uniform
-  bool saw_nan = false;
-  auto flush = [&]() {  // warp-wide
-    unsigned int base = 0;
-    if (lane == 0 && wcnt) base = atomicAdd(&s_cnt, wcnt);
-    base = __shfl_sync(0xffffffffu, base, 0);
-    __syncwarp();
-    for (unsigned int i = lane; i < wcnt; i += 32)
-      if (base + i < cand_cap) cand_key[base + i] = wkeys[i];
-    __syncwarp();
-    wcnt = 0;
-  };
-  const long long nchunks = ch.cstart[st.nseg];
-  for (long long cid = blockIdx.x; cid < nchunks; cid += gridDim.x) {
-    const int s = find_seg(ch, st.nseg, cid);
-    const long long size = st.start[s + 1] - st.start[s];
-    const long long base = (cid - ch.cstart[s]) * CHUNK;
-    const float* p = st.ptr[s];
-    const bool aligned = (reinterpret_cast<uintptr_t>(p) & 15) == 0;
-    float4 q[ITERS];
-    int nvalid[ITERS];
-#pragma unroll
-    for (int it = 0; it < ITERS; ++it) {  // all loads in flight before the first use
-      const long long i = base + ((long long)it * THREADS + threadIdx.x) * 4;
-      q[it] = make_float4(0.f, 0.f, 0.f, 0.f);
-      nvalid[it] = 0;
-      if (aligned && i + 4 <= size) {
-        q[it] = ld_stream_f4(reinterpret_cast<const float4*>(p + i));
-        nvalid[it] = 4;
-      } else if (i < size) {
-        float v[4] = {0.f, 0.f, 0.f, 0.f};
-        for (int j = 0; j < 4; ++j)
-          if (i + j < size) { v[j] = p[i + j]; nvalid[it] = j + 1; }
-        q[it] = make_float4(v[0], v[1], v[2], v[3]);
-      }
-    }
-    unsigned int keys[4 * ITERS];
-    unsigned int hits = 0;
-#pragma unroll
-    for (int it = 0; it < ITERS; ++it) {
-      const float v[4] = {q[it].x, q[it].y, q[it].z, q[it].w};
-#pragma unroll
-      for (int j = 0; j < 4; ++j) {
-        const unsigned int key = absbits(v[j]);
-        keys[it * 4 + j] = key;
-        if (j < nvalid[it]) {
-          if (MODE == 2) {
-            saw_nan |= key > 0x7f800000u;
-            atomicAdd(&s_mem[key >> 19], 1u);
-          } else if (key >= lo && key <= hi) {
-            hits |= 1u << (it * 4 + j);
-          }
-        }
-      }
-    }
-    if (MODE == 2) continue;
-    if (wcnt > STG_X - 32 * 4 * ITERS) flush();
-    const unsigned int cnt = __popc(hits);
-    unsigned int incl = cnt;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-      const unsigned int t = __shfl_up_sync(0xffffffffu, incl, o);
-      if (lane >= o) incl += t;
-    }
-    unsigned int pos = wcnt + (incl - cnt);
-#pragma unroll
-    for (int j = 0; j < 4 * ITERS; ++j)
-      if (hits & (1u << j)) wkeys[pos++] = keys[j];
-    wcnt += __shfl_sync(0xffffffffu, incl, 31);
+// ---- the select tail, shared by both paths --------------------------------------------------------------------
+// sorted[k+1] given key_a = sorted[k]: count(key <= key_a) and min(key > key_a) over the keys visit(f) hands to f,
+// plus `below` keys known to lie under key_a.  Collective over the grid; `slot` is the path's SelState slot.
+template <typename Visit>
+__device__ unsigned int select_key_b(cg::grid_group& grid, SelState* state, int slot, unsigned int key_a,
+                                     unsigned long long k, unsigned long long below, Visit visit) {
+  unsigned long long cnt = 0;
+  unsigned int mx = 0;  // max of ~key over keys > key_a  ==  ~(min key > key_a)
+  visit([&](unsigned int key) {
+    if (key <= key_a) ++cnt;
+    else if (~key > mx) mx = ~key;
+  });
+  for (int o = 16; o > 0; o >>= 1) {
+    cnt += __shfl_xor_sync(0xffffffffu, cnt, o);
+    const unsigned int other = __shfl_xor_sync(0xffffffffu, mx, o);
+    mx = other > mx ? other : mx;
   }
-  if (MODE == 1) {
-    flush();
-    __syncthreads();
-    if (threadIdx.x == 0) state->blk_cnt[1][blockIdx.x] = s_cnt < cand_cap ? s_cnt : cand_cap;  // cannot overflow
+  if ((threadIdx.x & 31) == 0) {
+    if (cnt) atomicAdd(&state->cnt_le[slot], cnt);
+    if (mx) atomicMax(&state->min_gt[slot], mx);
   }
-  if (MODE == 2) {
-    // has_nan may hold a "maybe" from the fast pass (Inf also trips it): the exact pass decides
-    if (saw_nan) atomicOr(&state->has_nan, 2u);
-  }
+  grid.sync();
+  const unsigned long long cnt_le = below + __ldcg(&state->cnt_le[slot]);
+  const unsigned int mg = __ldcg(&state->min_gt[slot]);
+  return (cnt_le <= k + 1ull && mg) ? ~mg : key_a;
 }
 
 // NumPy's _lerp (numpy/lib/_function_base_impl.py) in float32, no FMA contraction:
@@ -612,17 +635,20 @@ __device__ __forceinline__ float np_lerp_f32(float a, float b, float gamma) {
   return r;
 }
 
-// count(key <= key_a) and max(~key) over keys > key_a, warp-reduced and accumulated into the state
-__device__ __forceinline__ void succ_accumulate(SelState* state, int slot, unsigned long long cnt, unsigned int mx) {
-  for (int o = 16; o > 0; o >>= 1) {
-    cnt += __shfl_xor_sync(0xffffffffu, cnt, o);
-    const unsigned int other = __shfl_xor_sync(0xffffffffu, mx, o);
-    mx = other > mx ? other : mx;
+// out3 = (thr, a, b) and the diagnostics flag; returns thr.  np.percentile of data holding a NaN is NaN (only the exact
+// pass records a certain NaN, and the fast path never finishes when it saw one).
+__device__ float select_finish(SelState* state, unsigned int key_a, unsigned int key_b, float gamma, bool fast,
+                               float* out3) {
+  float fa = __uint_as_float(key_a), fb = __uint_as_float(key_b);
+  float thr = np_lerp_f32(fa, fb, gamma);
+  if (__ldcg(&state->has_nan) & 2u) thr = fa = fb = __uint_as_float(0x7fc00000u);
+  if (blockIdx.x == 0 && threadIdx.x == 0) {
+    out3[0] = thr;
+    out3[1] = fa;
+    out3[2] = fb;
+    state->used_fast = fast ? 1u : 0u;
   }
-  if ((threadIdx.x & 31) == 0) {
-    if (cnt) atomicAdd(&state->cnt_le[slot], cnt);
-    if (mx) atomicMax(&state->min_gt[slot], mx);
-  }
+  return thr;
 }
 
 template <bool WRITE_MASK>
@@ -630,7 +656,7 @@ __global__ void __launch_bounds__(THREADS, 4) weight_prune_kernel(const SegTable
                                                                unsigned int* cand, unsigned long long region_words,
                                                                unsigned long long k, float gamma, int use_fast,
                                                                float* out3) {
-  __shared__ __align__(16) unsigned int s_mem[SMEM_WORDS];  // 40 KB: staging | sample keys | histograms
+  __shared__ __align__(16) unsigned int s_mem[SMEM_WORDS];  // 40 KB: held values + staging | sample keys | histograms
   static_assert(SMEM_WORDS >= SAMPLE && SMEM_WORDS >= BINS0, "shared scratch too small");
   cg::grid_group grid = cg::this_grid();
   const long long n = st.start[st.nseg];
@@ -640,7 +666,6 @@ __global__ void __launch_bounds__(THREADS, 4) weight_prune_kernel(const SegTable
   const unsigned int fast_cap = (unsigned int)(region_words / 2);
   unsigned int* my_idx = region + fast_cap;
   const int need_b = (gamma != 0.f && (long long)k + 1 < n) ? 1 : 0;
-  unsigned int key_a = 0, key_b = 0;
   stamp(state, 0);
 
   if (use_fast) {
@@ -686,23 +711,13 @@ __global__ void __launch_bounds__(THREADS, 4) weight_prune_kernel(const SegTable
                     (k + (unsigned long long)need_b - below) < m;
     if (ok) {  // grid-uniform
       // ---- R: exact rank among the candidates (level 0 was binned during the pass) ----
-      key_a = resolve_rank(grid, &state->lvl_hist[0][0][0], my_keys, my_cnt, lo, hi - lo, k - below, s_mem, true);
+      const unsigned int key_a =
+          resolve_rank(grid, &state->lvl_hist[0][0][0], my_keys, my_cnt, lo, hi - lo, k - below, s_mem, true);
       stamp(state, 5);
-      key_b = key_a;
-      if (need_b) {
-        unsigned long long cnt = 0;
-        unsigned int mx = 0;  // max of ~key over keys > key_a  ==  ~(min key > key_a)
-        for_each_own(my_keys, my_cnt, [&](unsigned int key, unsigned int) {
-          if (key <= key_a) ++cnt;
-          else if (~key > mx) mx = ~key;
-        });
-        succ_accumulate(state, 0, cnt, mx);
-        grid.sync();
-        const unsigned long long cnt_le = below + __ldcg(&state->cnt_le[0]);
-        const unsigned int mg = __ldcg(&state->min_gt[0]);
-        if (cnt_le <= k + 1ull && mg) key_b = ~mg;
-      }
-      const float thr = np_lerp_f32(__uint_as_float(key_a), __uint_as_float(key_b), gamma);
+      const unsigned int key_b = need_b ? select_key_b(grid, state, 0, key_a, k, below, [&](auto f) {
+        for_each_own(my_keys, my_cnt, [&](unsigned int key, unsigned int) { f(key); });
+      }) : key_a;
+      const float thr = select_finish(state, key_a, key_b, gamma, true, out3);
       // ---- F: candidates whose provisional mask (|w| > mid) differs from the final one (|w| > thr) ----
       if (WRITE_MASK) {
         const float mid_f = __uint_as_float(mid);
@@ -716,21 +731,25 @@ __global__ void __launch_bounds__(THREADS, 4) weight_prune_kernel(const SegTable
           }
         });
       }
-      if (blockIdx.x == 0 && threadIdx.x == 0) {
-        out3[0] = thr;
-        out3[1] = __uint_as_float(key_a);
-        out3[2] = __uint_as_float(key_b);
-        state->used_fast = 1;
-      }
       stamp(state, 6);
       return;
     }
   }
 
   // ---- exact path ----
+  // 4096-bin histogram of key >> 19; records NaNs (has_nan may hold a "maybe" from the fast pass, Inf also trips it:
+  // this pass decides)
   for (int i = threadIdx.x; i < BINS0; i += THREADS) s_mem[i] = 0;
   __syncthreads();
-  exact_pass<2>(st, ch, state, 0u, 0u, nullptr, 0u, s_mem);
+  bool saw_nan = false;
+  walk_chunks<false, false>(st, ch, [&](const Where& w, const float4 (&q)[ITERS], auto full) {
+    for_each_valid<decltype(full)::value>(w, q, [&](float v, int) {
+      const unsigned int key = absbits(v);
+      saw_nan |= key > 0x7f800000u;
+      atomicAdd(&s_mem[key >> 19], 1u);
+    });
+  });
+  if (saw_nan) atomicOr(&state->has_nan, 2u);
   __syncthreads();
   for (int i = threadIdx.x; i < BINS0; i += THREADS)
     if (s_mem[i]) atomicAdd(&state->hist0[i], s_mem[i]);
@@ -739,111 +758,52 @@ __global__ void __launch_bounds__(THREADS, 4) weight_prune_kernel(const SegTable
   unsigned long long rem1;
   find_bin<BINS0>(state->hist0, k, &bin0, &rem1);
   const unsigned int lo = bin0 << 19, hi = lo + ((1u << 19) - 1u);
-  exact_pass<1>(st, ch, state, lo, hi, my_keys, (unsigned int)region_words, s_mem);
+  // compact the keys of that bin: the whole slice holds keys, which covers every element the block visits
+  {
+    __shared__ unsigned int s_cnt;
+    static_assert(HOLD_WORDS + STAGE_WORDS <= SMEM_WORDS, "exact compaction smem carve-up");
+    if (threadIdx.x == 0) s_cnt = 0;
+    __syncthreads();
+    CandSink<false> sink(s_mem, my_keys, nullptr, (unsigned int)region_words, &s_cnt);
+    walk_chunks<false, false>(st, ch, [&](const Where& w, const float4 (&q)[ITERS], auto full) {
+      unsigned int hits = 0;
+      for_each_valid<decltype(full)::value>(w, q, [&](float v, int b) {
+        const unsigned int key = absbits(v);
+        if (key >= lo && key <= hi) hits |= 1u << b;
+      });
+      sink.hold(q);
+      sink.append(hits, 0u, [](unsigned int) {});
+    });
+    sink.finish(&state->blk_cnt[1][blockIdx.x], &state->overflow);  // cannot overflow
+  }
   grid.sync();
   const unsigned int my_cnt = __ldcg(&state->blk_cnt[1][blockIdx.x]);
-  key_a = resolve_rank(grid, &state->lvl_hist[1][0][0], my_keys, my_cnt, lo, hi - lo, rem1, s_mem, false);
-  key_b = key_a;
-  if (need_b) {
-    // count(key <= key_a) and min(key > key_a) over the ORIGINAL data decide sorted[k+1]
-    unsigned long long cnt = 0;
-    unsigned int mx = 0;
-    for_each_element(st, ch, [&](float v, int, long long) {
-      const unsigned int key = absbits(v);
-      if (key <= key_a) ++cnt;
-      else if (~key > mx) mx = ~key;
+  const unsigned int key_a =
+      resolve_rank(grid, &state->lvl_hist[1][0][0], my_keys, my_cnt, lo, hi - lo, rem1, s_mem, false);
+  // the successor over the ORIGINAL data decides sorted[k+1]
+  const unsigned int key_b = need_b ? select_key_b(grid, state, 1, key_a, k, 0ull, [&](auto f) {
+    walk_chunks<false, false>(st, ch, [&](const Where& w, const float4 (&q)[ITERS], auto full) {
+      for_each_valid<decltype(full)::value>(w, q, [&](float v, int) { f(absbits(v)); });
     });
-    succ_accumulate(state, 1, cnt, mx);
-    grid.sync();
-    const unsigned long long cnt_le = __ldcg(&state->cnt_le[1]);
-    const unsigned int mg = __ldcg(&state->min_gt[1]);
-    if (cnt_le <= k + 1ull && mg) key_b = ~mg;
-  }
-  float thr = np_lerp_f32(__uint_as_float(key_a), __uint_as_float(key_b), gamma);
-  float fa = __uint_as_float(key_a), fb = __uint_as_float(key_b);
-  if (__ldcg(&state->has_nan) & 2u) thr = fa = fb = __uint_as_float(0x7fc00000u);  // np.percentile of data with NaN
-  if (blockIdx.x == 0 && threadIdx.x == 0) {
-    out3[0] = thr;
-    out3[1] = fa;
-    out3[2] = fb;
-  }
-  if (WRITE_MASK) {
-    for_each_element(st, ch, [&](float v, int s, long long i) { st.out[s][i] = fabsf(v) > thr ? 1.f : 0.f; });
-  }
+  }) : key_a;
+  const float thr = select_finish(state, key_a, key_b, gamma, false, out3);
+  if constexpr (WRITE_MASK) mask_pass<true, false>(st, ch, thr);
 }
 
-// ---- mask / apply ----------------------------------------------------------------------------------------
+// ---- stand-alone passes: one multi-tensor launch each ----------------------------------------------------------
 template <bool WRITE_MASK, bool APPLY>
 __global__ void __launch_bounds__(THREADS) mask_kernel(const SegTable st, const Chunks ch, const float* __restrict__ thr_p) {
-  const float thr = *thr_p;
-  const long long nchunks = ch.cstart[st.nseg];
-  for (long long cid = blockIdx.x; cid < nchunks; cid += gridDim.x) {
-    const int s = find_seg(ch, st.nseg, cid);
-    const long long size = st.start[s + 1] - st.start[s];
-    const long long base = (cid - ch.cstart[s]) * CHUNK;
-    float* w = const_cast<float*>(st.ptr[s]);
-    float* m = st.out[s];
-    const bool aligned = ((reinterpret_cast<uintptr_t>(w) | (WRITE_MASK ? reinterpret_cast<uintptr_t>(m) : 0)) & 15) == 0;
-#pragma unroll
-    for (int it = 0; it < ITERS; ++it) {
-      const long long i = base + ((long long)it * THREADS + threadIdx.x) * 4;
-      if (aligned && i + 4 <= size) {
-        const float4 v = ld_stream_f4(reinterpret_cast<const float4*>(w + i));
-        float4 mk;
-        mk.x = fabsf(v.x) > thr ? 1.f : 0.f;
-        mk.y = fabsf(v.y) > thr ? 1.f : 0.f;
-        mk.z = fabsf(v.z) > thr ? 1.f : 0.f;
-        mk.w = fabsf(v.w) > thr ? 1.f : 0.f;
-        if (WRITE_MASK) st_stream_f4(reinterpret_cast<float4*>(m + i), mk);
-        if (APPLY) {
-          float4 o;
-          o.x = __fmul_rn(v.x, mk.x);
-          o.y = __fmul_rn(v.y, mk.y);
-          o.z = __fmul_rn(v.z, mk.z);
-          o.w = __fmul_rn(v.w, mk.w);
-          st_stream_f4(reinterpret_cast<float4*>(w + i), o);
-        }
-      } else {
-        for (int j = 0; j < 4; ++j)
-          if (i + j < size) {
-            const float v = w[i + j];
-            const float mk = fabsf(v) > thr ? 1.f : 0.f;
-            if (WRITE_MASK) m[i + j] = mk;
-            if (APPLY) w[i + j] = __fmul_rn(v, mk);
-          }
-      }
-    }
-  }
+  mask_pass<WRITE_MASK, APPLY>(st, ch, *thr_p);
 }
 
 // w *= mask (out[] of the table holds the mask pointers)
 __global__ void __launch_bounds__(THREADS) apply_masks_kernel(const SegTable st, const Chunks ch) {
-  const long long nchunks = ch.cstart[st.nseg];
-  for (long long cid = blockIdx.x; cid < nchunks; cid += gridDim.x) {
-    const int s = find_seg(ch, st.nseg, cid);
-    const long long size = st.start[s + 1] - st.start[s];
-    const long long base = (cid - ch.cstart[s]) * CHUNK;
-    float* w = const_cast<float*>(st.ptr[s]);
-    const float* m = st.out[s];
-    const bool aligned = ((reinterpret_cast<uintptr_t>(w) | reinterpret_cast<uintptr_t>(m)) & 15) == 0;
+  walk_chunks<false, true>(st, ch, [&](const Where& w, const float4 (&q)[ITERS], auto full) {
+    constexpr bool FULL = decltype(full)::value;
 #pragma unroll
-    for (int it = 0; it < ITERS; ++it) {
-      const long long i = base + ((long long)it * THREADS + threadIdx.x) * 4;
-      if (aligned && i + 4 <= size) {
-        const float4 v = ld_stream_f4(reinterpret_cast<const float4*>(w + i));
-        const float4 k = ld_stream_f4(reinterpret_cast<const float4*>(m + i));
-        float4 o;
-        o.x = __fmul_rn(v.x, k.x);
-        o.y = __fmul_rn(v.y, k.y);
-        o.z = __fmul_rn(v.z, k.z);
-        o.w = __fmul_rn(v.w, k.w);
-        st_stream_f4(reinterpret_cast<float4*>(w + i), o);
-      } else {
-        for (int j = 0; j < 4; ++j)
-          if (i + j < size) w[i + j] = __fmul_rn(w[i + j], m[i + j]);
-      }
-    }
-  }
+    for (int it = 0; it < ITERS; ++it)
+      store4<FULL>(const_cast<float*>(w.p), w, it, mul4(q[it], load4<FULL>(w.out, w, it)));
+  });
 }
 
 __global__ void __launch_bounds__(THREADS) count_zeros_kernel(const SegTable st, const Chunks ch,
@@ -851,53 +811,37 @@ __global__ void __launch_bounds__(THREADS) count_zeros_kernel(const SegTable st,
   __shared__ unsigned int s_cnt[MC_MAX_SEGMENTS];
   if (threadIdx.x < MC_MAX_SEGMENTS) s_cnt[threadIdx.x] = 0;
   __syncthreads();
-  const long long nchunks = ch.cstart[st.nseg];
-  for (long long cid = blockIdx.x; cid < nchunks; cid += gridDim.x) {
-    const int s = find_seg(ch, st.nseg, cid);
-    const long long size = st.start[s + 1] - st.start[s];
-    const long long base = (cid - ch.cstart[s]) * CHUNK;
-    const float* p = st.ptr[s];
-    const bool aligned = (reinterpret_cast<uintptr_t>(p) & 15) == 0;
+  walk_chunks<false, false>(st, ch, [&](const Where& w, const float4 (&q)[ITERS], auto full) {
     unsigned int c = 0;
-#pragma unroll
-    for (int it = 0; it < ITERS; ++it) {
-      const long long i = base + ((long long)it * THREADS + threadIdx.x) * 4;
-      if (aligned && i + 4 <= size) {
-        const float4 v = ld_stream_f4(reinterpret_cast<const float4*>(p + i));
-        c += (v.x == 0.f) + (v.y == 0.f) + (v.z == 0.f) + (v.w == 0.f);
-      } else {
-        for (int j = 0; j < 4; ++j)
-          if (i + j < size) c += (p[i + j] == 0.f);
-      }
-    }
+    for_each_valid<decltype(full)::value>(w, q, [&](float v, int) { c += (v == 0.f); });
     for (int o = 16; o > 0; o >>= 1) c += __shfl_xor_sync(0xffffffffu, c, o);
-    if ((threadIdx.x & 31) == 0 && c) atomicAdd(&s_cnt[s], c);
-  }
+    if ((threadIdx.x & 31) == 0 && c) atomicAdd(&s_cnt[w.s], c);
+  });
   __syncthreads();
   if (threadIdx.x < st.nseg && s_cnt[threadIdx.x]) atomicAdd(&counts[threadIdx.x], (unsigned long long)s_cnt[threadIdx.x]);
 }
 
+// sum of w * |mask - 1| per segment: products in fp32, accumulated in fp64
 __global__ void __launch_bounds__(THREADS) masked_residual_kernel(const SegTable st, const Chunks ch,
                                                                   double* __restrict__ out) {
-  const long long nchunks = ch.cstart[st.nseg];
-  for (long long cid = blockIdx.x; cid < nchunks; cid += gridDim.x) {
-    const int s = find_seg(ch, st.nseg, cid);
-    const long long size = st.start[s + 1] - st.start[s];
-    const long long base = (cid - ch.cstart[s]) * CHUNK;
-    const float* w = st.ptr[s];
-    const float* m = st.out[s];
+  walk_chunks<false, true>(st, ch, [&](const Where& w, const float4 (&q)[ITERS], auto full) {
+    constexpr bool FULL = decltype(full)::value;
+    const unsigned int vm = valid_bits<FULL>(w);
     double acc = 0.0;
+#pragma unroll
     for (int it = 0; it < ITERS; ++it) {
-      const long long i = base + ((long long)it * THREADS + threadIdx.x) * 4;
+      const float4 m = load4<FULL>(w.out, w, it);
+#pragma unroll
       for (int j = 0; j < 4; ++j)
-        if (i + j < size) acc += (double)(w[i + j] * fabsf(m[i + j] - 1.f));
+        if (vm & (1u << (it * 4 + j))) acc += (double)(part(q[it], j) * fabsf(part(m, j) - 1.f));
     }
     for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
-    if ((threadIdx.x & 31) == 0 && acc != 0.0) atomicAdd(&out[s], acc);
-  }
+    if ((threadIdx.x & 31) == 0 && acc != 0.0) atomicAdd(&out[w.s], acc);
+  });
 }
 
-int build_tables(SegTable* st, Chunks* ch, const float* const* ptrs, float* const* outs, const int64_t* sizes,
+// Segment and chunk tables; every segment of a non-null outs table must have its mask.
+int build_tables(SegTable* st, Chunks* ch, const float* const* ptrs, const float* const* outs, const int64_t* sizes,
                  int nseg, const char* who) {
   if (nseg <= 0 || nseg > MC_MAX_SEGMENTS) return mc_set_error(MC_ERR_ARG, "%s: nseg %d out of range 1..%d", who, nseg, MC_MAX_SEGMENTS);
   if (!ptrs || !sizes) return mc_set_error(MC_ERR_ARG, "%s: null table", who);
@@ -906,8 +850,9 @@ int build_tables(SegTable* st, Chunks* ch, const float* const* ptrs, float* cons
   ch->cstart[0] = 0;
   for (int s = 0; s < nseg; ++s) {
     if (sizes[s] < 0 || (sizes[s] > 0 && !ptrs[s])) return mc_set_error(MC_ERR_ARG, "%s: segment %d invalid", who, s);
+    if (outs && sizes[s] > 0 && !outs[s]) return mc_set_error(MC_ERR_ARG, "%s: null mask %d", who, s);
     st->ptr[s] = ptrs[s];
-    st->out[s] = outs ? outs[s] : nullptr;
+    st->out[s] = outs ? const_cast<float*>(outs[s]) : nullptr;
     st->start[s + 1] = st->start[s] + sizes[s];
     ch->cstart[s + 1] = ch->cstart[s] + (sizes[s] + CHUNK - 1) / CHUNK;
   }
@@ -920,11 +865,15 @@ int build_tables(SegTable* st, Chunks* ch, const float* const* ptrs, float* cons
   return 0;
 }
 
-int stream_grid(long long nchunks) {
-  long long g = (long long)mc_num_sms() * 8;
-  if (g > nchunks) g = nchunks;
-  if (g < 1) g = 1;
-  return (int)g;
+// Tables and grid of a stand-alone pass: 8 blocks per SM, at most one per chunk; *grid = 0 when there is no chunk.
+int stream_tables(SegTable* st, Chunks* ch, int* grid, const float* const* ptrs, const float* const* masks,
+                  const int64_t* sizes, int nseg, const char* who) {
+  const int rc = build_tables(st, ch, ptrs, masks, sizes, nseg, who);
+  if (rc) return rc;
+  const long long nchunks = ch->cstart[nseg];
+  const long long g = (long long)mc_num_sms() * 8;
+  *grid = (int)(g < nchunks ? g : nchunks);
+  return 0;
 }
 
 }  // namespace
@@ -951,8 +900,6 @@ int launch_weight_prune(const float* const* h_w_ptrs, float* const* h_mask_ptrs,
   MC_CHECK_ARG(k >= 0 && k < n, "%s: rank %lld out of range [0,%lld)", who, (long long)k, n);
   MC_CHECK_ARG(d_out3 && d_ws, "%s: null output/workspace", who);
   MC_CHECK_ARG(gamma >= 0.f && gamma < 1.f, "%s: gamma must be in [0,1)", who);
-  if (h_mask_ptrs)
-    for (int s = 0; s < nseg; ++s) MC_CHECK_ARG(h_mask_ptrs[s] || h_seg_sizes[s] == 0, "%s: null mask %d", who, s);
   if (ws_bytes < mc_workspace_bytes_kth_abs_select(n))
     return mc_set_error(MC_ERR_WS, "%s: workspace %zu < required %zu", who, ws_bytes, mc_workspace_bytes_kth_abs_select(n));
   const size_t state_bytes = ((sizeof(SelState) + 255) / 256) * 256;
@@ -1026,13 +973,9 @@ extern "C" int mc_mask_apply_gt(float* const* h_w_ptrs, float* const* h_mask_ptr
   MC_CHECK_ARG(h_mask_ptrs != nullptr || apply, "mc_mask_apply_gt: nothing to do (no masks, no apply)");
   SegTable st;
   Chunks ch;
-  int rc = build_tables(&st, &ch, const_cast<const float* const*>(h_w_ptrs), h_mask_ptrs, h_seg_sizes, nseg,
-                        "mc_mask_apply_gt");
-  if (rc) return rc;
-  if (h_mask_ptrs)
-    for (int s = 0; s < nseg; ++s) MC_CHECK_ARG(h_mask_ptrs[s] || h_seg_sizes[s] == 0, "mc_mask_apply_gt: null mask %d", s);
-  if (ch.cstart[nseg] == 0) return 0;
-  const int grid = stream_grid(ch.cstart[nseg]);
+  int grid;
+  const int rc = stream_tables(&st, &ch, &grid, h_w_ptrs, h_mask_ptrs, h_seg_sizes, nseg, "mc_mask_apply_gt");
+  if (rc || !grid) return rc;
   if (h_mask_ptrs && apply) mask_kernel<true, true><<<grid, THREADS, 0, stream>>>(st, ch, d_thr);
   else if (h_mask_ptrs) mask_kernel<true, false><<<grid, THREADS, 0, stream>>>(st, ch, d_thr);
   else mask_kernel<false, true><<<grid, THREADS, 0, stream>>>(st, ch, d_thr);
@@ -1046,13 +989,10 @@ extern "C" int mc_apply_masks(float* const* h_w_ptrs, const float* const* h_mask
   MC_CHECK_ARG(h_mask_ptrs != nullptr, "mc_apply_masks: null mask table");
   SegTable st;
   Chunks ch;
-  int rc = build_tables(&st, &ch, const_cast<const float* const*>(h_w_ptrs),
-                        const_cast<float* const*>(reinterpret_cast<const float* const*>(h_mask_ptrs)), h_seg_sizes,
-                        nseg, "mc_apply_masks");
-  if (rc) return rc;
-  for (int s = 0; s < nseg; ++s) MC_CHECK_ARG(h_mask_ptrs[s] || h_seg_sizes[s] == 0, "mc_apply_masks: null mask %d", s);
-  if (ch.cstart[nseg] == 0) return 0;
-  apply_masks_kernel<<<stream_grid(ch.cstart[nseg]), THREADS, 0, stream>>>(st, ch);
+  int grid;
+  const int rc = stream_tables(&st, &ch, &grid, h_w_ptrs, h_mask_ptrs, h_seg_sizes, nseg, "mc_apply_masks");
+  if (rc || !grid) return rc;
+  apply_masks_kernel<<<grid, THREADS, 0, stream>>>(st, ch);
   MC_LAUNCH_CHECK("apply_masks_kernel");
   return 0;
 }
@@ -1063,12 +1003,12 @@ extern "C" int mc_count_zeros(const float* const* h_w_ptrs, const int64_t* h_seg
   MC_CHECK_ARG(d_counts != nullptr, "mc_count_zeros: null output");
   SegTable st;
   Chunks ch;
-  int rc = build_tables(&st, &ch, h_w_ptrs, nullptr, h_seg_sizes, nseg, "mc_count_zeros");
+  int grid;
+  const int rc = stream_tables(&st, &ch, &grid, h_w_ptrs, nullptr, h_seg_sizes, nseg, "mc_count_zeros");
   if (rc) return rc;
   MC_CUDA(cudaMemsetAsync(d_counts, 0, sizeof(int64_t) * nseg, stream));
-  if (ch.cstart[nseg] == 0) return 0;
-  count_zeros_kernel<<<stream_grid(ch.cstart[nseg]), THREADS, 0, stream>>>(st, ch,
-                                                                           reinterpret_cast<unsigned long long*>(d_counts));
+  if (!grid) return 0;
+  count_zeros_kernel<<<grid, THREADS, 0, stream>>>(st, ch, reinterpret_cast<unsigned long long*>(d_counts));
   MC_LAUNCH_CHECK("count_zeros_kernel");
   return 0;
 }
@@ -1079,12 +1019,12 @@ extern "C" int mc_masked_residual(const float* const* h_w_ptrs, const float* con
   MC_CHECK_ARG(d_out != nullptr && h_mask_ptrs != nullptr, "mc_masked_residual: null pointer");
   SegTable st;
   Chunks ch;
-  int rc = build_tables(&st, &ch, h_w_ptrs, const_cast<float* const*>(reinterpret_cast<const float* const*>(h_mask_ptrs)),
-                        h_seg_sizes, nseg, "mc_masked_residual");
+  int grid;
+  const int rc = stream_tables(&st, &ch, &grid, h_w_ptrs, h_mask_ptrs, h_seg_sizes, nseg, "mc_masked_residual");
   if (rc) return rc;
   MC_CUDA(cudaMemsetAsync(d_out, 0, sizeof(double) * nseg, stream));
-  if (ch.cstart[nseg] == 0) return 0;
-  masked_residual_kernel<<<stream_grid(ch.cstart[nseg]), THREADS, 0, stream>>>(st, ch, d_out);
+  if (!grid) return 0;
+  masked_residual_kernel<<<grid, THREADS, 0, stream>>>(st, ch, d_out);
   MC_LAUNCH_CHECK("masked_residual_kernel");
   return 0;
 }

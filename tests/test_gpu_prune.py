@@ -85,10 +85,11 @@ class _ParamBag(torch.nn.Module):
         self.ps = torch.nn.ParameterList([torch.nn.Parameter(t) for t in tensors])
 
 
-@pytest.mark.parametrize("sizes", [(70001,), (300000, 17, 700003), (1 << 20, 5)])
+@pytest.mark.parametrize("sizes", [(70001,), (300000, 17, 700003), (1 << 20, 5), (12000,)])
 def test_weight_prune_midsize_interpolated(sizes):
     # n < 2^24 so float32 np.percentile interpolates (gamma != 0) and n >= 8*SAMPLE so the fast path runs: the
-    # (k+1)-th order statistic is resolved among the bracketed candidates
+    # (k+1)-th order statistic is resolved among the bracketed candidates.  (12000,) is 36,000 elements in 9 chunks:
+    # a grid of 9 blocks, fewer than the 16 key groups of the sample ranking.
     from modelcompression_b200 import _lib
     from modelcompression_b200.pruning.weightPruning import methods
     gen = torch.Generator().manual_seed(5)
@@ -102,6 +103,8 @@ def test_weight_prune_midsize_interpolated(sizes):
             assert np.array_equal(a.cpu().numpy(), b), "perc %s" % perc
         out3 = methods.weight_threshold([p.data for p in bag.parameters()], perc).cpu().numpy()
         assert out3[0] == np.float32(thr_o), "perc %s" % perc
+        if sizes == (12000,) and perc in (12.5, 33.3, 70.0):
+            assert _used_fast() == 1, "perc %s" % perc
     # heavy ties: quantised weights (the k-th value is shared by thousands of elements)
     tq = [torch.round(t * 4) / 4 for t in ts]
     bagq = _ParamBag(tq).to(DEV)
@@ -317,3 +320,78 @@ def test_count_zeros_and_unaligned_segments():
     views = [v.clone() if False else v for v in views]
     got = count_zeros([v.contiguous() for v in views])
     assert got == [int((v == 0).sum()) for v in views]
+
+
+def test_weight_prune_more_tensors_than_one_launch_takes():
+    # 70 parameters > 64 segments: weight_prune selects on a flat copy (weight_threshold) and masks in groups
+    # (mc_mask_apply_gt); count_zeros launches once per 64 tensors
+    from modelcompression_b200.pruning.weightPruning.methods import weight_threshold
+    from modelcompression_b200.pruning.weightPruning.utils import count_zeros
+    gen = torch.Generator().manual_seed(12)
+    ts = [torch.randn(40 + 37 * i, 3, generator=gen) for i in range(70)]
+    for t in ts[::5]:
+        t[:7] = 0
+    bag = _ParamBag(ts).to(DEV)
+    ws = [t.numpy() for t in ts]
+    for perc in (10.0, 61.7, 95.0):
+        thr_o, masks_o = prune_oracle.weight_prune_np(ws, perc)
+        masks = mc.weight_prune(bag, perc)
+        assert len(masks) == 70
+        for a, b in zip(masks, masks_o):
+            assert np.array_equal(a.cpu().numpy(), b), "perc %s" % perc
+        out3 = weight_threshold([p.data for p in bag.parameters()], perc).cpu().numpy()
+        assert out3[0] == np.float32(thr_o), "perc %s" % perc
+    assert count_zeros([p.data for p in bag.parameters()]) == [int((w == 0).sum()) for w in ws]
+
+
+def _aligned_and_unaligned(gen, sizes):
+    """Fresh (16-byte aligned) tensors and views into one buffer that are only 4-byte aligned, of the same sizes."""
+    aligned = [torch.randn(n, generator=gen).to(DEV) for n in sizes]
+    buf = torch.randn(sum(sizes) + 4 * len(sizes), generator=gen).to(DEV)
+    unaligned, off = [], 1
+    for n in sizes:
+        unaligned.append(buf[off:off + n])
+        off += n + (1 - off - n) % 4  # every offset is 1 (mod 4) elements: 4 (mod 16) bytes
+    assert all(v.data_ptr() % 16 != 0 for v in unaligned)
+    return aligned, unaligned
+
+
+def test_mask_apply_gt_apply_bit_exact():
+    from modelcompression_b200 import _lib
+    lib = _lib.load()
+    gen = torch.Generator().manual_seed(13)
+    sizes = [70001, 3, 2 * 4096 + 5, 4096]
+    thr = torch.tensor([0.7], device=DEV)
+    for segs in _aligned_and_unaligned(gen, sizes):
+        for with_masks in (True, False):
+            w0 = [s.clone() for s in segs]
+            masks = [torch.full_like(s, 7.0) for s in segs] if with_masks else None
+            _lib.check(lib.mc_mask_apply_gt(_lib.ptr_array(segs), _lib.ptr_array(masks) if masks else None,
+                                            _lib.int64_array(sizes), len(segs), thr.data_ptr(), 1, _lib.stream_ptr()),
+                       "mc_mask_apply_gt")
+            for i, (w, s) in enumerate(zip(w0, segs)):
+                want_m = (w.abs() > thr).float()
+                assert torch.equal((w * want_m).view(torch.int32), s.view(torch.int32)), i
+                if with_masks:
+                    assert torch.equal(want_m.view(torch.int32), masks[i].view(torch.int32)), i
+
+
+def test_masked_residual_value():
+    # positive weights and a non-zero residual: no term cancels, so the fp64 sum of the fp32 products w * |m - 1| is
+    # the float64 torch sum up to the order of the additions
+    from modelcompression_b200 import _lib
+    lib = _lib.load()
+    gen = torch.Generator().manual_seed(14)
+    sizes = [70001, 3, 2 * 4096 + 5, 4096]
+    for ws in _aligned_and_unaligned(gen, sizes):
+        for w in ws:
+            w.abs_().add_(0.1)
+        ms = [(torch.rand(n, generator=gen) > 0.3).float().to(DEV) for n in sizes]
+        for m in ms:
+            m[::7] = 0
+        out = torch.zeros(len(ws), dtype=torch.float64, device=DEV)
+        _lib.check(lib.mc_masked_residual(_lib.ptr_array(ws), _lib.ptr_array(ms), _lib.int64_array(sizes), len(ws),
+                                          out.data_ptr(), _lib.stream_ptr()), "mc_masked_residual")
+        want = torch.stack([(w * (m - 1).abs()).double().sum() for w, m in zip(ws, ms)])
+        assert bool((want > 0).all())
+        assert torch.allclose(out, want, rtol=1e-12, atol=0), (out, want)

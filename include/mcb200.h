@@ -274,6 +274,20 @@ size_t mc_workspace_bytes_conv_chain(const mc_conv_desc* descs, int n);
  * info[5] = smem ring stages         info[6] = grid size                   info[7] = k-block (32 or 64)           */
 int mc_conv_last_plan(int info[8]);
 
+/* What mc_conv_fwd would launch for this descriptor on the current device, without launching (tests / reporting).
+ * The descriptor is checked as mc_conv_fwd checks it (same errors); buffers are not touched.
+ * info[0]  = 1 CTA-pair kernel, 0 single CTA       info[1]  = CTAs per SM (1..3; 1 for the pair)
+ * info[2]  = block_n                               info[3]  = block_k (32 or 64)
+ * info[4]  = B-tile (or A | B) ring stages         info[5]  = activation-box ring stages (0: no shared box)
+ * info[6]  = 1 shared activation box               info[7]  = CTAs launched
+ * info[8]  = 128-row m-tiles                       info[9]  = n-tiles
+ * info[10] = CTA pair: units in the stream-K tail (0: whole units only)
+ * info[11] = PNHWC store path: 2 TMA-store slabs, 1 staged through shared memory, 0 direct (and every other mode)
+ * info[12] = TMA-store slabs per epilogue warp     info[13] = 1: the epilogue loads 64 accumulator columns at a time
+ * info[14] = 1: 16-byte stores allowed (8-aligned ldc and ch_off; REORG2 also N % 8 == 0), 0: scalar stores
+ * info[15] = UMMA K steps (16 channels) issued for the last channel block of a tap                                  */
+int mc_conv_fwd_plan(const mc_conv_desc* desc, int info[16]);
+
 /* Small-channel direct convolution on CUDA cores, for layers too thin for a 128xNx64 tensor-core tile: the 3-channel
  * first layer (in_is_nchw_f32=1: d_in is the fp32 NCHW image [B,Cin,H,W]) and the first blocks of a filter-pruned
  * network (d_in PNHWC bf16, pitch Cin_ld).  d_w: fp32 [N,Cin,k,k] (already masked / gathered).  Fused scale/shift,

@@ -83,6 +83,7 @@ _SIGNATURES = {
     "mc_workspace_bytes_conv_chain": (c_size_t, [POINTER(mc_conv_desc), c_int]),
     "mc_workspace_bytes_conv_fwd": (c_size_t, [POINTER(mc_conv_desc)]),
     "mc_conv_last_plan": (c_int, [POINTER(c_int)]),
+    "mc_conv_fwd_plan": (c_int, [POINTER(mc_conv_desc), POINTER(c_int)]),
     "mc_conv_direct_supported": (c_int, [c_int, c_int, c_int]),
     "mc_conv_direct_fwd": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int,
                                    c_int, c_int, c_int, c_int, c_int, c_int, c_void_p]),

@@ -52,7 +52,7 @@ struct ConvKParams {
   int Wp, Hp, W, H;  // Wp = W+1, Hp = H+1
   int block_n, stages, tmem_cols, acc_stride;  // acc_stride: TMEM columns between accumulator stages
   int out_pitch;   // > 0: PNHWC epilogue stages each warp's 32 rows in shared memory (row pitch in bytes) and writes them out coalesced
-  int out_chunk;   // columns staged at a time (<= 64)
+  int out_chunk;   // columns staged at a time (= block_n: see epilogue_loop)
   int tma_bufs;    // > 0: PNHWC epilogue writes whole 64-column chunks with TMA stores from this many 4 KB slabs per warp
   float* stat_sum;    // training forward: per-channel sum / sum of squares of the STORED (bf16-rounded) outputs are
   float* stat_sumsq;  // accumulated from the TMA-store slabs (the batch statistics of BatchNorm); nullptr: off
@@ -637,8 +637,10 @@ __device__ __forceinline__ void epilogue_loop(const ConvKParams& p, const ConvSm
       // Staged store: a thread owns one output ROW, so direct stores are 16-byte pieces one row pitch apart (32 half-
       // filled sectors per warp instruction: measured ~38 cycles per output column and tile).  Instead the warp parks
       // its 32 rows x block_n bf16 in shared memory (pitch +16 B: conflict-free), hands the TMEM stage back at once,
-      // and writes the rows out with consecutive lanes on consecutive 16-byte chunks.
-      // Tiles wider than the staging buffer (64 columns) go through it in 64-column chunks.
+      // and writes the rows out with consecutive lanes on consecutive 16-byte chunks.  The planner stages only the 32-
+      // and 48-wide tiles (wider aligned tiles take the TMA stores), so out_chunk == block_n and the chunk loop runs
+      // once; written as one pass instead, the kernel spills more (ptxas, kernel<3>: 248 / 432 B of spill stores /
+      // loads instead of 224 / 328 B).
       const int pitch = p.out_pitch;
       const int chunk = p.out_chunk;
       uint8_t* wbuf = m.s_out + (size_t)quarter * 32 * pitch;
@@ -1416,23 +1418,16 @@ static int conv_plan(const mc_conv_desc* d, ConvPlan* L) {
   const int num_kb = ntaps * (Kc / BLOCK_K);
   constexpr size_t AUX_BYTES = 5120 + 1024;  // barriers (512), scale/shift staging (4096), pad to 1 KB; 1024-byte alignment slack
 
-  // staged epilogue (PNHWC, tiles up to 128 wide): 128 rows x (block_n bf16 + 16 B) of shared memory
-  // (measured: tiles 32..96 wide gain — dense conv2 396 -> 300 us, conv4' 60 -> 54, shrunk conv8 33 -> 29; 128-wide tiles
-  //  lose smem ring depth to the 34 KB staging buffer (133 -> 154 us) and 16-wide rows are two stores either way)
-  // Wider tiles go through the buffer in 64-column chunks where it was measured to pay: 3x3 layers at high resolution
-  // (dense conv3/conv5, 128 wide, 5513 tiles: 137 -> 123 us); wide 1x1 layers (conv7: 39 -> 47 us) and the short
-  // launches of the 26x26 / 13x13 stages do not.
-  const bool wide_ok = d->ksize == 3 && m_tiles >= 1024;
   // TMA-store epilogue (tiles >= 64 wide): whole 64-column chunks leave as bulk tensor stores from 4 KB slabs per
   // epilogue warp — two slabs per warp when the CTA has the SM to itself, one (16 KB per CTA) when several CTAs share
   // it (measured: dense conv4/conv6 at 104x104 run 113 us with 2 CTAs per SM + one slab, 158 us with one CTA + two
   // slabs, 125 us with the staged epilogue).
   const bool tma_out = d->epi_mode == MC_EPI_PNHWC && block_n >= 64 && ((d->ldc | d->ch_off) & 7) == 0;
   auto tma_bufs_for = [&](int ctas_) -> int { return tma_out ? (ctas_ == 1 ? 2 : 1) : 0; };
-  const bool stage_out = !tma_out && d->epi_mode == MC_EPI_PNHWC && block_n >= 32 && (block_n <= 96 || wide_ok) &&
-                         ((d->ldc | d->ch_off) & 7) == 0;
-  const int out_chunk = block_n <= 96 ? block_n : 64;
-  const int out_pitch = stage_out ? out_chunk * 2 + 16 : 0;
+  // staged epilogue (the aligned PNHWC tiles the TMA stores do not take: 32 and 48 wide): 128 rows x (block_n bf16 +
+  // 16 B) of shared memory (measured: dense conv2 396 -> 300 us; 16-wide rows are two stores either way)
+  const bool stage_out = !tma_out && d->epi_mode == MC_EPI_PNHWC && block_n >= 32 && ((d->ldc | d->ch_off) & 7) == 0;
+  const int out_pitch = stage_out ? block_n * 2 + 16 : 0;
   // (decode epilogue: 128 rows x (block_n + 1) floats of logits)
   auto out_stage_for = [&](int ctas_) -> size_t {
     return decode ? (size_t)128 * (block_n + 1) * 4
@@ -1556,7 +1551,7 @@ static int conv_plan(const mc_conv_desc* d, ConvPlan* L) {
   }
   p.a_stages = a_stages;
   p.out_pitch = use_pair ? 0 : out_pitch;
-  p.out_chunk = out_chunk;
+  p.out_chunk = block_n;
   p.tma_bufs = tma_bufs;
   p.stat_sum = d->d_stat_sum;
   p.stat_sumsq = d->d_stat_sumsq;
@@ -1701,6 +1696,32 @@ extern "C" int mc_conv_fwd(const mc_conv_desc* d, void* stream_) {
   else
     conv_gemm_tcgen05_kernel<1><<<L.grid, NUM_THREADS, L.smem_bytes, stream>>>(L.tm_a, L.tm_b, L.tm_abox, L.tm_out, p);
   MC_LAUNCH_CHECK("conv_gemm_tcgen05_kernel");
+  return 0;
+}
+
+extern "C" int mc_conv_fwd_plan(const mc_conv_desc* d, int info[16]) {
+  MC_CHECK_ARG(info != nullptr, "mc_conv_fwd_plan: null pointer");
+  ConvPlan L;
+  const int rc = conv_plan(d, &L);
+  if (rc) return rc;
+  const ConvKParams& p = L.p;
+  const bool pnhwc = p.epi_mode == MC_EPI_PNHWC;
+  info[0] = L.use_pair ? 1 : 0;
+  info[1] = L.ctas;
+  info[2] = p.block_n;
+  info[3] = p.block_k;
+  info[4] = p.stages;
+  info[5] = p.a_stages;
+  info[6] = p.share_dx;
+  info[7] = L.grid;
+  info[8] = p.m_tiles;
+  info[9] = p.n_tiles;
+  info[10] = p.sk_units;
+  info[11] = p.tma_bufs > 0 ? 2 : (p.out_pitch > 0 ? 1 : 0);
+  info[12] = p.tma_bufs;
+  info[13] = (pnhwc && (L.use_pair || L.ctas == 1)) ? 1 : 0;  // as the kernels instantiate epilogue_tile
+  info[14] = (((p.ldc | p.ch_off) & 7) == 0 && (p.epi_mode != MC_EPI_REORG2 || (p.N & 7) == 0)) ? 1 : 0;
+  info[15] = p.last_ksteps;
   return 0;
 }
 

@@ -63,6 +63,19 @@ def _thin_host_weights(wd, sc, sh, ct, nt):
     return _c_floats(wt), _c_floats(sct), _c_floats(sht)
 
 
+def _pool_window_weights(wd, rows, npos, cl):
+    """Weights of the pool-window GEMM (mc_conv_im2col_fwd with pool=1, mc_conv_window_fwd in_kind 1/2) from the fp32
+    [n, r, s, c] filters: fp32 [rows, 16*cl], row pos*npos + n, column (py*4+px)*cl + c = w[n,c,py-dy,px-dx] with
+    pos = dy*2+dx, zero elsewhere."""
+    n, _, _, c = wd.shape
+    wk = torch.zeros(rows, 4, 4, cl, device=wd.device)
+    for dy in range(2):
+        for dx in range(2):
+            r0 = (dy * 2 + dx) * npos
+            wk[r0:r0 + n, dy:dy + 3, dx:dx + 3, :c] = wd
+    return wk.reshape(rows, 16 * cl)
+
+
 class _TensorRef(object):
     """A logical activation: where it lives and how its physical channels map to the original channel space."""
 
@@ -450,11 +463,7 @@ class CompiledDarknet(object):
                 wk = torch.zeros(nb, 10, 8, device=dev)
                 wk[:n_phys, :9, :c_phys_in] = wd.reshape(n_phys, 9, c_phys_in)
             else:
-                wk = torch.zeros(nb, 4, 4, 4, device=dev)
-                for dy in range(2):
-                    for dx in range(2):
-                        r0 = (dy * 2 + dx) * npos
-                        wk[r0:r0 + n_phys, dy:dy + 3, dx:dx + 3, :c_phys_in] = wd
+                wk = _pool_window_weights(wd, nb, npos, 4)
             wk = wk.reshape(nb, kcols).to(torch.bfloat16).contiguous()
             Ho, Wo = (H // 2, W // 2) if pool else (H, W)
             ld = _pitch(n_phys)
@@ -480,12 +489,7 @@ class CompiledDarknet(object):
             wd = gathered_fp32().permute(0, 2, 3, 1)  # [n, r, s, c]
             nb_pad = _round_up(nb, 16)
             if pool:
-                wexp = torch.zeros(nb_pad, 4, 4, cl, device=dev)
-                for dy in range(2):
-                    for dx in range(2):
-                        r0 = (dy * 2 + dx) * npos
-                        wexp[r0:r0 + n_phys, dy:dy + 3, dx:dx + 3, :c_phys_in] = wd
-                wexp = wexp.reshape(nb_pad, 16 * cl)
+                wexp = _pool_window_weights(wd, nb_pad, npos, cl)
             else:
                 wexp = torch.zeros(nb_pad, 3, 3, cl, device=dev)
                 wexp[:n_phys, :, :, :c_phys_in] = wd

@@ -353,11 +353,8 @@ def _run_window(x, in_kind, w, scale, shift, leaky, pool):
         wk = torch.zeros(nb, 10, 8, device=DEV)
         wk[:N, :9, :C] = wd.reshape(N, 9, C)
     else:
-        wk = torch.zeros(nb, 4, 4, 4, device=DEV)
-        for dy in range(2):
-            for dx in range(2):
-                r0 = (dy * 2 + dx) * npos
-                wk[r0:r0 + N, dy:dy + 3, dx:dx + 3, :C] = wd
+        from modelcompression_b200.engine import _pool_window_weights
+        wk = _pool_window_weights(wd, nb, npos, 4)
     wk = wk.reshape(nb, kcols).to(torch.bfloat16).contiguous()
     nsc = max((npos + 15) // 16 * 16, 16)
     sc = torch.zeros(nsc, device=DEV)

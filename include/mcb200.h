@@ -484,6 +484,73 @@ int mc_sgd_momentum_step(float* const* h_param_ptrs, const float* const* h_grad_
                          const int64_t* h_sizes, int nseg, float lr, float momentum, float weight_decay,
                          int first_step, void* stream);
 
+/* ------------------------------------------------------------------------------------------
+ * Filter-shrunk retrain step (model.b200_shrink_train): the convolutions run over the ALIVE filters only (a filter is
+ * dead when its mask is zero over [C,kh,kw]).  A dead filter is not inert in training: its activation is the constant
+ * leaky(beta) inside the image (batch mean = var = 0), beta gets a gradient and the consumers' weights on it train.
+ * Each consumer therefore reads two extra "ones" input columns (1 at interior pixels, 0 at pads) whose packed weights
+ * are the high and low bf16 halves of S = sum over dead inputs c of bf16((W*mask)[o,c,tap]) * bf16(leaky(beta_c))
+ * (fp32; the dense step's products), and whose weight gradient G1[o,tap] gives
+ *   dW[o, c_dead, tap] = mask * leaky(beta_c) * G1[o,tap]
+ *   dbeta_c (dead)     = leaky'(beta_c) * sum over consumers of sum_{o,tap} (W*mask)[o, c_in, tap] * G1[o,tap]
+ * (c_in = every consumer input column carrying channel c: one per consumer, four through a Reorg).  DESIGN.md §1 a-12.
+ *
+ * One segment per convolution, in a device array built once per plan; per-step buffers are passed as base pointers and
+ * the segment holds offsets into them.  Index lists are offsets into one int32 device array `idx`.
+ * Every entry point is ONE launch over all segments (nseg <= MC_MAX_SEGMENTS).                                       */
+typedef struct mc_shrink_seg {
+  const float* w;          /* [O, C, taps] fp32 conv weight                                                       */
+  const float* mask;       /* same shape, or NULL                                                                 */
+  const float* gamma;      /* [O] BatchNorm weight / bias, NULL for a layer without BatchNorm                    */
+  const float* beta;
+  float* rmean;            /* [O] running statistics, NULL when not tracked                                       */
+  float* rvar;
+  float momentum;          /* running-statistics momentum                                                         */
+  int leaky;               /* 1: leaky(0.1) activation, 0: linear                                                 */
+  int O, C, taps;          /* full shape                                                                          */
+  int n_o;                 /* compact (alive) filters                                                             */
+  int n_col;               /* physical input columns (contraction width of the compact conv / wgrad)             */
+  int ones_col;            /* physical column of the first of the two ones columns, -1 none                       */
+  int npad, kc;            /* forward pack [npad, taps*kc] (kc = 0: this layer packs its weights itself)          */
+  int cpad, ko;            /* data-gradient pack [cpad, taps*ko]                                                  */
+  int n_dead;              /* dead input channels (length of dead_in)                                             */
+  int pad_;
+  int64_t oidx;            /* idx offset: [n_o] compact row -> filter                                             */
+  int64_t orow;            /* idx offset: [O] filter -> compact row, -1 dead                                      */
+  int64_t colmap;          /* idx offset: [n_col] physical column -> input channel, -1 zero column, -2 ones column */
+  int64_t cphys;           /* idx offset: [C] input channel -> physical column, -1 dead input                    */
+  int64_t clk;             /* idx offset: [C] dead input channel -> index into lk, -1 otherwise                  */
+  int64_t dead_in;         /* idx offset: [n_dead] the dead input channels                                        */
+  int64_t cons_ptr;        /* idx offset: [O+1] CSR row pointers of the consumer inputs of each dead filter       */
+  int64_t cons;            /* idx offset: pairs (consumer segment, consumer input channel)                        */
+  int64_t lk_off;          /* lk[lk_off + f] = act(beta[f]) for this layer's filters (BatchNorm layers)           */
+  int64_t cbn_off;         /* compact gamma, beta, running mean, running var at cbn_off + {0,1,2,3} * cbn_ld      */
+  int64_t cbn_ld;
+  int64_t wp_off, wpd_off; /* bf16 element offsets of the forward / data-gradient packs                           */
+  int64_t dwc_off;         /* float offset of the compact weight gradient [n_o, n_col, taps]                      */
+  int64_t cdgb_off;        /* float offset of the compact dbeta [n_o], then dgamma [n_o] (mc_bn_backward output)  */
+  int64_t dw_off;          /* float offset of the full dW [O, C, taps]                                            */
+  int64_t dbn_off;         /* float offset of the full dbeta [O], then dgamma [O]                                 */
+} mc_shrink_seg;
+
+/* Per training forward, first: lk[lk_off+f] = bf16(act(beta[f])) (a dead channel's stored activation) and the compact gamma/beta/running statistics gathered at
+ * cbn_off (which mc_bn_finalize / mc_bn_backward then use unchanged).                                                */
+int mc_shrink_prepare(const mc_shrink_seg* d_segs, int nseg, const int* d_idx, float* d_cbn, float* d_lk, void* stream);
+/* Forward weights: wp[wp_off + n*taps*kc + tap*kc + j] = bf16((W*mask)[oidx[n], colmap[j], tap]); the ones columns
+ * hold hi = bf16(S), lo = bf16(S - hi) of S above; zero rows / columns elsewhere.  d_wpd (may be NULL):
+ * the data-gradient weights at wpd_off, row = physical column (ones / zero columns get zero rows), column
+ * tap'*ko + n = (W*mask)[oidx[n], colmap[row], taps-1-tap'].                                                         */
+int mc_shrink_pack(const mc_shrink_seg* d_segs, int nseg, const int* d_idx, const float* d_lk, void* d_wp, void* d_wpd,
+                   void* stream);
+/* End of the training forward: compact running statistics (updated by mc_bn_finalize) back into the full buffers;
+ * dead channels decay as nn.BatchNorm2d with batch mean = var = 0, in mc_bn_finalize's fp32 operation order.         */
+int mc_shrink_stats(const mc_shrink_seg* d_segs, int nseg, const int* d_idx, const float* d_cbn, void* stream);
+/* End of the backward: full dW (alive entries from the compact gradient, dead input columns by the G1 rule, the mask
+ * applied, dead filters exactly 0) and full dgamma / dbeta (alive from the compact ones, dead: dgamma = 0 and dbeta by
+ * the rule above) into d_grad.                                                                                      */
+int mc_shrink_finish(const mc_shrink_seg* d_segs, int nseg, const int* d_idx, const float* d_lk, const float* d_dwc,
+                     float* d_grad, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -41,6 +41,19 @@ class mc_conv_desc(ctypes.Structure):
     ]
 
 
+class mc_shrink_seg(ctypes.Structure):
+    _fields_ = [
+        ("w", c_void_p), ("mask", c_void_p), ("gamma", c_void_p), ("beta", c_void_p), ("rmean", c_void_p),
+        ("rvar", c_void_p), ("momentum", c_float), ("leaky", c_int), ("O", c_int), ("C", c_int), ("taps", c_int),
+        ("n_o", c_int), ("n_col", c_int), ("ones_col", c_int), ("npad", c_int), ("kc", c_int), ("cpad", c_int),
+        ("ko", c_int), ("n_dead", c_int), ("pad_", c_int),
+        ("oidx", c_int64), ("orow", c_int64), ("colmap", c_int64), ("cphys", c_int64), ("clk", c_int64),
+        ("dead_in", c_int64), ("cons_ptr", c_int64), ("cons", c_int64), ("lk_off", c_int64), ("cbn_off", c_int64),
+        ("cbn_ld", c_int64), ("wp_off", c_int64), ("wpd_off", c_int64), ("dwc_off", c_int64), ("cdgb_off", c_int64),
+        ("dw_off", c_int64), ("dbn_off", c_int64),
+    ]
+
+
 # name -> (restype, argtypes); every symbol include/mcb200.h declares
 _SIGNATURES = {
     "mc_version": (c_int, []),
@@ -138,6 +151,10 @@ _SIGNATURES = {
     "mc_workspace_bytes_conv_wgrad_first": (c_size_t, [c_int, c_int, c_int, c_int, c_int]),
     "mc_sgd_momentum_step": (c_int, [POINTER(c_void_p), POINTER(c_void_p), POINTER(c_void_p), POINTER(c_int64), c_int,
                                      c_float, c_float, c_float, c_int, c_void_p]),
+    "mc_shrink_prepare": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "mc_shrink_pack": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "mc_shrink_stats": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p]),
+    "mc_shrink_finish": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
 }
 
 EXPORTED_SYMBOLS = tuple(sorted(_SIGNATURES))

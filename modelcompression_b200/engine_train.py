@@ -18,6 +18,10 @@ Per conv layer (all activations PNHWC bf16, include/mcb200.h):
 Masked weights get exactly zero gradient (dW is multiplied by the mask, layers.py:59), so with the reference's SGD
 (weight decay of a zero weight is zero) they stay zero: ``are_masks_consistent`` holds after the step.
 
+With ``model.b200_shrink_train`` (default off) the step runs over the filters the masks keep (shrink_layout): the same
+kernels on compact shapes, plus one launch each of mc_shrink_prepare / mc_shrink_pack / mc_shrink_stats per forward and
+mc_shrink_finish per backward, which carry what a dead filter still contributes in training mode (include/mcb200.h).
+
 No CPU / PyTorch fallback: a CPU tensor or an unsupported cfg raises.
 """
 import ctypes
@@ -46,7 +50,9 @@ class _Layer(object):
 class TrainPlan(object):
     """Static description of the cfg graph for training: layers, which buffer each reads/writes."""
 
-    def __init__(self, model):
+    def __init__(self, model, shrink=False):
+        """shrink=True: layers whose masks zero whole filters run over their alive filters (see shrink_layout); with
+        no such filter the plan is the dense one."""
         self.lib = _lib.load()
         blocks = model.blocks
         H, W = model.height, model.width
@@ -56,6 +62,7 @@ class TrainPlan(object):
         self.layers = []
         self.buf_specs = {}   # name -> (H, W, ld)
         self.grad_specs = {}  # name -> (H, W, ld) gradient buffers (same geometry as the activation they belong to)
+        self.cat_parts = {}   # concat buffer name -> (slot-0 producer, slot-1 producer)
         cat_of = {}
         ind = -2
         for block in blocks:
@@ -161,6 +168,7 @@ class TrainPlan(object):
                         if off1 != c0:
                             raise NotImplementedError("concat parts must be multiples of 8 channels")
                         name = 'cat%d' % route
+                        self.cat_parts[name] = (l0, l1)
                         self.buf_specs[name] = (h0, w0, ld)
                         self.grad_specs['d' + name] = (h0, w0, ld)
                         l0.act = _Act(name, h0, w0, c0, ld, 0)
@@ -200,6 +208,11 @@ class TrainPlan(object):
         for L in self.layers:
             if not L.is_head and L.act is None:
                 raise NotImplementedError("unresolved concat producer at block %d" % L.ind)
+        self.shrunk = False
+        self.ones_cols = {}  # activation buffer -> column holding the ones channel (written once per buffer set)
+        if shrink and shrink_layout(self, alive_filters(self.layers)):
+            self.seg_host, self.seg_idx, self.sizes = _seg_table(self)
+            self._tables = {}
         # Pooled layers whose full-resolution activation feeds nothing but the pool: BatchNorm + leaky + pool run as one
         # pass each way (mc_bn_apply_pool / mc_bn_pool_backward) and the activation / its gradient are never stored
         for L in self.layers:
@@ -209,6 +222,7 @@ class TrainPlan(object):
             if self.lib.mc_bn_pool_supported(L.O) != 1 or any(o.src is L.act for o in self.layers):
                 continue
             L.fused_pool = True
+            self.ones_cols.pop(L.act.name, None)
             del self.buf_specs[L.act.name]
             del self.grad_specs['d' + L.act.name]
             L.act = None
@@ -264,9 +278,250 @@ class TrainPlan(object):
             st = {'owner': None, 't': {}}
             for name, (H, W, ld) in list(self.buf_specs.items()) + list(self.grad_specs.items()):
                 st['t'][name] = torch.zeros(B * (H + 1) * (W + 1), ld, dtype=torch.bfloat16, device=dev)
+            # the two ones columns: 1 at interior pixels, 0 at pads.  No pass writes them again: mc_bn_apply /
+            # mc_bn_apply_pool write columns below C only, and mc_maxpool2x2 (whole 8-channel groups, run with C
+            # covering the ones columns) pools them into the ones columns of the pooled buffer, which hold the same values
+            for name, col in self.ones_cols.items():
+                H, W, ld = self.buf_specs[name]
+                st['t'][name].view(B, H + 1, W + 1, ld)[:, :H, :W, col:col + 2] = 1
             sets.append(st)
         st['owner'] = weakref.ref(owner) if owner is not None else None
         return st['t']
+
+
+def alive_filters(layers):
+    """Per layer: the sorted filters whose mask is non-zero somewhere over [C,kh,kw] (read once, on the host).  Dead is
+    decided by the mask, not the weights: a masked-in filter whose weights happen to be zero still trains.  The head keeps
+    every output (its dead rows produce the bias) and a layer with no alive filter keeps filter 0, whose masked weights
+    give the constant its consumers need through the ordinary arithmetic."""
+    alive = []
+    for L in layers:
+        conv = L.conv
+        if L.is_head or not getattr(conv, 'mask_flag', False):
+            alive.append(list(range(L.O)))
+            continue
+        keep = torch.nonzero(conv.mask.reshape(L.O, -1).ne(0).any(1)).flatten().tolist()
+        alive.append(keep or [0])
+    return alive
+
+
+def shrink_layout(plan, alive):
+    """Physical channel layout of the shrunk training plan (host only; the CPU tests call it).
+
+    Every activation buffer gets `plan.colmap[name]`: per physical column the channel of the full tensor it holds (the
+    inference plan's convention: -1 a zero pad column, -2 a ones column).  A producer writes its alive filters in
+    order; a Reorg producer writes 4 x its alive count (quadrant-major, like MC_EPI_REORG2); a concat holds its slot-0
+    part, padded to 8 columns, then its slot-1 part; two ones columns follow the last real column of a buffer with any
+    dead producer filter.  A consumer weights them with the high and low bf16 halves of its fp32 fold of the dead
+    inputs, so the dead constants reach z as exactly as the dense step's fp32 products do (one bf16 weight would put a
+    2^-9 relative error on what is often the largest part of z, and z is then rounded to bf16 around it).  Pitches and concat offsets are multiples of 8 (the BatchNorm passes require it); a consumer
+    contracts over the whole pitch, the pad columns meeting zero weights.  A layer's `L.O` / `L.C` become the compact
+    output count / contraction width.  No dead filter anywhere: the plan is left dense."""
+    layers = plan.layers
+    if all(len(a) == L.O for a, L in zip(alive, layers)):
+        return False
+    for L, a in zip(layers, alive):
+        if len(a) < L.O and L.bn is None:
+            # the constant of a dead filter is act(beta) of its BatchNorm; without one it would be act(bias)
+            raise NotImplementedError("block %d: dead filters in a convolution without BatchNorm" % L.ind)
+    for L, keep in zip(layers, alive):
+        L.keep = keep
+        L.O_full, L.C_full = L.O, L.C
+        L.has_dead = len(keep) < L.O
+        L.lkmap = {f: i for i, f in enumerate(keep)}
+
+    def part_cols(L):
+        if L.reorg:
+            return [q * L.O_full + f for q in range(4) for f in L.keep]
+        return list(L.keep)
+
+    colmap, prov = {}, {}  # prov[name](c) -> (producer layer, filter) of full channel c
+    for L in layers:
+        if L.is_head:
+            continue
+        names = [a.name for a in (L.act, L.pooled) if a is not None]
+        for name in names:
+            if name in plan.cat_parts:
+                continue
+            cols = part_cols(L) + ([-2, -2] if L.has_dead else [])
+            colmap[name] = cols + [-1] * (_round_up(len(cols), 8) - len(cols))
+            prov[name] = (lambda P: (lambda c: (P, c)))(L)
+    for name, (l0, l1) in plan.cat_parts.items():
+        c0 = part_cols(l0)
+        cols = c0 + [-1] * (_round_up(len(c0), 8) - len(c0))
+        off1 = len(cols)
+        base1 = 4 * l0.O_full if l0.reorg else l0.O_full
+        cols += [base1 + c for c in part_cols(l1)]
+        if l0.has_dead or l1.has_dead:
+            cols += [-2, -2]
+        colmap[name] = cols + [-1] * (_round_up(len(cols), 8) - len(cols))
+        l0.cat_off, l1.cat_off = 0, off1
+
+        def pv(c, l0=l0, l1=l1, base1=base1):
+            if c < base1:
+                return (l0, c % l0.O_full if l0.reorg else c)
+            return (l1, c - base1)
+        prov[name] = pv
+    plan.colmap = colmap
+    # geometry of every buffer and of every layer
+    for name, cols in colmap.items():
+        H, W, _ = plan.buf_specs[name]
+        plan.buf_specs[name] = (H, W, len(cols))
+        if ('d' + name) in plan.grad_specs:
+            plan.grad_specs['d' + name] = (H, W, len(cols))
+        if -2 in cols:
+            plan.ones_cols[name] = cols.index(-2)
+    for L in layers:
+        L.O = len(L.keep)
+        if not L.is_head:
+            ldz = _round_up(L.O, 8)
+            L.z.C, L.z.ld = L.O, ldz
+            plan.buf_specs[L.z.name] = (L.H, L.W, ldz)
+            plan.grad_specs['dz%d' % L.ind] = (L.H, L.W, ldz)
+            a = L.act
+            a.ld = len(colmap[a.name])
+            a.C = 4 * L.O if L.reorg else L.O
+            a.ch_off = getattr(L, 'cat_off', 0) if a.name in plan.cat_parts else 0
+            if L.pooled is not None:
+                L.pooled.C, L.pooled.ld = L.O, len(colmap[L.pooled.name])
+        if L.src is not None:
+            cols = colmap[L.src.name]
+            L.src.ld = len(cols)
+            L.C = len(cols)
+            L.colmap = cols
+            p = prov[L.src.name]
+            L.cphys = [-1] * L.C_full
+            for j, c in enumerate(cols):
+                if c >= 0:
+                    L.cphys[c] = j
+            L.dead_in = [(c, p(c)) for c in range(L.C_full) if L.cphys[c] < 0]
+            L.ones_col = cols.index(-2) if -2 in cols else -1
+            if L.dead_in and L.ones_col < 0:
+                raise RuntimeError("internal: block %d reads dead channels without a ones column" % L.ind)
+        else:
+            L.colmap, L.cphys, L.dead_in, L.ones_col = None, list(range(L.C)), [], -1
+    plan.shrunk = True
+    return True
+
+
+def _seg_table(plan):
+    """Offsets of the shrunk plan's per-step buffers and the host half of the mc_shrink_seg table (include/mcb200.h):
+    (segments, int32 index list, sizes).  Parameter pointers are filled in per device by _shrink_tables."""
+    idx, segs = [], []
+
+    def put(vals):
+        off = len(idx)
+        idx.extend(int(v) for v in vals)
+        return off
+    sizes = dict(lk=0, cbn=0, wp=0, wpd=0, dwc=0, grad=0)
+
+    def take(kind, n, align):
+        off = _round_up(sizes[kind], align)
+        sizes[kind] = off + n
+        return off
+    pos = {id(L): i for i, L in enumerate(plan.layers)}
+    for L in plan.layers:
+        L.lk_off = take('lk', L.O_full, 4) if L.bn is not None else 0
+    cons = {}  # (producer, filter) -> [(consumer segment, consumer input channel)]
+    for L in plan.layers:
+        for c, (P, f) in L.dead_in:
+            cons.setdefault((id(P), f), []).append((pos[id(L)], c))
+    for L in plan.layers:
+        s = _lib.mc_shrink_seg()
+        taps = L.k * L.k
+        s.O, s.C, s.taps, s.n_o, s.leaky = L.O_full, L.C_full, taps, L.O, L.leaky
+        s.n_col = L.C
+        s.ones_col = L.ones_col
+        s.oidx = put(L.keep)
+        orow = [-1] * L.O_full
+        for i, f in enumerate(L.keep):
+            orow[f] = i
+        s.orow = put(orow)
+        s.cphys = put(L.cphys)
+        clk = [-1] * L.C_full
+        for c, (P, f) in L.dead_in:
+            clk[c] = P.lk_off + f
+        s.clk = put(clk)
+        s.n_dead = len(L.dead_in)
+        s.dead_in = put([c for c, _ in L.dead_in])
+        ptr, pairs = [0], []
+        for f in range(L.O_full):
+            if orow[f] < 0:
+                pairs += cons.get((id(L), f), [])
+            ptr.append(len(pairs))
+        s.cons_ptr = put(ptr)
+        s.cons = put([v for pr in pairs for v in pr])
+        s.lk_off = L.lk_off
+        if L.src is not None:
+            s.colmap = put(L.colmap)
+            L.kb = _kblk(L.C, L.k)
+            s.npad, s.kc = _round_up(L.O, 16), _round_up(L.C, L.kb)
+            L.kbd = _kblk(L.O, L.k)
+            s.cpad, s.ko = _round_up(L.C, 16), _round_up(L.O, L.kbd)
+            s.wp_off = L.wp_off = take('wp', s.npad * taps * s.kc, 64)
+            s.wpd_off = L.wpd_off = take('wpd', s.cpad * taps * s.ko, 64)
+            L.npad, L.kc, L.cpad, L.ko = s.npad, s.kc, s.cpad, s.ko
+        else:
+            s.colmap, s.kc = put([]), 0
+        if L.bn is not None:
+            L.cbn_ld = s.cbn_ld = _round_up(L.O, 8)
+            L.cbn_off = s.cbn_off = take('cbn', 4 * L.cbn_ld, 8)
+            L.cdgb_off = s.cdgb_off = take('dwc', 2 * L.O, 4)
+            L.dbn_off = s.dbn_off = take('grad', 2 * L.O_full, 4)
+        L.dwc_off = s.dwc_off = take('dwc', L.O * L.C * taps, 4)
+        L.dw_off = s.dw_off = take('grad', L.O_full * L.C_full * taps, 4)
+        segs.append(s)
+    if len(segs) > _lib.MC_MAX_SEGMENTS:
+        raise NotImplementedError("shrunk training plans take at most %d convolutions" % _lib.MC_MAX_SEGMENTS)
+    return segs, idx, sizes
+
+
+def _shrink_tables(plan, dev):
+    """The device segment table (rebuilt when a parameter's storage moves) and the index list of this device."""
+    ptrs = []
+    for L in plan.layers:
+        conv, bn = L.conv, L.bn
+        ptrs += [conv.weight.data_ptr(), _masked(conv) or 0]
+        if bn is not None:
+            tracked = bn.track_running_stats and bn.running_mean is not None
+            ptrs += [bn.weight.data_ptr(), bn.bias.data_ptr(), bn.running_mean.data_ptr() if tracked else 0,
+                     bn.running_var.data_ptr() if tracked else 0]
+    key = (str(dev), tuple(ptrs))
+    cached = plan._tables.get(str(dev))
+    if cached is not None and cached[0] == key:
+        return cached[1], cached[2]
+    segs, idx = plan.seg_host, plan.seg_idx
+    for L, s in zip(plan.layers, segs):
+        conv, bn = L.conv, L.bn
+        s.w, s.mask = conv.weight.data_ptr(), _masked(conv)
+        if bn is not None:
+            tracked = bn.track_running_stats and bn.running_mean is not None
+            s.gamma, s.beta = bn.weight.data_ptr(), bn.bias.data_ptr()
+            s.rmean = bn.running_mean.data_ptr() if tracked else None
+            s.rvar = bn.running_var.data_ptr() if tracked else None
+            s.momentum = bn.momentum if bn.momentum is not None else 0.1
+    raw = b''.join(bytes(s) for s in segs)
+    table = torch.frombuffer(bytearray(raw), dtype=torch.uint8).to(dev)
+    idx_t = torch.tensor(idx if idx else [0], dtype=torch.int32, device=dev)
+    plan._tables[str(dev)] = (key, table, idx_t)
+    return table, idx_t
+
+
+def train_plan(model):
+    """The model's cached training plan, rebuilt when ``model.b200_shrink_train`` or (with it on) the masks change."""
+    want = bool(getattr(model, 'b200_shrink_train', False))
+    key = (want,)
+    if want:
+        key += tuple((c.mask.data_ptr(), c.mask._version, getattr(c, '_mask_epoch', 0)) if c.mask_flag else None
+                     for c in model.masked_convs())
+    plan = model.__dict__.get('_b200_train_plan')
+    if plan is None or getattr(plan, 'key', (False,)) != key:
+        old = plan
+        plan = model.__dict__['_b200_train_plan'] = TrainPlan(model, shrink=want)
+        plan.key = key
+        if old is not None:
+            plan.dp_group, plan.dp_world = old.dp_group, old.dp_world
+    return plan
 
 
 def _kblk(C, k=1):
@@ -313,6 +568,20 @@ def _forward(plan, x, training_stats=True, after_layer=None, needs_backward=True
     s = _lib.stream_ptr()
     y = None
     fuse_stats = bool(getattr(plan, 'fuse_stats', True))
+    if plan.shrunk:
+        # compact BatchNorm parameters, the dead channels' constants and every packed weight matrix: three launches
+        table, idx = _shrink_tables(plan, dev)
+        sz = plan.sizes
+        sv.cbn = torch.empty(max(sz['cbn'], 1), device=dev)
+        sv.lk = torch.empty(max(sz['lk'], 1), device=dev)
+        sv.wp = torch.empty(max(sz['wp'], 1), dtype=torch.bfloat16, device=dev)
+        sv.wpd = torch.empty(max(sz['wpd'], 1), dtype=torch.bfloat16, device=dev) if needs_backward else None
+        nseg = len(plan.layers)
+        _lib.check(lib.mc_shrink_prepare(table.data_ptr(), nseg, idx.data_ptr(), sv.cbn.data_ptr(), sv.lk.data_ptr(), s),
+                   "mc_shrink_prepare")
+        _lib.check(lib.mc_shrink_pack(table.data_ptr(), nseg, idx.data_ptr(), sv.lk.data_ptr(), sv.wp.data_ptr(),
+                                      sv.wpd.data_ptr() if sv.wpd is not None else None, s), "mc_shrink_pack")
+        any_upd = False
     for L in plan.layers:
         stats_done = False
         st = None
@@ -332,6 +601,8 @@ def _forward(plan, x, training_stats=True, after_layer=None, needs_backward=True
             _lib.check(lib.mc_conv_im2col_geometry(C, 1, O, 0, ctypes.byref(cl), ctypes.byref(npos), ctypes.byref(nb),
                                                    ctypes.byref(kpad)), "mc_conv_im2col_geometry")
             weff = w if mask_ptr is None else w * conv.mask
+            if plan.shrunk:
+                weff = weff[L.keep]
             nb_pad = _round_up(nb.value, 16)
             # expanded weights: the zero padding is written once, the 27 real columns are refreshed in place
             wexp = plan.scratch(dev, 'wexp1', (nb_pad, kpad.value // cl.value, cl.value), zero=True)
@@ -347,9 +618,12 @@ def _forward(plan, x, training_stats=True, after_layer=None, needs_backward=True
         else:
             kb = _kblk(C, k)
             Kc = _round_up(C, kb)
-            wpack = torch.empty(Npad, k * k * Kc, dtype=torch.bfloat16, device=dev)
-            _lib.check(lib.mc_pack_conv_weights(w.data_ptr(), mask_ptr, O, C, k, None, O, None, C, wpack.data_ptr(), Npad,
-                                                Kc, s), "mc_pack_conv_weights")
+            if plan.shrunk:
+                wpack = sv.wp[L.wp_off:L.wp_off + Npad * k * k * Kc]
+            else:
+                wpack = torch.empty(Npad, k * k * Kc, dtype=torch.bfloat16, device=dev)
+                _lib.check(lib.mc_pack_conv_weights(w.data_ptr(), mask_ptr, O, C, k, None, O, None, C, wpack.data_ptr(),
+                                                    Npad, Kc, s), "mc_pack_conv_weights")
             src = L.src
             in_ptr = bufs[src.name].data_ptr() + 2 * src.ch_off
             if L.is_head:
@@ -378,10 +652,11 @@ def _forward(plan, x, training_stats=True, after_layer=None, needs_backward=True
                        "mc_col_stats")
         upd = training_stats and bn.track_running_stats and bn.running_mean is not None
         mom = bn.momentum if bn.momentum is not None else 0.1
-        _lib.check(lib.mc_bn_finalize(st[0].data_ptr(), st[1].data_ptr(), O, float(B * L.H * L.W), bn.weight.data_ptr(),
-                                      bn.bias.data_ptr(), bn.eps, mom,
-                                      bn.running_mean.data_ptr() if upd else None,
-                                      bn.running_var.data_ptr() if upd else None,
+        gamma, beta, rmean, rvar = _bn_ptrs(plan, L, sv)
+        if plan.shrunk:
+            any_upd = any_upd or upd
+        _lib.check(lib.mc_bn_finalize(st[0].data_ptr(), st[1].data_ptr(), O, float(B * L.H * L.W), gamma, beta, bn.eps,
+                                      mom, rmean if upd else None, rvar if upd else None,
                                       st[2].data_ptr(), st[3].data_ptr(), st[4].data_ptr(), st[5].data_ptr(), s),
                    "mc_bn_finalize")
         if upd and bn.num_batches_tracked is not None:
@@ -397,11 +672,27 @@ def _forward(plan, x, training_stats=True, after_layer=None, needs_backward=True
         _lib.check(lib.mc_bn_apply(z.data_ptr(), L.z.ld, B, L.H, L.W, O, st[2].data_ptr(), st[3].data_ptr(), L.leaky,
                                    bufs[a.name].data_ptr(), a.ld, a.ch_off, int(L.reorg), s), "mc_bn_apply")
         if L.pool:
-            _lib.check(lib.mc_maxpool2x2(bufs[a.name].data_ptr(), bufs[L.pooled.name].data_ptr(), B, L.H, L.W, O, a.ld,
+            # the two ones columns (right after the O real channels) are pooled with them
+            cp = O + 2 if a.name in plan.ones_cols else O
+            _lib.check(lib.mc_maxpool2x2(bufs[a.name].data_ptr(), bufs[L.pooled.name].data_ptr(), B, L.H, L.W, cp, a.ld,
                                          L.pooled.ld, s), "mc_maxpool2x2")
         if after_layer is not None:
             after_layer(L, bufs)
+    if plan.shrunk and any_upd:
+        _lib.check(lib.mc_shrink_stats(table.data_ptr(), nseg, idx.data_ptr(), sv.cbn.data_ptr(), s), "mc_shrink_stats")
     return y, sv
+
+
+def _bn_ptrs(plan, L, sv):
+    """gamma, beta, running mean, running var of a BatchNorm layer: the parameters themselves, or their compact
+    copies in a shrunk plan."""
+    bn = L.bn
+    if not plan.shrunk:
+        return (bn.weight.data_ptr(), bn.bias.data_ptr(),
+                bn.running_mean.data_ptr() if bn.running_mean is not None else None,
+                bn.running_var.data_ptr() if bn.running_var is not None else None)
+    base, ld = sv.cbn.data_ptr() + 4 * L.cbn_off, 4 * L.cbn_ld
+    return base, base + ld, base + 2 * ld, base + 3 * ld
 
 
 _WS = {}
@@ -426,10 +717,17 @@ def _backward(plan, sv, dy, before_bn=None):
     written = set()  # gradient buffers that already hold a contribution in this backward
     pending = []     # data-parallel: (work handle, tensor) of the gradient all-reduces in flight
 
+    shrunk = plan.shrunk
+    if shrunk:
+        # compact gradients (dgamma/dbeta of mc_bn_backward, the wgrad outputs) and the full ones they expand into
+        dwc = torch.empty(max(plan.sizes['dwc'], 1), device=dev)
+        gfull = torch.empty(max(plan.sizes['grad'], 1), device=dev)
+
     def reduce_async(t):
         # SURVEY.md §8f N4: the all-reduce of a layer's gradient is issued as soon as the layer's wgrad is queued, so NCCL
-        # (its own stream, NVLink/NVSwitch) overlaps the backward of the layers below
-        if plan.dp_world > 1:
+        # (its own stream, NVLink/NVSwitch) overlaps the backward of the layers below.  A shrunk plan has its full
+        # gradients only after mc_shrink_finish: it reduces them there.
+        if plan.dp_world > 1 and not shrunk:
             import torch.distributed as dist
             pending.append((dist.all_reduce(t, group=plan.dp_group, async_op=True), t))
         return t
@@ -455,11 +753,12 @@ def _backward(plan, sv, dy, before_bn=None):
             if before_bn is not None:
                 before_bn(L, bufs)
             dz = bufs['dz%d' % L.ind]
-            dgb = torch.empty(2, O, device=dev)
+            dgb = dwc[L.cdgb_off:L.cdgb_off + 2 * O].view(2, O) if shrunk else torch.empty(2, O, device=dev)
             bn = L.bn
+            gamma, beta, _, _ = _bn_ptrs(plan, L, sv)
             _lib.check(lib.mc_bn_pool_backward(bufs[L.z.name].data_ptr(), L.z.ld, bufs[dp_name].data_ptr(), L.pooled.ld, B,
                                                L.H, L.W, O, st[2].data_ptr(), st[3].data_ptr(), st[4].data_ptr(),
-                                               st[5].data_ptr(), bn.weight.data_ptr(), bn.bias.data_ptr(), L.leaky,
+                                               st[5].data_ptr(), gamma, beta, L.leaky,
                                                dgb[0].data_ptr(), dgb[1].data_ptr(), dz.data_ptr(), L.z.ld, s),
                        "mc_bn_pool_backward")
             reduce_async(dgb)
@@ -472,6 +771,7 @@ def _backward(plan, sv, dy, before_bn=None):
             da_name = 'd' + a.name
             if L.pool:
                 dp = bufs['d' + L.pooled.name]
+                # (pool backward over the O real channels only: nothing reads the ones columns' gradient)
                 if ('d' + L.pooled.name) not in written:
                     raise RuntimeError("internal: pooled gradient of block %d was never produced" % L.ind)
                 _lib.check(lib.mc_maxpool2x2_backward(bufs[a.name].data_ptr(), a.ld, dp.data_ptr(), L.pooled.ld, B, L.H,
@@ -483,18 +783,24 @@ def _backward(plan, sv, dy, before_bn=None):
             if before_bn is not None:
                 before_bn(L, bufs)
             dz = bufs['dz%d' % L.ind]
-            dgb = torch.empty(2, O, device=dev)
+            dgb = dwc[L.cdgb_off:L.cdgb_off + 2 * O].view(2, O) if shrunk else torch.empty(2, O, device=dev)
             bn = L.bn
+            gamma, beta, _, _ = _bn_ptrs(plan, L, sv)
             _lib.check(lib.mc_bn_backward(bufs[L.z.name].data_ptr(), L.z.ld, bufs[da_name].data_ptr(), a.ld, a.ch_off,
                                           int(L.reorg), B, L.H, L.W, O, st[4].data_ptr(), st[5].data_ptr(),
-                                          bn.weight.data_ptr(), bn.bias.data_ptr(), L.leaky, dgb[0].data_ptr(),
+                                          gamma, beta, L.leaky, dgb[0].data_ptr(),
                                           dgb[1].data_ptr(), dz.data_ptr(), L.z.ld, s), "mc_bn_backward")
             reduce_async(dgb)
             grads[id(bn.bias)] = dgb[0]
             grads[id(bn.weight)] = dgb[1]
             dz_ptr, ld_dz = dz.data_ptr(), L.z.ld
-        # ---- weight gradient
-        dw = torch.empty_like(conv.weight.data)
+        # ---- weight gradient (shrunk: compact, unmasked; mc_shrink_finish expands it and applies the mask; the two
+        #      ones columns get the same gradient G1, the first one is used)
+        if shrunk:
+            dw = dwc[L.dwc_off:L.dwc_off + O * C * k * k]
+            mask_ptr = None
+        else:
+            dw = torch.empty_like(conv.weight.data)
         if L.src is None:
             # image layer: bf16 im2col rows in the workspace + the 1x1 tcgen05 weight gradient over them
             nbytes = lib.mc_workspace_bytes_conv_wgrad_first(B, L.H, L.W, C, O)
@@ -508,7 +814,8 @@ def _backward(plan, sv, dy, before_bn=None):
             ws = _workspace(dev, nbytes)
             _lib.check(lib.mc_conv_wgrad(bufs[src.name].data_ptr() + 2 * src.ch_off, src.ld, C, dz_ptr, ld_dz, O, B, L.H,
                                          L.W, k, mask_ptr, dw.data_ptr(), 0, ws.data_ptr(), nbytes, s), "mc_conv_wgrad")
-        grads[id(conv.weight)] = reduce_async(dw)
+        if not shrunk:
+            grads[id(conv.weight)] = reduce_async(dw)
         # ---- data gradient: the same tcgen05 conv kernel on the flipped / transposed filter
         if L.src is not None:
             src = L.src
@@ -517,15 +824,33 @@ def _backward(plan, sv, dy, before_bn=None):
                 raise NotImplementedError("two convolutions consume the same activation slice (block %d)" % L.ind)
             kb = _kblk(O, k)
             Cpad, Ko = _round_up(C, 16), _round_up(O, kb)
-            wpack = torch.empty(Cpad, k * k * Ko, dtype=torch.bfloat16, device=dev)
-            _lib.check(lib.mc_pack_conv_weights_dgrad(conv.weight.data_ptr(), mask_ptr, O, C, k, wpack.data_ptr(), Cpad, Ko,
-                                                      s), "mc_pack_conv_weights_dgrad")
+            if shrunk:
+                wpack = sv.wpd[L.wpd_off:L.wpd_off + Cpad * k * k * Ko]
+            else:
+                wpack = torch.empty(Cpad, k * k * Ko, dtype=torch.bfloat16, device=dev)
+                _lib.check(lib.mc_pack_conv_weights_dgrad(conv.weight.data_ptr(), mask_ptr, O, C, k, wpack.data_ptr(), Cpad,
+                                                          Ko, s), "mc_pack_conv_weights_dgrad")
             ones = plan.const(dev, 1.0, Cpad)
             zeros = plan.const(dev, 0.0, Cpad)
             d = _conv_desc(dz_ptr, wpack.data_ptr(), ones.data_ptr(), zeros.data_ptr(), bufs[dname].data_ptr(), B, L.H, L.W,
                            O, ld_dz, C, Cpad, k, 0, _lib.MC_EPI_PNHWC, src.ld, src.ch_off, kb, plan, dev)
             _lib.check(lib.mc_conv_fwd(ctypes.byref(d), s), "dgrad (block %d)" % L.ind)
             written.add(dname)
+    if shrunk:
+        table, idx = _shrink_tables(plan, dev)
+        _lib.check(lib.mc_shrink_finish(table.data_ptr(), len(plan.layers), idx.data_ptr(), sv.lk.data_ptr(),
+                                        dwc.data_ptr(), gfull.data_ptr(), s), "mc_shrink_finish")
+        for L in plan.layers:
+            n = L.O_full * L.C_full * L.k * L.k
+            grads[id(L.conv.weight)] = gfull[L.dw_off:L.dw_off + n].view_as(L.conv.weight)
+            if L.bn is not None:
+                grads[id(L.bn.bias)] = gfull[L.dbn_off:L.dbn_off + L.O_full]
+                grads[id(L.bn.weight)] = gfull[L.dbn_off + L.O_full:L.dbn_off + 2 * L.O_full]
+        if plan.dp_world > 1:  # every full gradient in one all-reduce, then the head bias
+            import torch.distributed as dist
+            hb = grads[id(head.conv.bias)]
+            for t in (gfull, hb):
+                pending.append((dist.all_reduce(t, group=plan.dp_group, async_op=True), t))
     for work, t in pending:  # the current stream waits for NCCL; gradients become the mean over the replicas
         work.wait()
         t.div_(plan.dp_world)
@@ -556,9 +881,7 @@ def darknet_train_forward(model, x):
     _lib.require_cuda(x, "Darknet.forward (training)")
     if x.dim() != 4:
         raise ValueError("expected [B,3,H,W] input")
-    plan = model.__dict__.get('_b200_train_plan')
-    if plan is None:
-        plan = model.__dict__['_b200_train_plan'] = TrainPlan(model)
+    plan = train_plan(model)
     params = plan.parameters()
     for p in params:
         _lib.require_cuda(p, "Darknet.forward (training)")

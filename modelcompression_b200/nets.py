@@ -142,6 +142,8 @@ class Darknet(nn.Module):
         self._b200_plan_key = None
         self._b200_watch = None
         self.b200_shrink = True      # physically drop filters whose (masked) weights are all zero
+        # training mode: run the retrain step over the filters the masks keep (engine_train.shrink_layout)
+        self.b200_shrink_train = False
         self.b200_keep_blocks = False  # keep every block's activation buffer alive for per-block parity checks
 
     # ------------------------------------------------------------------ graph construction (nets.py:779-895)

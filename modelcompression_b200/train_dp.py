@@ -15,16 +15,14 @@ every rank, so they stay zero after the averaged step.
 import torch
 import torch.distributed as dist
 
-from .engine_train import TrainPlan
+from .engine_train import train_plan
 
 
 def enable(model, group=None):
     """Average gradients across the process group inside Darknet's training backward."""
     if not (dist.is_available() and dist.is_initialized()):
         raise RuntimeError("train_dp.enable: torch.distributed is not initialised")
-    plan = model.__dict__.get('_b200_train_plan')
-    if plan is None:
-        plan = model.__dict__['_b200_train_plan'] = TrainPlan(model)
+    plan = train_plan(model)
     plan.dp_group = group
     plan.dp_world = dist.get_world_size(group)
     return model
